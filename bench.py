@@ -2,7 +2,7 @@
 """Benchmark of the rb_align query path on B200 (BASELINE.json metric: 150bp reads/s).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--mode count|locate|markers|all]
-                  [--impl reference] [--config c2|medium|small] [--reads R]
+                  [--impl reference] [--config c2|medium|small] [--reads R] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic reads (the whole
 BASELINE config: 10M x 150bp reads against the 50 Mbp x 64 haplotype pfbwt-f index,
@@ -40,25 +40,24 @@ MODES = {"count": 0, "locate": 1, "markers": 2, "all": 3}
 
 
 # ------------------------------------------------------------------------------------------
-def workload(config: str, log):
-    """(name, index prefix, panel).  The index is built once by tools/synth.py through the
-    unmodified reference builder and cached under data/ (git-ignored, travels with the repo)."""
+def workload(config: str, log, tmpdir):
+    """(name, index prefix, panel).  A config built by tools/synth.py and cached under data/ (git-ignored) is
+    used as it is; otherwise `small` is built into tmpdir without the reference (synth.build_index_gpu, about a
+    minute), so that a fresh checkout benchmarks the same index every time and writes nothing into the tree."""
     order = [config] if config != "auto" else ["c2", "medium", "small"]
     for cfg in order:
         prefix = os.path.join(DATA, cfg, cfg)
         if os.path.exists(prefix + ".rbwt"):
             L, H = synth.CONFIGS[cfg]
             return cfg, prefix, synth.make_panel(L, H)
-    # nothing cached: build the largest config that builds in about a minute
     cfg = order[-1] if config != "auto" else "small"
-    if cfg == "c2":
-        raise SystemExit("data/c2 is not built: run `python tools/synth.py c2 data/c2` (~45 min CPU)")
+    if cfg != "small":
+        raise SystemExit("data/%s is not built: run `python tools/synth.py %s data/%s`" % (cfg, cfg, cfg))
     L, H = synth.CONFIGS[cfg]
     panel = synth.make_panel(L, H)
-    os.makedirs(os.path.join(DATA, cfg), exist_ok=True)
-    prefix = os.path.join(DATA, cfg, cfg)
-    print("bench: building %s index with the reference builder ..." % cfg, file=log)
-    synth.build_index(panel, prefix, markers=True, log=log)
+    prefix = os.path.join(tmpdir, cfg)
+    print("bench: building the %s index in %s ..." % (cfg, tmpdir), file=log)
+    synth.build_index_gpu(panel, prefix, markers=True, device=int(os.environ.get("LOCAL_RANK", "0")), log=log)
     return cfg, prefix, panel
 
 
@@ -173,7 +172,7 @@ def run_reference_shards(prefix, reads, mode, procs, tmpdir):
     return len(reads) / max(qt), max(qt)
 
 
-def reference_arm(args, rank, world, log, emit):
+def reference_arm(args, rank, world, log, emit, tmpdir):
     if rank != 0:
         return
     mode = MODES[args.mode]
@@ -183,7 +182,7 @@ def reference_arm(args, rank, world, log, emit):
     if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "rb_align")):
         emit({"impl": "reference", "unavailable": "oracle/_ref/rb_align not built (run make -C oracle ref where /root/reference exists)"})
         return
-    cfg, prefix, panel = workload(args.config, log)
+    cfg, prefix, panel = workload(args.config, log, tmpdir)
     cores = os.cpu_count() or 1
     procs = max(1, min(cores, args.ref_procs or cores))
     per_proc = args.ref_reads_per_proc
@@ -279,9 +278,10 @@ class Workload:
         self._keep, self.sets = [], {}
 
 
-def run_leg(w, read_set, mode, steps, warmup, barrier, ascii_e2e=True):
+def run_leg(w, read_set, mode, steps, warmup, barrier, ascii_e2e=True, fetch=False):
     """One leg of the metric on this rank: device-resident steps (raw input: pack_kernel inside; and 2-bit input),
-    then end to end through rbg_query_packed / rbg_query with pinned host buffers.  Returns per-rank numbers."""
+    then end to end through rbg_query_packed / rbg_query with pinned host buffers.  Returns per-rank numbers; with
+    `fetch`, also out["result"]: what the last timed device-resident step computed, copied to the host after the timing."""
     ix, rs = w.ix, w.sets[read_set]
     e2e_mode = mode | (w.rb.RBG_NARROW_LOCS if mode & 1 else 0) | w.rb.RBG_NARROW_RANGES     # the narrow wire forms rb_align asks for
     out = {}
@@ -303,6 +303,8 @@ def run_leg(w, read_set, mode, steps, warmup, barrier, ascii_e2e=True):
     out.update(dev_ms=float(np.mean(dev_ms)), search_ms=float(np.mean(search_ms)), phi_ms=float(np.mean(phi_ms)), launches=launches,
                lf_steps=st.lf_steps, lf_lines=st.lf_lines, phi_steps=st.phi_steps, marker_words=st.marker_words,
                kernel_ms={k: getattr(st, k) for k in ("ms_pack", "ms_search", "ms_locate", "ms_phi", "ms_markers", "ms_total")})
+    if fetch:
+        out["result"] = ix.fetch(staged, mode)
     out["checksum"] = ix.query_staged(staged, mode, checksum=True)
     staged.free()
     # the same kernels over a batch that arrived 2-bit packed (no pack_kernel), locations narrow
@@ -340,6 +342,40 @@ def run_leg(w, read_set, mode, steps, warmup, barrier, ascii_e2e=True):
         out[key] = (time.perf_counter() - e0) * 1e3 / steps
         out[key + "_stages"] = {k: getattr(ix.stats(), k) for k in ("ms_h2d", "ms_search", "ms_d2h", "ms_total")}
     return out
+
+
+def dump_outputs(out_dir, res, budget=64 << 20):
+    """Writes a QueryResult as float64 .npy files under out_dir: lo / hi (and toehold, per-read location counts and the
+    locations; per-read marker counts and the marker words split into 32-bit halves, which float64 holds exactly) of a
+    fixed seeded sample of reads -- all of them when everything fits in `budget` bytes -- plus the sampled read indices."""
+    n = res.n
+    # (name, offsets, values, float64 words per value)
+    segs = [s for s in (("loc", res.loc_off, res.locs, 1), ("marker", res.mk_off, res.markers, 2)) if s[1] is not None]
+    k = n
+    while True:
+        idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        counts = [(off[idx + 1] - off[idx]).astype(np.int64) for _, off, _, _ in segs]
+        per_read = 3 + (res.toehold is not None) + len(segs)
+        total = 8 * (k * per_read + sum(int(c.sum()) * words for c, (_, _, _, words) in zip(counts, segs)))
+        if total <= budget or k == 1:
+            break
+        k //= 2
+    arrays = {"read_index": idx, "lo": res.lo[idx], "hi": res.hi[idx]}
+    if res.toehold is not None:
+        arrays["toehold"] = res.toehold[idx]
+    for (name, off, vals, _), cnt in zip(segs, counts):
+        first = np.repeat(off[idx].astype(np.int64) - np.concatenate([[0], np.cumsum(cnt)[:-1]]), cnt)
+        picked = vals[first + np.arange(int(cnt.sum()))]
+        arrays[name + "_count"] = cnt
+        if name == "marker":
+            arrays["markers_lo32"] = picked & np.uint64(0xFFFFFFFF)
+            arrays["markers_hi32"] = picked >> np.uint64(32)
+        else:
+            arrays["locs"] = picked
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a).astype(np.float64))
+    return {"dir": out_dir, "reads": int(k), "of": int(n), "bytes": int(sum(8 * len(a) for a in arrays.values()))}
 
 
 def leg_record(w, name, read_set, mode, m, world, peak, peak_src, gather):
@@ -419,8 +455,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gather", action="store_true")
     ap.add_argument("--ftab-k", type=int, default=10, help="k of the k-mer seed table built on the GPU at open (0 = none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the headline leg's results of its last "
+                    "step as DIR/<name>.npy (float64; a fixed sample of reads when all of them exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     log = sys.stderr
+    tmp = tempfile.TemporaryDirectory(prefix="rowbowt_bench_")      # an index built at run time; removed at exit
     # stdout carries exactly ONE line, the JSON record: whatever a library prints there (NCCL's version banner, torchrun
     # notices) is sent to stderr for the whole run, the record is written to the saved descriptor at the end
     sys.stdout.flush()
@@ -436,7 +477,7 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
-        reference_arm(args, rank, world, log, emit)
+        reference_arm(args, rank, world, log, emit, tmp.name)
         return
 
     import torch
@@ -466,7 +507,7 @@ def main():
         m.update({k: float(v) for k, v in zip(keys, t.tolist())})
         return m
 
-    cfg, prefix, panel = workload(args.config, log)
+    cfg, prefix, panel = workload(args.config, log, tmp.name)
     w = Workload(rb, lib, cfg, prefix, panel, local, rank, args.reads, args.ftab_k, log)
     info = w.info
     exact = w.add_reads("exact", 3)
@@ -495,7 +536,8 @@ def main():
     sampler.start()
     measured = {}
     for name, rset, mode in plan:
-        measured[name] = max_over_ranks(run_leg(w, rset, mode, args.steps, args.warmup, barrier))
+        measured[name] = max_over_ranks(run_leg(w, rset, mode, args.steps, args.warmup, barrier,
+                                                fetch=bool(args.dump_outputs) and name == args.mode and rank == 0))
     clocks = sampler.summary()
 
     # ---- BASELINE config 5 family (n > 2^32), -s [-m], when its index travelled with the repo --------------------
@@ -519,7 +561,7 @@ def main():
         if not args.no_gather and rank == 0:
             g5["dir"] = lib.rbg_gather_roofline(local, max(int(w5.info.dir_bytes), 1 << 20), 64, 256)
             g5["phi"] = lib.rbg_gather_roofline(local, max(int(w5.info.phi_bytes), 1 << 20), 32, 256)
-        m5 = max_over_ranks(run_leg(w5, "exact", mode5, max(2, args.steps // 2), 2, barrier, ascii_e2e=False))
+        m5 = max_over_ranks(run_leg(w5, "exact", mode5, args.steps, 2, barrier, ascii_e2e=False))
         if rank == 0:
             peak, peak_src = measured_peaks()
             c5 = leg_record(w5, "all" if mode5 == 3 else "locate", "exact", mode5, m5, world, peak, peak_src, g5)
@@ -569,6 +611,8 @@ def main():
             out["roofline_locate"] = head["roofline_locate"]
         if c5:
             out["legs"]["c5"] = c5
+        if args.dump_outputs:
+            out["dump_outputs"] = dump_outputs(args.dump_outputs, m.pop("result"))
         # CPU baseline beside it: the unmodified reference on a bounded sample, one process (as shipped)
         if not args.no_cpu_baseline and world == 1 and os.path.exists(os.path.join(ROOT, "oracle", "_ref", "rb_align")):
             k = k_cpu

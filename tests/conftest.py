@@ -42,6 +42,19 @@ def golden():
     return GOLDEN
 
 
+@pytest.fixture(scope="session")
+def small_index(tmp_path_factory):
+    """Prefix of the `small` benchmark index (1 Mbp x 16 haplotypes): data/small when it has been built, else the same
+    files built once per session without the reference (tools/synth.build_index_gpu, about a minute; needs a GPU)."""
+    prefix = os.path.join(ROOT, "data", "small", "small")
+    if os.path.exists(prefix + ".mab"):
+        return prefix
+    from tools import synth
+    prefix = str(tmp_path_factory.mktemp("small") / "small")
+    synth.build_index_gpu(synth.make_panel(*synth.CONFIGS["small"]), prefix, markers=True)
+    return prefix
+
+
 FIXTURES = {
     # name: (dir, prefix, query files, has markers)
     "toy": ("toy", "small.fa", ["simple_query.fq", "error_query.fq", "edge_query.fq"], True),

@@ -10,8 +10,8 @@ made (tools/synth.py), independently of any BWT code:
     sequence is followed by 10 'A's, pfbwt-f README "padding"), each with the right haplotype, and
   * markers reported by -m are words of the panel sites within wsize of the read start (allele of h').
 Plus: a sample of the batch bit-exact against the oracle; seed table on/off and 1 vs N chunks give the
-same device digest.  Falls back to data/small when data/c2 has not been built; skipped when neither
-exists (they are built by tools/synth.py through the unmodified reference builder).
+same device digest.  Falls back to the `small` index when data/c2 has not been built: data/small when present,
+else built once per session without the reference (conftest.small_index).
 """
 import os
 
@@ -36,7 +36,7 @@ def _workloads():
     if os.environ.get("RBG_TEST_CONFIG"):
         return [(os.environ["RBG_TEST_CONFIG"], int(os.environ.get("RBG_TEST_READS", "1000000")))]
     have = lambda cfg: os.path.exists(os.path.join(ROOT, "data", cfg, cfg + ".rbwt"))
-    out = [("c2", 2_000_000)] if have("c2") else ([("small", 500_000)] if have("small") else [])
+    out = [("c2", 2_000_000)] if have("c2") else [("small", 500_000)]
     if have("c5w"):
         out.append(("c5w", 100_000))
     return out
@@ -60,12 +60,10 @@ def _carriers(panel, hs, starts):
     return same
 
 
-@pytest.fixture(scope="module", params=_workloads() or [None], ids=lambda w: w[0] if w else "none")
+@pytest.fixture(scope="module", params=_workloads(), ids=lambda w: w[0])
 def full(request):
-    if request.param is None:
-        pytest.skip("no benchmark index under data/ (python tools/synth.py small data/small)")
     cfg, n_reads = request.param
-    prefix = os.path.join(ROOT, "data", cfg, cfg)
+    prefix = os.path.join(ROOT, "data", cfg, cfg) if cfg != "small" else request.getfixturevalue("small_index")
     L, H = synth.CONFIGS[cfg]
     panel = synth.make_panel(L, H)
     reads, hs, starts = synth.make_reads(panel, n_reads, READ_LEN, seed=3)

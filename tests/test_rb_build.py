@@ -53,6 +53,17 @@ def test_writers_reproduce_benchmark_index_files(tmp_path, cfg):
         assert filecmp.cmp(src + suf, out + suf, shallow=False), suf
 
 
+def test_raw_inputs_without_the_reference_equal_pfbwt_output(tmp_path):
+    """tools/synth.write_raw_index (what bench.py and the full-size tests build their index from when data/ is empty)
+    writes the reference pfbwt-f64 / mps_to_ma files of the `tiny` panel byte for byte."""
+    from tools import synth
+    pre = str(tmp_path / "tiny")
+    synth.write_raw_index(synth.make_panel(*synth.CONFIGS["tiny"]), pre, markers=True)
+    for suf in (".bwt", ".ssa", ".esa", ".ma"):
+        assert filecmp.cmp(RAW + suf, pre + suf, shallow=False), suf
+    assert filecmp.cmp(TINY + ".docs", pre + ".docs", shallow=False)
+
+
 @pytest.mark.gpu
 def test_build_index_is_byte_identical_to_reference(tmp_path):
     out = str(tmp_path / "b")

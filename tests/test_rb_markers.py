@@ -176,13 +176,11 @@ def test_gpu_greedy_edge_cases():
 
 
 @pytest.mark.gpu
-def test_gpu_greedy_larger_index_sample():
-    """data/small (1 Mbp x 16 haplotypes, built by tools/synth.py) when present: 3000 noisy 150 bp reads, both
-    the plain and the ftab-seeded walk, against the oracle."""
+def test_gpu_greedy_larger_index_sample(small_index):
+    """The `small` index (1 Mbp x 16 haplotypes): 3000 noisy 150 bp reads, both the plain and the ftab-seeded walk,
+    against the oracle."""
     from tools import synth
-    prefix = os.path.join(ROOT, "data", "small", "small")
-    if not os.path.exists(prefix + ".mab"):
-        pytest.skip("data/small not built")
+    prefix = small_index
     panel = synth.make_panel(*synth.CONFIGS["small"])
     reads, _, _ = synth.make_reads(panel, 3000, 150, seed=17, err_rate=0.01, n_rate=0.001)
     ix = rb.GpuIndex.open(prefix, markers=True)

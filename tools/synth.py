@@ -144,6 +144,87 @@ def build_index(panel: Panel, prefix: str, markers: bool = True, wsize: int = 10
     return t
 
 
+def panel_text(panel: Panel) -> np.ndarray:
+    """The text pfbwt-f indexes: every sequence followed by PAD 'A's, then the terminator (byte 0)."""
+    pad = np.full(PAD, ord("A"), np.uint8)
+    return np.concatenate([x for h in range(panel.nseq) for x in (panel.sequence(h), pad)] + [np.zeros(1, np.uint8)])
+
+
+def suffix_array(text: np.ndarray) -> np.ndarray:
+    """int64 suffix array of an ACGT text ending in a unique byte 0, by prefix doubling from 27-mer keys."""
+    n = len(text)
+    code = np.searchsorted(np.frombuffer(b"\0ACGT", np.uint8), text).astype(np.int64)
+    K = 27                                                   # 27 base-5 digits fit in 63 bits
+    padded = np.concatenate([code, np.zeros(K, np.int64)])
+    key = np.zeros(n, np.int64)
+    for j in range(K):
+        key = key * 5 + padded[j:j + n]
+    rank = np.empty(n, np.int64)
+    h = K
+    while True:
+        order = np.argsort(key, kind="stable")
+        sk = key[order]
+        rank[order] = np.concatenate([[0], np.cumsum(sk[1:] != sk[:-1])])
+        if rank[order[-1]] == n - 1:
+            return order
+        nxt = np.zeros(n, np.int64)
+        nxt[:n - h] = rank[h:] + 1
+        key = rank * (n + 1) + nxt
+        h *= 2
+
+
+def write_raw_index(panel: Panel, prefix: str, markers: bool = True, wsize: int = 10) -> None:
+    """rb_build's inputs as pfbwt-f64 / mps_to_ma write them, computed here without the reference:
+    <prefix>.bwt (one byte per row), .ssa / .esa (row, SA) at the first / last row of every run, .docs and,
+    with markers, .ma (`first_row last_row marker* ~0` for every maximal block of consecutive rows whose
+    suffix starts within wsize before the same panel-site markers).  tests/test_rb_build.py checks the files
+    against the reference's own for the `tiny` panel, byte for byte."""
+    text = panel_text(panel)
+    n = len(text)
+    sa = suffix_array(text)
+    bwt = text[sa - 1]                                        # sa - 1 = -1 at the terminator's row wraps to it
+    bwt.tofile(prefix + ".bwt")
+    starts = np.concatenate([[0], np.nonzero(bwt[1:] != bwt[:-1])[0] + 1])
+    ends = np.concatenate([starts[1:] - 1, [n - 1]])
+    for suf, rows in ((".ssa", starts), (".esa", ends)):
+        np.stack([rows, sa[rows]], axis=1).astype(np.uint64).tofile(prefix + suf)
+    with open(prefix + ".docs", "w") as f:
+        f.write("".join("%s %d\n" % ("ref" if h == 0 else "h%d" % h, panel.seq_start(h)) for h in range(panel.nseq)))
+    if not markers:
+        return
+    # MarkerT words (pfbwt-f/include/marker.hpp): allele << 60 | reference position, in text order
+    pos = np.concatenate([panel.sites + panel.seq_start(h) for h in range(panel.nseq)])
+    alleles = np.concatenate([np.zeros(len(panel.sites), np.uint64)] + [g.astype(np.uint64) for g in panel.gt])
+    words = (alleles << np.uint64(60)) | np.tile(panel.sites.astype(np.uint64), panel.nseq)
+    a, b = np.searchsorted(pos, sa), np.searchsorted(pos, sa + wsize)
+    out, block = [], None
+    for row in np.nonzero(b > a)[0].tolist():
+        ws = words[a[row]:b[row]].tolist()
+        if block and block[1] == row - 1 and block[2] == ws:
+            block[1] = row
+            continue
+        if block:
+            out += block[:2] + block[2] + [0xFFFFFFFFFFFFFFFF]
+        block = [row, row, ws]
+    if block:
+        out += block[:2] + block[2] + [0xFFFFFFFFFFFFFFFF]
+    np.array(out, np.uint64).tofile(prefix + ".ma")
+
+
+def build_index_gpu(panel: Panel, prefix: str, markers: bool = True, device: int = 0, log=sys.stderr) -> dict:
+    """The same index files as build_index, without the reference: write_raw_index, then the project's own
+    rb_build on the GPU (rowbowt_b200.build_index).  Returns timings."""
+    import rowbowt_b200 as rb
+    t = {}
+    t0 = time.time(); write_raw_index(panel, prefix, markers=markers); t["raw"] = time.time() - t0
+    t0 = time.time(); rb.build_index(prefix, prefix, sa=True, markers=markers, device=device); t["rb_build"] = time.time() - t0
+    for suf in (".bwt", ".ssa", ".esa", ".ma"):
+        if os.path.exists(prefix + suf):
+            os.remove(prefix + suf)
+    print("build_index_gpu %s: %s" % (prefix, {k: round(v, 1) for k, v in t.items()}), file=log)
+    return t
+
+
 def make_reads(panel: Panel, n_reads: int, read_len: int = 150, seed: int = 3,
                err_rate: float = 0.0, n_rate: float = 0.0, chunk: int = 1 << 20):
     """uint8[n_reads, read_len] ASCII reads: uniform substrings of uniformly
