@@ -1261,10 +1261,13 @@ void run_greedy(rbg_index* ix, Lane& L, rbg_stats& s, const rbg_batch* in, const
     const uint64_t n_items = 2 * n;
     for (DBuf* d : {&g.item_seeds, &g.item_words, &g.seed_off, &g.word_off}) d->reserve((n_items + 2) * 8);
     rd->scan_tmp.reserve(scan_tmp_bytes(n_items + 1));
+    // Every A/C/G/T gets its code even when the index lacks that base: the minus strand complements the code, so a base
+    // the index lacks may stand for one it has.  A code the index lacks ends its seed through LF (an empty range), as
+    // in the reference; only 'N' after seq_ntoa has no code.
     CodeTable ct;
     for (int c = 0; c < 256; ++c) {
-        const int8_t code = ix->codes.code_of[seq_ntoa((uint8_t) c)];
-        ct.code_of[c] = (code >= 0 && code < 4) ? code : (int8_t) -1;
+        const uint8_t a = seq_ntoa((uint8_t) c);
+        ct.code_of[c] = a == 'A' ? 0 : a == 'C' ? 1 : a == 'G' ? 2 : a == 'T' ? 3 : (int8_t) -1;
     }
     DevBatch b{rd->bases.as<uint8_t>(), rd->offs.as<uint64_t>(), n, rd->n_bytes, 0, n, rd->packed.as<uint64_t>(),
                rd->flags.as<uint8_t>(), g.bad.as<uint32_t>()};

@@ -214,6 +214,8 @@ void validate_toehold(const ToeholdArrays& t, const std::string& what) {
     for (uint64_t k = 0; k < t.r; ++k) {
         if (t.pred[k] >= t.n || (k && t.pred[k] <= t.pred[k - 1])) throw format_error("sampled positions not ascending below n in " + what);
         if (t.pred_to_run[k] > t.r) throw format_error("pred_to_run value beyond r in " + what);
+        // a sample becomes a toehold and then a phi argument, which indexes the phi directory without a bound
+        if (t.samples_last[k] >= t.n) throw format_error("run-end sample beyond n in " + what);
     }
 }
 
@@ -226,6 +228,8 @@ void validate_markers(const MarkerArrays& m, const std::string& what) {
     ascending_below(m.ends, m.size_ends, "window ends");
     ascending_below(m.idxs, m.size_idxs, "window indexes");
     if (!m.idxs.empty() && m.idxs.back() > m.arr.size()) throw format_error("marker array: window index beyond the marker words in " + what);
+    // the select past the last window returns size_idxs: it ends the last window's gather
+    if (m.size_idxs > m.arr.size()) throw format_error("marker array: index universe beyond the marker words in " + what);
 }
 
 RunsBwt read_rbwt(const std::string& path) {

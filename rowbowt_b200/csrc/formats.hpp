@@ -51,8 +51,9 @@ struct MarkerArrays {
 // Consistency of decoded (or caller-supplied) arrays, checked before any layout is built from them: a corrupted file must end
 // as format_error, never as an out-of-range access in the layout builders or on the device.  `what` names the source in the message.
 //   runs:    R heads and lengths, every length in [1, n - (sum so far)], lengths sum to n
-//   toehold: r sorted sample positions < n, r samples, pred_to_run values <= r
-//   markers: window starts / ends / indexes ascending inside their universes, indexes <= the number of marker words
+//   toehold: r sorted sample positions < n, r samples < n, pred_to_run values <= r
+//   markers: window starts / ends / indexes ascending inside their universes, indexes and their universe <= the number of
+//            marker words
 void validate_runs(const RunsBwt& b, const std::string& what);
 void validate_toehold(const ToeholdArrays& t, const std::string& what);
 void validate_markers(const MarkerArrays& m, const std::string& what);

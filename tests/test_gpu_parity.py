@@ -302,12 +302,11 @@ def test_ftab_of_another_index_is_rejected_and_load_flag(tmp_path):
         rb.GpuIndex.open(tiny, ftab=True)           # no tiny.ftab: "bad file"
 
 
-def _wide_synthetic_index():
+def _wide_synthetic_index(monkeypatch):
     """(GpuIndex, OracleIndex, reads) over a synthetic run sequence with n ~ 5.5*10^10 and fabricated toehold arrays."""
     from oracle import rbformats as F
-    old = os.environ.get("RBG_PHI_SHIFT")
-    os.environ["RBG_PHI_SHIFT"] = "14"                    # 2^14-position buckets: 3 M slots instead of 400 M
-    try:
+    with monkeypatch.context() as mp:
+        mp.setenv("RBG_PHI_SHIFT", "14")                  # 2^14-position buckets: 3 M slots instead of 400 M
         rng = np.random.default_rng(17)
         R = 200_000
         heads = np.frombuffer(b"ACGT", np.uint8)[np.cumsum(rng.integers(1, 4, R)) % 4].copy()      # adjacent runs differ
@@ -324,11 +323,6 @@ def _wide_synthetic_index():
         tsa = F.Toehold(r=R, n=n, pred=pred, samples_last=samples_last, pred_to_run=pred_to_run)
         orc = O.OracleIndex(bwt, tsa)
         ix = rb.GpuIndex.from_arrays(n, heads, lens, tsa=(pred, samples_last, pred_to_run))
-    finally:
-        if old is None:
-            os.environ.pop("RBG_PHI_SHIFT", None)
-        else:
-            os.environ["RBG_PHI_SHIFT"] = old
     acgt = np.frombuffer(b"ACGT", np.uint8)
     seqs = [acgt[rng.integers(0, 4, int(m))].tobytes() for m in rng.integers(1, 22, 4000)]
     seqs += [b"A", b"C", b"G", b"T", b"\x01", b"A\x01", b"N"]
@@ -336,11 +330,11 @@ def _wide_synthetic_index():
 
 
 @pytest.mark.parametrize("ftab_k", [0, 8])
-def test_wide_positions_synthetic_index(ftab_k):
+def test_wide_positions_synthetic_index(ftab_k, monkeypatch):
     """Positions beyond 2^32 (BASELINE config 5 needs 38 bits; SURVEY §7 'position width'): a synthetic run
     sequence with n ~ 5.5*10^10 and fabricated toehold arrays.  find_range / LF_w_loc / phi are pure rank
     arithmetic over the arrays, so the oracle defines the answer for any such input."""
-    ix, orc, seqs, n = _wide_synthetic_index()
+    ix, orc, seqs, n = _wide_synthetic_index(monkeypatch)
     ix.build_ftab(ftab_k)
     info = ix.info()
     assert info.n == n and info.window == 32767

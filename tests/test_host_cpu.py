@@ -649,3 +649,80 @@ def test_public_header_compiles_as_c_and_cpp_and_links(compiler, std, tmp_path):
     p = subprocess.run([exe], capture_output=True)
     assert p.returncode == 0, (p.stdout, p.stderr)
     assert b"bad file" in p.stdout
+
+
+FAST_DIV_HARNESS = r"""
+#include <vector_types.h>
+#include <cstdio>
+#include <thread>
+#include <vector>
+#include "device_index.cuh"
+
+// set_fast_div for window W over n positions; the quotient x / m (m = odd part of W) for x = p >> div_k < 2^31
+static rbg::DevLeafDir div_for(uint32_t W, uint64_t n) {
+    rbg::DevLeafDir D{};
+    D.window = W;
+    D.n = n;
+    rbg::set_fast_div(D);
+    return D;
+}
+
+int main() {
+    const uint64_t top = 1ull << 31;
+    long long bad = 0;
+    std::vector<uint32_t> mul_of(32768, 0), s_of(32768, 0);
+    for (uint32_t W = 16; W <= 32767; ++W) {
+        uint32_t k = 0;
+        while (!((W >> k) & 1u)) ++k;
+        const uint64_t m = W >> k, n_max = (top << k) - 1;       // the largest n with (n >> k) < 2^31
+        const rbg::DevLeafDir D = div_for(W, n_max);
+        if (!D.div_fast || D.div_k != k) { printf("W=%u: no fast path at n=%llu\n", W, (unsigned long long) n_max); ++bad; continue; }
+        if (div_for(W, n_max + 1).div_fast) { printf("W=%u: fast path at n=%llu\n", W, (unsigned long long) (n_max + 1)); ++bad; }
+        for (uint64_t x = top - (1ull << 16); x < top; ++x)
+            if (((x * D.div_mul) >> D.div_s) != x / m && bad++ < 20) printf("W=%u x=%llu\n", W, (unsigned long long) x);
+        if (mul_of[m] && (mul_of[m] != D.div_mul || s_of[m] != D.div_s)) { printf("W=%u: multiplier differs\n", W); ++bad; }
+        mul_of[m] = D.div_mul;
+        s_of[m] = D.div_s;
+    }
+    // every x = 0 and x = -1 (mod m) among the top 2^24 values below 2^31, once per odd part m (div_mul / div_s depend on m only)
+    const unsigned T = std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    std::vector<long long> wrong(T, 0);
+    std::vector<std::thread> th;
+    for (unsigned t = 0; t < T; ++t)
+        th.emplace_back([&, t] {
+            for (uint64_t m = 1 + 2 * t; m < 32768; m += 2 * T) {
+                if (!mul_of[m]) continue;
+                const uint64_t mul = mul_of[m], s = s_of[m], q0 = (top - (1ull << 24)) / m;
+                for (uint64_t q = q0, x = q0 * m; x < top; ++q, x += m) {
+                    wrong[t] += ((x * mul) >> s) != q;
+                    if (x + m - 1 < top) wrong[t] += (((x + m - 1) * mul) >> s) != q;
+                }
+            }
+        });
+    for (auto& x : th) x.join();
+    for (long long w : wrong) bad += w;
+    printf("%lld wrong\n", bad);
+    return bad ? 1 : 0;
+}
+"""
+
+
+def test_fast_window_division_is_exact(tmp_path):
+    """line_of divides a BWT position by the window with set_fast_div's 32-bit multiplier whenever (n >> k) < 2^31
+    (W = m * 2^k, m odd).  The real set_fast_div (device_index.cuh) against exact division for every window in [16, 32767]
+    at the largest n that enables the fast path: the top 2^16 quotient arguments below 2^31 and every multiple of m and
+    every x = -1 (mod m) among the top 2^24; one step past that n the fast path must be off."""
+    import shutil
+    cxx = shutil.which("g++") or shutil.which("c++")
+    cuda_inc = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "include")      # vector_types.h: ulonglong2
+    if not cxx or not os.path.exists(os.path.join(cuda_inc, "vector_types.h")):
+        pytest.skip("no host C++ compiler or CUDA toolkit headers")
+    src = tmp_path / "fast_div.cpp"
+    src.write_text(FAST_DIV_HARNESS)
+    exe = str(tmp_path / "fast_div")
+    p = subprocess.run([cxx, "-O2", "-std=c++17", "-pthread", "-I", cuda_inc, "-I", os.path.join(ROOT, "rowbowt_b200", "csrc"),
+                        str(src), "-o", exe], capture_output=True)
+    assert p.returncode == 0, p.stderr.decode()
+    p = subprocess.run([exe], capture_output=True)
+    assert p.returncode == 0, p.stdout.decode()
+    assert p.stdout.decode().strip() == "0 wrong"

@@ -208,10 +208,10 @@ def test_rb_align_stdout_to_a_file_is_the_same_report(d, pre, fq, tag, sa, ma, t
     assert open(out, "rb").read() == b"header line\n" + want + b"trailer\n" + want
 
 
-def test_wide_index_narrow_locations_have_a_high_plane():
+def test_wide_index_narrow_locations_have_a_high_plane(monkeypatch):
     """An index with n > 2^32 (fabricated arrays as in test_wide_positions_synthetic_index): 5-byte locations."""
     from test_gpu_parity import _wide_synthetic_index
-    ix, orc, seqs, n = _wide_synthetic_index()
+    ix, orc, seqs, n = _wide_synthetic_index(monkeypatch)
     wide = ix.query(seqs, RBG_LOCATE, max_hits=6)
     narrow = ix.query(seqs, RBG_LOCATE | RBG_NARROW_LOCS, max_hits=6)
     assert narrow.narrow_bytes == 5
