@@ -142,8 +142,8 @@ typedef struct {
     uint32_t ftab_k;                /* FTab::get_k() of the resident k-mer seed table, 0 = none */
     uint32_t layout;                /* GPU layout of the rank directory: 4 (24 runs per line + L2-resident superblock counts) or 5 (20 runs, u32 counts in the line) */
     uint64_t ftab_bytes;            /* seed table footprint */
-    uint64_t hot_bytes;             /* superblock counts + seed table: the region under the L2 access-policy window */
-    uint64_t l2_pinned_bytes;       /* persisting-L2 set-aside granted for it (0 = window off) */
+    uint64_t hot_bytes;             /* superblock counts + seed table, held in one device allocation */
+    uint64_t l2_pinned_bytes;       /* always 0: no persisting-L2 window is set (the field keeps the struct layout) */
     uint32_t phi_shift;             /* GPU layout: one 32-byte phi slot per 2^phi_shift text positions */
     uint32_t from_cache;            /* 1: this handle was opened from <prefix>.rbgcache (RBG_LOAD_CACHE) */
     uint64_t phi_overflow;          /* slots whose bucket holds more than 3 samples (side array, binary search) */

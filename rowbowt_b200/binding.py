@@ -90,7 +90,8 @@ class Stats(C.Structure):
 
 
 def lib_path() -> str:
-    # RBG_LIB: another build of the SAME library (A/B runs of kernel variants in tools/); never a fallback
+    # RBG_LIB: another build of the SAME library, e.g. one made at another commit, so that bench.py or a tool can A/B
+    # the two on the same inputs; never a fallback
     return os.environ.get("RBG_LIB") or os.path.join(HERE, "librowbowt_gpu.so")
 
 

@@ -228,10 +228,8 @@ struct rbg_index {
     CodeTable codes{};
     DevFtab ft{};                        // k-mer seed table (k == 0: none)
     std::vector<ulonglong2> ft_host;     // host copy of ft.range (rbg_ftab_save / rbg_ftab_lookup)
-    void* hot = nullptr;                 // one allocation: superblock counts + ftab, covered by the L2 access-policy window
+    void* hot = nullptr;                 // one allocation: superblock counts + ftab
     size_t hot_bytes = 0;
-    bool l2_window = false;              // an access-policy window is configured (RBG_L2_PIN)
-    cudaStreamAttrValue l2_attr{};
     rbg_info info{};
     rbg_stats stats{};                   // of the call that finished last
     std::mutex mu;                       // lanes, result pools, stats
@@ -255,7 +253,6 @@ struct rbg_index {
             std::unique_ptr<Lane> fresh(new Lane);
             CU(cudaSetDevice(device));
             fresh->create();
-            if (l2_window) CU(cudaStreamSetAttribute(fresh->stream, cudaStreamAttributeAccessPolicyWindow, &l2_attr));
             l = fresh.get();
             lanes.push_back(std::move(fresh));
         }
@@ -299,11 +296,10 @@ struct LaneHold {
 };
 
 // The small, hot arrays -- superblock counts (read by every LF step) and the k-mer seed table (read
-// once per read) -- live in ONE allocation, (re)built whenever the ftab changes.  An access-policy window can mark
-// it persisting in L2 (RBG_L2_PIN=1).  Measured on the BASELINE batch with the final 158 MB directory the window
-// LOSES 4 % (22.9 vs 21.9 ms: both arrays are hot enough to stay under plain LRU, and the carve-out is taken from
-// the lines), and a window over the directory itself (RBG_L2_PIN=2, 83 MB persisting) loses 6 % and starves the
-// phi slots (locate 12.7 -> 51 ms) -- so the default is no window.
+// once per read) -- live in ONE allocation, (re)built whenever the ftab changes.  No L2 access-policy window is set:
+// measured on the BASELINE batch with the final 158 MB directory, a window marking this region persisting LOST 4 %
+// (22.9 vs 21.9 ms: both arrays are hot enough to stay under plain LRU, and the carve-out is taken from the lines), and
+// a window over the directory itself (83 MB persisting) lost 6 % and starved the phi slots (locate 12.7 -> 51 ms).
 void rebuild_hot_region(rbg_index* ix, uint32_t k, bool with_toe) {
     const size_t super_bytes = (size_t) ix->dir.n_super * 4 * sizeof(uint64_t);
     const size_t entries = k ? (size_t) 1 << (2 * k) : 0;
@@ -328,30 +324,6 @@ void rebuild_hot_region(rbg_index* ix, uint32_t k, bool with_toe) {
     ix->info.ftab_bytes = 0;
     ix->info.hot_bytes = total;
     ix->info.l2_pinned_bytes = 0;
-    const char* e = getenv("RBG_L2_PIN");
-    if (!e || atoi(e) == 0) return;
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, ix->device));
-    if (prop.persistingL2CacheMaxSize <= 0 || prop.accessPolicyMaxWindowSize <= 0) return;
-    size_t set_aside = std::min<size_t>(total, (size_t) prop.persistingL2CacheMaxSize);
-    cudaStreamAttrValue attr{};
-    attr.accessPolicyWindow.base_ptr = region;
-    attr.accessPolicyWindow.num_bytes = std::min<size_t>(total, (size_t) prop.accessPolicyMaxWindowSize);
-    if (e && atoi(e) == 2) {
-        // experiment (RBG_L2_PIN=2): the window over the rank directory instead -- a fixed pseudo-random share of its
-        // lines (hitRatio) persists in the whole carve-out; seed table and superblock counts stay under plain LRU
-        set_aside = (size_t) prop.persistingL2CacheMaxSize;
-        attr.accessPolicyWindow.base_ptr = const_cast<uint32_t*>(ix->dir.lines);
-        attr.accessPolicyWindow.num_bytes = std::min<size_t>((size_t) ix->info.n_lines * 64, (size_t) prop.accessPolicyMaxWindowSize);
-    }
-    CU(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, set_aside));
-    attr.accessPolicyWindow.hitRatio = (float) std::min(1.0, (double) set_aside / (double) attr.accessPolicyWindow.num_bytes);
-    attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-    ix->l2_attr = attr;
-    ix->l2_window = true;
-    for (auto& l : ix->lanes) CU(cudaStreamSetAttribute(l->stream, cudaStreamAttributeAccessPolicyWindow, &attr));
-    ix->info.l2_pinned_bytes = set_aside;
 }
 
 // RowBowt::build_ftab(k), include/rowbowt.hpp:726-743, as one kernel over all 4^k k-mers; with the
@@ -1039,7 +1011,6 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
     auto cut = [&](int c) { return (uint64_t) ((__uint128_t) n * (uint64_t) c / (uint64_t) n_chunks); };
 
     uint32_t launches = 0;
-    const bool two_streams = !(getenv("RBG_SEARCH_STREAMS") && atoi(getenv("RBG_SEARCH_STREAMS")) == 1);
     // tests: RBG_TEST_STALL="a,b" stalls even chunks' stream for a microseconds in front of their pack and odd chunks' stream for
     // b microseconds between their pack and their search
     unsigned long long stall_ns[2] = {0, 0};
@@ -1047,7 +1018,6 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         unsigned long long a = 0, bb = 0;
         if (sscanf(e, "%llu,%llu", &a, &bb) >= 1) { stall_ns[0] = a * 1000ull; stall_ns[1] = bb * 1000ull; }
     }
-    const bool order_packs = two_streams && !getenv("RBG_TEST_UNORDERED_PACKS");      // tools/exp_pack_race.py: the race, on purpose
     CU(cudaEventRecord(L.ev_span[0], si));
     // offsets first (pack's flagging searches them), re-based to 0 when the caller's are not
     std::vector<uint64_t> rebased;
@@ -1138,8 +1108,8 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         CU(cudaEventRecord(L.ev_in[c], si));
         // pack + search of consecutive chunks alternate between two streams, so that the next chunk's CTAs take the SMs
         // the tail of this one leaves idle (16 launches per batch: their tails were ~8 % of the end-to-end step)
-        cudaStream_t ss = two_streams ? L.s_srch[c & 1] : sc;
-        if (two_streams && c < 2) CU(cudaStreamWaitEvent(ss, L.ev_span[2], 0));      // counters and flags are zeroed on sc
+        cudaStream_t ss = L.s_srch[c & 1];
+        if (c < 2) CU(cudaStreamWaitEvent(ss, L.ev_span[2], 0));                     // counters and flags are zeroed on sc
         CU(cudaStreamWaitEvent(ss, L.ev_in[c], 0));
         b.r0 = r0;
         b.r1 = r1;
@@ -1151,9 +1121,9 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
             // compute-sanitizer's timing; RBG_TEST_STALL reproduces the order).  A search reading the word while the next
             // chunk's pack rewrites it sees the same bits for its own bases either way.
             if (stall_ns[0] && !(c & 1)) launch_stall(stall_ns[0], ss);
-            if (order_packs && c > 0) CU(cudaStreamWaitEvent(ss, L.ev_pack[c - 1], 0));
+            if (c > 0) CU(cudaStreamWaitEvent(ss, L.ev_pack[c - 1], 0));
             launches += launch_pack(b, ix->codes, b1 - b0, ss);
-            if (order_packs) CU(cudaEventRecord(L.ev_pack[c], ss));
+            CU(cudaEventRecord(L.ev_pack[c], ss));
             if (stall_ns[1] && (c & 1)) launch_stall(stall_ns[1], ss);
         }
         launches += launch_search(ix->dir, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[c], ss);
@@ -1161,7 +1131,7 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         if (narrow_rg) launches += launch_narrow_ranges(r.lo, r.hi, rd->lo32.as<uint32_t>(), rd->hi32.as<uint32_t>(), r0, r1, ss);
         CU(cudaEventRecord(L.ev_cmp[c], ss));
         CU(cudaStreamWaitEvent(so, L.ev_cmp[c], 0));
-        if (two_streams) CU(cudaStreamWaitEvent(sc, L.ev_cmp[c], 0));                 // what follows on sc (counts, scans, phi, markers) needs this chunk's ranges
+        CU(cudaStreamWaitEvent(sc, L.ev_cmp[c], 0));                                  // what follows on sc (counts, scans, phi, markers) needs this chunk's ranges
         if (c == 0) CU(cudaEventRecord(L.ev_span[4], so));
         if (narrow_rg) {
             CU(cudaMemcpyAsync(out->lo32 + r0, rd->lo32.as<uint32_t>() + r0, (r1 - r0) * 4, cudaMemcpyDeviceToHost, so));

@@ -296,11 +296,7 @@ __device__ __forceinline__ bool lf_step_lines(const DevLeafDir& D, const uint64_
         // only shrink at variant sites) the answer is yes without looking; the third rank is computed only in warp
         // steps where some lane's range shrank -- about one warp step in six on the BASELINE workload.
         const bool whole = new_end - new_lo == h - l + 1;
-#ifdef RBG_TOE_ALWAYS                                            // A/B build (make alt): the third rank in every step
-        const bool unsure = act;
-#else
         const bool unsure = act && !whole && new_end != new_lo;
-#endif
         hi_is_c = whole;
         if (__any_sync(0xFFFFFFFFu, unsure)) {
             uint32_t rc = leaf_rank_x<V>(B, xb, xs, qb - 1u), rel_c = leaf_rel_count<V>(B, c);
@@ -310,67 +306,6 @@ __device__ __forceinline__ bool lf_step_lines(const DevLeafDir& D, const uint64_
                 if ((fl & kFlagTerm) && c == 0) term_fix(D, B, h, qb - 1u, sk_c, rc);
             }
             if (unsure) hi_is_c = (rel_b + rb) != (rel_c + rc);
-        }
-    }
-    if (!act || new_end == new_lo) return false;
-    lo = new_lo;
-    hi = new_end - 1;
-    return true;
-}
-
-// ---- lane-PAIR form (search_pair_kernel): two lanes per read, one rank each ---------------------------------
-// The even lane of a pair answers rank_c(lo), the odd lane rank_c(hi+1); each holds ONE directory line in registers
-// (16 instead of 32), decodes one rank (10 packed mins + 20 dot products instead of 20 + 40) and the two exchange
-// their results with one 64-bit shuffle.  When lo and hi fall into the same window (~94 % of the steps behind the seed
-// table) both lanes load the same 64 bytes and the L1 coalescer merges the two requests, so the traffic is that of
-// lf_step_lines.  Per read and step the pair issues ~2 x 110 instructions against ~260 for one thread doing both
-// ranks, and the kernel needs 48 registers instead of 64+: more warps per scheduler AND shorter steps.
-// Every lane of the warp must call; both lanes of a pair pass the same c, lo, hi, act and get the same results
-// (hi_is_c is only meaningful on the odd lane).  `lines_touched` counts the pair's distinct lines, split over its lanes.
-template <bool TOEHOLD, int V>
-__device__ __forceinline__ bool lf_step_pair(const DevLeafDir& D, const uint64_t* sup_all, uint32_t c, uint64_t& lo, uint64_t& hi, bool act,
-                                             uint32_t odd, bool& hi_is_c, uint32_t& lines_touched) {
-    constexpr uint32_t kFull = 0xFFFFFFFFu;
-    uint32_t L[16];
-    const uint64_t pos = act ? (odd ? hi : lo) : 0ull;
-    const uint64_t w = line_of(D, pos);
-    const uint32_t q = (uint32_t) pos - (uint32_t) w * D.window + odd;      // rank position inside the window: lo, or hi + 1
-    load_line(D.lines + w * 16, L);
-    const uint64_t* sup = sup_all + (uint64_t) c * D.n_super;
-    const uint64_t base = V == 5 ? sup[w >> D.sb_shift] : __ldg(sup + (w >> D.sb_shift));
-    uint32_t xb[6], xs[6];
-    leaf_match<V>(L, leaf_cpat(c), xb, xs);
-    uint32_t rk = leaf_rank_x<V>(L, xb, xs, q);
-    uint32_t rel = leaf_rel_count<V>(L, c);
-    const uint32_t fl = act ? L[15] & kFlagAny : 0u;
-    const bool any_fl = __any_sync(kFull, fl != 0u);              // warp-uniform: some lane sees a variant cluster / the terminator
-    if (any_fl) {
-        uint32_t sk = 0;
-        coop_cluster_fix<V>(D, L, c, q, fl && leaf_inside_cluster(L, q), rk, rel, sk);
-        if ((fl & kFlagTerm) && c == 0) term_fix(D, L, pos + odd, q, sk, rk);
-    }
-    const uint64_t val = base + rel + rk;                          // even: F[c] + #c in BWT[0,lo); odd: F[c] + #c in BWT[0,hi]
-    const uint64_t other = __shfl_xor_sync(kFull, val, 1);
-    const uint32_t w_other = __shfl_xor_sync(kFull, (uint32_t) w, 1);
-    const uint64_t new_lo = odd ? other : val, new_end = odd ? val : other;
-    lines_touched += !act ? 0u : (odd ? (w_other != (uint32_t) w ? 1u : 0u) : 1u);
-    hi_is_c = false;
-    if (TOEHOLD) {
-        // BWT[hi] == c, as in lf_step_lines: known when the whole range maps (count grows by the range size), otherwise the
-        // odd lane (which holds hi's line) ranks once more at hi -- only in warp steps where some range shrank.
-        const bool whole = new_end - new_lo == hi - lo + 1;
-        const bool unsure = act && !whole && new_end != new_lo;
-        hi_is_c = whole;
-        if (__any_sync(kFull, unsure)) {
-            const bool mine = unsure && odd;
-            const uint32_t qc = mine ? q - 1u : 0u;
-            uint32_t rc = leaf_rank_x<V>(L, xb, xs, qc), rel_c = leaf_rel_count<V>(L, c);
-            if (any_fl) {
-                uint32_t sk_c = 0;
-                coop_cluster_fix<V>(D, L, c, qc, mine && fl && leaf_inside_cluster(L, qc), rc, rel_c, sk_c);
-                if (mine && (fl & kFlagTerm) && c == 0) term_fix(D, L, pos, qc, sk_c, rc);
-            }
-            if (mine) hi_is_c = (rel + rk) != (rel_c + rc);
         }
     }
     if (!act || new_end == new_lo) return false;

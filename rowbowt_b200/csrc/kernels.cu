@@ -9,7 +9,6 @@
 //   marker_*_kernel  rle_window_arr::at_range (pfbwt-f/include/rle_window_array.hpp:130-154)
 #include "kernels.cuh"
 
-#include <algorithm>
 #include <cstdlib>
 
 #include <cub/device/device_scan.cuh>
@@ -32,7 +31,9 @@ int grid_for(uint64_t work_items, int block, int per_sm) {
 namespace {
 
 constexpr int kBlock = 256;
-constexpr int kPairMinB = 5;          // CTAs per SM search_pair_kernel is compiled for by default (RBG_SEARCH_MINB overrides)
+// Resident CTAs per SM search_kernel is built and launched for: 4 x 256 threads at 64 registers.  5 x 256 at 48 registers
+// and 9 x 128 at 56 registers spill and measured 26.8 / 22.7 ms against 21.2 ms (profiles/r2_search_occupancy_variants.jsonl).
+constexpr int kSearchCtas = 4;
 
 __device__ __forceinline__ uint64_t mix64(uint64_t z) {
     z += 0x9E3779B97F4A7C15ull;
@@ -159,9 +160,9 @@ struct ToeholdTrack {
 // whole warp (device_index.cuh).
 // Layout 5 (V == 5): the superblock bases (<= 4 x 256 u64) are copied to shared memory once per CTA, so an LF step
 // issues no load besides its one or two directory lines.
-template <bool TOEHOLD, int MINB, int V>
-__global__ void __launch_bounds__(kBlock, MINB) search_kernel(DevLeafDir D, DevToehold T, DevFtab ft, DevBatch b, DevResult r, DevCounters* ctr,
-                                                             unsigned long long* cursor) {
+template <bool TOEHOLD, int V>
+__global__ void __launch_bounds__(kBlock, kSearchCtas) search_kernel(DevLeafDir D, DevToehold T, DevFtab ft, DevBatch b, DevResult r,
+                                                                     DevCounters* ctr, unsigned long long* cursor) {
     constexpr uint32_t kFull = 0xFFFFFFFFu;
     __shared__ uint64_t s_base[V == 5 ? 4 * kMaxSuper5Dev : 1];
     const uint64_t* sup = D.super;
@@ -178,11 +179,7 @@ __global__ void __launch_bounds__(kBlock, MINB) search_kernel(DevLeafDir D, DevT
     ToeholdTrack tt;
     tt.init();
     bool exhausted = false;                                 // warp-uniform: the launch has handed out its last read
-#ifdef RBG_NO_REFILL                                        // A/B build (make alt): a warp takes 32 reads, finishes all, takes the next 32
-    constexpr int kRefillAt = 32;
-#else
     constexpr int kRefillAt = 8;
-#endif
     for (;;) {
         const uint32_t idle = __ballot_sync(kFull, !have);
         if (!exhausted && (idle == kFull || __popc(idle) >= kRefillAt)) {
@@ -259,111 +256,6 @@ __global__ void __launch_bounds__(kBlock, MINB) search_kernel(DevLeafDir D, DevT
         }
     }
     const unsigned long long st = warp_sum((unsigned long long) steps), ln = warp_sum((unsigned long long) lines);
-    if (lane == 0 && st) {
-        atomicAdd(&ctr->lf_steps, st);
-        atomicAdd(&ctr->lf_lines, ln);
-    }
-}
-
-// The same search with TWO LANES PER READ (lf_step_pair, device_index.cuh): the even lane carries rank(lo), the odd lane
-// rank(hi+1) and the toehold bookkeeping; both keep the read's state (identical values), so the set-up and the step
-// loop are uniform code and the loads of a pair coalesce.  16 reads per warp, refilled when a quarter of the pairs is idle.
-template <bool TOEHOLD, int MINB, int V>
-__global__ void __launch_bounds__(kBlock, MINB) search_pair_kernel(DevLeafDir D, DevToehold T, DevFtab ft, DevBatch b, DevResult r, DevCounters* ctr,
-                                                                   unsigned long long* cursor) {
-    constexpr uint32_t kFull = 0xFFFFFFFFu;
-    __shared__ uint64_t s_base[V == 5 ? 4 * kMaxSuper5Dev : 1];
-    const uint64_t* sup = D.super;
-    if (V == 5) {
-        for (uint32_t i = threadIdx.x; i < 4u * (uint32_t) D.n_super; i += blockDim.x) s_base[i] = __ldg(D.super + i);
-        __syncthreads();
-        sup = s_base;
-    }
-    const uint32_t lane = threadIdx.x & 31u, odd = lane & 1u;
-    uint32_t steps = 0, lines = 0;                          // per lane: far below 2^32
-    bool have = false;                                      // this pair owns a read that is not finished
-    uint64_t i = 0, lo = 0, hi = 0, x = 0, word = 0;
-    uint32_t left = 0;
-    ToeholdTrack tt;
-    tt.init();
-    bool exhausted = false;                                 // warp-uniform: the launch has handed out its last read
-    constexpr int kRefillAt = 4;                            // idle pairs that trigger a refill
-    for (;;) {
-        const uint32_t idle = __ballot_sync(kFull, !have);
-        const uint32_t n_idle = (uint32_t) __popc(idle) >> 1;
-        if (!exhausted && (idle == kFull || n_idle >= (uint32_t) kRefillAt)) {
-            unsigned long long base = 0;
-            const int leader = __ffs(idle) - 1;
-            if ((int) lane == leader) base = atomicAdd(cursor, (unsigned long long) n_idle);
-            base = __shfl_sync(kFull, base, leader);
-            exhausted = b.r0 + base + (unsigned long long) n_idle >= b.r1;
-            if (!have) {
-                i = b.r0 + base + (uint64_t) ((uint32_t) __popc(idle & ((1u << lane) - 1u)) >> 1);
-                const uint32_t fl = i < b.r1 ? (uint32_t) b.flags[i] : (uint32_t) kReadExotic;
-                if (!(fl & kReadExotic)) {                  // search_bytes_kernel owns exotic reads
-                    have = true;
-                    lo = 0;
-                    hi = D.n - 1;                           // full_range, rowbowt.hpp:115-118
-                    bool alive = !(fl & kReadDead);
-                    tt.init();
-                    left = 0;
-                    if (alive) {
-                        const uint64_t beg = b.offs[i], end = b.offs[i + 1];
-                        x = end;
-                        if (ft.k && end - beg >= ft.k) {    // seed table, as in search_kernel
-                            x = end - ft.k;
-                            const uint32_t sh = 2u * (uint32_t) (x & 31);
-                            uint64_t key = __ldg(b.packed + (x >> 5)) >> sh;
-                            if (sh + 2u * ft.k > 64u) key |= __ldg(b.packed + (x >> 5) + 1) << (64u - sh);
-                            key &= (1ull << (2u * ft.k)) - 1;
-                            const ulonglong2 seed = __ldg(ft.range + key);
-                            lo = seed.x;
-                            hi = seed.y;
-                            alive = lo <= hi;
-                            if (TOEHOLD && alive) tt.unpack(__ldg(ft.toe + key));
-                        }
-                        left = alive ? (uint32_t) (x - beg) : 0u;
-                        if (left) word = __ldg(b.packed + ((x - 1) >> 5));
-                    }
-                    if (!alive) { lo = 1; hi = 0; }         // the empty range is exactly (1,0)
-                }
-            }
-        }
-        if (!__any_sync(kFull, have)) {
-            if (exhausted) break;
-            continue;
-        }
-        const bool act = have && left != 0u;
-        uint32_t c = 0;
-        if (act) {
-            --x;
-            if ((x & 31) == 31) word = __ldg(b.packed + (x >> 5));
-            c = (uint32_t) (word >> (2 * (x & 31))) & 3u;
-        }
-        bool hi_is_c;
-        const bool ok = lf_step_pair<TOEHOLD, V>(D, sup, c, lo, hi, act, odd, hi_is_c, lines);
-        if (act) {
-            --left;
-            ++steps;                                        // the failing step is counted, the rest of the read is not searched
-            if (!ok) {
-                left = 0;
-                lo = 1;
-                hi = 0;
-            } else if (TOEHOLD) {
-                tt.step(hi_is_c, hi);
-            }
-        }
-        if (have && left == 0u) {                           // finished: the even lane reports lo, the odd lane hi and the toehold
-            if (odd) {
-                r.hi[i] = hi;
-                if (TOEHOLD) r.toehold[i] = hi >= lo ? tt.finish(T) : 0;   // cleared LFData on failure, rowbowt.hpp:176-179
-            } else {
-                r.lo[i] = lo;
-            }
-            have = false;
-        }
-    }
-    unsigned long long st = warp_sum(odd ? 0ull : (unsigned long long) steps), ln = warp_sum((unsigned long long) lines);
     if (lane == 0 && st) {
         atomicAdd(&ctr->lf_steps, st);
         atomicAdd(&ctr->lf_lines, ln);
@@ -658,44 +550,18 @@ int launch_pack(const DevBatch& b, const CodeTable& ct, uint64_t approx_bytes, c
     return 1;
 }
 
-template <int V>
-static void launch_search_pair_v(int grid, const DevLeafDir& D, const DevToehold* T, const DevFtab& ft, const DevBatch& b,
-                                 const DevResult& r, DevCounters* ctr, unsigned long long* cursor, cudaStream_t st) {
-    DevToehold t0{};
-    if (T) search_pair_kernel<true, kPairMinB, V><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-    else search_pair_kernel<false, kPairMinB, V><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
-}
-
 int launch_search(const DevLeafDir& D, const DevToehold* T, const DevFtab& ft, const DevBatch& b, const DevResult& r,
                   DevCounters* ctr, unsigned long long* cursor, cudaStream_t st) {
     if (b.r1 <= b.r0) return 0;
-    // tuning knobs, read at every launch so that one process can sweep them (tools/exp_r2d.py)
-    const char *e_pair = getenv("RBG_SEARCH_PAIR"), *e_minb = getenv("RBG_SEARCH_MINB");
-    const bool pair = e_pair && atoi(e_pair) != 0;               // default: one thread per read (measured faster, profiles/r2_pair_sweep.jsonl)
-    const int minb_env = e_minb ? atoi(e_minb) : 0;               // CTAs/SM the kernel is compiled for
-    if (pair) {                                     // compiled for 5 CTAs per SM: the best of 4 / 5 / 6 / 8 (profiles/r2_pair_sweep.jsonl)
-        const int grid = grid_for(2 * (b.r1 - b.r0), kBlock, kPairMinB);
-        if (D.version == 5) launch_search_pair_v<5>(grid, D, T, ft, b, r, ctr, cursor, st);
-        else launch_search_pair_v<4>(grid, D, T, ft, b, r, ctr, cursor, st);
-        return 1;
-    }
     DevToehold t0{};
-    const int minb = minb_env ? minb_env : 4;
     // reads are handed out by the device cursor, so ONE wave of CTAs is the whole grid: resident CTAs per SM x SMs.
-    // 4 CTAs of 256 threads at 64 registers; 5 x 256 at 48 registers and 9 x 128 at 56 registers spill and measured
-    // 26.8 / 22.7 ms against 21.2 ms (profiles/r2_search_occupancy_variants.jsonl); 3 x 256 (no spills at all) is kept as the A/B knob.
-    const int grid = grid_for(b.r1 - b.r0, kBlock, minb == 3 ? 3 : 4);
+    const int grid = grid_for(b.r1 - b.r0, kBlock, kSearchCtas);
     if (D.version == 5) {
-        if (minb == 3) {
-            if (T) search_kernel<true, 3, 5><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-            else search_kernel<false, 3, 5><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
-        } else {
-            if (T) search_kernel<true, 4, 5><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-            else search_kernel<false, 4, 5><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
-        }
+        if (T) search_kernel<true, 5><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
+        else search_kernel<false, 5><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
     } else {
-        if (T) search_kernel<true, 4, 4><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-        else search_kernel<false, 4, 4><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
+        if (T) search_kernel<true, 4><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
+        else search_kernel<false, 4><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
     }
     return 1;
 }
@@ -727,35 +593,31 @@ int launch_locate_counts(const DevResult& r, uint64_t r0, uint64_t r1, uint64_t 
 // (profiles/r2_locate_ctas.jsonl; BASELINE batch / c5w): u64 locations are bound by their store requests and want FEWER warps
 // (4: 10.7 ms, 6: 12.7 ms); narrow locations are latency-bound and want more -- the static kernel 6 (6.5 -> 6.0 ms; 40 registers,
 // no spills without the high plane), the drawing kernel and the high-plane builds 5 (c5w: 14.3 -> 12.4 ms; 6 would spill).
-__host__ inline int default_loc_ctas(bool narrow, bool hi_plane, bool draw) { return !narrow ? 4 : (draw || hi_plane) ? 5 : 6; }
+constexpr int default_loc_ctas(bool narrow, bool hi_plane, bool draw) { return !narrow ? 4 : (draw || hi_plane) ? 5 : 6; }
+// The build whose register budget lets that many CTAs of 256 threads be resident: 64 registers for 4 (and for 5, where the
+// kernel needs <= 48), 40 for 6.  Each form is instantiated for its own count only.
+constexpr int loc_minb(int ctas) { return ctas == 6 ? 6 : 4; }
 
-template <int MINB>
-static void launch_locate_v(bool draw, int grid, const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, DevCounters* ctr,
-                            unsigned long long* cursor, cudaStream_t st) {
+template <bool NARROW, bool HI>
+static void launch_locate_form(bool draw, const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, DevCounters* ctr,
+                               unsigned long long* cursor, cudaStream_t st) {
     if (draw) {
-        if (r.locs_lo && r.locs_hi) locate_draw_kernel<true, true, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr, cursor);
-        else if (r.locs_lo) locate_draw_kernel<true, false, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr, cursor);
-        else locate_draw_kernel<false, false, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr, cursor);
+        constexpr int ctas = default_loc_ctas(NARROW, HI, true);
+        locate_draw_kernel<NARROW, HI, loc_minb(ctas)><<<grid_for(r1 - r0, kBlock, ctas), kBlock, 0, st>>>(P, r, r0, r1, ctr, cursor);
     } else {
-        if (r.locs_lo && r.locs_hi) locate_kernel<true, true, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr);
-        else if (r.locs_lo) locate_kernel<true, false, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr);
-        else locate_kernel<false, false, MINB><<<grid, kBlock, 0, st>>>(P, r, r0, r1, ctr);
+        constexpr int ctas = default_loc_ctas(NARROW, HI, false);
+        locate_kernel<NARROW, HI, loc_minb(ctas)><<<grid_for(r1 - r0, kBlock, ctas), kBlock, 0, st>>>(P, r, r0, r1, ctr);
     }
 }
 
 int launch_locate(const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, uint64_t n_locs, DevCounters* ctr,
                   unsigned long long* cursor, cudaStream_t st) {
     if (r1 <= r0) return 0;
-    const char* d = getenv("RBG_LOC_DRAW");                  // 0 / 1 forces the static / drawing form
+    const char* d = getenv("RBG_LOC_DRAW");                  // test override: 0 / 1 forces the static / drawing form
     const bool draw = d ? atoi(d) != 0 : n_locs / (r1 - r0) >= 256;
-    const char* e = getenv("RBG_LOC_CTAS");                  // tuning knob (tools/exp_r2g.py): resident CTAs per SM
-    const int per_sm = e ? std::max(1, std::min(8, atoi(e))) : default_loc_ctas(r.locs_lo != nullptr, r.locs_hi != nullptr, draw);
-    const int grid = grid_for(r1 - r0, kBlock, per_sm);
-    // the build whose register budget lets per_sm CTAs of 256 threads be resident: 64 registers up to 4 (5 where the kernel
-    // needs <= 48), 40 for 6, 32 for 8
-    if (per_sm <= 5) launch_locate_v<4>(draw, grid, P, r, r0, r1, ctr, cursor, st);
-    else if (per_sm == 6) launch_locate_v<6>(draw, grid, P, r, r0, r1, ctr, cursor, st);
-    else launch_locate_v<8>(draw, grid, P, r, r0, r1, ctr, cursor, st);
+    if (r.locs_lo && r.locs_hi) launch_locate_form<true, true>(draw, P, r, r0, r1, ctr, cursor, st);
+    else if (r.locs_lo) launch_locate_form<true, false>(draw, P, r, r0, r1, ctr, cursor, st);
+    else launch_locate_form<false, false>(draw, P, r, r0, r1, ctr, cursor, st);
     return 1;
 }
 

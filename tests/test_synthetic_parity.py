@@ -4,9 +4,9 @@ terminators (at 0, at n-1, on a window boundary, inside a collapsed CLUSTER stre
 without 'T', phi buckets with more than three samples -- opened with GpuIndex.from_arrays.  The oracle is pure rank / phi
 arithmetic over the same arrays, so it defines the answer for any such input, bit for bit.
 
-Every build runs the search forms (one thread per read, the 3-CTA build, lane pairs) with and without the toehold and
-the seed table, the locate forms (static / drawing, 4 / 5 / 6 / 8 CTAs per SM, u64 / narrow locations), every entry point
-(query, query_packed, staged + checksum, 1 and 16 chunks, narrow ranges) and greedy seeding.  What each case is meant to
+Every build runs the search with and without the toehold and the seed table, both locate forms (static / drawing, each at
+the CTAs per SM it is built for, u64 / narrow locations), every entry point (query, query_packed, staged + checksum, 1 and
+16 chunks, narrow ranges) and greedy seeding.  What each case is meant to
 reach (layout, window, CLUSTER lines, phi overflow slots, the high planes) is asserted, not assumed."""
 import numpy as np
 import pytest
@@ -276,32 +276,25 @@ def test_synthetic_index_equals_oracle(name, layout, window, monkeypatch):
             assert _fast_div(n, info.window)
         mode = RBG_LOCATE | RBG_MARKERS
 
-        # search forms x toehold x seed table
+        # search x toehold x seed table
         for k in (0, 1, 7, 13):
             ix.build_ftab(k)
             assert ix.info().ftab_k == k
-            for form in ({}, {"RBG_SEARCH_MINB": "3"}, {"RBG_SEARCH_PAIR": "1"}):
-                with monkeypatch.context() as mp:
-                    for key, val in form.items():
-                        mp.setenv(key, val)
-                    s.check(ix.query(s.seqs, mode, max_hits=MAX_HITS))
-                    st = ix.stats()
-                    assert st.lf_steps > 0 and st.phi_steps > 0
-                    s.check_count(ix.query(s.count_seqs, RBG_COUNT))
+            s.check(ix.query(s.seqs, mode, max_hits=MAX_HITS))
+            st = ix.stats()
+            assert st.lf_steps > 0 and st.phi_steps > 0
+            s.check_count(ix.query(s.count_seqs, RBG_COUNT))
         ix.build_ftab(0)
 
-        # locate forms: static / drawing kernel, resident CTAs, u64 / narrow locations (+ the high plane above 2^32)
+        # locate forms: static / drawing kernel, u64 / narrow locations (+ the high plane above 2^32)
         for draw in ("0", "1"):
-            for ctas in (None, "4", "6", "8"):
-                with monkeypatch.context() as mp:
-                    mp.setenv("RBG_LOC_DRAW", draw)
-                    if ctas:
-                        mp.setenv("RBG_LOC_CTAS", ctas)
-                    s.check(ix.query(s.seqs, RBG_LOCATE, max_hits=MAX_HITS), markers=False)
-                    assert ix.stats().phi_steps == len(s.locs) - int(np.count_nonzero(np.diff(s.loc_off)))
-                    r = ix.query(s.seqs, RBG_LOCATE | RBG_NARROW_LOCS, max_hits=MAX_HITS)
-                    s.check(r, markers=False)
-                    assert r.narrow_bytes == (5 if n >> 32 else 4)
+            with monkeypatch.context() as mp:
+                mp.setenv("RBG_LOC_DRAW", draw)
+                s.check(ix.query(s.seqs, RBG_LOCATE, max_hits=MAX_HITS), markers=False)
+                assert ix.stats().phi_steps == len(s.locs) - int(np.count_nonzero(np.diff(s.loc_off)))
+                r = ix.query(s.seqs, RBG_LOCATE | RBG_NARROW_LOCS, max_hits=MAX_HITS)
+                s.check(r, markers=False)
+                assert r.narrow_bytes == (5 if n >> 32 else 4)
 
         # entry points
         for threads in (1, 3):

@@ -1,19 +1,13 @@
 #!/usr/bin/env python3
-"""Runs ON THE GPU BOX: (1) random-gather ceilings around the directory footprints, whole-line-per-thread vs lane-pair
-loads; (2) locate_kernel at 1..4 CTAs per SM, narrow / wide; (3) end-to-end count step with one vs two search streams.
-One JSON line per measurement."""
+"""Runs ON THE GPU BOX: random-gather ceilings around the directory footprints, whole-line-per-thread vs lane-pair
+loads.  One JSON line per measurement."""
 import json
 import os
 import sys
-import time
-
-import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import rowbowt_b200 as rb  # noqa: E402
-from rowbowt_b200 import RBG_LOCATE, RBG_NARROW_LOCS  # noqa: E402
-from tools import synth  # noqa: E402
 
 lib = rb.lib()
 for mb in (64, 128, 160, 192, 224, 256, 384):
@@ -21,36 +15,3 @@ for mb in (64, 128, 160, 192, 224, 256, 384):
         g = lib.rbg_gather_roofline(0, mb << 20, line, 256)
         print(json.dumps({"kind": "gather", "footprint_MB": mb, "line_bytes": abs(line), "lane_pairs": line < 0, "gbs": round(g, 1),
                           "glines_per_s": round(g / abs(line), 2)}), flush=True)
-
-cfg, n_reads = "c2", 10_000_000
-prefix = os.path.join(ROOT, "data", cfg, cfg)
-panel = synth.make_panel(*synth.CONFIGS[cfg])
-exact = synth.make_reads(panel, n_reads, 150, seed=3)[0]
-ix = rb.GpuIndex.open(prefix, sa=True, markers=False)
-ix.build_ftab(10)
-st = ix.upload(exact)
-for ctas in ("1", "2", "3", "4"):
-    for narrow in (1, 0):
-        os.environ["RBG_LOC_CTAS"] = ctas
-        mode = RBG_LOCATE | (RBG_NARROW_LOCS if narrow else 0)
-        ix.query_staged(st, mode)
-        ms = []
-        for _ in range(3):
-            ix.query_staged(st, mode)
-            ms.append(ix.stats().ms_phi)
-        s = ix.stats()
-        print(json.dumps({"kind": "locate", "ctas": int(ctas), "narrow": narrow, "ms_phi": float(np.mean(ms)), "phi_steps": s.phi_steps,
-                          "g_phi_per_s": s.phi_steps / float(np.mean(ms)) / 1e6}), flush=True)
-os.environ.pop("RBG_LOC_CTAS")
-st.free()
-pb, keep = ix.pack(exact, threads=8)
-for streams in ("1", "2"):
-    for mode, name in ((0, "count"), (RBG_LOCATE | RBG_NARROW_LOCS, "locate")):
-        os.environ["RBG_SEARCH_STREAMS"] = streams
-        ix.query_raw(pb, mode)
-        t0 = time.perf_counter()
-        for _ in range(5):
-            ix.query_raw(pb, mode)
-        ms = (time.perf_counter() - t0) * 1e3 / 5
-        print(json.dumps({"kind": "e2e", "mode": name, "search_streams": int(streams), "ms_per_step": ms}), flush=True)
-ix.close()

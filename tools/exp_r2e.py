@@ -1,7 +1,6 @@
 #!/usr/bin/env python3
-"""Runs ON THE GPU BOX: (1) latency of one rbg_query_packed call against the batch size (what rb_align's GPU worker pays per
-parsed chunk), alone and with 2 / 4 host threads calling on the same handle; (2) search kernel variants on the BASELINE
-batch (one thread per read / lane pairs).  One JSON line per measurement."""
+"""Runs ON THE GPU BOX: latency of one rbg_query_packed call against the batch size (what rb_align's GPU worker pays per
+parsed chunk), alone and with 2 / 4 host threads calling on the same handle.  One JSON line per measurement."""
 import concurrent.futures as cf
 import ctypes as C
 import json
@@ -51,25 +50,4 @@ for n in (10_000, 53_000, 212_000, 1_000_000):
             print(json.dumps({"kind": "call", "mode": name, "reads": n, "host_threads": threads, "calls": reps * threads,
                               "ms_per_call": dt * 1e3 / reps, "reads_per_s": n * reps * threads / dt}), flush=True)
 
-n_reads = 10_000_000
-sets = {"exact": synth.make_reads(panel, n_reads, 150, seed=3)[0],
-        "noisy": synth.make_reads(panel, n_reads, 150, seed=5, err_rate=0.01, n_rate=0.001)[0]}
-want = {}
-for name, reads in sets.items():
-    st = ix.upload(reads)
-    for v in (sys.argv[1].split(",") if len(sys.argv) > 1 else ["0:4", "1:4", "1:5"]):
-        pair, minb = v.split(":")
-        os.environ["RBG_SEARCH_PAIR"], os.environ["RBG_SEARCH_MINB"] = pair, minb
-        for kind, mode in (("count", 0), ("toehold", RBG_LOCATE | RBG_NARROW_LOCS)):
-            cs = ix.query_staged(st, mode, checksum=True)
-            ms = []
-            for _ in range(4):
-                ix.query_staged(st, mode)
-                ms.append(ix.stats().ms_search)
-            s = ix.stats()
-            ref = want.setdefault((name, kind), cs)
-            print(json.dumps({"kind": kind, "reads_set": name, "pair": int(pair), "minb": int(minb), "ms_search": float(np.mean(ms)),
-                              "ms_min": float(np.min(ms)), "lf_steps": s.lf_steps, "lf_lines": s.lf_lines, "checksum": cs,
-                              "same_digest": cs == ref}), flush=True)
-    st.free()
 ix.close()

@@ -1,5 +1,5 @@
 #!/bin/bash
-# Runs ON THE GPU BOX: parity tests, default bench (all legs), microbenchmarks / knob sweeps, binary-level end to end, ncu captures.
+# Runs ON THE GPU BOX: parity tests, default bench (all legs), gather microbenchmark, binary-level end to end, ncu captures.
 mkdir -p gpurun_out; O=gpurun_out; T=${1:-r2c}
 ( timeout 1700 python -m pytest tests -m gpu -x -q 2>&1 | tail -15 ) | tee $O/${T}_pytest.log
 timeout 900 python bench.py --steps 5 --warmup 3 > $O/${T}_bench.json 2> $O/${T}_bench.err || tail -20 $O/${T}_bench.err

@@ -31,9 +31,9 @@ CLASSES = [
 ]
 
 
-def sass_of(variant, kernel="search_kernel"):
+def sass_of(variant):
     names = subprocess.run(["cuobjdump", "-sass", OBJ], capture_output=True, text=True).stdout
-    m = re.search(r"Function : (\S*%s%s\S*)" % (kernel, variant), names)
+    m = re.search(r"Function : (\S*search_kernel%s\S*)" % variant, names)
     if not m:
         raise SystemExit("kernel variant %s not found" % variant)
     txt = subprocess.run(["cuobjdump", "-sass", "-fun", m.group(1), OBJ], capture_output=True, text=True).stdout
@@ -103,14 +103,12 @@ def main():
            "variants the `common path` column also holds the block of the third rank, which runs in about one warp step in six.",
            "`common path` = what every warp step executes; `rare path` = the forward-branched block that runs only when some lane's",
            "rank position lies inside a collapsed variant cluster / the terminator window (warp-cooperative child-line walk).", ""]
-    for kernel, variant, label in (("search_kernel", "ILb0ELi4ELi5", "one thread per read, count, layout 5 (the default)"),
-                                   ("search_kernel", "ILb1ELi4ELi5", "one thread per read, toehold (-s), layout 5"),
-                                   ("search_kernel", "ILb0ELi4ELi4", "one thread per read, count, layout 4"),
-                                   ("search_pair_kernel", "ILb0ELi5ELi5", "two lanes per read (RBG_SEARCH_PAIR=1), count, layout 5, 5 CTAs/SM"),
-                                   ("search_pair_kernel", "ILb1ELi5ELi5", "two lanes per read, toehold (-s), layout 5, 5 CTAs/SM")):
-        ins = sass_of(variant, kernel)
+    for variant, label in (("ILb0ELi5EE", "count, layout 5 (the default)"),
+                           ("ILb1ELi5EE", "toehold (-s), layout 5"),
+                           ("ILb0ELi4EE", "count, layout 4")):
+        ins = sass_of(variant)
         (start, end, step_start, rare), refill, common, rare_ins = loop_parts(ins)
-        out += ["## %s — `%s<%s>`" % (label, kernel, variant), "",
+        out += ["## %s — `search_kernel<%s>`" % (label, variant), "",
                 "loop 0x%04x..0x%04x; LF step from 0x%04x: **%d instructions on the common path** of a step, %d in the rare block "
                 "(0x%04x..0x%04x), %d in the read refill in front of the step (runs when a quarter of the warp is idle)" % (
                     start, end, step_start, len(common), len(rare_ins), rare[0], rare[1], len(refill)), "",
@@ -119,7 +117,7 @@ def main():
         for name in sorted(set(cc) | set(rc) | set(fc), key=lambda k: -cc.get(k, 0)):
             out.append("| %s | %d | %d | %d |" % (name, cc.get(name, 0), rc.get(name, 0), fc.get(name, 0)))
         out.append("")
-        if variant == "ILb0ELi4ELi5" and kernel == "search_kernel":
+        if variant == "ILb0ELi5EE":
             out += ["<details><summary>common path, full listing</summary>", "", "```"]
             out += ["/*%04x*/ %s ;" % (x[0], x[1]) for x in common]
             out += ["```", "", "</details>", ""]
