@@ -194,6 +194,28 @@ typedef struct {
 int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flags, uint32_t ftab_k, int device, rbg_build_stats* stats);
 int rbg_index_open_raw(const char* prefix, uint32_t flags, int device, rbg_index** out);
 
+/* mps_to_ma (pfbwt-f/src/mps_to_ma.cpp) with SA taken from the index's phi instead of a suffix-array stream: the marker
+ * array (.ma) of a .mps (`first last word* ~0` records over inclusive ranges of text positions).  Row i gets the words of
+ * the record whose range holds SA[i]; a .ma record is a maximal run of rows whose lists are non-empty and equal by value.
+ * Index from <prefix>.rbwt + .tsa when present, else the raw <prefix>.bwt/.ssa/.esa (as rb_build --ftab-only chooses).
+ * Rows [row_begin, min(row_end, n)); blocks are cut at the window edges.  mab_path may be NULL; otherwise the .mab
+ * that rb_build -m would make from this .ma is written too.  Outputs are written to a temporary file and renamed.
+ * Errors: no .tsa (.ssa/.esa) RBG_E_IO; r != R or an empty window RBG_E_ARG; a malformed .mps RBG_E_FORMAT naming the
+ * record (checked, with the index files read, before any CUDA call except for the raw .bwt); with mab_path, a .ma
+ * record at row 0 RBG_E_FORMAT as rb_build -m refuses it (the .ma is still written).
+ * RBG_MA_CHUNK_ROWS in the environment caps the rows of one device pass (tests: many chunk seams). */
+typedef struct {
+    uint64_t n, r, rows, phi_steps;          /* rows walked in the window; phi_step calls */
+    uint64_t mps_records, lists, ma_records, ma_words;
+    double s_read, s_layout, s_write, s_total;
+    float ms_rows_kernel, ms_blocks;          /* CUDA-event time, summed over chunks */
+} rbg_ma_stats;
+int rbg_build_marker_array(const char* index_prefix, const char* mps_path, const char* ma_path, const char* mab_path,
+                           uint64_t row_begin, uint64_t row_end, int device, rbg_ma_stats* stats);
+/* Same over flat arrays (tests): desc needs the runs and the toehold arrays with r == R; its marker fields are ignored. */
+int rbg_build_marker_array_arrays(const rbg_index_desc* desc, const char* mps_path, const char* ma_path, const char* mab_path,
+                                  uint64_t row_begin, uint64_t row_end, int device, rbg_ma_stats* stats);
+
 /* The k-mer seed table (FTab, include/ftab.hpp:12-40).  Once resident, every query of a read of
  * at least k bases starts from the table entry of its last k bases instead of k LF steps; results
  * are identical by construction (entry = find_range(kmer), rb_tests.cpp:147-173).

@@ -78,6 +78,16 @@ class BuildStats(C.Structure):
                 ("s_write", C.c_double), ("s_total", C.c_double)]
 
 
+class MaStats(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("r", C.c_uint64), ("rows", C.c_uint64), ("phi_steps", C.c_uint64),
+                ("mps_records", C.c_uint64), ("lists", C.c_uint64), ("ma_records", C.c_uint64), ("ma_words", C.c_uint64),
+                ("s_read", C.c_double), ("s_layout", C.c_double), ("s_write", C.c_double), ("s_total", C.c_double),
+                ("ms_rows_kernel", C.c_float), ("ms_blocks", C.c_float)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
 class Stats(C.Structure):
     _fields_ = [("reads", C.c_uint64), ("bases", C.c_uint64), ("lf_steps", C.c_uint64), ("lf_lines", C.c_uint64),
                 ("phi_steps", C.c_uint64), ("marker_words", C.c_uint64),
@@ -111,6 +121,10 @@ def lib():
         L.rbg_index_open_arrays.argtypes = [C.POINTER(_Desc), C.c_int, C.POINTER(C.c_void_p)]
         L.rbg_index_open_raw.argtypes = [C.c_char_p, C.c_uint32, C.c_int, C.POINTER(C.c_void_p)]
         L.rbg_build_index.argtypes = [C.c_char_p, C.c_char_p, C.c_uint32, C.c_uint32, C.c_int, C.POINTER(BuildStats)]
+        L.rbg_build_marker_array.argtypes = [C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64, C.c_int,
+                                             C.POINTER(MaStats)]
+        L.rbg_build_marker_array_arrays.argtypes = [C.POINTER(_Desc), C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64,
+                                                    C.c_int, C.POINTER(MaStats)]
         L.rbg_index_close.argtypes = [C.c_void_p]
         L.rbg_index_info.argtypes = [C.c_void_p, C.POINTER(Info)]
         L.rbg_last_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
@@ -210,6 +224,34 @@ def build_index(in_prefix: str, out_prefix: str, sa: bool = False, markers: bool
     st = BuildStats()
     flags = (RBG_LOAD_SA if sa else 0) | (RBG_LOAD_MA if markers else 0) | (RBG_LOAD_FT if ftab_k else 0)
     _check(lib().rbg_build_index(in_prefix.encode(), out_prefix.encode(), flags, ftab_k, device, C.byref(st)))
+    return st
+
+
+def _ma_window(rows):
+    return (0, U64_MAX) if rows is None else (int(rows[0]), int(rows[1]))
+
+
+def build_marker_array(prefix: str, mps: str, ma: str, mab: str | None = None, rows=None, device: int = 0) -> "MaStats":
+    """mps_to_ma on the GPU: <mps> -> <ma> (and, with `mab`, the .mab rb_build -m makes from it), SA taken from the index's
+    phi (<prefix>.rbwt + .tsa, else the raw <prefix>.bwt/.ssa/.esa).  rows = (begin, end): only rows [begin, min(end, n))."""
+    st = MaStats()
+    r0, r1 = _ma_window(rows)
+    _check(lib().rbg_build_marker_array(prefix.encode(), mps.encode(), ma.encode(), mab.encode() if mab else None, r0, r1, device,
+                                        C.byref(st)))
+    return st
+
+
+def build_marker_array_arrays(n, heads, lens, tsa, mps: str, ma: str, mab: str | None = None, rows=None,
+                              device: int = 0) -> "MaStats":
+    """The same over flat arrays: runs (heads, lens) and tsa = (pred, samples_last, pred_to_run) with one sample per run."""
+    keep = [np.ascontiguousarray(heads, np.uint8), np.ascontiguousarray(lens, np.uint64)] + [np.ascontiguousarray(x, np.uint64) for x in tsa]
+    d = _Desc()
+    d.n, d.R, d.r = int(n), len(keep[0]), len(keep[2])
+    d.run_heads, d.run_lens, d.pred, d.samples_last, d.pred_to_run = (x.ctypes.data for x in keep)
+    st = MaStats()
+    r0, r1 = _ma_window(rows)
+    _check(lib().rbg_build_marker_array_arrays(C.byref(d), mps.encode(), ma.encode(), mab.encode() if mab else None, r0, r1, device,
+                                               C.byref(st)))
     return st
 
 

@@ -26,6 +26,7 @@
 #include "sdsl_writer.hpp"
 #include "kernels.cuh"
 #include "layout.hpp"
+#include "ma_build.hpp"
 
 using namespace rbg;
 
@@ -1469,6 +1470,105 @@ int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flag
         st.s_total = wall_s() - t_begin;
         if (stats) *stats = st;
         return (int) RBG_OK;
+    });
+}
+
+namespace {
+// What the two rbg_build_marker_array entries share once the index arrays are in hand: the device check, then the build.
+// `mps` was read and checked against n (check_ma_inputs) before any CUDA call.
+int build_ma_from(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsRecords& mps, uint64_t row_begin, uint64_t row_end,
+                  int device, const char* ma_path, const char* mab_path, rbg_ma_stats& st, double t_begin, rbg_ma_stats* out) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        return fail(RBG_E_CUDA, "no CUDA device: librowbowt_gpu has no CPU fallback");
+    }
+    if (device < 0 || device >= ndev) return fail(RBG_E_ARG, "device ordinal out of range");
+    st.n = bwt.n;
+    st.r = bwt.R;
+    st.mps_records = mps.first.size();
+    st.lists = mps.list_off.size() - 1;
+    try {
+        build_marker_array(bwt, tsa, mps, row_begin, row_end, device, ma_path, mab_path ? mab_path : "", st);
+    } catch (const cuda_error_ma& e) {
+        cudaGetLastError();
+        return fail(RBG_E_CUDA, e.what());
+    }
+    st.s_total = wall_s() - t_begin;
+    if (out) *out = st;
+    return (int) RBG_OK;
+}
+
+// The window [row_begin, min(row_end, n)) must hold a row, the index r == R samples; then the .mps is read against n.
+int check_ma_inputs(uint64_t n, uint64_t R, uint64_t r, uint64_t row_begin, uint64_t& row_end, const char* mps_path, MpsRecords& mps) {
+    if (r != R) return fail(RBG_E_ARG, "the toehold arrays hold " + std::to_string(r) + " samples for " + std::to_string(R) + " runs");
+    row_end = std::min(row_end, n);
+    if (row_begin >= row_end) return fail(RBG_E_ARG, "empty row window");
+    mps = read_mps(mps_path, n);
+    return (int) RBG_OK;
+}
+}  // namespace
+
+int rbg_build_marker_array(const char* index_prefix, const char* mps_path, const char* ma_path, const char* mab_path,
+                           uint64_t row_begin, uint64_t row_end, int device, rbg_ma_stats* stats) {
+    if (!index_prefix || !mps_path || !ma_path) return fail(RBG_E_ARG, "null argument");
+    return guarded([&] {
+        rbg_ma_stats st;
+        memset(&st, 0, sizeof st);
+        const double t_begin = wall_s();
+        const std::string pre(index_prefix);
+        struct stat sb;
+        MpsRecords mps;
+        RawParts p;
+        if (stat((pre + ".rbwt").c_str(), &sb) == 0) {
+            if (stat((pre + ".tsa").c_str(), &sb) != 0) return fail(RBG_E_IO, "no toehold samples: " + pre + ".tsa");
+            p.bwt = read_rbwt(pre + ".rbwt");
+            p.tsa = read_tsa(pre + ".tsa");
+            const int rc = check_ma_inputs(p.bwt.n, p.bwt.R, p.tsa.r, row_begin, row_end, mps_path, mps);
+            if (rc != RBG_OK) return rc;
+        } else {           // the raw inputs: n is the size of the .bwt (one byte per row); decoded on the GPU afterwards
+            struct stat bwt_st;
+            if (stat((pre + ".bwt").c_str(), &bwt_st) != 0) return fail(RBG_E_IO, "no index: neither " + pre + ".rbwt nor " + pre + ".bwt");
+            for (const char* suf : {".ssa", ".esa"})
+                if (stat((pre + suf).c_str(), &sb) != 0) return fail(RBG_E_IO, "no toehold samples: " + pre + suf);
+            const uint64_t n = (uint64_t) bwt_st.st_size;
+            row_end = std::min(row_end, n);
+            if (row_begin >= row_end) return fail(RBG_E_ARG, "empty row window");
+            mps = read_mps(mps_path, n);
+            load_raw(pre, RBG_LOAD_SA, device, p, nullptr);
+        }
+        st.s_read = wall_s() - t_begin;
+        return build_ma_from(p.bwt, p.tsa, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
+    });
+}
+
+int rbg_build_marker_array_arrays(const rbg_index_desc* d, const char* mps_path, const char* ma_path, const char* mab_path,
+                                  uint64_t row_begin, uint64_t row_end, int device, rbg_ma_stats* stats) {
+    if (!d || !mps_path || !ma_path) return fail(RBG_E_ARG, "null argument");
+    return guarded([&] {
+        rbg_ma_stats st;
+        memset(&st, 0, sizeof st);
+        const double t_begin = wall_s();
+        if (!d->run_heads || !d->run_lens) return fail(RBG_E_ARG, "run_heads/run_lens missing");
+        if (!d->r || !d->pred || !d->samples_last || !d->pred_to_run) return fail(RBG_E_ARG, "toehold arrays missing");
+        RunsBwt bwt;
+        bwt.n = d->n;
+        bwt.R = d->R;
+        bwt.heads.assign(d->run_heads, d->run_heads + d->R);
+        bwt.lens.assign(d->run_lens, d->run_lens + d->R);
+        ToeholdArrays tsa;
+        tsa.r = d->r;
+        tsa.n = d->n;
+        tsa.pred.assign(d->pred, d->pred + d->r);
+        tsa.samples_last.assign(d->samples_last, d->samples_last + d->r);
+        tsa.pred_to_run.assign(d->pred_to_run, d->pred_to_run + d->r);
+        MpsRecords mps;
+        const int rc = check_ma_inputs(bwt.n, bwt.R, tsa.r, row_begin, row_end, mps_path, mps);
+        if (rc != RBG_OK) return rc;
+        validate_runs(bwt, "the BWT runs");
+        validate_toehold(tsa, "the toehold arrays");
+        st.s_read = wall_s() - t_begin;
+        return build_ma_from(bwt, tsa, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
     });
 }
 

@@ -5,6 +5,7 @@
 #include <thread>
 #include <cstdio>
 #include <cstring>
+#include <unordered_map>
 #include <fcntl.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
@@ -52,6 +53,8 @@ class FileView {
     uint8_t u8() { return *take(1); }
     int32_t i32() { int32_t v; memcpy(&v, take(4), 4); return v; }
     bool done() const { return pos_ == size_; }
+    size_t left() const { return size_ - pos_; }
+    const uint8_t* at(size_t pos) const { return data_ + pos; }
     const std::string& path() const { return path_; }
 
   private:
@@ -570,6 +573,47 @@ MarkerArrays read_mab(const std::string& path) {
     m.wsize = f.i32();
     if (!f.done()) throw format_error("mab: trailing bytes in " + path);
     validate_markers(m, path);
+    return m;
+}
+
+MpsRecords read_mps(const std::string& path, uint64_t n) {
+    FileView f(path);
+    const uint64_t delim = ~0ull;
+    MpsRecords m;
+    m.list_off.push_back(0);
+    std::unordered_map<std::string, uint32_t> ids;      // word list (raw bytes) -> list id
+    for (uint64_t k = 0; !f.done(); ++k) {
+        const std::string at = ".mps record " + std::to_string(k) + " in " + path;
+        if (f.left() < 16) throw format_error("truncated " + at);
+        const uint64_t first = f.u64(), last = f.u64();
+        const size_t w0 = f.pos();
+        for (;;) {
+            if (f.done()) throw format_error("no delimiter at the end of " + at);
+            if (f.left() < 8) throw format_error("truncated " + at);
+            if (f.u64() == delim) break;
+        }
+        if (first > last) throw format_error("first > last in " + at);
+        if (last >= n) throw format_error("last position beyond the text length " + std::to_string(n) + " in " + at);
+        if (!m.last.empty() && m.last.back() >= first) throw format_error("not after the previous record (ranges must ascend without overlap) in " + at);
+        const size_t bytes = f.pos() - 8 - w0;
+        uint32_t id = kNoList;
+        if (bytes) {
+            std::string key((const char*) f.at(w0), bytes);
+            auto it = ids.find(key);
+            if (it == ids.end()) {
+                if (ids.size() >= (size_t) kNoList) throw format_error("2^32 - 1 or more distinct word lists in " + path);
+                it = ids.emplace(std::move(key), (uint32_t) ids.size()).first;
+                const size_t w = m.words.size();
+                m.words.resize(w + bytes / 8);
+                memcpy(m.words.data() + w, f.at(w0), bytes);
+                m.list_off.push_back(m.words.size());
+            }
+            id = it->second;
+        }
+        m.first.push_back(first);
+        m.last.push_back(last);
+        m.list.push_back(id);
+    }
     return m;
 }
 

@@ -66,4 +66,17 @@ RunsBwt read_rbwt_fbb(const std::string& path);
 ToeholdArrays read_tsa(const std::string& path);
 MarkerArrays read_mab(const std::string& path);
 
+// A .mps (pfbwt-f's MarkerPositionsWriter; SURVEY.md A.1): records `first last word* ~0`, [first, last] an inclusive range
+// of text positions.  Word lists are deduplicated by value into list ids; a record without words has kNoList.
+constexpr uint32_t kNoList = 0xFFFFFFFFu;
+struct MpsRecords {
+    std::vector<uint64_t> first, last;  // [records] ascending, last[k] < first[k + 1]
+    std::vector<uint32_t> list;         // [records] list id or kNoList
+    std::vector<uint64_t> list_off;     // list i is words[list_off[i] .. list_off[i + 1])
+    std::vector<uint64_t> words;
+};
+// Refuses (format_error naming the record) a truncated record or missing delimiter, first > last, records that do not
+// ascend without overlap, last >= n, and 2^32 - 1 or more distinct lists.  No CUDA call.
+MpsRecords read_mps(const std::string& path, uint64_t n);
+
 }  // namespace rbg

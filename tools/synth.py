@@ -211,6 +211,61 @@ def write_raw_index(panel: Panel, prefix: str, markers: bool = True, wsize: int 
     np.array(out, np.uint64).tofile(prefix + ".ma")
 
 
+def _marker_words(panel: Panel):
+    """Text positions of every marker (reference included, text order) and their MarkerT words."""
+    pos = np.concatenate([panel.sites + panel.seq_start(h) for h in range(panel.nseq)])
+    alleles = np.concatenate([np.zeros(len(panel.sites), np.uint64)] + [g.astype(np.uint64) for g in panel.gt])
+    return pos, (alleles << np.uint64(60)) | np.tile(panel.sites.astype(np.uint64), panel.nseq)
+
+
+def write_mps(panel: Panel, path: str, wsize: int = 10) -> None:
+    """The panel's .mps without the reference: `first last word* ~0` for every maximal run of text positions p with the same
+    non-empty list of markers in [p, p + wsize).  The list only changes where a marker at q enters (p = q - wsize + 1) or
+    leaves (p = q + 1), so the records come from those breakpoints, never from the n positions."""
+    n = panel.nseq * (panel.L + PAD) + 1
+    pos, words = _marker_words(panel)
+    cuts = np.unique(np.clip(np.concatenate([[0], pos - wsize + 1, pos + 1]), 0, n - 1))    # segment i: [cuts[i], cuts[i + 1])
+    a, b = np.searchsorted(pos, cuts), np.searchsorted(pos, cuts + wsize)
+    keep = b > a
+    same = np.zeros(len(cuts) + 1, bool)                     # segment i continues the record of segment i - 1
+    same[1:-1] = keep[1:] & keep[:-1] & (a[1:] == a[:-1]) & (b[1:] == b[:-1])
+    first, last = np.nonzero(keep & ~same[:-1])[0], np.nonzero(keep & ~same[1:])[0]
+    seg_end = np.append(cuts[1:], n) - 1
+    out = []
+    for f, l in zip(first.tolist(), last.tolist()):
+        out += [int(cuts[f]), int(seg_end[l])] + words[a[f]:b[f]].tolist() + [0xFFFFFFFFFFFFFFFF]
+    np.array(out, np.uint64).tofile(path)
+
+
+def ma_from_mps(sa_rows: np.ndarray, row0: int, mps_words: np.ndarray) -> np.ndarray:
+    """The .ma of rows [row0, row0 + len(sa_rows)) with SA values sa_rows, from the words of a .mps: row i gets the list of the
+    record whose [first, last] holds SA[i] (none without one); a .ma record is a maximal run of consecutive rows whose lists
+    are non-empty and equal by value, words in the .mps record's order."""
+    w = np.asarray(mps_words, np.uint64)
+    ends = np.nonzero(w == np.uint64(0xFFFFFFFFFFFFFFFF))[0]
+    starts = np.concatenate([[0], ends[:-1] + 1]).astype(np.int64)
+    firsts, lasts = w[starts], w[starts + 1]
+    lists, lid = {}, np.empty(len(starts), np.int64)
+    for k, (s, e) in enumerate(zip(starts.tolist(), ends.tolist())):
+        ws = tuple(w[s + 2:e].tolist())
+        lid[k] = lists.setdefault(ws, len(lists)) if ws else -1
+    by_id = {v: list(k) for k, v in lists.items()}
+    sa = np.asarray(sa_rows, np.uint64)
+    ids = np.full(len(sa), -1, np.int64)
+    if len(firsts):
+        k = np.searchsorted(firsts, sa, side="right") - 1
+        hit = (k >= 0) & (sa <= lasts[np.clip(k, 0, None)])
+        ids[hit] = lid[k[hit]]
+    change = np.nonzero(np.diff(ids) != 0)[0] + 1
+    b0 = np.concatenate([[0], change])
+    b1 = np.append(change, len(ids)) - 1
+    out = []
+    for f, l in zip(b0.tolist(), b1.tolist()):
+        if ids[f] >= 0:
+            out += [row0 + f, row0 + l] + by_id[int(ids[f])] + [0xFFFFFFFFFFFFFFFF]
+    return np.array(out, np.uint64)
+
+
 def build_index_gpu(panel: Panel, prefix: str, markers: bool = True, device: int = 0, log=sys.stderr) -> dict:
     """The same index files as build_index, without the reference: write_raw_index, then the project's own
     rb_build on the GPU (rowbowt_b200.build_index).  Returns timings."""
