@@ -20,6 +20,7 @@
 #include <string>
 #include <vector>
 
+#include "cuda_host.hpp"
 #include "formats.hpp"
 #include "host_pack.hpp"
 #include "raw_build.hpp"
@@ -39,87 +40,50 @@ int fail(int code, const std::string& msg) {
     return code;
 }
 
-struct cuda_error : std::runtime_error { using std::runtime_error::runtime_error; };
-
-#define CU(call)                                                                                   \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess)                                                                     \
-            throw cuda_error(std::string(#call) + ": " + cudaGetErrorString(e_));                  \
-    } while (0)
-
-// growable device buffer
-struct DBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    void reserve(size_t bytes) {
-        if (bytes <= cap) return;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        CU(cudaMalloc(&p, want));
-        cap = want;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    template <class T> T* as() const { return (T*) p; }
-};
-
-// growable pinned host buffer
-struct HBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    void reserve(size_t bytes) {
-        if (bytes <= cap) return;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        CU(cudaHostAlloc(&p, want, cudaHostAllocDefault));
-        cap = want;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
-thread_local std::vector<size_t>* g_upload_sizes = nullptr;      // set by open_from_arrays: payload bytes of every upload, for the layout cache
-
-template <class T>
-T* upload(const std::vector<T>& v, std::vector<void*>& owned, size_t* bytes_acc) {
-    void* p = nullptr;
-    size_t bytes = std::max<size_t>(v.size() * sizeof(T), 64);
-    CU(cudaMalloc(&p, bytes));
-    owned.push_back(p);
-    if (g_upload_sizes) g_upload_sizes->push_back(v.size() * sizeof(T));
-    if (!v.empty()) CU(cudaMemcpy(p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    if (bytes_acc) *bytes_acc += bytes;
-    return (T*) p;
-}
+// Reserves with headroom: the next slightly larger batch reuses the buffer.
+template <class B>
+void reserve(B& b, size_t bytes) { b.reserve(bytes, bytes + bytes / 8 + 256); }
 
 struct HostSeedResult {  // pinned buffers behind one rbg_seed_result
-    HBuf seed_off, seeds, markers;
+    PinnedBuf seed_off, seeds, markers;
     rbg_index* ix = nullptr;
-    void release() { seed_off.release(); seeds.release(); markers.release(); }
 };
 
 struct GreedyScratch {   // device buffers of rbg_markers_greedy
-    DBuf bad, item_seeds, item_words, seed_off, word_off, seeds, words;
-    void release() { for (DBuf* b : {&bad, &item_seeds, &item_words, &seed_off, &word_off, &seeds, &words}) b->release(); }
+    DevBuf bad, item_seeds, item_words, seed_off, word_off, seeds, words;
 };
 
 static_assert(sizeof(DevSeed) == sizeof(rbg_seed) && sizeof(rbg_seed) == 40, "rbg_seed layout");
 
 struct HostResult {      // pinned buffers behind one rbg_result
-    HBuf lo, hi, toehold, loc_off, locs, locs_hi, mk_off, markers;      // lo / hi hold u32 planes with RBG_NARROW_RANGES
+    PinnedBuf lo, hi, toehold, loc_off, locs, locs_hi, mk_off, markers;      // lo / hi hold u32 planes with RBG_NARROW_RANGES
     rbg_index* ix = nullptr;
-    void release() { lo.release(); hi.release(); toehold.release(); loc_off.release(); locs.release(); locs_hi.release(); mk_off.release(); markers.release(); }
+};
+
+// Results handed to callers through `_owner`; up to 4 given back are kept for the next call.
+template <class H>
+class ResultPool {
+    std::mutex mu;
+    std::vector<std::unique_ptr<H>> kept;
+  public:
+    H* take(rbg_index* ix) {
+        {
+            std::lock_guard<std::mutex> lock(mu);
+            if (!kept.empty()) {
+                H* h = kept.back().release();
+                kept.pop_back();
+                return h;
+            }
+        }
+        H* h = new H;
+        h->ix = ix;
+        return h;
+    }
+    void give_back(H* h) {
+        std::lock_guard<std::mutex> lock(mu);
+        if (kept.size() < 4) kept.emplace_back(h);
+        else delete h;
+    }
 };
 
 }  // namespace
@@ -129,17 +93,12 @@ struct rbg_reads {
     uint64_t n_reads = 0, n_bytes = 0;
     bool prepacked = false;              // `packed` / `flags` came from the host (rbg_reads_upload_packed): no pack_kernel
     bool has_bases = false;
-    DBuf bases, offs, packed, flags;
-    DBuf lo, hi, toehold, loc_cnt, loc_off, locs, locs_hi, mk_cnt, mk_off, mk_first, markers, scan_tmp;
-    DBuf lo32, hi32;                     // RBG_NARROW_RANGES: what leaves the device instead of lo / hi
+    DevBuf bases, offs, packed, flags;
+    DevBuf lo, hi, toehold, loc_cnt, loc_off, locs, locs_hi, mk_cnt, mk_off, mk_first, markers, scan_tmp;
+    DevBuf lo32, hi32;                   // RBG_NARROW_RANGES: what leaves the device instead of lo / hi
     uint64_t n_locs = 0, n_markers = 0;
     uint32_t last_mode = 0;
     bool ran = false;
-    void release() {
-        for (DBuf* b : {&bases, &offs, &packed, &flags, &lo, &hi, &toehold, &loc_cnt, &loc_off, &locs, &locs_hi, &mk_cnt, &mk_off,
-                        &mk_first, &markers, &scan_tmp, &lo32, &hi32})
-            b->release();
-    }
 };
 
 namespace {
@@ -195,8 +154,6 @@ struct Lane {
         CU(cudaHostAlloc(&h_ctr, sizeof(DevCounters), cudaHostAllocDefault));
     }
     ~Lane() {
-        scratch.release();
-        greedy.release();
         if (d_ctr) cudaFree(d_ctr);
         if (h_ctr) cudaFreeHost(h_ctr);
         for (auto& e : ev) if (e) cudaEventDestroy(e);
@@ -220,8 +177,7 @@ struct Lane {
 
 struct rbg_index {
     int device = 0;
-    std::vector<void*> owned;
-    std::vector<size_t> owned_bytes;     // payload bytes of owned[i] (layout cache)
+    std::vector<Upload> owned;
     DevLeafDir dir{};
     DevToehold toe{};
     DevPhi phi{};
@@ -233,14 +189,14 @@ struct rbg_index {
     size_t hot_bytes = 0;
     rbg_info info{};
     rbg_stats stats{};                   // of the call that finished last
-    std::mutex mu;                       // lanes, result pools, stats
+    std::mutex mu;                       // lanes, stats
     std::condition_variable cv;
     std::vector<std::unique_ptr<Lane>> lanes;
     int max_lanes = 2;
     int n_busy = 0;
     bool exclusive = false;              // an ftab rebuild owns the handle
-    std::vector<HostResult*> free_results;
-    std::vector<HostSeedResult*> free_seed_results;
+    ResultPool<HostResult> results;
+    ResultPool<HostSeedResult> seed_results;
     // One free lane (creating it on first use); with `all`, waits until no call is in flight and keeps others out.
     Lane* acquire(bool all = false) {
         std::unique_lock<std::mutex> lock(mu);
@@ -275,12 +231,23 @@ struct rbg_index {
     ~rbg_index() {
         cudaSetDevice(device);
         lanes.clear();
-        for (auto* h : free_results) { h->release(); delete h; }
-        for (auto* h : free_seed_results) { h->release(); delete h; }
-        for (void* p : owned) cudaFree(p);
         if (hot) cudaFree(hot);
     }
 };
+
+namespace rbg {
+DevPhi upload_phi(const PhiDir& pd, uint64_t n, std::vector<Upload>& owned, size_t* acc) {
+    DevPhi P{};
+    P.l1 = upload(pd.l1, owned, acc);
+    P.slots = upload(pd.slots, owned, acc);
+    P.ovf_keys = upload(pd.ovf_keys, owned, acc);
+    P.ovf_prev_lo = upload(pd.ovf_prev.lo, owned, acc);
+    P.ovf_prev_hi = pd.ovf_prev.wide ? upload(pd.ovf_prev.hi, owned, acc) : nullptr;
+    P.n = n;
+    P.shift = pd.shift;
+    return P;
+}
+}  // namespace rbg
 
 namespace {
 
@@ -468,12 +435,12 @@ void cache_fields(rbg_index* ix, const void*** f) {
 // After open_from_arrays: dir.super already points into the hot region; its blob is the second upload (owned[1]).
 void write_layout_cache(rbg_index* ix, const std::string& pre, uint32_t flags) {
     CacheHeader h = cache_stamp(pre, flags);
-    if (ix->owned.size() != ix->owned_bytes.size() || ix->owned.size() < 2) return;
+    if (ix->owned.size() < 2) return;
     const void** f[15];
     cache_fields(ix, f);
     for (int i = 0; i < 15; ++i) {
         h.field_blob[i] = -1;
-        for (size_t b = 0; b < ix->owned.size(); ++b) if (*f[i] == ix->owned[b]) h.field_blob[i] = (int32_t) b;
+        for (size_t b = 0; b < ix->owned.size(); ++b) if (*f[i] == ix->owned[b].mem.p) h.field_blob[i] = (int32_t) b;
     }
     h.field_blob[1] = 1;                                       // dir.super: the blob behind the hot region's copy
     h.n_blobs = (uint32_t) ix->owned.size();
@@ -490,11 +457,11 @@ void write_layout_cache(rbg_index* ix, const std::string& pre, uint32_t flags) {
     try {
         std::vector<char> buf;
         for (size_t b = 0; ok && b < ix->owned.size(); ++b) {
-            const uint64_t bytes = ix->owned_bytes[b];
+            const uint64_t bytes = ix->owned[b].bytes;
             ok = fwrite(&bytes, 8, 1, fp) == 1;
             if (!bytes) continue;
             buf.resize(bytes);
-            CU(cudaMemcpy(buf.data(), ix->owned[b], bytes, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(buf.data(), ix->owned[b].mem.p, bytes, cudaMemcpyDeviceToHost));
             ok = ok && fwrite(buf.data(), 1, bytes, fp) == bytes;
         }
     } catch (...) {
@@ -507,8 +474,17 @@ void write_layout_cache(rbg_index* ix, const std::string& pre, uint32_t flags) {
     if (!ok) remove(tmp.c_str());
 }
 
+// A handle on `device` (after the device checks) that answers queries with RBG_LANES lanes at most.
+std::unique_ptr<rbg_index> new_index(int device) {
+    select_device(device);
+    std::unique_ptr<rbg_index> ix(new rbg_index);
+    ix->device = device;
+    if (const char* e = getenv("RBG_LANES")) ix->max_lanes = std::max(1, std::min(8, atoi(e)));
+    return ix;
+}
+
 // nullptr when there is no valid cache for (prefix, flags)
-rbg_index* open_layout_cache(const std::string& pre, uint32_t flags, int device) {
+std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t flags, int device) {
     const std::string path = pre + ".rbgcache";
     const int fd = open(path.c_str(), O_RDONLY);
     if (fd < 0) return nullptr;
@@ -528,13 +504,7 @@ rbg_index* open_layout_cache(const std::string& pre, uint32_t flags, int device)
     size_t at = sizeof h;
     const size_t pods = sizeof(DevLeafDir) + sizeof(DevToehold) + sizeof(DevPhi) + sizeof(DevMarkers) + sizeof(CodeTable) + sizeof(rbg_info);
     if (at + pods > size || h.n_blobs < 2 || h.n_blobs > 64) return nullptr;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) throw cuda_error("no CUDA device: librowbowt_gpu has no CPU fallback");
-    if (device < 0 || device >= ndev) throw std::invalid_argument("device ordinal out of range");
-    CU(cudaSetDevice(device));
-    std::unique_ptr<rbg_index> ix(new rbg_index);
-    ix->device = device;
-    if (const char* e = getenv("RBG_LANES")) ix->max_lanes = std::max(1, std::min(8, atoi(e)));
+    std::unique_ptr<rbg_index> ix = new_index(device);
     memcpy(&ix->dir, m + at, sizeof ix->dir); at += sizeof ix->dir;
     memcpy(&ix->toe, m + at, sizeof ix->toe); at += sizeof ix->toe;
     memcpy(&ix->phi, m + at, sizeof ix->phi); at += sizeof ix->phi;
@@ -547,39 +517,25 @@ rbg_index* open_layout_cache(const std::string& pre, uint32_t flags, int device)
         memcpy(&bytes, m + at, 8);
         at += 8;
         if (bytes > size - at) return nullptr;                 // truncated file
-        void* p = nullptr;
-        CU(cudaMalloc(&p, std::max<size_t>(bytes, 64)));
-        ix->owned.push_back(p);
-        ix->owned_bytes.push_back(bytes);
-        if (bytes) CU(cudaMemcpy(p, m + at, bytes, cudaMemcpyHostToDevice));
+        ix->owned.push_back(Upload{DevBuf(std::max<size_t>(bytes, 64)), bytes});
+        if (bytes) CU(cudaMemcpy(ix->owned.back().mem.p, m + at, bytes, cudaMemcpyHostToDevice));
         at += bytes;
     }
     const void** f[15];
     cache_fields(ix.get(), f);
     for (int i = 0; i < 15; ++i) {
         if (h.field_blob[i] >= (int32_t) h.n_blobs) return nullptr;
-        *f[i] = h.field_blob[i] < 0 ? nullptr : ix->owned[h.field_blob[i]];
+        *f[i] = h.field_blob[i] < 0 ? nullptr : ix->owned[h.field_blob[i]].mem.p;
     }
     ix->hot = nullptr;
     CU(cudaDeviceSynchronize());
     rebuild_hot_region(ix.get(), 0, false);                    // superblock counts into the hot region, no seed table yet
     ix->info.from_cache = 1;
-    return ix.release();
+    return ix;
 }
 
-int open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerArrays* ma, int device, rbg_index** out) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0)
-        return fail(RBG_E_CUDA, "no CUDA device: librowbowt_gpu has no CPU fallback");
-    if (device < 0 || device >= ndev) return fail(RBG_E_ARG, "device ordinal out of range");
-    CU(cudaSetDevice(device));
-    std::unique_ptr<rbg_index> ix(new rbg_index);
-    ix->device = device;
-    if (const char* e = getenv("RBG_LANES")) ix->max_lanes = std::max(1, std::min(8, atoi(e)));
-    struct SizeRecorder {
-        explicit SizeRecorder(std::vector<size_t>* v) { g_upload_sizes = v; }
-        ~SizeRecorder() { g_upload_sizes = nullptr; }
-    } recorder(&ix->owned_bytes);
+std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerArrays* ma, int device) {
+    std::unique_ptr<rbg_index> ix = new_index(device);
 
     // caller-supplied arrays (rbg_index_open_arrays) and raw builds come here without passing a file reader
     validate_runs(bwt, "the BWT runs");
@@ -593,9 +549,7 @@ int open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerA
     // the phi directory depends on the toehold arrays only: built on another host thread while this one lays out the BWT
     std::future<PhiDir> phi_job;
     if (tsa) {
-        size_t free_b = 0, total_b = 0;
-        CU(cudaMemGetInfo(&free_b, &total_b));
-        const uint64_t budget = (uint64_t) free_b / 4;          // slots may take a quarter of the free memory
+        const uint64_t budget = phi_slot_budget();
         phi_job = std::async(std::launch::async, [tsa, budget] { return build_phi_dir(*tsa, 0, budget); });
     }
     {
@@ -635,13 +589,7 @@ int open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerA
         info.toehold0 = td.toehold0;
         PhiDir pd = phi_job.get();
         acc = 0;
-        ix->phi.l1 = upload(pd.l1, ix->owned, &acc);
-        ix->phi.slots = upload(pd.slots, ix->owned, &acc);
-        ix->phi.ovf_keys = upload(pd.ovf_keys, ix->owned, &acc);
-        ix->phi.ovf_prev_lo = upload(pd.ovf_prev.lo, ix->owned, &acc);
-        ix->phi.ovf_prev_hi = pd.ovf_prev.wide ? upload(pd.ovf_prev.hi, ix->owned, &acc) : nullptr;
-        ix->phi.n = tsa->n;
-        ix->phi.shift = pd.shift;
+        ix->phi = upload_phi(pd, tsa->n, ix->owned, &acc);
         info.phi_shift = pd.shift;
         info.phi_overflow = pd.n_overflow;
         info.phi_bytes = acc;
@@ -665,8 +613,7 @@ int open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerA
     }
     CU(cudaDeviceSynchronize());
     rebuild_hot_region(ix.get(), 0, false);
-    *out = ix.release();
-    return RBG_OK;
+    return ix;
 }
 
 template <class Fn>
@@ -724,10 +671,10 @@ void reserve_input(rbg_reads* rd, rbg_index* ix, uint64_t n, uint64_t n_bytes, b
     rd->ran = false;
     rd->prepacked = false;
     rd->has_bases = with_bases;
-    if (with_bases) rd->bases.reserve(n_bytes + 64);
-    rd->offs.reserve((n + 1) * 8);
-    rd->packed.reserve(((n_bytes + 31) / 32 + 1) * 8);
-    rd->flags.reserve(n + 8);
+    if (with_bases) reserve(rd->bases, n_bytes + 64);
+    reserve(rd->offs, (n + 1) * 8);
+    reserve(rd->packed, ((n_bytes + 31) / 32 + 1) * 8);
+    reserve(rd->flags, n + 8);
 }
 
 // Raw bytes of the reads flagged RBG_READ_EXOTIC among [r0, r1) of a packed batch (normally none).
@@ -738,6 +685,15 @@ void copy_exotic_bases(const BatchIn& in, rbg_reads* rd, uint64_t r0, uint64_t r
             const uint64_t a = in.offsets[i], z = in.offsets[i + 1];
             if (z > a) CU(cudaMemcpyAsync(rd->bases.as<uint8_t>() + a, in.bases + a, z - a, cudaMemcpyHostToDevice, st));
         }
+}
+
+// The batch's offsets re-based so that offs[0] == 0: the caller's own array when they already are, else a copy in `tmp`.
+const uint64_t* rebased_offsets(const BatchIn& in, std::vector<uint64_t>& tmp) {
+    const uint64_t base = in.n ? in.offsets[0] : 0;
+    if (base == 0) return in.offsets;
+    tmp.resize(in.n + 1);
+    for (uint64_t i = 0; i <= in.n; ++i) tmp[i] = in.offsets[i] - base;
+    return tmp.data();
 }
 
 // H2D of one whole batch into `rd` (raw: bases re-based so that offs[0] == 0; packed: words + flags as given).
@@ -756,14 +712,9 @@ void stage_batch(rbg_index* ix, cudaStream_t st, const BatchIn& in, rbg_reads* r
         return;
     }
     if (n_bytes) CU(cudaMemcpyAsync(rd->bases.p, in.bases + base, n_bytes, cudaMemcpyHostToDevice, st));
-    if (base == 0) {
-        CU(cudaMemcpyAsync(rd->offs.p, in.offsets, (n + 1) * 8, cudaMemcpyHostToDevice, st));
-    } else {
-        std::vector<uint64_t> tmp(n + 1);
-        for (uint64_t i = 0; i <= n; ++i) tmp[i] = in.offsets[i] - base;
-        CU(cudaMemcpyAsync(rd->offs.p, tmp.data(), (n + 1) * 8, cudaMemcpyHostToDevice, st));
-        CU(cudaStreamSynchronize(st));
-    }
+    std::vector<uint64_t> tmp;
+    CU(cudaMemcpyAsync(rd->offs.p, rebased_offsets(in, tmp), (n + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (!tmp.empty()) CU(cudaStreamSynchronize(st));      // the copy reads `tmp`
 }
 
 float ev_ms(cudaEvent_t a, cudaEvent_t b) {
@@ -780,19 +731,19 @@ Views prepare(rbg_index* ix, rbg_reads* rd, uint32_t mode) {
     if (locate && !ix->info.has_sa) throw std::invalid_argument("RBG_LOCATE needs an index opened with RBG_LOAD_SA");
     if (markers && !ix->info.has_ma) throw std::invalid_argument("RBG_MARKERS needs an index opened with RBG_LOAD_MA");
     const uint64_t n = rd->n_reads;
-    rd->lo.reserve((n + 1) * 8);
-    rd->hi.reserve((n + 1) * 8);
+    reserve(rd->lo, (n + 1) * 8);
+    reserve(rd->hi, (n + 1) * 8);
     if (locate) {
-        rd->toehold.reserve((n + 1) * 8);
-        rd->loc_cnt.reserve((n + 2) * 8);
-        rd->loc_off.reserve((n + 2) * 8);
+        reserve(rd->toehold, (n + 1) * 8);
+        reserve(rd->loc_cnt, (n + 2) * 8);
+        reserve(rd->loc_off, (n + 2) * 8);
     }
     if (markers) {
-        rd->mk_cnt.reserve((n + 2) * 8);
-        rd->mk_off.reserve((n + 2) * 8);
-        rd->mk_first.reserve((n + 1) * 8);
+        reserve(rd->mk_cnt, (n + 2) * 8);
+        reserve(rd->mk_off, (n + 2) * 8);
+        reserve(rd->mk_first, (n + 1) * 8);
     }
-    if (locate || markers) rd->scan_tmp.reserve(std::max(scan_tmp_bytes(n + 1), scan_from_tmp_bytes(n + 1)));
+    if (locate || markers) reserve(rd->scan_tmp, std::max(scan_tmp_bytes(n + 1), scan_from_tmp_bytes(n + 1)));
     Views v{};
     v.b = DevBatch{rd->bases.as<uint8_t>(), rd->offs.as<uint64_t>(), n, rd->n_bytes, 0, n, rd->packed.as<uint64_t>(), rd->flags.as<uint8_t>()};
     v.r.lo = rd->lo.as<uint64_t>();
@@ -807,11 +758,25 @@ Views prepare(rbg_index* ix, rbg_reads* rd, uint32_t mode) {
     return v;
 }
 
-// Location planes of `rd` into the kernel view: u64 each, or (narrow) a u32 plane + a u8 plane when n > 2^32.
-void point_locs(const rbg_index* ix, rbg_reads* rd, DevResult& r, bool narrow) {
-    r.locs = narrow ? nullptr : rd->locs.as<uint64_t>();
-    r.locs_lo = narrow ? rd->locs.as<uint32_t>() : nullptr;
-    r.locs_hi = narrow && (ix->info.n >> 32) ? rd->locs_hi.as<uint8_t>() : nullptr;
+// How locations leave the device: u64 each, or with RBG_NARROW_LOCS a u32 plane plus, when n > 2^32, a u8 plane.
+struct LocForm {
+    bool narrow, hi_plane;
+    LocForm(uint32_t mode, uint64_t n) : narrow((mode & RBG_LOCATE) && (mode & RBG_NARROW_LOCS)), hi_plane(narrow && (n >> 32)) {}
+    size_t item() const { return narrow ? 4 : 8; }
+};
+
+// Location planes of `rd` into the kernel view.
+void point_locs(const rbg_reads* rd, DevResult& r, LocForm f) {
+    r.locs = f.narrow ? nullptr : rd->locs.as<uint64_t>();
+    r.locs_lo = f.narrow ? rd->locs.as<uint32_t>() : nullptr;
+    r.locs_hi = f.hi_plane ? rd->locs_hi.as<uint8_t>() : nullptr;
+}
+
+// Location planes of `h` into the caller's result.
+void point_locs(const HostResult* h, rbg_result* out, LocForm f) {
+    out->locs = f.narrow ? nullptr : h->locs.as<uint64_t>();
+    out->locs_lo32 = f.narrow ? h->locs.as<uint32_t>() : nullptr;
+    out->locs_hi8 = f.hi_plane ? h->locs_hi.as<uint8_t>() : nullptr;
 }
 
 // Occurrence / marker-word counts of every read -> offsets; returns the total (one host sync).
@@ -836,7 +801,8 @@ void collect_counters(Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t launches) {
 // All kernels of one query over a staged batch, one launch per stage (the kernel-only measurement
 // path).  Leaves results on the device.
 void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mode, uint64_t max_hits, bool want_checksum) {
-    const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS, narrow = locate && (mode & RBG_NARROW_LOCS);
+    const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS;
+    const LocForm lf(mode, ix->info.n);
     Views v = prepare(ix, rd, mode);
     DevBatch& b = v.b;
     DevResult& r = v.r;
@@ -858,9 +824,9 @@ void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mo
         launches += launch_locate_counts(r, 0, n, max_hits, st);
         rd->n_locs = scan_counts(L, rd, r.loc_cnt, r.loc_off, n, st);
         launches += 1;
-        rd->locs.reserve((rd->n_locs + 1) * (narrow ? 4 : 8));
-        if (narrow && (ix->info.n >> 32)) rd->locs_hi.reserve(rd->n_locs + 8);
-        point_locs(ix, rd, r, narrow);
+        reserve(rd->locs, (rd->n_locs + 1) * lf.item());
+        if (lf.hi_plane) reserve(rd->locs_hi, rd->n_locs + 8);
+        point_locs(rd, r, lf);
         CU(cudaEventRecord(L.ev[6], st));
         launches += launch_locate(ix->phi, r, 0, n, rd->n_locs, L.d_ctr, &L.d_ctr->loc_cursor[0], st);
     }
@@ -869,7 +835,7 @@ void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mo
         launches += launch_marker_counts(ix->mk, r, 0, n, st);
         rd->n_markers = scan_counts(L, rd, r.mk_cnt, r.mk_off, n, st);
         launches += 1;
-        rd->markers.reserve((rd->n_markers + 1) * 8);
+        reserve(rd->markers, (rd->n_markers + 1) * 8);
         r.markers = rd->markers.as<uint64_t>();
         launches += launch_marker_gather(ix->mk, r, 0, n, L.d_ctr, st);
     }
@@ -892,63 +858,39 @@ void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mo
     rd->ran = true;
 }
 
-HostResult* take_host_result(rbg_index* ix) {
-    {
-        std::lock_guard<std::mutex> lock(ix->mu);
-        if (!ix->free_results.empty()) {
-            HostResult* h = ix->free_results.back();
-            ix->free_results.pop_back();
-            return h;
-        }
-    }
-    HostResult* h = new HostResult;
-    h->ix = ix;
-    return h;
-}
-
-void give_back_host_result(rbg_index* ix, HostResult* h) {
-    std::lock_guard<std::mutex> lock(ix->mu);
-    if (ix->free_results.size() < 4) ix->free_results.push_back(h);
-    else { h->release(); delete h; }
-}
-
 // D2H of a staged run's results into pinned buffers.
 void fetch_staged(rbg_index* ix, Lane& L, rbg_reads* rd, uint32_t mode, rbg_result* out) {
     if (!rd->ran) throw std::invalid_argument("no staged run to fetch");
-    const bool narrow = (rd->last_mode & RBG_LOCATE) && (rd->last_mode & RBG_NARROW_LOCS);
+    const LocForm lf(rd->last_mode, ix->info.n);
     mode = rd->last_mode & mode;
     const uint64_t n = rd->n_reads;
     cudaStream_t st = L.stream;
-    HostResult* h = take_host_result(ix);
+    HostResult* h = ix->results.take(ix);
     memset(out, 0, sizeof *out);
     out->_owner = h;
     out->n_reads = n;
-    h->lo.reserve((n + 1) * 8);
-    h->hi.reserve((n + 1) * 8);
+    reserve(h->lo, (n + 1) * 8);
+    reserve(h->hi, (n + 1) * 8);
     CU(cudaMemcpyAsync(h->lo.p, rd->lo.p, n * 8, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(h->hi.p, rd->hi.p, n * 8, cudaMemcpyDeviceToHost, st));
     out->lo = (uint64_t*) h->lo.p;
     out->hi = (uint64_t*) h->hi.p;
     if (mode & RBG_LOCATE) {
-        const size_t item = narrow ? 4 : 8;
-        const bool hi_plane = narrow && (ix->info.n >> 32);
-        h->toehold.reserve((n + 1) * 8);
-        h->loc_off.reserve((n + 2) * 8);
-        h->locs.reserve((rd->n_locs + 1) * item);
-        if (hi_plane) h->locs_hi.reserve(rd->n_locs + 8);
+        reserve(h->toehold, (n + 1) * 8);
+        reserve(h->loc_off, (n + 2) * 8);
+        reserve(h->locs, (rd->n_locs + 1) * lf.item());
+        if (lf.hi_plane) reserve(h->locs_hi, rd->n_locs + 8);
         CU(cudaMemcpyAsync(h->toehold.p, rd->toehold.p, n * 8, cudaMemcpyDeviceToHost, st));
         CU(cudaMemcpyAsync(h->loc_off.p, rd->loc_off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, st));
-        if (rd->n_locs) CU(cudaMemcpyAsync(h->locs.p, rd->locs.p, rd->n_locs * item, cudaMemcpyDeviceToHost, st));
-        if (hi_plane && rd->n_locs) CU(cudaMemcpyAsync(h->locs_hi.p, rd->locs_hi.p, rd->n_locs, cudaMemcpyDeviceToHost, st));
+        if (rd->n_locs) CU(cudaMemcpyAsync(h->locs.p, rd->locs.p, rd->n_locs * lf.item(), cudaMemcpyDeviceToHost, st));
+        if (lf.hi_plane && rd->n_locs) CU(cudaMemcpyAsync(h->locs_hi.p, rd->locs_hi.p, rd->n_locs, cudaMemcpyDeviceToHost, st));
         out->toehold = (uint64_t*) h->toehold.p;
         out->loc_off = (uint64_t*) h->loc_off.p;
-        out->locs = narrow ? nullptr : (uint64_t*) h->locs.p;
-        out->locs_lo32 = narrow ? (uint32_t*) h->locs.p : nullptr;
-        out->locs_hi8 = hi_plane ? (uint8_t*) h->locs_hi.p : nullptr;
+        point_locs(h, out, lf);
     }
     if (mode & RBG_MARKERS) {
-        h->mk_off.reserve((n + 2) * 8);
-        h->markers.reserve((rd->n_markers + 1) * 8);
+        reserve(h->mk_off, (n + 2) * 8);
+        reserve(h->markers, (rd->n_markers + 1) * 8);
         CU(cudaMemcpyAsync(h->mk_off.p, rd->mk_off.p, (n + 1) * 8, cudaMemcpyDeviceToHost, st));
         if (rd->n_markers) CU(cudaMemcpyAsync(h->markers.p, rd->markers.p, rd->n_markers * 8, cudaMemcpyDeviceToHost, st));
         out->mk_off = (uint64_t*) h->mk_off.p;
@@ -963,9 +905,9 @@ void fetch_staged(rbg_index* ix, Lane& L, rbg_reads* rd, uint32_t mode, rbg_resu
 // skips pack_kernel: its words and flags are copied as they are.
 // Locate / marker output sizes are data dependent: see the comments at the locate and marker stages below.
 void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint32_t mode, uint64_t max_hits, rbg_result* out) {
-    const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS, narrow = locate && (mode & RBG_NARROW_LOCS);
-    const bool hi_plane = narrow && (ix->info.n >> 32);
-    const size_t loc_item = narrow ? 4 : 8;
+    const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS;
+    const LocForm lf(mode, ix->info.n);
+    const size_t loc_item = lf.item();
     const bool narrow_rg = (mode & RBG_NARROW_RANGES) && !(ix->info.n >> 32);       // u32 planes of lo / hi on the wire
     rbg_reads* rd = &L.scratch;
     const uint64_t n = in.n;
@@ -979,29 +921,29 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
     DevResult r = v.r;
     cudaStream_t sc = L.stream, si = L.s_in, so = L.s_out;
 
-    HostResult* h = take_host_result(ix);
+    HostResult* h = ix->results.take(ix);
     memset(out, 0, sizeof *out);
     out->_owner = h;
     out->n_reads = n;
-    h->lo.reserve((n + 1) * 8);
-    h->hi.reserve((n + 1) * 8);
+    reserve(h->lo, (n + 1) * 8);
+    reserve(h->hi, (n + 1) * 8);
     if (narrow_rg) {
         out->lo32 = (uint32_t*) h->lo.p;
         out->hi32 = (uint32_t*) h->hi.p;
-        rd->lo32.reserve((n + 1) * 4);
-        rd->hi32.reserve((n + 1) * 4);
+        reserve(rd->lo32, (n + 1) * 4);
+        reserve(rd->hi32, (n + 1) * 4);
     } else {
         out->lo = (uint64_t*) h->lo.p;
         out->hi = (uint64_t*) h->hi.p;
     }
     if (locate) {
-        h->toehold.reserve((n + 1) * 8);
-        h->loc_off.reserve((n + 2) * 8);
+        reserve(h->toehold, (n + 1) * 8);
+        reserve(h->loc_off, (n + 2) * 8);
         out->toehold = (uint64_t*) h->toehold.p;
         out->loc_off = (uint64_t*) h->loc_off.p;
     }
     if (markers) {
-        h->mk_off.reserve((n + 2) * 8);
+        reserve(h->mk_off, (n + 2) * 8);
         out->mk_off = (uint64_t*) h->mk_off.p;
     }
 
@@ -1022,12 +964,7 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
     CU(cudaEventRecord(L.ev_span[0], si));
     // offsets first (pack's flagging searches them), re-based to 0 when the caller's are not
     std::vector<uint64_t> rebased;
-    const uint64_t* offs_h = in.offsets;
-    if (base != 0) {
-        rebased.resize(n + 1);
-        for (uint64_t i = 0; i <= n; ++i) rebased[i] = in.offsets[i] - base;
-        offs_h = rebased.data();
-    }
+    const uint64_t* offs_h = rebased_offsets(in, rebased);
     if (n) CU(cudaMemcpyAsync(rd->offs.p, offs_h, (n + 1) * 8, cudaMemcpyHostToDevice, si));
     CU(cudaMemsetAsync(L.d_ctr, 0, sizeof(DevCounters), sc));
     if (!packed_in || !in.flags) CU(cudaMemsetAsync(b.flags, 0, n + 4, sc));
@@ -1037,41 +974,37 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
     // 8-byte total comes back.  Once the host knows it (one chunk later, so the GPU queue never drains) it sizes the
     // buffers, launches the phi kernel of that chunk and queues the D2H of its locations behind it -- the locations
     // of the BASELINE batch (565 M: 2.3 GB narrow, 4.5 GB as u64) leave the device while later chunks are searched.
-    HBuf& loc_h = h->locs;
-    HBuf& loc_hi_h = h->locs_hi;
-    DBuf& loc_d = rd->locs;
-    DBuf& loc_hi_d = rd->locs_hi;
+    PinnedBuf& loc_h = h->locs;
+    PinnedBuf& loc_hi_h = h->locs_hi;
+    DevBuf& loc_d = rd->locs;
+    DevBuf& loc_hi_d = rd->locs_hi;
     uint64_t loc_done = 0;                                        // locations whose D2H has been queued
-    auto grow_dev = [&](DBuf& d, size_t want, size_t keep) {
+    auto grow_dev = [&](DevBuf& d, size_t want, size_t keep) {
         if (want <= d.cap) return;
         CU(cudaStreamSynchronize(sc));                             // phi kernels write the old buffer
         CU(cudaStreamSynchronize(so));                             // ... and copies read it
-        DBuf bigger;
-        bigger.reserve(want + want / 4);
+        DevBuf bigger;
+        reserve(bigger, want + want / 4);
         if (keep) CU(cudaMemcpy(bigger.p, d.p, keep, cudaMemcpyDeviceToDevice));
-        d.release();
-        d = bigger;
+        d = std::move(bigger);
     };
-    auto grow_host = [&](HBuf& hb, size_t want, size_t keep) {
+    auto grow_host = [&](PinnedBuf& hb, size_t want, size_t keep) {
         if (want <= hb.cap) return;
         CU(cudaStreamSynchronize(so));                             // copies in flight target the old buffer
-        HBuf bigger;
-        bigger.reserve(want + want / 4);
+        PinnedBuf bigger;
+        reserve(bigger, want + want / 4);
         if (keep) memcpy(bigger.p, hb.p, keep);
-        hb.release();
-        hb = bigger;
+        hb = std::move(bigger);
     };
     auto grow_locs = [&](uint64_t want_items) {                    // keeps [0, loc_done) on both sides
         grow_dev(loc_d, (size_t) (want_items + 1) * loc_item, loc_done * loc_item);
         grow_host(loc_h, (size_t) (want_items + 1) * loc_item, loc_done * loc_item);
-        if (hi_plane) {
+        if (lf.hi_plane) {
             grow_dev(loc_hi_d, (size_t) want_items + 8, loc_done);
             grow_host(loc_hi_h, (size_t) want_items + 8, loc_done);
         }
-        point_locs(ix, rd, r, narrow);
-        out->locs = narrow ? nullptr : (uint64_t*) loc_h.p;
-        out->locs_lo32 = narrow ? (uint32_t*) loc_h.p : nullptr;
-        out->locs_hi8 = hi_plane ? (uint8_t*) loc_hi_h.p : nullptr;
+        point_locs(rd, r, lf);
+        point_locs(h, out, lf);
     };
     auto locate_chunk = [&](int c) {
         const uint64_t r0 = cut(c), r1 = cut(c + 1);
@@ -1089,7 +1022,7 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         if (end > begin) {
             CU(cudaMemcpyAsync((char*) loc_h.p + begin * loc_item, (const char*) loc_d.p + begin * loc_item, (end - begin) * loc_item,
                                cudaMemcpyDeviceToHost, so));
-            if (hi_plane) CU(cudaMemcpyAsync((char*) loc_hi_h.p + begin, (const char*) loc_hi_d.p + begin, end - begin, cudaMemcpyDeviceToHost, so));
+            if (lf.hi_plane) CU(cudaMemcpyAsync((char*) loc_hi_h.p + begin, (const char*) loc_hi_d.p + begin, end - begin, cudaMemcpyDeviceToHost, so));
         }
         loc_done = end;
     };
@@ -1165,8 +1098,8 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         const uint64_t total = scan_counts(L, rd, cnt, off, n, sc);           // syncs sc
         launches += 1;
         CU(cudaMemcpyAsync(off_h, off, (n + 1) * 8, cudaMemcpyDeviceToHost, sc));
-        rd->markers.reserve((total + 1) * 8);
-        h->markers.reserve((total + 1) * 8);
+        reserve(rd->markers, (total + 1) * 8);
+        reserve(h->markers, (total + 1) * 8);
         rd->n_markers = total;
         r.markers = rd->markers.as<uint64_t>();
         out->markers = (uint64_t*) h->markers.p;
@@ -1228,10 +1161,10 @@ void run_greedy(rbg_index* ix, Lane& L, rbg_stats& s, const rbg_batch* in, const
     CU(cudaEventRecord(L.ev[0], st));
     stage_batch(ix, st, BatchIn::raw(in), rd);
     const uint64_t n_words = (rd->n_bytes + 31) / 32 + 1;
-    g.bad.reserve(n_words * 4);
+    reserve(g.bad, n_words * 4);
     const uint64_t n_items = 2 * n;
-    for (DBuf* d : {&g.item_seeds, &g.item_words, &g.seed_off, &g.word_off}) d->reserve((n_items + 2) * 8);
-    rd->scan_tmp.reserve(scan_tmp_bytes(n_items + 1));
+    for (DevBuf* d : {&g.item_seeds, &g.item_words, &g.seed_off, &g.word_off}) reserve(*d, (n_items + 2) * 8);
+    reserve(rd->scan_tmp, scan_tmp_bytes(n_items + 1));
     // Every A/C/G/T gets its code even when the index lacks that base: the minus strand complements the code, so a base
     // the index lacks may stand for one it has.  A code the index lacks ends its seed through LF (an empty range), as
     // in the reference; only 'N' after seq_ntoa has no code.
@@ -1254,8 +1187,8 @@ void run_greedy(rbg_index* ix, Lane& L, rbg_stats& s, const rbg_batch* in, const
     const uint64_t total_seeds = scan_counts(L, rd, o.item_seeds, o.seed_off, n_items, st);
     const uint64_t total_words = scan_counts(L, rd, o.item_words, o.word_off, n_items, st);
     launches += 2;
-    g.seeds.reserve((total_seeds + 1) * sizeof(DevSeed));
-    g.words.reserve((total_words + 1) * 8);
+    reserve(g.seeds, (total_seeds + 1) * sizeof(DevSeed));
+    reserve(g.words, (total_words + 1) * 8);
     o.seeds = g.seeds.as<DevSeed>();
     o.words = g.words.as<uint64_t>();
     launches += launch_greedy(ix->dir, ix->ft, ix->mk, b, P, o, true, L.d_ctr, st);
@@ -1263,20 +1196,15 @@ void run_greedy(rbg_index* ix, Lane& L, rbg_stats& s, const rbg_batch* in, const
     launches += launch_seed_sort(o, total_seeds, st);
     CU(cudaEventRecord(L.ev[4], st));
 
-    HostSeedResult* h = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(ix->mu);
-        if (!ix->free_seed_results.empty()) { h = ix->free_seed_results.back(); ix->free_seed_results.pop_back(); }
-    }
-    if (!h) { h = new HostSeedResult; h->ix = ix; }
+    HostSeedResult* h = ix->seed_results.take(ix);
     memset(out, 0, sizeof *out);
     out->_owner = h;
     out->n_reads = n;
     out->n_seeds = total_seeds;
     out->n_marker_words = total_words;
-    h->seed_off.reserve((n_items + 1) * 8);
-    h->seeds.reserve((total_seeds + 1) * sizeof(rbg_seed));
-    h->markers.reserve((total_words + 1) * 8);
+    reserve(h->seed_off, (n_items + 1) * 8);
+    reserve(h->seeds, (total_seeds + 1) * sizeof(rbg_seed));
+    reserve(h->markers, (total_words + 1) * 8);
     out->seed_off = (uint64_t*) h->seed_off.p;
     out->seeds = (rbg_seed*) h->seeds.p;
     out->markers = (uint64_t*) h->markers.p;
@@ -1316,99 +1244,81 @@ int rbg_index_open(const char* prefix, uint32_t flags, int device, rbg_index** o
         const std::string pre(prefix);
         if ((flags & RBG_LOAD_FBB) && (flags & RBG_LOAD_SA))
             return fail(RBG_E_ARG, "fbb_string does not support loading toehold suffix array");     // include/rowbowt_io.hpp:107
-        if (flags & RBG_LOAD_CACHE) {
-            if (rbg_index* cached = open_layout_cache(pre, flags, device)) {
-                *out = cached;
-                if (flags & RBG_LOAD_FT) {
-                    try {
-                        LaneHold hold(*out, true);
-                        load_ftab(*out, hold.lane->stream, pre + ".ftab");
-                    } catch (...) {
-                        delete *out;
-                        *out = nullptr;
-                        throw;
-                    }
-                }
-                return (int) RBG_OK;
+        std::unique_ptr<rbg_index> ix;
+        if (flags & RBG_LOAD_CACHE) ix = open_layout_cache(pre, flags, device);
+        if (!ix) {
+            // the three files are decoded at the same time (each reader is itself multi-threaded over its components)
+            std::future<ToeholdArrays> tsa_job;
+            std::future<MarkerArrays> ma_job;
+            if (flags & RBG_LOAD_SA) tsa_job = std::async(std::launch::async, [&pre] { return read_tsa(pre + ".tsa"); });   // tsa_suffix :18
+            if (flags & RBG_LOAD_MA) ma_job = std::async(std::launch::async, [&pre] { return read_mab(pre + ".mab"); });    // ma_suffix  :19
+            RunsBwt bwt = (flags & RBG_LOAD_FBB) ? read_rbwt_fbb(pre + ".rbwt") : read_rbwt(pre + ".rbwt");   // rbwt_suffix, include/rowbowt_io.hpp:17
+            ToeholdArrays tsa;
+            MarkerArrays ma;
+            if (flags & RBG_LOAD_SA) tsa = tsa_job.get();
+            if (flags & RBG_LOAD_MA) ma = ma_job.get();
+            ix = open_from_arrays(bwt, (flags & RBG_LOAD_SA) ? &tsa : nullptr, (flags & RBG_LOAD_MA) ? &ma : nullptr, device);
+            if (flags & RBG_LOAD_FBB) ix->codes.code_of[1] = -1;   // wt_fbb: terminator is byte 0, byte 1 is no symbol
+            if (flags & RBG_LOAD_CACHE) {
+                try { write_layout_cache(ix.get(), pre, flags); } catch (...) { cudaGetLastError(); }      // best effort: the index is open either way
             }
         }
-        // the three files are decoded at the same time (each reader is itself multi-threaded over its components)
-        std::future<ToeholdArrays> tsa_job;
-        std::future<MarkerArrays> ma_job;
-        if (flags & RBG_LOAD_SA) tsa_job = std::async(std::launch::async, [&pre] { return read_tsa(pre + ".tsa"); });   // tsa_suffix :18
-        if (flags & RBG_LOAD_MA) ma_job = std::async(std::launch::async, [&pre] { return read_mab(pre + ".mab"); });    // ma_suffix  :19
-        RunsBwt bwt = (flags & RBG_LOAD_FBB) ? read_rbwt_fbb(pre + ".rbwt") : read_rbwt(pre + ".rbwt");   // rbwt_suffix, include/rowbowt_io.hpp:17
-        ToeholdArrays tsa;
-        MarkerArrays ma;
-        if (flags & RBG_LOAD_SA) tsa = tsa_job.get();
-        if (flags & RBG_LOAD_MA) ma = ma_job.get();
-        int rc = open_from_arrays(bwt, (flags & RBG_LOAD_SA) ? &tsa : nullptr, (flags & RBG_LOAD_MA) ? &ma : nullptr, device, out);
-        if (rc == RBG_OK && (flags & RBG_LOAD_FBB)) (*out)->codes.code_of[1] = -1;   // wt_fbb: terminator is byte 0, byte 1 is no symbol
-        if (rc == RBG_OK && (flags & RBG_LOAD_CACHE)) {
-            try { write_layout_cache(*out, pre, flags); } catch (...) { cudaGetLastError(); }      // best effort: the index is open either way
+        if (flags & RBG_LOAD_FT) {                  // ft_suffix :21, LoadRbwtFlag::FT :151
+            LaneHold hold(ix.get(), true);
+            load_ftab(ix.get(), hold.lane->stream, pre + ".ftab");
         }
-        if (rc == RBG_OK && (flags & RBG_LOAD_FT)) {                  // ft_suffix :21, LoadRbwtFlag::FT :151
-            try {
-                LaneHold hold(*out, true);
-                load_ftab(*out, hold.lane->stream, pre + ".ftab");
-            } catch (...) {
-                delete *out;
-                *out = nullptr;
-                throw;
-            }
-        }
-        return rc;
-    });
-}
-
-int rbg_index_open_arrays(const rbg_index_desc* d, int device, rbg_index** out) {
-    if (!d || !out) return fail(RBG_E_ARG, "null argument");
-    *out = nullptr;
-    return guarded([&] {
-        RunsBwt bwt;
-        bwt.n = d->n;
-        bwt.R = d->R;
-        if (!d->run_heads || !d->run_lens) return fail(RBG_E_ARG, "run_heads/run_lens missing");
-        bwt.heads.assign(d->run_heads, d->run_heads + d->R);
-        bwt.lens.assign(d->run_lens, d->run_lens + d->R);
-        ToeholdArrays tsa;
-        const bool has_sa = d->r && d->pred && d->samples_last && d->pred_to_run;
-        if (has_sa) {
-            tsa.r = d->r;
-            tsa.n = d->n;
-            tsa.pred.assign(d->pred, d->pred + d->r);
-            tsa.samples_last.assign(d->samples_last, d->samples_last + d->r);
-            tsa.pred_to_run.assign(d->pred_to_run, d->pred_to_run + d->r);
-        }
-        MarkerArrays ma;
-        const bool has_ma = d->win_starts && d->win_ends && d->win_idxs;
-        if (has_ma) {
-            ma.starts.assign(d->win_starts, d->win_starts + d->n_windows);
-            ma.ends.assign(d->win_ends, d->win_ends + d->n_windows);
-            ma.idxs.assign(d->win_idxs, d->win_idxs + d->n_windows);
-            if (d->arr_size) ma.arr.assign(d->arr, d->arr + d->arr_size);
-            ma.size_starts = d->size_starts;
-            ma.size_ends = d->size_ends;
-            ma.size_idxs = d->size_idxs;
-        }
-        return open_from_arrays(bwt, has_sa ? &tsa : nullptr, has_ma ? &ma : nullptr, device, out);
+        *out = ix.release();
+        return (int) RBG_OK;
     });
 }
 
 namespace {
-double wall_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-
-struct RawParts {
+// The arrays an index is laid out from; the toehold / marker arrays only with has_sa / has_ma.
+struct IndexArrays {
     RunsBwt bwt;
     ToeholdArrays tsa;
     MarkerArrays ma;
+    bool has_sa = false, has_ma = false;
 };
 
+// The arrays of a caller's rbg_index_desc: toehold arrays when all four of their pointers are set, marker arrays when all
+// three are.  With `tsa_only` (the marker-array build) the toehold arrays are required and marker arrays are not read.
+IndexArrays index_arrays_from_desc(const rbg_index_desc* d, bool tsa_only) {
+    if (!d->run_heads || !d->run_lens) throw std::invalid_argument("run_heads/run_lens missing");
+    IndexArrays p;
+    p.has_sa = d->r && d->pred && d->samples_last && d->pred_to_run;
+    if (tsa_only && !p.has_sa) throw std::invalid_argument("toehold arrays missing");
+    p.bwt.n = d->n;
+    p.bwt.R = d->R;
+    p.bwt.heads.assign(d->run_heads, d->run_heads + d->R);
+    p.bwt.lens.assign(d->run_lens, d->run_lens + d->R);
+    if (p.has_sa) {
+        p.tsa.r = d->r;
+        p.tsa.n = d->n;
+        p.tsa.pred.assign(d->pred, d->pred + d->r);
+        p.tsa.samples_last.assign(d->samples_last, d->samples_last + d->r);
+        p.tsa.pred_to_run.assign(d->pred_to_run, d->pred_to_run + d->r);
+    }
+    p.has_ma = !tsa_only && d->win_starts && d->win_ends && d->win_idxs;
+    if (p.has_ma) {
+        p.ma.starts.assign(d->win_starts, d->win_starts + d->n_windows);
+        p.ma.ends.assign(d->win_ends, d->win_ends + d->n_windows);
+        p.ma.idxs.assign(d->win_idxs, d->win_idxs + d->n_windows);
+        if (d->arr_size) p.ma.arr.assign(d->arr, d->arr + d->arr_size);
+        p.ma.size_starts = d->size_starts;
+        p.ma.size_ends = d->size_ends;
+        p.ma.size_idxs = d->size_idxs;
+    }
+    return p;
+}
+
+std::unique_ptr<rbg_index> open_from_arrays(const IndexArrays& p, int device) {
+    return open_from_arrays(p.bwt, p.has_sa ? &p.tsa : nullptr, p.has_ma ? &p.ma : nullptr, device);
+}
+
 // rb_build's inputs (src/rb_build.cpp:76-87): <prefix>.bwt, .ssa/.esa, .ma
-void load_raw(const std::string& pre, uint32_t flags, int device, RawParts& p, rbg_build_stats* st) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) throw cuda_error("no CUDA device: librowbowt_gpu has no CPU fallback");
-    if (device < 0 || device >= ndev) throw std::invalid_argument("device ordinal out of range");
+void load_raw(const std::string& pre, uint32_t flags, int device, IndexArrays& p, rbg_build_stats* st) {
+    select_device(device);
     RawBuildStats rs;
     double t0 = wall_s();
     p.bwt = rle_bwt_gpu(pre + ".bwt", device, &rs);
@@ -1419,12 +1329,14 @@ void load_raw(const std::string& pre, uint32_t flags, int device, RawParts& p, r
         st->ms_rle_kernels = rs.ms_kernels;
         st->s_rle = wall_s() - t0;
     }
-    if (flags & RBG_LOAD_SA) {
+    p.has_sa = flags & RBG_LOAD_SA;
+    if (p.has_sa) {
         t0 = wall_s();
         p.tsa = toehold_from_raw(pre + ".ssa", pre + ".esa", p.bwt.n, p.bwt.R, device);
         if (st) st->s_samples = wall_s() - t0;
     }
-    if (flags & RBG_LOAD_MA) {
+    p.has_ma = flags & RBG_LOAD_MA;
+    if (p.has_ma) {
         t0 = wall_s();
         p.ma = markers_from_ma(pre + ".ma");
         if (st) st->s_markers = wall_s() - t0;
@@ -1432,13 +1344,23 @@ void load_raw(const std::string& pre, uint32_t flags, int device, RawParts& p, r
 }
 }  // namespace
 
+int rbg_index_open_arrays(const rbg_index_desc* d, int device, rbg_index** out) {
+    if (!d || !out) return fail(RBG_E_ARG, "null argument");
+    *out = nullptr;
+    return guarded([&] {
+        *out = open_from_arrays(index_arrays_from_desc(d, false), device).release();
+        return (int) RBG_OK;
+    });
+}
+
 int rbg_index_open_raw(const char* prefix, uint32_t flags, int device, rbg_index** out) {
     if (!prefix || !out) return fail(RBG_E_ARG, "null argument");
     *out = nullptr;
     return guarded([&] {
-        RawParts p;
+        IndexArrays p;
         load_raw(prefix, flags, device, p, nullptr);
-        return open_from_arrays(p.bwt, (flags & RBG_LOAD_SA) ? &p.tsa : nullptr, (flags & RBG_LOAD_MA) ? &p.ma : nullptr, device, out);
+        *out = open_from_arrays(p, device).release();
+        return (int) RBG_OK;
     });
 }
 
@@ -1448,7 +1370,7 @@ int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flag
         rbg_build_stats st;
         memset(&st, 0, sizeof st);
         const double t_begin = wall_s();
-        RawParts p;
+        IndexArrays p;
         load_raw(in_prefix, flags, device, p, &st);
         const std::string out(out_prefix);
         double t0 = wall_s();
@@ -1457,15 +1379,12 @@ int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flag
         if (flags & RBG_LOAD_SA) write_tsa(p.tsa, out + ".tsa");           // :65-72
         st.s_write = wall_s() - t0;
         if (flags & RBG_LOAD_FT) {                                         // :82-88 (rb_build -f): build_ftab(k) + FTab::serialize
-            rbg_index* ix = nullptr;
-            int rc = open_from_arrays(p.bwt, nullptr, nullptr, device, &ix);
-            if (rc != RBG_OK) return rc;
-            std::unique_ptr<rbg_index> own(ix);
+            std::unique_ptr<rbg_index> ix = open_from_arrays(p.bwt, nullptr, nullptr, device);
             {
-                LaneHold hold(ix, true);
-                build_ftab(ix, hold.lane->stream, ftab_k ? ftab_k : 10);
+                LaneHold hold(ix.get(), true);
+                build_ftab(ix.get(), hold.lane->stream, ftab_k ? ftab_k : 10);
             }
-            save_ftab(ix, out + ".ftab");
+            save_ftab(ix.get(), out + ".ftab");
         }
         st.s_total = wall_s() - t_begin;
         if (stats) *stats = st;
@@ -1475,37 +1394,29 @@ int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flag
 
 namespace {
 // What the two rbg_build_marker_array entries share once the index arrays are in hand: the device check, then the build.
-// `mps` was read and checked against n (check_ma_inputs) before any CUDA call.
-int build_ma_from(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsRecords& mps, uint64_t row_begin, uint64_t row_end,
-                  int device, const char* ma_path, const char* mab_path, rbg_ma_stats& st, double t_begin, rbg_ma_stats* out) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        return fail(RBG_E_CUDA, "no CUDA device: librowbowt_gpu has no CPU fallback");
-    }
-    if (device < 0 || device >= ndev) return fail(RBG_E_ARG, "device ordinal out of range");
-    st.n = bwt.n;
-    st.r = bwt.R;
+// `mps` was read and checked against n (read_mps_window) before any CUDA call.
+int build_ma_from(const IndexArrays& p, const MpsRecords& mps, uint64_t row_begin, uint64_t row_end, int device, const char* ma_path,
+                  const char* mab_path, rbg_ma_stats& st, double t_begin, rbg_ma_stats* out) {
+    select_device(device);
+    st.n = p.bwt.n;
+    st.r = p.bwt.R;
     st.mps_records = mps.first.size();
     st.lists = mps.list_off.size() - 1;
-    try {
-        build_marker_array(bwt, tsa, mps, row_begin, row_end, device, ma_path, mab_path ? mab_path : "", st);
-    } catch (const cuda_error_ma& e) {
-        cudaGetLastError();
-        return fail(RBG_E_CUDA, e.what());
-    }
+    build_marker_array(p.bwt, p.tsa, mps, row_begin, row_end, device, ma_path, mab_path ? mab_path : "", st);
     st.s_total = wall_s() - t_begin;
     if (out) *out = st;
     return (int) RBG_OK;
 }
 
-// The window [row_begin, min(row_end, n)) must hold a row, the index r == R samples; then the .mps is read against n.
-int check_ma_inputs(uint64_t n, uint64_t R, uint64_t r, uint64_t row_begin, uint64_t& row_end, const char* mps_path, MpsRecords& mps) {
-    if (r != R) return fail(RBG_E_ARG, "the toehold arrays hold " + std::to_string(r) + " samples for " + std::to_string(R) + " runs");
+void check_sample_count(uint64_t r, uint64_t R) {
+    if (r != R) throw std::invalid_argument("the toehold arrays hold " + std::to_string(r) + " samples for " + std::to_string(R) + " runs");
+}
+
+// The window [row_begin, min(row_end, n)) must hold a row; then the .mps is read against n.
+MpsRecords read_mps_window(const char* mps_path, uint64_t n, uint64_t row_begin, uint64_t& row_end) {
     row_end = std::min(row_end, n);
-    if (row_begin >= row_end) return fail(RBG_E_ARG, "empty row window");
-    mps = read_mps(mps_path, n);
-    return (int) RBG_OK;
+    if (row_begin >= row_end) throw std::invalid_argument("empty row window");
+    return read_mps(mps_path, n);
 }
 }  // namespace
 
@@ -1518,27 +1429,25 @@ int rbg_build_marker_array(const char* index_prefix, const char* mps_path, const
         const double t_begin = wall_s();
         const std::string pre(index_prefix);
         struct stat sb;
-        MpsRecords mps;
-        RawParts p;
-        if (stat((pre + ".rbwt").c_str(), &sb) == 0) {
+        IndexArrays p;
+        uint64_t n;
+        const bool raw = stat((pre + ".rbwt").c_str(), &sb) != 0;
+        if (!raw) {
             if (stat((pre + ".tsa").c_str(), &sb) != 0) return fail(RBG_E_IO, "no toehold samples: " + pre + ".tsa");
             p.bwt = read_rbwt(pre + ".rbwt");
             p.tsa = read_tsa(pre + ".tsa");
-            const int rc = check_ma_inputs(p.bwt.n, p.bwt.R, p.tsa.r, row_begin, row_end, mps_path, mps);
-            if (rc != RBG_OK) return rc;
+            check_sample_count(p.tsa.r, p.bwt.R);
+            n = p.bwt.n;
         } else {           // the raw inputs: n is the size of the .bwt (one byte per row); decoded on the GPU afterwards
-            struct stat bwt_st;
-            if (stat((pre + ".bwt").c_str(), &bwt_st) != 0) return fail(RBG_E_IO, "no index: neither " + pre + ".rbwt nor " + pre + ".bwt");
+            if (stat((pre + ".bwt").c_str(), &sb) != 0) return fail(RBG_E_IO, "no index: neither " + pre + ".rbwt nor " + pre + ".bwt");
+            n = (uint64_t) sb.st_size;
             for (const char* suf : {".ssa", ".esa"})
                 if (stat((pre + suf).c_str(), &sb) != 0) return fail(RBG_E_IO, "no toehold samples: " + pre + suf);
-            const uint64_t n = (uint64_t) bwt_st.st_size;
-            row_end = std::min(row_end, n);
-            if (row_begin >= row_end) return fail(RBG_E_ARG, "empty row window");
-            mps = read_mps(mps_path, n);
-            load_raw(pre, RBG_LOAD_SA, device, p, nullptr);
         }
+        const MpsRecords mps = read_mps_window(mps_path, n, row_begin, row_end);
+        if (raw) load_raw(pre, RBG_LOAD_SA, device, p, nullptr);
         st.s_read = wall_s() - t_begin;
-        return build_ma_from(p.bwt, p.tsa, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
+        return build_ma_from(p, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
     });
 }
 
@@ -1549,26 +1458,13 @@ int rbg_build_marker_array_arrays(const rbg_index_desc* d, const char* mps_path,
         rbg_ma_stats st;
         memset(&st, 0, sizeof st);
         const double t_begin = wall_s();
-        if (!d->run_heads || !d->run_lens) return fail(RBG_E_ARG, "run_heads/run_lens missing");
-        if (!d->r || !d->pred || !d->samples_last || !d->pred_to_run) return fail(RBG_E_ARG, "toehold arrays missing");
-        RunsBwt bwt;
-        bwt.n = d->n;
-        bwt.R = d->R;
-        bwt.heads.assign(d->run_heads, d->run_heads + d->R);
-        bwt.lens.assign(d->run_lens, d->run_lens + d->R);
-        ToeholdArrays tsa;
-        tsa.r = d->r;
-        tsa.n = d->n;
-        tsa.pred.assign(d->pred, d->pred + d->r);
-        tsa.samples_last.assign(d->samples_last, d->samples_last + d->r);
-        tsa.pred_to_run.assign(d->pred_to_run, d->pred_to_run + d->r);
-        MpsRecords mps;
-        const int rc = check_ma_inputs(bwt.n, bwt.R, tsa.r, row_begin, row_end, mps_path, mps);
-        if (rc != RBG_OK) return rc;
-        validate_runs(bwt, "the BWT runs");
-        validate_toehold(tsa, "the toehold arrays");
+        const IndexArrays p = index_arrays_from_desc(d, true);
+        check_sample_count(p.tsa.r, p.bwt.R);
+        const MpsRecords mps = read_mps_window(mps_path, p.bwt.n, row_begin, row_end);
+        validate_runs(p.bwt, "the BWT runs");
+        validate_toehold(p.tsa, "the toehold arrays");
         st.s_read = wall_s() - t_begin;
-        return build_ma_from(bwt, tsa, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
+        return build_ma_from(p, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
     });
 }
 
@@ -1651,7 +1547,7 @@ int query_any(rbg_index* ix, const BatchIn& in, uint32_t mode, uint64_t max_hits
             for (auto& st : hold.lane->s_srch) cudaStreamSynchronize(st);
             cudaStreamSynchronize(hold.lane->stream);
             cudaStreamSynchronize(hold.lane->s_out);
-            if (out->_owner) { give_back_host_result(ix, (HostResult*) out->_owner); memset(out, 0, sizeof *out); }
+            if (out->_owner) { ix->results.give_back((HostResult*) out->_owner); memset(out, 0, sizeof *out); }
             throw;
         }
         hold.stats.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1676,7 +1572,7 @@ int rbg_query_packed(rbg_index* ix, const rbg_packed_batch* in, uint32_t mode, u
 void rbg_result_free(rbg_result* res) {
     if (!res || !res->_owner) return;
     HostResult* h = (HostResult*) res->_owner;
-    give_back_host_result(h->ix, h);
+    h->ix->results.give_back(h);
     memset(res, 0, sizeof *res);
 }
 
@@ -1692,11 +1588,7 @@ int rbg_markers_greedy(rbg_index* ix, const rbg_batch* in, const rbg_greedy_para
             run_greedy(ix, *hold.lane, hold.stats, in, params, out);
         } catch (...) {
             cudaStreamSynchronize(hold.lane->stream);
-            if (out->_owner) {
-                std::lock_guard<std::mutex> lock(ix->mu);
-                ix->free_seed_results.push_back((HostSeedResult*) out->_owner);
-                memset(out, 0, sizeof *out);
-            }
+            if (out->_owner) { ix->seed_results.give_back((HostSeedResult*) out->_owner); memset(out, 0, sizeof *out); }
             throw;
         }
         hold.stats.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -1708,12 +1600,7 @@ int rbg_markers_greedy(rbg_index* ix, const rbg_batch* in, const rbg_greedy_para
 void rbg_seed_result_free(rbg_seed_result* res) {
     if (!res || !res->_owner) return;
     HostSeedResult* h = (HostSeedResult*) res->_owner;
-    rbg_index* ix = h->ix;
-    {
-        std::lock_guard<std::mutex> lock(ix->mu);
-        if (ix->free_seed_results.size() < 4) ix->free_seed_results.push_back(h);
-        else { h->release(); delete h; }
-    }
+    h->ix->seed_results.give_back(h);
     memset(res, 0, sizeof *res);
 }
 
@@ -1724,10 +1611,8 @@ int upload_any(rbg_index* ix, const BatchIn& in, rbg_reads** out) {
         CU(cudaSetDevice(ix->device));
         LaneHold hold(ix);
         std::unique_ptr<rbg_reads> rd(new rbg_reads);
-        try {
-            stage_batch(ix, hold.lane->stream, in, rd.get());
-            CU(cudaStreamSynchronize(hold.lane->stream));
-        } catch (...) { rd->release(); throw; }
+        stage_batch(ix, hold.lane->stream, in, rd.get());
+        CU(cudaStreamSynchronize(hold.lane->stream));
         *out = rd.release();
         return (int) RBG_OK;
     });
@@ -1771,7 +1656,6 @@ int rbg_reads_fetch(rbg_index* ix, rbg_reads* reads, uint32_t mode, rbg_result* 
 void rbg_reads_free(rbg_reads* reads) {
     if (!reads) return;
     if (reads->ix) cudaSetDevice(reads->ix->device);
-    reads->release();
     delete reads;
 }
 
@@ -1807,9 +1691,7 @@ double rbg_gather_roofline(int device, size_t footprint_bytes, int line_bytes, i
     if (line_bytes != 32 && line_bytes != 64 && line_bytes != 128) { g_err = "line_bytes must be 32, 64 or 128"; return -1.0; }
     double gbs = -1.0;
     int rc = guarded([&] {
-        int ndev = 0;
-        if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) throw cuda_error("no CUDA device");
-        CU(cudaSetDevice(device));
+        select_device(device);
         void* buf = nullptr;
         CU(cudaMalloc(&buf, footprint_bytes));
         CU(cudaMemset(buf, 0x5A, footprint_bytes));

@@ -17,25 +17,18 @@
 #include <unistd.h>
 
 #include <algorithm>
-#include <chrono>
 #include <cstdio>
 #include <cstdlib>
-#include <memory>
 #include <string>
 #include <vector>
 
 #include "ma_build.hpp"
+#include "cuda_host.hpp"
 #include "device_index.cuh"
 #include "raw_build.hpp"
 #include "sdsl_writer.hpp"
 
 namespace rbg {
-
-#define CUM(call)                                                                                              \
-    do {                                                                                                       \
-        cudaError_t e_ = (call);                                                                               \
-        if (e_ != cudaSuccess) throw cuda_error_ma(std::string(#call) + ": " + cudaGetErrorString(e_));        \
-    } while (0)
 
 // Kernels outside the anonymous namespace: their names stay the same from build to build (traces, profiles).
 constexpr int kMaBlock = 256;
@@ -96,24 +89,7 @@ __global__ void __launch_bounds__(kMaBlock) ma_blocks_kernel(const uint32_t* __r
 
 namespace {
 
-struct DevMem {
-    void* p = nullptr;
-    DevMem() = default;
-    explicit DevMem(size_t bytes) { CUM(cudaMalloc(&p, std::max<size_t>(bytes, 64))); }
-    ~DevMem() { if (p) cudaFree(p); }
-    DevMem(const DevMem&) = delete;
-    DevMem& operator=(const DevMem&) = delete;
-    template <class T> T* as() const { return (T*) p; }
-};
-
-template <class T>
-T* put(std::vector<std::unique_ptr<DevMem>>& owned, const std::vector<T>& v) {
-    owned.emplace_back(new DevMem(v.size() * sizeof(T)));
-    if (!v.empty()) CUM(cudaMemcpy(owned.back()->p, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
-    return owned.back()->as<T>();
-}
-
-double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+DevBuf dev_mem(size_t bytes) { return DevBuf(std::max<size_t>(bytes, 64)); }
 
 struct Block {
     uint64_t first, last;
@@ -153,26 +129,16 @@ void write_ma(const std::vector<Block>& blocks, const MpsRecords& mps, const std
 void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsRecords& mps, uint64_t row_begin, uint64_t row_end,
                         int device, const std::string& ma_path, const std::string& mab_path, rbg_ma_stats& st) {
     const uint64_t n = bwt.n, R = bwt.R;
-    const double t_layout = now_s();
-    CUM(cudaSetDevice(device));
+    const double t_layout = wall_s();
+    CU(cudaSetDevice(device));
     // run starts, and the runs the window [row_begin, row_end) overlaps: [j0, j1]
     std::vector<uint64_t> start(R + 1, 0);
     for (uint64_t j = 0; j < R; ++j) start[j + 1] = start[j] + bwt.lens[j];
     const uint64_t j0 = (uint64_t) (std::upper_bound(start.begin(), start.end(), row_begin) - start.begin()) - 1;
     const uint64_t j1 = (uint64_t) (std::upper_bound(start.begin(), start.end(), row_end - 1) - start.begin()) - 1;
 
-    std::vector<std::unique_ptr<DevMem>> owned;
-    size_t free_b = 0, total_b = 0;
-    CUM(cudaMemGetInfo(&free_b, &total_b));
-    PhiDir pd = build_phi_dir(tsa, 0, (uint64_t) free_b / 4);          // the budget open_from_arrays gives the slots
-    DevPhi P{};
-    P.l1 = put(owned, pd.l1);
-    P.slots = put(owned, pd.slots);
-    P.ovf_keys = put(owned, pd.ovf_keys);
-    P.ovf_prev_lo = put(owned, pd.ovf_prev.lo);
-    P.ovf_prev_hi = pd.ovf_prev.wide ? put(owned, pd.ovf_prev.hi) : nullptr;
-    P.n = n;
-    P.shift = pd.shift;
+    std::vector<Upload> owned;
+    const DevPhi P = upload_phi(build_phi_dir(tsa, 0, phi_slot_budget()), n, owned);
 
     // directory over text positions: about one record per bucket, so it costs no more than the records themselves
     const uint64_t m = mps.first.size();
@@ -183,10 +149,11 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
         while (k < m && mps.last[k] < (b << shift)) ++k;
         dir[b] = k;
     }
-    DevRecords D{put(owned, mps.first), put(owned, mps.last), put(owned, mps.list), put(owned, dir), m, shift};
+    DevRecords D{upload(mps.first, owned), upload(mps.last, owned), upload(mps.list, owned), upload(dir, owned), m, shift};
 
     // chunk buffers: the id array plus, per row at worst, one run of the encoder, its scan and two blocks
-    CUM(cudaMemGetInfo(&free_b, &total_b));
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
     const uint64_t per_row = 4 * 4 + 2 * sizeof(MaBlock);
     uint64_t cap = std::min<uint64_t>(kMaxChunkRows, (uint64_t) free_b / 2 / per_row);
     if (const char* e = getenv("RBG_MA_CHUNK_ROWS")) cap = std::max<uint64_t>(1, std::min<uint64_t>(cap, strtoull(e, nullptr, 10)));
@@ -202,21 +169,22 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
         runs_alloc = std::max(runs_alloc, e - a);
         a = e;
     }
-    DevMem d_ids(rows_alloc * 4), d_unique(rows_alloc * 4), d_lens(rows_alloc * 4), d_offs(rows_alloc * 4);
-    DevMem d_blocks(rows_alloc * sizeof(MaBlock)), d_sel(rows_alloc * sizeof(MaBlock));
-    DevMem d_run_last(runs_alloc * 8), d_run_sa(runs_alloc * 8), d_ctr(4 * 8);
+    DevBuf d_ids = dev_mem(rows_alloc * 4), d_unique = dev_mem(rows_alloc * 4), d_lens = dev_mem(rows_alloc * 4),
+           d_offs = dev_mem(rows_alloc * 4);
+    DevBuf d_blocks = dev_mem(rows_alloc * sizeof(MaBlock)), d_sel = dev_mem(rows_alloc * sizeof(MaBlock));
+    DevBuf d_run_last = dev_mem(runs_alloc * 8), d_run_sa = dev_mem(runs_alloc * 8), d_ctr = dev_mem(4 * 8);
     size_t tmp_a = 0, tmp_b = 0, tmp_c = 0;
     const int items = (int) rows_alloc;
-    CUM(cub::DeviceRunLengthEncode::Encode(nullptr, tmp_a, d_ids.as<uint32_t>(), d_unique.as<uint32_t>(), d_lens.as<uint32_t>(),
+    CU(cub::DeviceRunLengthEncode::Encode(nullptr, tmp_a, d_ids.as<uint32_t>(), d_unique.as<uint32_t>(), d_lens.as<uint32_t>(),
                                           d_ctr.as<int>(), items));
-    CUM(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, d_lens.as<uint32_t>(), d_offs.as<uint32_t>(), items));
-    CUM(cub::DeviceSelect::If(nullptr, tmp_c, d_blocks.as<MaBlock>(), d_sel.as<MaBlock>(), d_ctr.as<int>() + 1, items, HasList()));
+    CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, d_lens.as<uint32_t>(), d_offs.as<uint32_t>(), items));
+    CU(cub::DeviceSelect::If(nullptr, tmp_c, d_blocks.as<MaBlock>(), d_sel.as<MaBlock>(), d_ctr.as<int>() + 1, items, HasList()));
     const size_t tmp_bytes = std::max(tmp_a, std::max(tmp_b, tmp_c));
-    DevMem d_tmp(tmp_bytes);
+    DevBuf d_tmp = dev_mem(tmp_bytes);
     cudaStream_t s;
-    CUM(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
     cudaEvent_t ev[3];
-    for (auto& e : ev) CUM(cudaEventCreate(&e));
+    for (auto& e : ev) CU(cudaEventCreate(&e));
     struct Cleanup {
         cudaStream_t s;
         cudaEvent_t* ev;
@@ -227,10 +195,10 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
     std::vector<Block> blocks;
     unsigned long long* ctr = d_ctr.as<unsigned long long>();     // [0] run cursor, [1] phi steps; [2..3] the encoder / select counts
     int* counts = (int*) (ctr + 2);
-    CUM(cudaMemsetAsync(ctr + 1, 0, 8, s));
+    CU(cudaMemsetAsync(ctr + 1, 0, 8, s));
     int sms = 0;
-    CUM(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-    st.s_layout = now_s() - t_layout;
+    CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    st.s_layout = wall_s() - t_layout;
 
     // chunks of whole runs, at most `cap` window rows each (or one run)
     for (uint64_t a = j0; a <= j1;) {
@@ -242,40 +210,40 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
             h_last[j - a] = start[j + 1] - 1;
             h_sa[j - a] = tsa.samples_last[j] + 1 == n ? 0 : tsa.samples_last[j] + 1;
         }
-        CUM(cudaMemcpyAsync(d_run_last.p, h_last.data(), (e - a) * 8, cudaMemcpyHostToDevice, s));
-        CUM(cudaMemcpyAsync(d_run_sa.p, h_sa.data(), (e - a) * 8, cudaMemcpyHostToDevice, s));
-        CUM(cudaMemsetAsync(ctr, 0, 8, s));
-        CUM(cudaEventRecord(ev[0], s));
+        CU(cudaMemcpyAsync(d_run_last.p, h_last.data(), (e - a) * 8, cudaMemcpyHostToDevice, s));
+        CU(cudaMemcpyAsync(d_run_sa.p, h_sa.data(), (e - a) * 8, cudaMemcpyHostToDevice, s));
+        CU(cudaMemsetAsync(ctr, 0, 8, s));
+        CU(cudaEventRecord(ev[0], s));
         const uint64_t want = (e - a + kMaBlock - 1) / kMaBlock;
         const int grid = (int) std::min<uint64_t>(want, (uint64_t) sms * 8);
         ma_rows_kernel<<<grid, kMaBlock, 0, s>>>(P, D, d_run_last.as<uint64_t>(), d_run_sa.as<uint64_t>(), e - a, start[a], row0, row_end,
                                                  d_ids.as<uint32_t>(), ctr, ctr + 1);
-        CUM(cudaGetLastError());
-        CUM(cudaEventRecord(ev[1], s));
+        CU(cudaGetLastError());
+        CU(cudaEventRecord(ev[1], s));
         size_t tb = tmp_bytes;
-        CUM(cub::DeviceRunLengthEncode::Encode(d_tmp.p, tb, d_ids.as<uint32_t>(), d_unique.as<uint32_t>(), d_lens.as<uint32_t>(), counts,
+        CU(cub::DeviceRunLengthEncode::Encode(d_tmp.p, tb, d_ids.as<uint32_t>(), d_unique.as<uint32_t>(), d_lens.as<uint32_t>(), counts,
                                               (int) rows, s));
         int n_runs = 0;
-        CUM(cudaMemcpyAsync(&n_runs, counts, 4, cudaMemcpyDeviceToHost, s));
-        CUM(cudaStreamSynchronize(s));
+        CU(cudaMemcpyAsync(&n_runs, counts, 4, cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
         tb = tmp_bytes;
-        CUM(cub::DeviceScan::ExclusiveSum(d_tmp.p, tb, d_lens.as<uint32_t>(), d_offs.as<uint32_t>(), n_runs, s));
+        CU(cub::DeviceScan::ExclusiveSum(d_tmp.p, tb, d_lens.as<uint32_t>(), d_offs.as<uint32_t>(), n_runs, s));
         ma_blocks_kernel<<<(n_runs + kMaBlock - 1) / kMaBlock, kMaBlock, 0, s>>>(d_unique.as<uint32_t>(), d_lens.as<uint32_t>(),
                                                                                  d_offs.as<uint32_t>(), (uint32_t) n_runs, d_blocks.as<MaBlock>());
-        CUM(cudaGetLastError());
+        CU(cudaGetLastError());
         tb = tmp_bytes;
-        CUM(cub::DeviceSelect::If(d_tmp.p, tb, d_blocks.as<MaBlock>(), d_sel.as<MaBlock>(), counts + 1, n_runs, HasList(), s));
-        CUM(cudaEventRecord(ev[2], s));
+        CU(cub::DeviceSelect::If(d_tmp.p, tb, d_blocks.as<MaBlock>(), d_sel.as<MaBlock>(), counts + 1, n_runs, HasList(), s));
+        CU(cudaEventRecord(ev[2], s));
         int n_sel = 0;
-        CUM(cudaMemcpyAsync(&n_sel, counts + 1, 4, cudaMemcpyDeviceToHost, s));
-        CUM(cudaStreamSynchronize(s));
+        CU(cudaMemcpyAsync(&n_sel, counts + 1, 4, cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
         h_sel.resize(n_sel);
-        if (n_sel) CUM(cudaMemcpyAsync(h_sel.data(), d_sel.p, (size_t) n_sel * sizeof(MaBlock), cudaMemcpyDeviceToHost, s));
-        CUM(cudaStreamSynchronize(s));
+        if (n_sel) CU(cudaMemcpyAsync(h_sel.data(), d_sel.p, (size_t) n_sel * sizeof(MaBlock), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
         float ms = 0;
-        CUM(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+        CU(cudaEventElapsedTime(&ms, ev[0], ev[1]));
         st.ms_rows_kernel += ms;
-        CUM(cudaEventElapsedTime(&ms, ev[1], ev[2]));
+        CU(cudaEventElapsedTime(&ms, ev[1], ev[2]));
         st.ms_blocks += ms;
         for (int i = 0; i < n_sel; ++i) {
             const MaBlock& b = h_sel[i];
@@ -287,11 +255,11 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
         a = e;
     }
     unsigned long long steps = 0;
-    CUM(cudaMemcpy(&steps, ctr + 1, 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&steps, ctr + 1, 8, cudaMemcpyDeviceToHost));
     st.phi_steps = steps;
     st.ma_records = blocks.size();
 
-    const double t_write = now_s();
+    const double t_write = wall_s();
     write_ma(blocks, mps, ma_path, st.ma_words);
     if (!mab_path.empty()) {             // rb_build -m over the .ma just written (the .ma stays even when this refuses it)
         MarkerArrays ma = markers_from_ma(ma_path);
@@ -307,7 +275,7 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
             throw io_error("cannot write " + mab_path);
         }
     }
-    st.s_write = now_s() - t_write;
+    st.s_write = wall_s() - t_write;
 }
 
 }  // namespace rbg

@@ -1,7 +1,6 @@
 // The marker array (.ma) from a .mps and the index's own phi (ma_build.cu).
 #pragma once
 #include <cstdint>
-#include <stdexcept>
 #include <string>
 
 #include "../../include/rowbowt_gpu.h"
@@ -9,8 +8,6 @@
 #include "layout.hpp"
 
 namespace rbg {
-
-struct cuda_error_ma : std::runtime_error { using std::runtime_error::runtime_error; };
 
 // Rows [row_begin, row_end) (row_begin < row_end <= n; tsa.r == bwt.R): writes ma_path and, when mab_path is not empty, the
 // .mab rb_build -m makes from it.  Fills the row, step, record, layout, write and kernel fields of `st` (adding to them).

@@ -17,13 +17,13 @@
 #include <cub/cub.cuh>
 
 #include <algorithm>
-#include <chrono>
 #include <cstdio>
 #include <cstring>
 #include <memory>
 #include <string>
 #include <vector>
 
+#include "cuda_host.hpp"
 #include "formats.hpp"
 #include "layout.hpp"
 #include "raw_build.hpp"
@@ -31,13 +31,6 @@
 namespace rbg {
 
 namespace {
-
-struct cuda_error_rb : std::runtime_error { using std::runtime_error::runtime_error; };
-#define CUR(call)                                                                                              \
-    do {                                                                                                       \
-        cudaError_t e_ = (call);                                                                               \
-        if (e_ != cudaSuccess) throw cuda_error_rb(std::string(#call) + ": " + cudaGetErrorString(e_));        \
-    } while (0)
 
 constexpr int kThreads = 256;
 constexpr int kVecPerThread = 8;                                   // 16-byte vectors per thread
@@ -161,27 +154,13 @@ __global__ void widen_kernel(const uint32_t* __restrict__ in, uint64_t* __restri
     if (i < n) out[i] = in[i];
 }
 
+// Room for n items of T, growing by at least half of what `b` holds.
 template <class T>
-struct DevBuf {
-    T* p = nullptr;
-    size_t cap = 0;
-    ~DevBuf() { if (p) cudaFree(p); }
-    void reserve(size_t n) {
-        if (n <= cap) return;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = std::max(n, cap + cap / 2);
-        CUR(cudaMalloc(&p, cap * sizeof(T)));
-    }
-};
-
-struct Pinned {
-    uint8_t* p = nullptr;
-    explicit Pinned(size_t n) { CUR(cudaHostAlloc(&p, n, cudaHostAllocDefault)); }
-    ~Pinned() { if (p) cudaFreeHost(p); }
-};
-
-double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+T* grow(DevBuf& b, size_t n) {
+    const size_t held = b.cap / sizeof(T);
+    b.reserve(n * sizeof(T), std::max(n, held + held / 2) * sizeof(T));
+    return b.as<T>();
+}
 
 std::vector<uint64_t> read_u64_file(const std::string& path) {
     FILE* f = fopen(path.c_str(), "rb");
@@ -201,30 +180,26 @@ std::vector<uint64_t> read_u64_file(const std::string& path) {
 RunsBwt rle_bwt_gpu(const std::string& path, int device, RawBuildStats* st) {
     FILE* f = fopen(path.c_str(), "rb");
     if (!f) throw io_error("bad file: " + path);
-    CUR(cudaSetDevice(device));
+    CU(cudaSetDevice(device));
     const size_t chunk = (size_t) 64 << 20;
-    Pinned hb[2] = {Pinned(chunk + 16), Pinned(chunk + 16)};
-    DevBuf<uint8_t> d_bytes[2];
-    d_bytes[0].reserve(chunk + 16);
-    d_bytes[1].reserve(chunk + 16);
+    PinnedBuf hb_mem[2] = {PinnedBuf(chunk + 16), PinnedBuf(chunk + 16)};
+    uint8_t* hb[2] = {hb_mem[0].as<uint8_t>(), hb_mem[1].as<uint8_t>()};
+    DevBuf d_bytes_mem[2], d_cnt_mem, d_cnt64_mem, d_off_mem, d_space_mem, d_tmp_mem, d_starts, d_heads;
+    uint8_t* d_bytes[2] = {grow<uint8_t>(d_bytes_mem[0], chunk + 16), grow<uint8_t>(d_bytes_mem[1], chunk + 16)};
     const uint32_t max_tiles = (uint32_t) ((chunk + kTileBytes - 1) / kTileBytes);
-    DevBuf<uint32_t> d_cnt;
-    DevBuf<uint64_t> d_cnt64, d_off, d_starts;
-    DevBuf<uint8_t> d_heads, d_tmp;
-    DevBuf<unsigned long long> d_space;
-    d_cnt.reserve(max_tiles);
-    d_cnt64.reserve(max_tiles + 1);
-    d_off.reserve(max_tiles + 1);
-    d_space.reserve(1);
+    uint32_t* d_cnt = grow<uint32_t>(d_cnt_mem, max_tiles);
+    uint64_t* d_cnt64 = grow<uint64_t>(d_cnt64_mem, max_tiles + 1);
+    uint64_t* d_off = grow<uint64_t>(d_off_mem, max_tiles + 1);
+    unsigned long long* d_space = grow<unsigned long long>(d_space_mem, 1);
     size_t tmp_bytes = 0;
-    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt64.p, d_off.p, max_tiles + 1);
-    d_tmp.reserve(tmp_bytes);
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, d_cnt64, d_off, max_tiles + 1);
+    uint8_t* d_tmp = grow<uint8_t>(d_tmp_mem, tmp_bytes);
     cudaStream_t s;
-    CUR(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-    CUR(cudaMemsetAsync(d_space.p, 0, 8, s));
+    CU(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    CU(cudaMemsetAsync(d_space, 0, 8, s));
     cudaEvent_t e0, e1;
-    CUR(cudaEventCreate(&e0));
-    CUR(cudaEventCreate(&e1));
+    CU(cudaEventCreate(&e0));
+    CU(cudaEventCreate(&e1));
 
     RunsBwt out;
     std::vector<uint64_t> starts;
@@ -233,51 +208,51 @@ RunsBwt rle_bwt_gpu(const std::string& path, int device, RawBuildStats* st) {
     uint64_t row0 = 0;
     uint32_t carry = 0x100;
     int cur = 0;
-    double t0 = now_s();
-    size_t got = fread(hb[0].p, 1, chunk, f);
-    t_read += now_s() - t0;
+    double t0 = wall_s();
+    size_t got = fread(hb[0], 1, chunk, f);
+    t_read += wall_s() - t0;
     std::vector<uint64_t> h_starts;
     std::vector<uint8_t> h_heads;
     while (got) {
         const uint64_t n_vec = (got + 15) / 16;
-        memset(hb[cur].p + got, hb[cur].p[got - 1], n_vec * 16 - got);           // pad: no new run starts
+        memset(hb[cur] + got, hb[cur][got - 1], n_vec * 16 - got);           // pad: no new run starts
         const uint32_t tiles = (uint32_t) ((n_vec * 16 + kTileBytes - 1) / kTileBytes);
-        CUR(cudaMemcpyAsync(d_bytes[cur].p, hb[cur].p, n_vec * 16, cudaMemcpyHostToDevice, s));
-        CUR(cudaEventRecord(e0, s));
-        rle_kernel<false><<<tiles, kThreads, 0, s>>>((const uint4*) d_bytes[cur].p, n_vec, carry, row0, d_cnt.p, nullptr, nullptr,
-                                                     nullptr, d_space.p);
-        widen_kernel<<<(tiles + 1 + 255) / 256, 256, 0, s>>>(d_cnt.p, d_cnt64.p, tiles);
-        cub::DeviceScan::ExclusiveSum(d_tmp.p, tmp_bytes, d_cnt64.p, d_off.p, tiles + 1, s);
+        CU(cudaMemcpyAsync(d_bytes[cur], hb[cur], n_vec * 16, cudaMemcpyHostToDevice, s));
+        CU(cudaEventRecord(e0, s));
+        rle_kernel<false><<<tiles, kThreads, 0, s>>>((const uint4*) d_bytes[cur], n_vec, carry, row0, d_cnt, nullptr, nullptr,
+                                                     nullptr, d_space);
+        widen_kernel<<<(tiles + 1 + 255) / 256, 256, 0, s>>>(d_cnt, d_cnt64, tiles);
+        cub::DeviceScan::ExclusiveSum(d_tmp, tmp_bytes, d_cnt64, d_off, tiles + 1, s);
         uint64_t n_runs = 0;
-        CUR(cudaMemcpyAsync(&n_runs, d_off.p + tiles, 8, cudaMemcpyDeviceToHost, s));
+        CU(cudaMemcpyAsync(&n_runs, d_off + tiles, 8, cudaMemcpyDeviceToHost, s));
         // overlap: read the next chunk while the GPU counts
-        t0 = now_s();
-        const size_t got_next = fread(hb[cur ^ 1].p, 1, chunk, f);
-        t_read += now_s() - t0;
-        t0 = now_s();
-        CUR(cudaStreamSynchronize(s));
-        t_gpu_wait += now_s() - t0;
-        d_starts.reserve(n_runs + 1);
-        d_heads.reserve(n_runs + 1);
-        rle_kernel<true><<<tiles, kThreads, 0, s>>>((const uint4*) d_bytes[cur].p, n_vec, carry, row0, nullptr, d_off.p, d_starts.p,
-                                                    d_heads.p, nullptr);
-        CUR(cudaEventRecord(e1, s));
+        t0 = wall_s();
+        const size_t got_next = fread(hb[cur ^ 1], 1, chunk, f);
+        t_read += wall_s() - t0;
+        t0 = wall_s();
+        CU(cudaStreamSynchronize(s));
+        t_gpu_wait += wall_s() - t0;
+        uint64_t* d_starts_p = grow<uint64_t>(d_starts, n_runs + 1);
+        uint8_t* d_heads_p = grow<uint8_t>(d_heads, n_runs + 1);
+        rle_kernel<true><<<tiles, kThreads, 0, s>>>((const uint4*) d_bytes[cur], n_vec, carry, row0, nullptr, d_off, d_starts_p,
+                                                    d_heads_p, nullptr);
+        CU(cudaEventRecord(e1, s));
         h_starts.resize(n_runs);
         h_heads.resize(n_runs);
         if (n_runs) {
-            CUR(cudaMemcpyAsync(h_starts.data(), d_starts.p, n_runs * 8, cudaMemcpyDeviceToHost, s));
-            CUR(cudaMemcpyAsync(h_heads.data(), d_heads.p, n_runs, cudaMemcpyDeviceToHost, s));
+            CU(cudaMemcpyAsync(h_starts.data(), d_starts_p, n_runs * 8, cudaMemcpyDeviceToHost, s));
+            CU(cudaMemcpyAsync(h_heads.data(), d_heads_p, n_runs, cudaMemcpyDeviceToHost, s));
         }
-        t0 = now_s();
-        CUR(cudaStreamSynchronize(s));
-        t_gpu_wait += now_s() - t0;
-        CUR(cudaGetLastError());
+        t0 = wall_s();
+        CU(cudaStreamSynchronize(s));
+        t_gpu_wait += wall_s() - t0;
+        CU(cudaGetLastError());
         float ms = 0;
         cudaEventElapsedTime(&ms, e0, e1);
         ms_kernels += ms;
         starts.insert(starts.end(), h_starts.begin(), h_starts.end());
         out.heads.insert(out.heads.end(), h_heads.begin(), h_heads.end());
-        const uint8_t last = hb[cur].p[got - 1];
+        const uint8_t last = hb[cur][got - 1];
         carry = last > 1 ? last : 1;
         row0 += got;
         cur ^= 1;
@@ -285,7 +260,7 @@ RunsBwt rle_bwt_gpu(const std::string& path, int device, RawBuildStats* st) {
     }
     fclose(f);
     unsigned long long n_space = 0;
-    CUR(cudaMemcpy(&n_space, d_space.p, 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&n_space, d_space, 8, cudaMemcpyDeviceToHost));
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     cudaStreamDestroy(s);
@@ -326,21 +301,20 @@ ToeholdArrays toehold_from_raw(const std::string& ssa_path, const std::string& e
         t.samples_last[i] = z ? z - 1 : n - 1;                        // :152
         if (keys[i] >= n || t.samples_last[i] >= n) throw format_error("suffix-array sample beyond the text length");
     }
-    CUR(cudaSetDevice(device));
-    DevBuf<uint64_t> k_in, k_out, v_in, v_out;
-    DevBuf<uint8_t> tmp;
-    k_in.reserve(r); k_out.reserve(r); v_in.reserve(r); v_out.reserve(r);
-    CUR(cudaMemcpy(k_in.p, keys.data(), r * 8, cudaMemcpyHostToDevice));
-    CUR(cudaMemcpy(v_in.p, vals.data(), r * 8, cudaMemcpyHostToDevice));
+    CU(cudaSetDevice(device));
+    DevBuf k_mem[2], v_mem[2], tmp_mem;
+    uint64_t *k_in = grow<uint64_t>(k_mem[0], r), *k_out = grow<uint64_t>(k_mem[1], r);
+    uint64_t *v_in = grow<uint64_t>(v_mem[0], r), *v_out = grow<uint64_t>(v_mem[1], r);
+    CU(cudaMemcpy(k_in, keys.data(), r * 8, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(v_in, vals.data(), r * 8, cudaMemcpyHostToDevice));
     size_t tb = 0;
     const int end_bit = 64 - __builtin_clzll(n | 1);
-    cub::DeviceRadixSort::SortPairs(nullptr, tb, k_in.p, k_out.p, v_in.p, v_out.p, (int64_t) r, 0, end_bit);
-    tmp.reserve(tb);
-    cub::DeviceRadixSort::SortPairs(tmp.p, tb, k_in.p, k_out.p, v_in.p, v_out.p, (int64_t) r, 0, end_bit);
+    cub::DeviceRadixSort::SortPairs(nullptr, tb, k_in, k_out, v_in, v_out, (int64_t) r, 0, end_bit);
+    cub::DeviceRadixSort::SortPairs(grow<uint8_t>(tmp_mem, tb), tb, k_in, k_out, v_in, v_out, (int64_t) r, 0, end_bit);
     t.pred_to_run.resize(r);
-    CUR(cudaMemcpy(keys.data(), k_out.p, r * 8, cudaMemcpyDeviceToHost));
-    CUR(cudaMemcpy(t.pred_to_run.data(), v_out.p, r * 8, cudaMemcpyDeviceToHost));
-    CUR(cudaGetLastError());
+    CU(cudaMemcpy(keys.data(), k_out, r * 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(t.pred_to_run.data(), v_out, r * 8, cudaMemcpyDeviceToHost));
+    CU(cudaGetLastError());
     keys.erase(std::unique(keys.begin(), keys.end()), keys.end());   // pred_ is a bit vector: duplicates collapse
     t.pred = std::move(keys);
     return t;

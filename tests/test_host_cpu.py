@@ -12,6 +12,7 @@ import pytest
 
 from conftest import GOLDEN, ROOT, read_fastx
 from oracle import oracle as O
+from tools import synth
 
 import rowbowt_b200 as rb
 
@@ -82,10 +83,23 @@ def test_layout_selftest_rejects_missing_file():
 
 
 @pytest.mark.skipif(rb.lib().rbg_device_count() > 0, reason="a GPU is present")
-def test_fails_loudly_without_gpu():
+def test_fails_loudly_without_gpu(tmp_path):
     with pytest.raises(rb.RbgError) as e:
         rb.GpuIndex.open(os.path.join(GOLDEN, "toy", "small.fa"))
     assert e.value.code == -4 and "no CPU fallback" in str(e.value)
+    raw = os.path.join(GOLDEN, "raw", "tiny")
+    for call in (lambda: rb.GpuIndex.open_raw(raw, sa=True, markers=True),
+                 lambda: rb.build_index(raw, str(tmp_path / "built"), sa=True, markers=True),
+                 lambda: rb.GpuIndex.from_arrays(100, [ord("A"), ord("C")], [50, 50])):
+        with pytest.raises(rb.RbgError) as e:
+            call()
+        assert e.value.code == -4 and "no CPU fallback" in str(e.value)
+    mps = str(tmp_path / "tiny.mps")
+    synth.write_mps(synth.make_panel(*synth.CONFIGS["tiny"]), mps)
+    with pytest.raises(rb.RbgError) as e:                                     # the raw-input branch
+        rb.build_marker_array(raw, mps, str(tmp_path / "o.ma"))
+    assert e.value.code == -4 and "no CPU fallback" in str(e.value)
+    assert not os.path.exists(str(tmp_path / "built.rbwt")) and not os.path.exists(str(tmp_path / "o.ma"))
     p = subprocess.run([RB_ALIGN, os.path.join(GOLDEN, "toy", "small.fa"), os.path.join(GOLDEN, "toy", "simple_query.fq")],
                        capture_output=True, text=True)
     assert p.returncode == 1 and p.stdout == "" and "no CUDA device" in p.stderr
