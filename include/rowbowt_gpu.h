@@ -147,6 +147,8 @@ typedef struct {
     uint32_t phi_shift;             /* GPU layout: one 32-byte phi slot per 2^phi_shift text positions */
     uint32_t from_cache;            /* 1: this handle was opened from <prefix>.rbgcache (RBG_LOAD_CACHE) */
     uint64_t phi_overflow;          /* slots whose bucket holds more than 3 samples (side array, binary search) */
+    uint64_t pair_bytes;            /* pair directory (two bases per LF step in the count search); 0 = not built, see RBG_PAIR */
+    uint32_t pair_window;           /* its BWT positions per line */
 } rbg_info;
 
 typedef struct {

@@ -69,7 +69,7 @@ class Info(C.Structure):
                 ("phi_bytes", C.c_uint64), ("toehold_bytes", C.c_uint64), ("marker_bytes", C.c_uint64),
                 ("ftab_k", C.c_uint32), ("layout", C.c_uint32), ("ftab_bytes", C.c_uint64), ("hot_bytes", C.c_uint64),
                 ("l2_pinned_bytes", C.c_uint64), ("phi_shift", C.c_uint32), ("from_cache", C.c_uint32),
-                ("phi_overflow", C.c_uint64)]
+                ("phi_overflow", C.c_uint64), ("pair_bytes", C.c_uint64), ("pair_window", C.c_uint32)]
 
 
 class BuildStats(C.Structure):
@@ -153,6 +153,7 @@ def lib():
         L.rbg_selftest_phi.argtypes = [C.c_char_p, C.c_uint32, C.c_uint64, u64p, u64p, u64p]
         L.rbg_selftest_rewrite.argtypes = [C.c_char_p, C.c_char_p, C.c_uint32]
         L.rbg_selftest_toehold.argtypes = [C.c_char_p, C.c_uint32, u64p, u64p]
+        L.rbg_selftest_pair.argtypes = [C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_void_p, u64p, u64p, u64p]
         L.rbg_selftest_pack.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p,
                                         C.c_void_p, u64p]
         _lib = L

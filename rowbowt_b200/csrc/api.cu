@@ -179,6 +179,8 @@ struct rbg_index {
     int device = 0;
     std::vector<Upload> owned;
     DevLeafDir dir{};
+    DevPairDir pair{};                   // lines == nullptr: the count search takes one base per step
+    std::vector<Upload> pair_owned;      // kept out of `owned`: a layout cache does not carry the pair directory
     DevToehold toe{};
     DevPhi phi{};
     DevMarkers mk{};
@@ -531,7 +533,45 @@ std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t fl
     CU(cudaDeviceSynchronize());
     rebuild_hot_region(ix.get(), 0, false);                    // superblock counts into the hot region, no seed table yet
     ix->info.from_cache = 1;
+    ix->info.pair_bytes = 0;                                   // not rebuilt from a cache: the count search steps base by base
+    ix->info.pair_window = 0;
     return ix;
+}
+
+// The pair directory, when the count search gains from it: a layout-5 index with n < 2^32 whose pair directory stays
+// within kPairBudget -- small enough to stay resident in L2 beside the single-base directory, where the search is bound by
+// instructions and two bases per step take fewer of them than two steps -- and whose superblock table fits shared memory.
+// Larger indexes are bound by their line gathers, which the pair directory would only multiply.  RBG_PAIR=0|1 (tests)
+// forces either form; 1 still needs layout 5, n < 2^32 and the shared-memory table.
+constexpr uint64_t kPairBudget = 64ull << 20;
+void build_pair(rbg_index* ix, const RunsBwt& bwt, const LeafDir& ld) {
+    const char* e = getenv("RBG_PAIR");
+    const int force = e && *e ? atoi(e) : -1;
+    if (force == 0 || ld.version != 5 || (bwt.n >> 32)) return;
+    // a line holds at most 12 runs of P, and P has at least as many runs as the BWT: skip what cannot fit without building it
+    if (force != 1 && bwt.R * 64 / LeafFmt<6>::E > kPairBudget) return;
+    PairDir pd = build_pair_dir(bwt, ld);
+    if (64 * pd.n_super > kPairMaxShared || (force != 1 && pd.bytes() > kPairBudget)) return;
+    size_t acc = 0;
+    DevPairDir& P = ix->pair;
+    P.lines = upload(pd.lines, ix->pair_owned, &acc);
+    P.super = upload(pd.super, ix->pair_owned, &acc);
+    P.n_super = (uint32_t) pd.n_super;
+    P.window = pd.window;
+    P.sb_shift = pd.sb_shift;
+    DevLeafDir div{};
+    div.window = pd.window;
+    div.n = pd.n;
+    set_fast_div(div);
+    if (!div.div_fast) throw std::logic_error("pair directory: no 32-bit division");
+    P.div_k = div.div_k;
+    P.div_mul = div.div_mul;
+    P.div_s = div.div_s;
+    P.n_child = (pd.window + kPairRawSymbols - 1) / kPairRawSymbols;
+    P.n_bad = pd.n_bad;
+    for (int t = 0; t < kPairMaxBad; ++t) P.bad_pos[t] = pd.bad_pos[t];
+    ix->info.pair_bytes = acc;
+    ix->info.pair_window = pd.window;
 }
 
 std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerArrays* ma, int device) {
@@ -572,6 +612,7 @@ std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArr
         set_fast_div(ix->dir);
         for (int t = 0; t < kMaxTerm; ++t) ix->dir.term_pos[t] = ld.term_pos[t];
         memcpy(ix->codes.code_of, ld.code_of, 256);
+        build_pair(ix.get(), bwt, ld);
     }
     memcpy(info.F, F, sizeof info.F);
 
@@ -816,7 +857,7 @@ void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mo
         launches += launch_pack(b, ix->codes, rd->n_bytes, st);
     }
     CU(cudaEventRecord(L.ev[1], st));
-    launches += launch_search(ix->dir, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[0], st);
+    launches += launch_search(ix->dir, ix->pair, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[0], st);
     if (rd->has_bases) launches += launch_search_bytes(ix->dir, locate ? &ix->toe : nullptr, b, r, ix->codes, L.d_ctr, st);
     CU(cudaEventRecord(L.ev[2], st));
     rd->n_locs = rd->n_markers = 0;
@@ -1060,7 +1101,7 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
             CU(cudaEventRecord(L.ev_pack[c], ss));
             if (stall_ns[1] && (c & 1)) launch_stall(stall_ns[1], ss);
         }
-        launches += launch_search(ix->dir, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[c], ss);
+        launches += launch_search(ix->dir, ix->pair, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[c], ss);
         if (rd->has_bases) launches += launch_search_bytes(ix->dir, locate ? &ix->toe : nullptr, b, r, ix->codes, L.d_ctr, ss);
         if (narrow_rg) launches += launch_narrow_ranges(r.lo, r.hi, rd->lo32.as<uint32_t>(), rd->hi32.as<uint32_t>(), r0, r1, ss);
         CU(cudaEventRecord(L.ev_cmp[c], ss));

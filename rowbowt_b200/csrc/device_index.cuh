@@ -10,6 +10,7 @@ namespace rbg {
 
 constexpr int kDevMaxTerm = 8;
 constexpr int kMaxSuper5Dev = 256;      // == kMaxSuper5 (layout.hpp): layout 5 keeps at most 4 x 256 superblock bases
+constexpr uint64_t kPairMaxShared = 48 << 10;   // the pair superblock table search_kernel holds in shared memory (16 x 4 x n_super bytes)
 
 // The rank directory (LeafDir, layout.hpp): the line of BWT position p is p >> g.
 struct DevLeafDir {
@@ -46,6 +47,19 @@ inline void set_fast_div(DevLeafDir& D) {
     D.div_s = 31 + l;
     D.div_fast = 1;
 }
+
+// The pair directory (PairDir, layout.hpp; lines: leaf.cuh LeafFmt<6>), n < 2^32.  lines == nullptr: not built.
+struct DevPairDir {
+    const uint32_t* lines;
+    const uint32_t* super;      // [16][n_super]: K[p] + #p in P[0, superblock_start), copied to shared memory per CTA
+    uint32_t n_super;
+    uint32_t window;            // even, so i / window == ((i >> div_k) * div_mul) >> div_s for every i < 2^32 (set_fast_div)
+    uint32_t sb_shift;
+    uint32_t div_k, div_mul, div_s;
+    uint32_t n_child;           // RAW children of a CLUSTER window: ceil(window / 128)
+    uint32_t n_bad;
+    uint32_t bad_pos[kPairMaxBad];
+};
 
 // ToeholdDir (layout.hpp): bucket table over the rows that are LF images of run ends, keys reduced to their low
 // `shift` bits, samples as a u32 plane (+ a u8 plane when n > 2^32).
@@ -311,6 +325,86 @@ __device__ __forceinline__ bool lf_step_lines(const DevLeafDir& D, const uint64_
     if (!act || new_end == new_lo) return false;
     lo = new_lo;
     hi = new_end - 1;
+    return true;
+}
+
+// ---- two bases per LF step (count search on the pair directory) ----------------------------------
+// For a read ...c1 c2 (c2 consumed first) and p = 4 c1 + c2:
+//   LF(c1, LF(c2, lo)) = F[c1] + rank_c1(F[c2] + rank_c2(lo))
+//                      = F[c1] + rank_c1(F[c2]) + #{i in [F[c2], F[c2] + rank_c2(lo)) : BWT[i] = c1}
+//                      = K[p] + #{j < lo : BWT[j] = c2, BWT[LF(j)] = c1} = K[p] + rank_p(lo) over P
+// because LF maps the c2-rows below lo, in order, onto the first rank_c2(lo) rows of block c2.  The same holds for hi + 1,
+// and the range is empty after both steps exactly when this one is empty.
+
+// A whole warp answers the ranks that fall in CLUSTER windows, one lane's position at a time: lanes 0..31 load the (at most
+// 32) words of the window's RAW children, count code p before q in their word, REDUX adds them up.
+__device__ __forceinline__ void coop_pair_raw(const DevPairDir& P, const uint32_t (&w)[16], uint32_t p, uint32_t q, bool in, uint32_t& r) {
+    uint32_t need = __ballot_sync(0xFFFFFFFFu, in);
+    if (!need) return;                                             // warp-uniform
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t child = in ? pair_child_ptr(w) : 0u, qp = q | (p << 16);
+    do {
+        const int src = __ffs(need) - 1;
+        need &= need - 1u;
+        const uint32_t sc = __shfl_sync(0xFFFFFFFFu, child, src), sqp = __shfl_sync(0xFFFFFFFFu, qp, src);
+        const uint32_t word = lane < 16u * P.n_child ? __ldg(P.lines + (uint64_t) sc * 16 + lane) : 0u;
+        const uint32_t cnt = pair_raw_word_count(word, pair_pat(sqp >> 16), 8 * (int) lane, (int) (sqp & 0xFFFFu));
+        const uint32_t total = __reduce_add_sync(0xFFFFFFFFu, cnt);
+        if ((int) lane == src) r = total;
+    } while (need);
+}
+
+// TERM window, code 0: the rows stored as code 0 for a pair with the terminator, in [pos_end - q, pos_end)
+__device__ __forceinline__ void pair_term_fix(const DevPairDir& P, const uint32_t (&w)[16], uint32_t pos_end, uint32_t q, uint32_t& r) {
+    if (!(w[15] & kFlagTerm)) return;
+    const uint32_t from = pos_end - q;
+#pragma unroll
+    for (uint32_t t = 0; t < (uint32_t) kPairMaxBad; ++t)
+        r -= (t < P.n_bad && P.bad_pos[t] >= from && P.bad_pos[t] < pos_end) ? 1u : 0u;
+}
+
+__device__ __forceinline__ uint32_t pair_line_of(const DevPairDir& P, uint32_t i) {
+    return (uint32_t) (((uint64_t) (i >> P.div_k) * P.div_mul) >> P.div_s);
+}
+
+// Two LF steps (code p = 4 c1 + c2) for a whole warp; `sup` is the pair superblock table in shared memory.  Every lane calls;
+// an inactive lane reads line 0 and keeps its range.  Returns false when the range after both steps is empty.
+__device__ __forceinline__ bool lf_pair_warp(const DevPairDir& P, const uint32_t* sup, uint32_t p, uint64_t& lo, uint64_t& hi, bool act,
+                                             uint32_t& lines_touched) {
+    uint32_t A[16], B[16];
+    const uint32_t l = act ? (uint32_t) lo : 0u, h = act ? (uint32_t) hi : 0u;
+    const uint32_t wa = pair_line_of(P, l), wb = pair_line_of(P, h);
+    const uint32_t qa = l - wa * P.window, qb = h - wb * P.window + 1u;
+    load_line(P.lines + (uint64_t) wa * 16, A);
+    const uint32_t* sp = sup + p * P.n_super;
+    const uint32_t base_a = sp[wa >> P.sb_shift];
+    uint32_t base_b = base_a;
+    if (wb == wa) {
+#pragma unroll
+        for (int i = 0; i < 16; ++i) B[i] = A[i];
+        lines_touched += act ? 1u : 0u;
+    } else {
+        load_line(P.lines + (uint64_t) wb * 16, B);
+        base_b = sp[wb >> P.sb_shift];
+        lines_touched += 2;
+    }
+    const uint32_t ppat = pair_pat(p);
+    uint32_t ra = pair_rank(A, ppat, qa);
+    uint32_t rb = pair_rank(B, ppat, qb);
+    const uint32_t rel_a = pair_rel_count(A, p), rel_b = pair_rel_count(B, p);
+    const uint32_t fl = act ? (A[15] | B[15]) & kFlagAny : 0u;
+    if (__any_sync(0xFFFFFFFFu, fl != 0u)) {                       // warp-uniform: some lane sees a CLUSTER / TERM window
+        coop_pair_raw(P, A, p, qa, fl && (A[15] & kFlagCluster), ra);
+        coop_pair_raw(P, B, p, qb, fl && (B[15] & kFlagCluster), rb);
+        if ((fl & kFlagTerm) && p == 0) {
+            pair_term_fix(P, A, l, qa, ra);
+            pair_term_fix(P, B, h + 1u, qb, rb);
+        }
+    }
+    const uint32_t new_lo = base_a + rel_a + ra, new_end = base_b + rel_b + rb;
+    if (!act || new_end == new_lo) return false;
+    lo = new_lo;
+    hi = new_end - 1u;
     return true;
 }
 

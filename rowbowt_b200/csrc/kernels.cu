@@ -10,6 +10,7 @@
 #include "kernels.cuh"
 
 #include <cstdlib>
+#include <stdexcept>
 
 #include <cub/device/device_scan.cuh>
 
@@ -160,13 +161,20 @@ struct ToeholdTrack {
 // whole warp (device_index.cuh).
 // Layout 5 (V == 5): the superblock bases (<= 4 x 256 u64) are copied to shared memory once per CTA, so an LF step
 // issues no load besides its one or two directory lines.
-template <bool TOEHOLD, int V>
-__global__ void __launch_bounds__(kBlock, kSearchCtas) search_kernel(DevLeafDir D, DevToehold T, DevFtab ft, DevBatch b, DevResult r,
-                                                                     DevCounters* ctr, unsigned long long* cursor) {
+// PAIR (count search only): two bases per step from the pair directory (lf_pair_warp), whose superblock table (16 x n_super
+// u32, <= kPairMaxShared bytes) is the kernel's dynamic shared memory.  A lane whose read has an odd number of bases left
+// first takes one step on the single-base directory, which then reads its superblock bases from global memory.
+template <bool TOEHOLD, int V, bool PAIR>
+__global__ void __launch_bounds__(kBlock, kSearchCtas) search_kernel(DevLeafDir D, DevPairDir PD, DevToehold T, DevFtab ft, DevBatch b,
+                                                                     DevResult r, DevCounters* ctr, unsigned long long* cursor) {
     constexpr uint32_t kFull = 0xFFFFFFFFu;
-    __shared__ uint64_t s_base[V == 5 ? 4 * kMaxSuper5Dev : 1];
+    __shared__ uint64_t s_base[V == 5 && !PAIR ? 4 * kMaxSuper5Dev : 1];
+    extern __shared__ uint32_t s_pair[];
     const uint64_t* sup = D.super;
-    if (V == 5) {
+    if (PAIR) {
+        for (uint32_t i = threadIdx.x; i < 16u * PD.n_super; i += blockDim.x) s_pair[i] = __ldg(PD.super + i);
+        __syncthreads();
+    } else if (V == 5) {
         for (uint32_t i = threadIdx.x; i < 4u * (uint32_t) D.n_super; i += blockDim.x) s_base[i] = __ldg(D.super + i);
         __syncthreads();
         sup = s_base;
@@ -229,23 +237,54 @@ __global__ void __launch_bounds__(kBlock, kSearchCtas) search_kernel(DevLeafDir 
         }
         // one LF step for every lane with bases left; an empty range has left == 0
         const bool act = have && left != 0u;
-        uint32_t c = 0;
-        if (act) {
-            --x;
-            if ((x & 31) == 31) word = __ldg(b.packed + (x >> 5));
-            c = (uint32_t) (word >> (2 * (x & 31))) & 3u;
-        }
-        bool hi_is_c;
-        const bool ok = lf_step_warp<TOEHOLD, V>(D, sup, c, lo, hi, act, hi_is_c, lines);
-        if (act) {
-            --left;
-            ++steps;                                        // the failing step is counted, the rest of the read is not searched
-            if (!ok) {
+        const bool single = PAIR ? act && (left & 1u) : act;
+        if (!PAIR || __any_sync(kFull, single)) {
+            uint32_t c = 0;
+            if (single) {
+                --x;
+                if ((x & 31) == 31) word = __ldg(b.packed + (x >> 5));
+                c = (uint32_t) (word >> (2 * (x & 31))) & 3u;
+            }
+            bool hi_is_c;
+            const bool ok = lf_step_warp<TOEHOLD, V>(D, sup, c, lo, hi, single, hi_is_c, lines);
+            if (single) {
+                --left;
+                ++steps;                                    // the failing step is counted, the rest of the read is not searched
+                if (!ok) {
+                    left = 0;
+                    lo = 1;
+                    hi = 0;
+                } else if (TOEHOLD) {
+                    tt.step(hi_is_c, hi);
+                }
+            }
+        } else {
+            uint32_t c1 = 0, c2 = 0;
+            if (act) {
+                --x;
+                if ((x & 31) == 31) word = __ldg(b.packed + (x >> 5));
+                c2 = (uint32_t) (word >> (2 * (x & 31))) & 3u;
+                --x;
+                if ((x & 31) == 31) word = __ldg(b.packed + (x >> 5));
+                c1 = (uint32_t) (word >> (2 * (x & 31))) & 3u;
+            }
+            const bool ok = lf_pair_warp(PD, s_pair, 4u * c1 + c2, lo, hi, act, lines);     // leaves lo, hi as they were when it fails
+            const bool failed = act && !ok;
+            if (act) {
+                left -= 2;
+                steps += 2;
+            }
+            if (__any_sync(kFull, failed)) {
+                // lf_steps counts the step that emptied the range and none after it: when the range was already empty after
+                // c2 that is one step, not two (statistics only: the result is (1,0) either way)
+                bool unused;
+                const bool ok2 = lf_step_warp<false, V>(D, sup, c2, lo, hi, failed, unused, lines);
+                if (failed && !ok2) --steps;
+            }
+            if (failed) {
                 left = 0;
                 lo = 1;
                 hi = 0;
-            } else if (TOEHOLD) {
-                tt.step(hi_is_c, hi);
             }
         }
         if (have && left == 0u) {                           // finished: report and free the lane
@@ -550,18 +589,21 @@ int launch_pack(const DevBatch& b, const CodeTable& ct, uint64_t approx_bytes, c
     return 1;
 }
 
-int launch_search(const DevLeafDir& D, const DevToehold* T, const DevFtab& ft, const DevBatch& b, const DevResult& r,
+int launch_search(const DevLeafDir& D, const DevPairDir& PD, const DevToehold* T, const DevFtab& ft, const DevBatch& b, const DevResult& r,
                   DevCounters* ctr, unsigned long long* cursor, cudaStream_t st) {
     if (b.r1 <= b.r0) return 0;
     DevToehold t0{};
     // reads are handed out by the device cursor, so ONE wave of CTAs is the whole grid: resident CTAs per SM x SMs.
     const int grid = grid_for(b.r1 - b.r0, kBlock, kSearchCtas);
-    if (D.version == 5) {
-        if (T) search_kernel<true, 5><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-        else search_kernel<false, 5><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
+    if (!T && PD.lines) {                                   // the pair directory is built only over a layout-5 directory
+        if (D.version != 5 || 64ull * PD.n_super > kPairMaxShared) throw std::logic_error("pair directory without its layout");
+        search_kernel<false, 5, true><<<grid, kBlock, 64 * PD.n_super, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
+    } else if (D.version == 5) {
+        if (T) search_kernel<true, 5, false><<<grid, kBlock, 0, st>>>(D, PD, *T, ft, b, r, ctr, cursor);
+        else search_kernel<false, 5, false><<<grid, kBlock, 0, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
     } else {
-        if (T) search_kernel<true, 4><<<grid, kBlock, 0, st>>>(D, *T, ft, b, r, ctr, cursor);
-        else search_kernel<false, 4><<<grid, kBlock, 0, st>>>(D, t0, ft, b, r, ctr, cursor);
+        if (T) search_kernel<true, 4, false><<<grid, kBlock, 0, st>>>(D, PD, *T, ft, b, r, ctr, cursor);
+        else search_kernel<false, 4, false><<<grid, kBlock, 0, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
     }
     return 1;
 }

@@ -49,8 +49,8 @@ struct DevResult {
 int grid_for(uint64_t work_items, int block, int per_sm);
 
 int launch_pack(const DevBatch& b, const CodeTable& ct, uint64_t approx_bytes, cudaStream_t st);   // reads [b.r0, b.r1)
-int launch_search(const DevLeafDir& D, const DevToehold* T, const DevFtab& ft, const DevBatch& b, const DevResult& r,
-                  DevCounters* ctr, unsigned long long* cursor, cudaStream_t st);     // T == nullptr -> count only; ft.k == 0 -> no seed table; cursor: zeroed device counter of this launch; returns #launches
+int launch_search(const DevLeafDir& D, const DevPairDir& PD, const DevToehold* T, const DevFtab& ft, const DevBatch& b, const DevResult& r,
+                  DevCounters* ctr, unsigned long long* cursor, cudaStream_t st);     // T == nullptr -> count only (on PD when PD.lines is set); ft.k == 0 -> no seed table; cursor: zeroed device counter of this launch; returns #launches
 int launch_ftab_build(const DevLeafDir& D, uint32_t k, bool toehold, ulonglong2* range, uint64_t* toe, cudaStream_t st);
 int launch_search_bytes(const DevLeafDir& D, const DevToehold* T, const DevBatch& b, const DevResult& r,
                         const CodeTable& ct, DevCounters* ctr, cudaStream_t st);   // reads flagged kReadExotic

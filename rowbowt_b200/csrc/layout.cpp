@@ -279,6 +279,171 @@ LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window) {
     return d;
 }
 
+namespace {
+int8_t sym_code(uint8_t h) { return h == 'A' ? 0 : h == 'C' ? 1 : h == 'G' ? 2 : h == 'T' ? 3 : 4; }      // validated by build_leaf_dir
+}  // namespace
+
+void pair_runs(const RunsBwt& bwt, const LeafDir& d, std::vector<uint32_t>& lens, std::vector<uint8_t>& codes) {
+    if (bwt.n >> 32) throw std::runtime_error("pair directory: n >= 2^32");
+    std::vector<uint64_t> start(bwt.R + 1, 0);
+    for (uint64_t k = 0; k < bwt.R; ++k) start[k + 1] = start[k] + bwt.lens[k];
+    lens.clear();
+    codes.clear();
+    lens.reserve(2 * bwt.R);
+    codes.reserve(2 * bwt.R);
+    auto push = [&](uint64_t len, uint8_t code) {
+        if (!codes.empty() && codes.back() == code && code != kPairBad) lens.back() += (uint32_t) len;
+        else { lens.push_back((uint32_t) len); codes.push_back(code); }
+    };
+    uint64_t cum[4] = {0, 0, 0, 0};
+    for (uint64_t k = 0; k < bwt.R; ++k) {
+        const int8_t c = sym_code(bwt.heads[k]);
+        if (c == 4) { push(bwt.lens[k], kPairBad); continue; }
+        // rows [start[k], start[k+1]) map onto [a, a + len): the first symbols of their pairs are BWT[a, a + len)
+        uint64_t a = d.Fcode[c] + cum[c], left = bwt.lens[k];
+        cum[c] += left;
+        uint64_t m = (uint64_t) (std::upper_bound(start.begin(), start.end(), a) - start.begin()) - 1;
+        while (left) {
+            const uint64_t take = std::min(left, start[m + 1] - a);
+            const int8_t c1 = sym_code(bwt.heads[m]);
+            push(take, c1 == 4 ? kPairBad : (uint8_t) (4 * c1 + c));
+            a += take;
+            left -= take;
+            ++m;
+        }
+    }
+}
+
+namespace {
+
+struct PairCount { uint64_t children = 0, clusters = 0, positions = 0; };
+
+// Walks the runs of P window by window (as LeafWalker does for the BWT).  out == nullptr: only counts.
+PairCount pair_walk(const std::vector<uint32_t>& lens, const std::vector<uint8_t>& codes, uint64_t n, uint32_t W,
+                    uint32_t sb_shift, const uint32_t K[16], PairDir* out) {
+    constexpr int E = LeafFmt<6>::E;
+    const uint64_t n_direct = (n + W - 1) / W, n_child = (W + kPairRawSymbols - 1) / kPairRawSymbols;
+    PairCount pc;
+    uint64_t j = 0, jstart = 0, cum[16] = {0}, sb[16] = {0};
+    for (uint64_t t = 0; t < n_direct; ++t) {
+        const uint64_t P = t * W, Pend = std::min(P + W, n);
+        while (jstart + lens[j] <= P) {
+            if (codes[j] < kPairBad) cum[codes[j]] += lens[j];
+            jstart += lens[j];
+            ++j;
+        }
+        uint64_t at[16];
+        for (int p = 0; p < 16; ++p) at[p] = cum[p];
+        if (codes[j] < kPairBad) at[codes[j]] += P - jstart;
+        if ((t & ((1ull << sb_shift) - 1)) == 0) {
+            for (int p = 0; p < 16; ++p) sb[p] = at[p];
+            if (out) for (int p = 0; p < 16; ++p) out->super[(uint64_t) p * out->n_super + (t >> sb_shift)] = (uint32_t) (K[p] + at[p]);
+        }
+        size_t np = 0;
+        bool term = false;
+        for (uint64_t i = j, st = jstart; i < lens.size() && st < Pend; st += lens[i], ++i) { ++np; term |= codes[i] == kPairBad; }
+        const bool cluster = np > (size_t) E;
+        if (cluster) { ++pc.clusters; pc.positions += Pend - P; }
+        if (out) {
+            uint32_t* w = out->lines.data() + t * kLineWords;
+            memset(w, 0, 64);
+            for (int p = 0; p < 16; ++p) {
+                const uint64_t rel = at[p] - sb[p];
+                if (rel > 0xFFFFu) throw std::logic_error("pair line: superblock-relative count exceeds 16 bits");
+                w[p >> 1] |= (uint32_t) rel << (16 * (p & 1));
+            }
+            for (int e = 0; e < E / 2; ++e) w[LeafFmt<6>::S0 + e] = 0xFFFFFFFFu;
+            if (!cluster) {
+                uint64_t st = jstart;
+                for (uint64_t i = j, e = 0; e < np; st += lens[i], ++i, ++e) {
+                    const uint32_t s = (uint32_t) (st > P ? st - P : 0);
+                    uint32_t& sw = w[LeafFmt<6>::S0 + e / 2];
+                    sw = (sw & ~(0xFFFFu << (16 * (e & 1)))) | (s << (16 * (e & 1)));
+                    w[e < 8 ? 14 : 15] |= (uint32_t) (codes[i] & 15u) << pair_head_bit((uint32_t) e);
+                }
+            } else {
+                const uint64_t child0 = n_direct + pc.children;
+                if ((child0 + n_child) >> 32) throw std::runtime_error("pair directory exceeds 2^32 lines");
+                w[LeafFmt<6>::S0] = (uint32_t) child0;
+                uint32_t* cw = out->lines.data() + child0 * kLineWords;
+                memset(cw, 0, 64 * n_child);
+                uint64_t st = jstart;
+                for (uint64_t i = j; i < lens.size() && st < Pend; st += lens[i], ++i)
+                    for (uint64_t r = std::max(st, P); r < std::min(st + lens[i], Pend); ++r)
+                        cw[(r - P) >> 3] |= (uint32_t) (codes[i] & 15u) << (4 * ((r - P) & 7));
+                w[15] |= kFlagCluster;
+            }
+            if (term) w[15] |= kFlagTerm;
+        }
+        if (cluster) pc.children += n_child;
+    }
+    return pc;
+}
+
+uint32_t pair_sb_shift(uint32_t W) {                  // largest s with (2^s - 1) * W <= 65535: the u16 counts of a line
+    uint32_t s = 0;
+    while (((2ull << s) - 1) * W <= 65535ull) ++s;
+    return s;
+}
+
+}  // namespace
+
+PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window) {
+    PairDir P;
+    P.n = bwt.n;
+    std::vector<uint32_t> lens;
+    std::vector<uint8_t> codes;
+    pair_runs(bwt, d, lens, codes);
+    P.n_runs = lens.size();
+    uint64_t pos = 0;
+    for (size_t i = 0; i < lens.size(); ++i) {
+        if (codes[i] == kPairBad)
+            for (uint32_t t = 0; t < lens[i]; ++t) {
+                if (P.n_bad >= (uint32_t) kPairMaxBad) throw std::logic_error("pair directory: more than 16 terminator rows");
+                P.bad_pos[P.n_bad++] = (uint32_t) (pos + t);
+            }
+        pos += lens[i];
+    }
+    // K[4 c1 + c2] = F[c1] + rank_c1(F[c2]): where the rows of c1 that precede block c2 end
+    uint32_t K[16];
+    for (int c2 = 0; c2 < 4; ++c2) {
+        uint64_t before[4] = {0, 0, 0, 0}, at = 0;
+        for (uint64_t k = 0; k < bwt.R && at < d.Fcode[c2]; ++k) {
+            const int8_t c = sym_code(bwt.heads[k]);
+            const uint64_t take = std::min<uint64_t>(bwt.lens[k], d.Fcode[c2] - at);
+            if (c < 4) before[c] += take;
+            at += take;
+        }
+        for (int c1 = 0; c1 < 4; ++c1) K[4 * c1 + c2] = (uint32_t) (d.Fcode[c1] + before[c1]);
+    }
+    uint32_t W = window;
+    if (W == 0) if (const char* e = getenv("RBG_PAIR_WINDOW")) W = (uint32_t) atoi(e);
+    if (W == 0) {
+        // the ladder of build_leaf_dir with E = 12; a rank in a CLUSTER window is answered by the whole warp from its raw
+        // children, so those windows weigh as in the single-base cost model
+        const double target = (17.0 * LeafFmt<6>::E / 24.0) * (double) bwt.n / (double) lens.size();
+        const uint32_t unit = std::max<uint32_t>(2, 1u << (uint32_t) std::max(1.0, std::floor(std::log2(target)) - 3.0));
+        double best = 1e300;
+        for (int k = 0; k < 8; ++k) {
+            const int64_t c64 = ((int64_t) (target / unit) + (k - 3)) * (int64_t) unit;
+            const uint32_t cand = (uint32_t) std::min<int64_t>(kPairMaxWindow, std::max<int64_t>(kMinWindow, c64)) & ~1u;
+            const PairCount c = pair_walk(lens, codes, bwt.n, cand, pair_sb_shift(cand), K, nullptr);
+            const double cost = (double) ((bwt.n + cand - 1) / cand + c.children) * (1.0 + 20.0 * (double) c.positions / (double) bwt.n);
+            if (cost < best) { best = cost; W = cand; }
+        }
+    }
+    if (W < kMinWindow || W > kPairMaxWindow || (W & 1u)) throw std::runtime_error("pair window must be even, in [16,256]");
+    P.window = W;
+    P.sb_shift = pair_sb_shift(W);
+    P.n_direct = (bwt.n + W - 1) / W;
+    P.n_super = (P.n_direct + (1ull << P.sb_shift) - 1) >> P.sb_shift;
+    const PairCount c = pair_walk(lens, codes, bwt.n, W, P.sb_shift, K, nullptr);
+    P.lines.assign((P.n_direct + c.children) * kLineWords, 0);
+    P.super.assign(16 * P.n_super, 0);
+    P.n_cluster = pair_walk(lens, codes, bwt.n, W, P.sb_shift, K, &P).clusters;
+    return P;
+}
+
 ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const ToeholdArrays& tsa) {
     if (tsa.r != bwt.R || tsa.n != bwt.n) throw format_error("toehold SA does not match the BWT (r/n differ)");
     ToeholdDir t;

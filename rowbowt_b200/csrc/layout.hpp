@@ -18,6 +18,7 @@
 #include <vector>
 
 #include "formats.hpp"
+#include "leaf.cuh"
 
 namespace rbg {
 
@@ -51,6 +52,27 @@ struct LeafDir {
 
 // Validates the alphabet and builds the rank directory.  window = 0 -> choose automatically.
 LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window = 0);
+
+// Pair directory (leaf.cuh, LeafFmt<6>): a rank directory over P[j] = (BWT[LF(j)], BWT[j]) with which the count search
+// takes two bases per LF step.  Built from the runs alone: the rows of BWT run k map under LF onto one contiguous interval
+// of rows, and the first symbols of their pairs are the BWT over that interval -- so the runs of P are each run's image
+// interval cut at BWT run boundaries (R2 <= 2R + a few).
+struct PairDir {
+    uint64_t n = 0;
+    uint32_t window = 0;                 // even, <= kPairMaxWindow
+    uint32_t sb_shift = 0;               // a superblock is 2^sb_shift windows, (2^sb_shift - 1) * window <= 65535
+    uint64_t n_direct = 0, n_super = 0, n_cluster = 0, n_runs = 0;
+    std::vector<uint32_t> lines;         // [(n_direct + raw children) * 16]
+    std::vector<uint32_t> super;         // [16][n_super]: K[p] + #p in P[0, superblock_start)
+    uint32_t n_bad = 0;
+    uint32_t bad_pos[kPairMaxBad] = {0}; // rows whose pair holds the terminator, ascending (stored as code 0)
+    uint64_t bytes() const { return lines.size() * 4 + super.size() * 4; }
+};
+// Runs of P in row order: code 0..15, or kPairBad for a row whose pair holds the terminator.
+constexpr uint8_t kPairBad = 16;
+void pair_runs(const RunsBwt& bwt, const LeafDir& d, std::vector<uint32_t>& lens, std::vector<uint8_t>& codes);
+// window = 0 -> choose (RBG_PAIR_WINDOW overrides).  Needs n < 2^32.
+PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window = 0);
 
 // Sorted u64 keys with a radix table: table[b] = #keys < (b << shift), b in [0, (universe>>shift)+1].
 struct PredTable {

@@ -51,6 +51,7 @@ namespace rbg {
 template <int V> struct LeafFmt;
 template <> struct LeafFmt<4> { static constexpr int E = 24, S0 = 3, H0 = 2, NX = 6, CE = 20; };   // entries, first start word, head word, match words, entries of a CLUSTER line
 template <> struct LeafFmt<5> { static constexpr int E = 20, S0 = 5, H0 = 4, NX = 5, CE = 16; };
+template <> struct LeafFmt<6> { static constexpr int E = 12, S0 = 8, H0 = 14, NX = 3, CE = 0; };    // pair line, below
 
 constexpr int kLeafEntries = 24;                    // layout 4 (the larger of the two)
 constexpr int kClusterEntries = 20;                 // w[13], w[14] of a CLUSTER line: stretch bounds, child pointer
@@ -187,6 +188,68 @@ RBG_HD uint32_t raw_rank(const uint32_t* cw, uint32_t cpat, uint32_t p) {
 RBG_HD uint32_t raw_rel_count(const uint32_t* cw, uint32_t c) {
     const uint32_t pair = cw[c >> 1];
     return (c & 1u) ? pair >> 16 : pair & 0xFFFFu;
+}
+
+// ---- pair lines (LeafFmt<6>) ------------------------------------------------------------------
+// The pair directory (PairDir, layout.hpp) is a rank directory over the sequence P[j] = (BWT[LF(j)], BWT[j]), code
+// p = 4 c1 + c2, so that one rank answers two LF steps (derivation beside lf_pair_warp, device_index.cuh).  One line:
+//   w[0..7]   16 x u16: #p in P[superblock_start, window_start), code p in the (p&1) half of w[p/2]; the absolute part
+//             (K[p] + #p before the superblock) is one u32 per code and superblock, kept in shared memory
+//   w[8..13]  12 x u16 run starts, entry e in the (e&1) half of w[8 + e/2], as in the single-base lines
+//   w[14]     4-bit heads of entries 0..7, TRANSPOSED: entry e at bit 8*(e&3) + 4*(e>>2), so that (eq >> 4i) & 0x01010101
+//             is the byte vector of entries 4i..4i+3
+//   w[15]     heads of entries 8..11 at bits 8*(e&3) (low nibble of each byte); byte 0 bit 4: CLUSTER, bit 6: TERM
+// The rank is leaf_rank_x<6>: the same mins and dot products as the single-base lines, over 12 entries.
+// CLUSTER: a window of more than 12 runs keeps its counts, and w[8] holds the index of its first RAW child: the whole
+// window's codes at 4 bits (symbol i at bits 4*(i&7) of word i/8 of child i/128; windows are <= 256, so <= 2 children).
+// TERM: rows whose pair has a terminator (BWT[j] or BWT[LF(j)] is '$', at most 16) are stored as code 0 in the heads and
+// the children but are not counted anywhere else; a rank of code 0 in such a window subtracts them (pair_bad list).
+constexpr uint32_t kPairMaxWindow = 256;
+constexpr uint32_t kPairRawSymbols = 128;          // 16 words x 8 codes in a pair RAW child line
+constexpr int kPairMaxBad = 16;
+
+RBG_HD uint32_t pair_head_bit(uint32_t e) { return e < 8u ? 8u * (e & 3u) + 4u * (e >> 2) : 8u * (e & 3u); }
+RBG_HD uint32_t pair_pat(uint32_t p) { return p * 0x11111111u; }
+
+RBG_HD uint32_t pair_rel_count(const uint32_t (&w)[16], uint32_t p) {
+    const bool b1 = p & 2u, b2 = p & 4u, b3 = p & 8u;
+    const uint32_t w01 = b1 ? w[1] : w[0], w23 = b1 ? w[3] : w[2], w45 = b1 ? w[5] : w[4], w67 = b1 ? w[7] : w[6];
+    const uint32_t w03 = b2 ? w23 : w01, w47 = b2 ? w67 : w45;
+    const uint32_t x = b3 ? w47 : w03;
+    return (p & 1u) ? x >> 16 : x & 0xFFFFu;
+}
+
+// 1 in bit 0 of each nibble of x ^ pat that is zero
+RBG_HD uint32_t pair_eq_nibbles(uint32_t x) {
+    const uint32_t t = x | (x >> 1);
+    return ~(t | (t >> 2));
+}
+
+RBG_HD void pair_match(const uint32_t (&w)[16], uint32_t ppat, uint32_t (&xb)[6], uint32_t (&xs)[6]) {
+    const uint32_t eq = pair_eq_nibbles(w[14] ^ ppat), eq2 = pair_eq_nibbles(w[15] ^ ppat);
+    xb[0] = eq & 0x01010101u;
+    xb[1] = (eq >> 4) & 0x01010101u;
+    xb[2] = eq2 & 0x01010101u;
+    xb[3] = xb[4] = xb[5] = 0u;
+    xs[0] = xb[0] << 8;
+    xs[1] = rbg_funnel_l8(xb[0], xb[1]);
+    xs[2] = rbg_funnel_l8(xb[1], xb[2]);
+    xs[3] = xs[4] = xs[5] = 0u;
+}
+
+RBG_HD uint32_t pair_rank(const uint32_t (&w)[16], uint32_t ppat, uint32_t q) {
+    uint32_t xb[6], xs[6];
+    pair_match(w, ppat, xb, xs);
+    return leaf_rank_x<6>(w, xb, xs, q);
+}
+
+RBG_HD uint32_t pair_child_ptr(const uint32_t (&w)[16]) { return w[8]; }
+
+// #p among the first q codes of one word of a pair RAW child whose first code is code `first` of the window
+RBG_HD uint32_t pair_raw_word_count(uint32_t word, uint32_t ppat, int first, int q) {
+    const int rem = q - first;
+    const uint32_t m = rem >= 8 ? 0xFFFFFFFFu : (rem <= 0 ? 0u : (1u << (4 * rem)) - 1u);
+    return rbg_popc(pair_eq_nibbles(word ^ ppat) & 0x11111111u & m);
 }
 
 }  // namespace rbg

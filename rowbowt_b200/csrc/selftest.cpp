@@ -255,3 +255,63 @@ extern "C" int rbg_selftest_rewrite(const char* prefix, const char* out_prefix, 
         return -1;
     }
 }
+
+// Pair directory (PairDir, leaf.cuh LeafFmt<6>) over caller-supplied runs: K[p] + rank_p(pos) decoded from the lines -- the
+// decode lf_pair_warp runs, CLUSTER children and the terminator correction included -- equals a direct count over the pair
+// sequence at every stride-th position (and n) for all 16 codes.  codes_out (n bytes, optional) receives P[j] row by row
+// (16 = a pair with the terminator), expanded from the runs the directory was built from.
+extern "C" int rbg_selftest_pair(uint64_t n, const uint8_t* heads, const uint64_t* lens, uint64_t R, uint32_t window, uint64_t stride,
+                                 uint8_t* codes_out, uint64_t* checked, uint64_t* n_lines, uint64_t* n_cluster) {
+    try {
+        RunsBwt bwt;
+        bwt.n = n;
+        bwt.R = R;
+        bwt.heads.assign(heads, heads + R);
+        bwt.lens.assign(lens, lens + R);
+        setenv("RBG_LAYOUT", "5", 1);
+        LeafDir d = build_leaf_dir(bwt);
+        unsetenv("RBG_LAYOUT");
+        PairDir P = build_pair_dir(bwt, d, window);
+        if (n_lines) *n_lines = P.lines.size() / kLineWords;
+        if (n_cluster) *n_cluster = P.n_cluster;
+        std::vector<uint32_t> rl;
+        std::vector<uint8_t> rc;
+        pair_runs(bwt, d, rl, rc);
+        std::vector<uint8_t> code(n);
+        uint64_t at = 0;
+        for (size_t i = 0; i < rl.size(); ++i) for (uint32_t t = 0; t < rl[i]; ++t) code[at++] = rc[i];
+        if (at != n) return 2;
+        if (codes_out) memcpy(codes_out, code.data(), n);
+        const uint32_t W = P.window;
+        uint64_t cnt[16] = {0}, chk = 0;
+        if (stride == 0) stride = 1;
+        for (uint64_t pos = 0; pos <= n; ++pos) {
+            if (pos % stride == 0 || pos == n) {
+                // rank at pos from the window of `a` with offset q; also the "hi" form (q = W) at every other boundary
+                const bool prev = pos == n || (pos % W == 0 && pos > 0 && ((pos / W) & 1));
+                const uint64_t a = prev ? pos - 1 : pos, widx = a / W;
+                const uint32_t q = (uint32_t) (a - widx * W) + (prev ? 1u : 0u);
+                uint32_t w[16];
+                memcpy(w, P.lines.data() + widx * 16, 64);
+                for (uint32_t p = 0; p < 16; ++p) {
+                    uint32_t r = pair_rank(w, pair_pat(p), q);
+                    if (w[15] & kFlagCluster) {
+                        const uint32_t* cw = P.lines.data() + (uint64_t) pair_child_ptr(w) * 16;
+                        r = 0;
+                        for (uint32_t k = 0; 8 * k < q; ++k) r += pair_raw_word_count(cw[k], pair_pat(p), 8 * (int) k, (int) q);
+                    }
+                    if ((w[15] & kFlagTerm) && p == 0)
+                        for (uint32_t t = 0; t < P.n_bad; ++t) r -= (P.bad_pos[t] >= pos - q && P.bad_pos[t] < pos) ? 1 : 0;
+                    const uint64_t got = (uint64_t) P.super[p * P.n_super + (widx >> P.sb_shift)] + pair_rel_count(w, p) + r;
+                    if (got != (uint64_t) P.super[p * P.n_super] + cnt[p]) return 1;
+                    ++chk;
+                }
+            }
+            if (pos < n && code[pos] < kPairBad) ++cnt[code[pos]];
+        }
+        if (checked) *checked = chk;
+        return 0;
+    } catch (...) {
+        return -1;
+    }
+}

@@ -103,9 +103,9 @@ def main():
            "variants the `common path` column also holds the block of the third rank, which runs in about one warp step in six.",
            "`common path` = what every warp step executes; `rare path` = the forward-branched block that runs only when some lane's",
            "rank position lies inside a collapsed variant cluster / the terminator window (warp-cooperative child-line walk).", ""]
-    for variant, label in (("ILb0ELi5EE", "count, layout 5 (the default)"),
-                           ("ILb1ELi5EE", "toehold (-s), layout 5"),
-                           ("ILb0ELi4EE", "count, layout 4")):
+    for variant, label in (("ILb0ELi5ELb0EE", "count, layout 5"),
+                           ("ILb1ELi5ELb0EE", "toehold (-s), layout 5"),
+                           ("ILb0ELi4ELb0EE", "count, layout 4")):
         ins = sass_of(variant)
         (start, end, step_start, rare), refill, common, rare_ins = loop_parts(ins)
         out += ["## %s — `search_kernel<%s>`" % (label, variant), "",
@@ -117,7 +117,7 @@ def main():
         for name in sorted(set(cc) | set(rc) | set(fc), key=lambda k: -cc.get(k, 0)):
             out.append("| %s | %d | %d | %d |" % (name, cc.get(name, 0), rc.get(name, 0), fc.get(name, 0)))
         out.append("")
-        if variant == "ILb0ELi5EE":
+        if variant == "ILb0ELi5ELb0EE":
             out += ["<details><summary>common path, full listing</summary>", "", "```"]
             out += ["/*%04x*/ %s ;" % (x[0], x[1]) for x in common]
             out += ["```", "", "</details>", ""]
