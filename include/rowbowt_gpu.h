@@ -218,6 +218,35 @@ int rbg_build_marker_array(const char* index_prefix, const char* mps_path, const
 int rbg_build_marker_array_arrays(const rbg_index_desc* desc, const char* mps_path, const char* ma_path, const char* mab_path,
                                   uint64_t row_begin, uint64_t row_end, int device, rbg_ma_stats* stats);
 
+/* The builder's raw outputs from a FASTA, on the GPU: what `pfbwt-f64 --non-acgt-to-a --print-docs -r -o P P.fa` writes and
+ * rbg_build_index / rbg_build_marker_array read.  The text T is, for each record in file order, its bases followed by 10 'A's,
+ * then one byte 0 (the terminator): n = sum(len + 10) + 1.
+ *   <out>.bwt   n bytes, BWT[i] = T[SA[i] - 1] (0 at the row where SA[i] = 0), bases as ASCII
+ *   <out>.ssa   per maximal run of equal BWT bytes, in row order: (first row, SA[first row]), two little-endian u64
+ *   <out>.esa   the same with the run's last row
+ *   <out>.docs  `name start` per record: the header up to the first whitespace, the offset of its first base in T
+ * Input: FASTA, plain, gzip or BGZF, multi-line records joined.  Uppercase A C G T are kept, any other uppercase letter
+ * becomes 'A'.  Refused before any CUDA call: a missing or unreadable file RBG_E_IO; no records, or a record without bases
+ * RBG_E_FORMAT; a lowercase letter or a non-letter byte in a sequence RBG_E_ALPHABET (record and offset named: soft-masked
+ * input must be uppercased first); n >= 2^32 RBG_E_ARG.  When the build does not fit the device's free memory RBG_E_NOMEM
+ * (the bytes needed are named), before anything is allocated.  Outputs are written to temporary files and renamed.
+ * rbg_build_bwt_text takes len ACGT bytes without the terminator (tests) and writes no .docs; len is checked before the
+ * buffer is read.  `stats` may be NULL. */
+#define RBG_BWT_MAX_ROUNDS 32
+typedef struct {
+    uint64_t n, r;                  /* text length (terminator included), BWT runs */
+    uint64_t records;               /* FASTA records (0 for rbg_build_bwt_text) */
+    uint32_t rounds;                /* prefix-doubling rounds after the initial sort by the first 27 symbols */
+    uint32_t _pad;
+    uint64_t max_active;            /* most suffixes one round sorted */
+    uint64_t active[RBG_BWT_MAX_ROUNDS];   /* suffixes round i sorted (i < rounds): those whose group was still larger than 1 */
+    double s_parse, s_sort, s_write, s_total;   /* wall time: FASTA -> text; upload, sort, BWT and samples back; file writes; all */
+    float ms_sort, ms_gather;       /* CUDA-event time of the initial sort + rounds, and of the BWT gather + run boundaries + samples */
+    uint64_t peak_bytes;            /* device memory the build allocates (checked against the free memory first) */
+} rbg_bwt_stats;
+int rbg_build_bwt(const char* fasta_path, const char* out_prefix, int device, rbg_bwt_stats* stats);
+int rbg_build_bwt_text(const uint8_t* text, uint64_t len, const char* out_prefix, int device, rbg_bwt_stats* stats);
+
 /* The k-mer seed table (FTab, include/ftab.hpp:12-40).  Once resident, every query of a read of
  * at least k bases starts from the table entry of its last k bases instead of k LF steps; results
  * are identical by construction (entry = find_range(kmer), rb_tests.cpp:147-173).

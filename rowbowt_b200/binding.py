@@ -88,6 +88,21 @@ class MaStats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+BWT_MAX_ROUNDS = 32       # RBG_BWT_MAX_ROUNDS
+
+
+class BwtStats(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("r", C.c_uint64), ("records", C.c_uint64), ("rounds", C.c_uint32), ("_pad", C.c_uint32),
+                ("max_active", C.c_uint64), ("active", C.c_uint64 * BWT_MAX_ROUNDS),
+                ("s_parse", C.c_double), ("s_sort", C.c_double), ("s_write", C.c_double), ("s_total", C.c_double),
+                ("ms_sort", C.c_float), ("ms_gather", C.c_float), ("peak_bytes", C.c_uint64)]
+
+    def as_dict(self):
+        d = {k: getattr(self, k) for k, _ in self._fields_ if k not in ("_pad", "active")}
+        d["active"] = list(self.active)[:min(self.rounds, BWT_MAX_ROUNDS)]
+        return d
+
+
 class Stats(C.Structure):
     _fields_ = [("reads", C.c_uint64), ("bases", C.c_uint64), ("lf_steps", C.c_uint64), ("lf_lines", C.c_uint64),
                 ("phi_steps", C.c_uint64), ("marker_words", C.c_uint64),
@@ -125,6 +140,8 @@ def lib():
                                              C.POINTER(MaStats)]
         L.rbg_build_marker_array_arrays.argtypes = [C.POINTER(_Desc), C.c_char_p, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64,
                                                     C.c_int, C.POINTER(MaStats)]
+        L.rbg_build_bwt.argtypes = [C.c_char_p, C.c_char_p, C.c_int, C.POINTER(BwtStats)]
+        L.rbg_build_bwt_text.argtypes = [C.c_void_p, C.c_uint64, C.c_char_p, C.c_int, C.POINTER(BwtStats)]
         L.rbg_index_close.argtypes = [C.c_void_p]
         L.rbg_index_info.argtypes = [C.c_void_p, C.POINTER(Info)]
         L.rbg_last_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
@@ -225,6 +242,22 @@ def build_index(in_prefix: str, out_prefix: str, sa: bool = False, markers: bool
     st = BuildStats()
     flags = (RBG_LOAD_SA if sa else 0) | (RBG_LOAD_MA if markers else 0) | (RBG_LOAD_FT if ftab_k else 0)
     _check(lib().rbg_build_index(in_prefix.encode(), out_prefix.encode(), flags, ftab_k, device, C.byref(st)))
+    return st
+
+
+def build_bwt(fasta: str, out_prefix: str, device: int = 0) -> "BwtStats":
+    """pfbwt-f64 --non-acgt-to-a --print-docs -r on the GPU: a FASTA (plain, gzip or BGZF) -> <out>.bwt/.ssa/.esa/.docs, the
+    files rb_build reads.  The text is every record followed by 10 'A's, then the terminator; it must have n < 2^32."""
+    st = BwtStats()
+    _check(lib().rbg_build_bwt(fasta.encode(), out_prefix.encode(), device, C.byref(st)))
+    return st
+
+
+def build_bwt_text(text: np.ndarray, out_prefix: str, device: int = 0) -> "BwtStats":
+    """The same for one ACGT text (uint8 ASCII, without the terminator, which is appended): <out>.bwt/.ssa/.esa, no .docs."""
+    t = np.ascontiguousarray(text, np.uint8)
+    st = BwtStats()
+    _check(lib().rbg_build_bwt_text(t.ctypes.data, len(t), out_prefix.encode(), device, C.byref(st)))
     return st
 
 

@@ -21,6 +21,7 @@
 #include <vector>
 
 #include "cuda_host.hpp"
+#include "bwt_build.hpp"
 #include "formats.hpp"
 #include "host_pack.hpp"
 #include "raw_build.hpp"
@@ -665,6 +666,7 @@ int guarded(Fn&& fn) {
     } catch (const format_error& e) { return fail(RBG_E_FORMAT, e.what());
     } catch (const alphabet_error& e) { return fail(RBG_E_ALPHABET, e.what());
     } catch (const cuda_error& e) { cudaGetLastError(); return fail(RBG_E_CUDA, e.what());
+    } catch (const nomem_error& e) { return fail(RBG_E_NOMEM, e.what());
     } catch (const std::bad_alloc&) { return fail(RBG_E_NOMEM, "out of host memory");
     } catch (const std::exception& e) { return fail(RBG_E_ARG, e.what()); }
 }
@@ -1506,6 +1508,44 @@ int rbg_build_marker_array_arrays(const rbg_index_desc* d, const char* mps_path,
         validate_toehold(p.tsa, "the toehold arrays");
         st.s_read = wall_s() - t_begin;
         return build_ma_from(p, mps, row_begin, row_end, device, ma_path, mab_path, st, t_begin, stats);
+    });
+}
+
+int rbg_build_bwt(const char* fasta_path, const char* out_prefix, int device, rbg_bwt_stats* stats) {
+    if (!fasta_path || !out_prefix) return fail(RBG_E_ARG, "null argument");
+    return guarded([&] {
+        rbg_bwt_stats st;
+        memset(&st, 0, sizeof st);
+        const double t_begin = wall_s();
+        const FastaText ft = read_fasta_text(fasta_path);
+        st.records = ft.names.size();
+        st.s_parse = wall_s() - t_begin;
+        select_device(device);
+        build_bwt_files(ft.text.data(), ft.text.size(), device, out_prefix, st);
+        const double t_docs = wall_s();
+        write_docs(ft, std::string(out_prefix) + ".docs");
+        st.s_write += wall_s() - t_docs;
+        st.s_total = wall_s() - t_begin;
+        if (stats) *stats = st;
+        return (int) RBG_OK;
+    });
+}
+
+int rbg_build_bwt_text(const uint8_t* text, uint64_t len, const char* out_prefix, int device, rbg_bwt_stats* stats) {
+    if (!text || !out_prefix) return fail(RBG_E_ARG, "null argument");
+    if (len == 0) return fail(RBG_E_ARG, "empty text");
+    return guarded([&] {
+        rbg_bwt_stats st;
+        memset(&st, 0, sizeof st);
+        const double t_begin = wall_s();
+        check_bwt_length(std::min(len, kBwtMaxN) + 1, "a text of " + std::to_string(len) + " bases");    // before the buffer is read
+        check_acgt(text, len);
+        st.s_parse = wall_s() - t_begin;
+        select_device(device);
+        build_bwt_files(text, len, device, out_prefix, st);
+        st.s_total = wall_s() - t_begin;
+        if (stats) *stats = st;
+        return (int) RBG_OK;
     });
 }
 

@@ -3,13 +3,13 @@
 
 Generates: a uniform-random reference, a SNP panel, H haplotypes, the FASTA the
 reference's index builder consumes, marker positions, and simulated reads.
-Index CONSTRUCTION is out of scope for this repo (SURVEY.md §2 rows 13, 20):
 `build_index` shells out to the UNMODIFIED reference builder binaries compiled
 by oracle/Makefile into oracle/_ref/ (pfbwt-f64, rb_build, mps_to_ma and the
 write_mps driver around MarkerPositionsWriter), following the reference's
-scripts/fa_to_rowbowt.sh.  The files produced (.rbwt/.tsa/.mab/.docs) are the
-reference's own on-disk formats and are what both the GPU library and the
-reference rb_align consume.
+scripts/fa_to_rowbowt.sh.  `build_index_from_fasta_gpu` (`--gpu`) builds the same
+files from the same FASTA with this project's GPU builders alone.  The files
+produced (.rbwt/.tsa/.mab/.docs) are the reference's own on-disk formats and are
+what both the GPU library and the reference rb_align consume.
 
 Seeds (§8(d)): reference seed=1, panel/genotypes seed=2, reads seed=3.
 """
@@ -280,6 +280,28 @@ def build_index_gpu(panel: Panel, prefix: str, markers: bool = True, device: int
     return t
 
 
+def build_index_from_fasta_gpu(panel: Panel, prefix: str, markers: bool = True, device: int = 0, log=sys.stderr) -> dict:
+    """The same index files as build_index, from the panel's FASTA with the project's GPU builders alone: write_fasta ->
+    build_bwt (.bwt/.ssa/.esa/.docs) -> build_index (.rbwt/.tsa) -> write_mps -> build_marker_array (.ma, .mab); the FASTA
+    and the raw files are removed afterwards.  Returns timings."""
+    import rowbowt_b200 as rb
+    t = {}
+    fa = prefix + ".fa"
+    t0 = time.time(); write_fasta(panel, fa); t["fasta"] = time.time() - t0
+    t0 = time.time(); rb.build_bwt(fa, prefix, device=device); t["bwt"] = time.time() - t0
+    t0 = time.time(); rb.build_index(prefix, prefix, sa=True, device=device); t["rb_build"] = time.time() - t0
+    if markers:
+        t0 = time.time(); write_mps(panel, prefix + ".mps"); t["mps"] = time.time() - t0
+        t0 = time.time()
+        rb.build_marker_array(prefix, prefix + ".mps", prefix + ".ma", mab=prefix + ".mab", device=device)
+        t["ma"] = time.time() - t0
+    for path in (fa, prefix + ".bwt", prefix + ".ssa", prefix + ".esa", prefix + ".mps", prefix + ".ma"):
+        if os.path.exists(path):
+            os.remove(path)
+    print("build_index_from_fasta_gpu %s: %s" % (prefix, {k: round(v, 1) for k, v in t.items()}), file=log)
+    return t
+
+
 def make_reads(panel: Panel, n_reads: int, read_len: int = 150, seed: int = 3,
                err_rate: float = 0.0, n_rate: float = 0.0, chunk: int = 1 << 20):
     """uint8[n_reads, read_len] ASCII reads: uniform substrings of uniformly
@@ -361,12 +383,18 @@ def main():
     ap.add_argument("--no-markers", action="store_true")
     ap.add_argument("--reads", type=int, default=0, help="also write N reads as FASTQ")
     ap.add_argument("--keep", action="store_true")
+    ap.add_argument("--gpu", action="store_true", help="build on the GPU with this project's builders, without the reference")
     a = ap.parse_args()
     L, H = CONFIGS[a.config]
     os.makedirs(a.outdir, exist_ok=True)
     prefix = os.path.join(a.outdir, a.config)
     panel = make_panel(L, H)
-    build_index(panel, prefix, markers=not a.no_markers, keep_fasta=a.keep)
+    if a.gpu:
+        if ROOT not in sys.path:          # run as a script from tools/: the package is imported from the repository root
+            sys.path.insert(0, ROOT)
+        build_index_from_fasta_gpu(panel, prefix, markers=not a.no_markers)
+    else:
+        build_index(panel, prefix, markers=not a.no_markers, keep_fasta=a.keep)
     if a.reads:
         reads, _, _ = make_reads(panel, a.reads)
         write_fastq(reads, prefix + ".reads.fq")
