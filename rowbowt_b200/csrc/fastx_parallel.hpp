@@ -74,8 +74,7 @@ struct ReadBatch {
     GrowBuf<uint64_t> offs;             // n + 1
     std::vector<char> names;            // concatenated names
     std::vector<uint64_t> name_off{0};  // n + 1
-    std::vector<std::string> out;       // formatted text, one string per formatter slice (rb_markers)
-    std::vector<OutBuf> text;           // rb_align: one buffer per formatter slice; keeps its pages across recycles
+    std::vector<OutBuf> text;           // formatted text, one buffer per formatter slice; keeps its pages across recycles
     size_t n_text = 0;                  // slices of `text` in use
     std::vector<uint8_t> aux;           // one driver-defined byte per read (rb_markers --heuristic: strand tried first)
     // 2-bit form of `bases` for rbg_query_packed, filled by the driver's on_batch hook (on the parser thread that built the batch)
@@ -90,7 +89,6 @@ struct ReadBatch {
         n = 0;
         names.clear();
         name_off.assign(1, 0);
-        out.clear();
         n_text = 0;
         aux.clear();
         n_exotic = 0;

@@ -6,33 +6,22 @@
 //
 //   rb_align [-s] [-m] [-o prefix] [--gpus N] [--threads T] [--batch READS] [--ftab | --ftab-k K] <index_prefix> <fastq>
 //
-// Pipeline: T parser threads over the mmap'ed FASTQ (fastx_parallel.hpp; a .gz or irregular
-// input goes through the sequential kseq-compatible reader) filling pinned batch buffers ->
-// N GPU workers (one index replica and one C-ABI handle per device) -> T formatter threads
-// (slices of a batch) -> one ordered writer.  No collective: batches are independent
-// (SURVEY.md §8(e)).
-#include <fcntl.h>
+// Pipeline (driver_pipeline.hpp): parser threads, which also pack the bases to 2 bits -> GPU
+// workers calling rbg_query_packed -> formatter pool (report_format.hpp) -> ordered writer.
 #include <getopt.h>
-#include <sys/stat.h>
-#include <unistd.h>
 
-#include <atomic>
 #include <chrono>
-#include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
-#include <deque>
+#include <cstring>
 #include <iostream>
-#include <map>
 #include <memory>
-#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
 
 #include "../../include/rowbowt_gpu.h"
-#include "fastx_parallel.hpp"
-#include "host_io.hpp"
+#include "driver_pipeline.hpp"
 
 namespace {
 
@@ -276,19 +265,6 @@ int format_selftest(long n_reads) {
     return 0;
 }
 
-using rbhost::Channel;
-
-// RBG_HOST_STATS=1: busy seconds of every stage of the host pipeline on stderr (before the reference's timing line)
-struct StageClock {
-    std::atomic<uint64_t> ns{0};
-    struct Scope {
-        StageClock& c;
-        std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
-        ~Scope() { c.ns += (uint64_t) std::chrono::duration_cast<std::chrono::nanoseconds>(std::chrono::steady_clock::now() - t0).count(); }
-    };
-    double s() const { return (double) ns.load() * 1e-9; }
-};
-
 [[noreturn]] void die_rbg(const char* what) {
     fprintf(stderr, "%s: %s\n", what, rbg_last_error());
     exit(1);
@@ -348,72 +324,43 @@ int main(int argc, char** argv) {
     if (args.ftab_file) flags |= RBG_LOAD_FT;
     if (args.fbb) flags |= RBG_LOAD_FBB;
     if (args.layout_cache) flags |= RBG_LOAD_CACHE;
-    int ndev = rbg_device_count();
-    if (ndev <= 0) {
-        fprintf(stderr, "no CUDA device available (this build has no CPU path)\n");
-        return 1;
-    }
-    // one GPU worker per requested GPU.  RBG_GPU_MODULO=1 (tests on a box with fewer devices): worker g shares the
-    // handle of device g % ndev -- calls on one handle run concurrently -- so that the ordered reassembly of a
-    // multi-worker run is exercised anywhere; otherwise the request is clamped to the visible devices.
-    const bool modulo = getenv("RBG_GPU_MODULO") && atoi(getenv("RBG_GPU_MODULO")) > 0;
-    const int n_gpus = modulo ? args.gpus : std::min(args.gpus, ndev);
-    const int n_handles = std::min(n_gpus, ndev);
+    rbhost::QueryPipeline<rbg_result>::Options po;
+    po.fastq = args.fastq;
+    po.threads = args.threads;
+    po.chunk_bytes = args.chunk_bytes;
+    po.batch_reads = args.batch_reads;
+    po.gpus = args.gpus;
     // A parser chunk is ~50 k reads: 0.4 ms on an idle GPU (0.12 ms of it kernel time, the rest the latency of 140 dependent
     // LF steps and three copies), so ONE caller per device leaves the GPU mostly idle and, at 10^7 reads, was the slowest
     // stage of the count / -m pipeline.  Two workers per device overlap their calls (the library runs concurrent calls on one
     // handle in separate lanes).  With -s the report writer is the bound and concurrent locate calls contend for the device
-    // allocator: one worker.  RBG_WORKERS_PER_GPU overrides.
-    const int wpg = getenv("RBG_WORKERS_PER_GPU") ? std::max(1, std::min(4, atoi(getenv("RBG_WORKERS_PER_GPU")))) : (args.sam ? 1 : 2);
-    const int gpus = n_gpus * wpg;                  // GPU workers; worker g calls on the handle of device g % n_handles
-    std::vector<rbg_index*> idx(n_handles, nullptr);
-    // parser threads -> GPU workers (one per device) -> formatter pool (slices of a batch) -> ordered writer
-    const size_t pool = 2 * (size_t) args.threads + 6 * (size_t) gpus + 4;
+    // allocator: one worker.
+    po.workers_per_gpu = args.sam ? 1 : 2;
+    po.slice_shift = 12;
     // the thread that parsed a batch also packs its bases to 2 bits (rbg_pack_bytes): 46 instead of 158 bytes per
     // 150 bp read cross PCIe, and the GPU skips pack_kernel (RBG_HOST_PACK=0: ship the bytes, pack on the device)
     const bool host_pack = !(getenv("RBG_HOST_PACK") && atoi(getenv("RBG_HOST_PACK")) == 0);
-    StageClock clk_pack, clk_query, clk_format, clk_write, clk_wait_gpu, clk_next;
-    uint64_t n_batches = 0, n_reads_total = 0;
-    std::function<void(ReadBatch&)> pack_hook;
     if (host_pack)
-        pack_hook = [&](ReadBatch& b) {
-            StageClock::Scope sc{clk_pack};
+        po.pack = [](rbg_index* ix, ReadBatch& b) {
             const uint64_t nb = b.n_bases();
             b.packed.reserve(nb / 32 + 2, 0);
             b.flags.reserve(b.n + 8, 0);
             memset(b.flags.p, 0, b.n);
             b.n_exotic = 0;
             uint64_t ex = 0;
-            if (rbg_pack_bytes(idx[0], b.bases.p, b.offs.p, b.n, 0, nb, b.packed.p, b.flags.p, &ex) != RBG_OK) die_rbg("rbg_pack_bytes");
+            if (rbg_pack_bytes(ix, b.bases.p, b.offs.p, b.n, 0, nb, b.packed.p, b.flags.p, &ex) != RBG_OK) die_rbg("rbg_pack_bytes");
             if (ex)
                 for (uint64_t i = 0; i < b.n; ++i) b.n_exotic += (b.flags.p[i] & RBG_READ_EXOTIC) ? 1 : 0;
         };
-    // The source is set up now but parses nothing before the index is loaded (start() below, inside the query time): only
-    // its pinned staging buffers are allocated meanwhile, on a thread of their own -- pinning is ~0.3 ms per MB under the
-    // CUDA context lock, which must not happen while the GPU worker is issuing copies and launches.  With host packing
-    // the raw bases never cross PCIe (only a read holding the terminator byte is copied, from pageable memory): plain malloc.
-    const rbhost::HostAlloc pinned{rbg_host_alloc, rbg_host_free}, pageable{malloc, free};
-    rbhost::FastxBatchSource src(args.fastq.c_str(), args.threads, args.chunk_bytes, args.batch_reads, pinned, pool, pack_hook,
-                                 /*start=*/false, host_pack ? &pageable : nullptr);
-    std::thread prewarm([&] { if (src.ok()) src.prewarm(host_pack); });
-    struct Joiner { std::thread& t; ~Joiner() { if (t.joinable()) t.join(); } } prewarm_joiner{prewarm};      // error exits below
-    {
-        std::vector<std::thread> th;
-        std::vector<int> rc(n_handles, 0);
-        std::vector<std::string> msg(n_handles);
-        for (int g = 0; g < n_handles; ++g)
-            th.emplace_back([&, g] {
-                rc[g] = rbg_index_open(args.inpre.c_str(), flags, g, &idx[g]);
-                if (!rc[g] && !args.ftab_file && args.ftab_k) rc[g] = rbg_ftab_build(idx[g], (uint32_t) args.ftab_k);
-                if (rc[g]) msg[g] = rbg_last_error();
-            });
-        for (auto& t : th) t.join();
-        for (int g = 0; g < n_handles; ++g)
-            if (rc[g]) {
-                // the reference prints "bad file" and exits for a missing part (rowbowt_io.hpp:166-169)
-                std::cerr << (rc[g] == RBG_E_IO ? "bad file" : msg[g]) << std::endl;
-                return 1;
-            }
+    rbhost::QueryPipeline<rbg_result> pipe(std::move(po));
+    std::string msg;
+    const int rc = pipe.open(args.inpre.c_str(), flags, [&](rbg_index* ix) {
+        return !args.ftab_file && args.ftab_k ? rbg_ftab_build(ix, (uint32_t) args.ftab_k) : RBG_OK;
+    }, msg);
+    if (rc) {
+        // the reference prints "bad file" and exits for a missing part (rowbowt_io.hpp:166-169)
+        std::cerr << (rc == RBG_E_IO ? "bad file" : msg) << std::endl;
+        return 1;
     }
     if (args.sam) {
         std::cerr << "loading: " << args.inpre + ".docs" << std::endl;
@@ -424,196 +371,29 @@ int main(int argc, char** argv) {
     }
     rbhost::DocResolver resolver;
     resolver.init(docs.names(), docs.starts());
-    prewarm.join();
+    const bool input_ok = pipe.finish_load();
     std::chrono::duration<double> load_time = clk::now() - t0;
-    if (!src.ok()) {                                  // src/rb_align.cpp:170-173 (after the index is loaded, as there)
+    if (!input_ok) {                                  // src/rb_align.cpp:170-173 (after the index is loaded, as there)
         fprintf(stderr, "invalid file\n");
         return 1;
     }
 
-    auto q0 = clk::now();
-    src.start();
     // narrow wire forms (u32 ranges / locations when n <= 2^32): half the D2H bytes, widened while formatting
     const uint32_t mode = (args.sam ? RBG_LOCATE | RBG_NARROW_LOCS : 0) | (args.markers ? RBG_MARKERS : 0) | RBG_NARROW_RANGES;
-
-    struct Job {                                   // one batch between its query and its last formatted slice
-        std::unique_ptr<ReadBatch> b;
-        rbg_result res;
-        std::atomic<int> left{0};
-        int gpu = 0;
-    };
-    struct Slice { Job* job; int s; uint64_t i0, i1; };
-    Channel<std::unique_ptr<ReadBatch>> to_gpu(2 * gpus), to_writer(pool);
-    Channel<Slice> to_format(64 * (size_t) args.threads);
-    std::mutex inflight_m;
-    std::condition_variable inflight_cv;
-    std::vector<int> inflight(gpus, 0);            // results of device g not yet freed (the library pools 4)
-
-    std::vector<std::thread> workers, formatters;
-    for (int g = 0; g < gpus; ++g)
-        workers.emplace_back([&, g] {
-            std::unique_ptr<ReadBatch> b;
-            while (to_gpu.pop(b)) {
-                {
-                    std::unique_lock<std::mutex> l(inflight_m);
-                    inflight_cv.wait(l, [&] { return inflight[g] < 3; });
-                    ++inflight[g];
-                }
-                Job* job = new Job;
-                rbg_index* ix = idx[g % n_handles];
-                StageClock::Scope sq{clk_query};
-                if (host_pack) {
-                    rbg_packed_batch in{b->n, b->packed.p, b->offs.p, b->flags.p, b->n_exotic, b->bases.p};
-                    if (rbg_query_packed(ix, &in, mode, UINT64_MAX, &job->res) != RBG_OK) die_rbg("rbg_query_packed");
-                } else {
-                    rbg_batch in{b->n, b->bases.p, b->offs.p};
-                    if (rbg_query(ix, &in, mode, UINT64_MAX, &job->res) != RBG_OK) die_rbg("rbg_query");
-                }
-                job->gpu = g;
-                const uint64_t n = b->n;
-                const int slices = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) args.threads, n >> 12));
-                if (b->text.size() < (size_t) slices) b->text.resize(slices);
-                b->n_text = (size_t) slices;
-                job->b = std::move(b);
-                job->left = slices;
-                for (int s = 0; s < slices; ++s)
-                    to_format.push(Slice{job, s, n * (uint64_t) s / slices, n * (uint64_t) (s + 1) / slices});
+    const double query_time = pipe.run(
+        [&](rbg_index* ix, ReadBatch& b, rbg_result& res) {
+            if (host_pack) {
+                rbg_packed_batch in{b.n, b.packed.p, b.offs.p, b.flags.p, b.n_exotic, b.bases.p};
+                if (rbg_query_packed(ix, &in, mode, UINT64_MAX, &res) != RBG_OK) die_rbg("rbg_query_packed");
+            } else {
+                rbg_batch in{b.n, b.bases.p, b.offs.p};
+                if (rbg_query(ix, &in, mode, UINT64_MAX, &res) != RBG_OK) die_rbg("rbg_query");
             }
+        },
+        rbg_result_free,
+        [&](const rbg_result& res, const ReadBatch& b, uint64_t i0, uint64_t i1, rbhost::OutBuf& out) {
+            rbhost::format_report(args.sam != 0, args.markers != 0, resolver, res, [&b](uint64_t i, size_t& nl) { return b.name(i, nl); }, i0, i1, out);
         });
-    for (int t = 0; t < args.threads; ++t)
-        formatters.emplace_back([&] {
-            Slice sl;
-            while (to_format.pop(sl)) {
-                Job* job = sl.job;
-                {
-                    StageClock::Scope sf{clk_format};
-                    const ReadBatch& rb_ = *job->b;
-                    rbhost::format_report(args.sam != 0, args.markers != 0, resolver, job->res,
-                                          [&rb_](uint64_t i, size_t& nl) { return rb_.name(i, nl); }, sl.i0, sl.i1, job->b->text[sl.s]);
-                }
-                if (job->left.fetch_sub(1) == 1) {
-                    const int g = job->gpu;
-                    rbg_result_free(&job->res);
-                    {
-                        std::lock_guard<std::mutex> l(inflight_m);
-                        --inflight[g];
-                    }
-                    inflight_cv.notify_all();
-                    to_writer.push(std::move(job->b));
-                    delete job;
-                }
-            }
-        });
-    // Ordered output.  A pipe / terminal / O_APPEND stdout gets one write(2) after the other from this thread.  When stdout is a
-    // regular file (the usual `rb_align ... > report.txt`; with -s that is 1.4 KB per read) the order is only a matter of
-    // OFFSETS: this thread hands every slice of the next batch its place in the file and a few writer threads pwrite(2) them
-    // concurrently -- one thread copying into the page cache moved 2.3 GB/s, a third of what the formatters produce.
-    struct WriteTask { ReadBatch* b; size_t k; off_t at; };
-    struct stat out_st;
-    const int out_fl = fcntl(1, F_GETFL);
-    const off_t out_pos = lseek(1, 0, SEEK_CUR);
-    const bool positional = !(getenv("RBG_SEQ_WRITE") && atoi(getenv("RBG_SEQ_WRITE")) > 0) && fstat(1, &out_st) == 0 && S_ISREG(out_st.st_mode) &&
-                            out_fl >= 0 && !(out_fl & O_APPEND) && out_pos >= 0;
-    const int n_writers = positional ? std::max(1, std::min(4, args.threads / 2)) : 0;
-    Channel<WriteTask> to_pwrite(256);
-    std::mutex left_m;
-    std::map<ReadBatch*, std::pair<size_t, std::unique_ptr<ReadBatch>>> writing;      // batch -> (slices not yet written, owner)
-    std::vector<std::thread> pwriters;
-    for (int t = 0; t < n_writers; ++t)
-        pwriters.emplace_back([&] {
-            WriteTask w;
-            while (to_pwrite.pop(w)) {
-                {
-                    StageClock::Scope sw{clk_write};
-                    const char* p = w.b->text[w.k].p;
-                    size_t left = w.b->text[w.k].len;
-                    off_t at = w.at;
-                    while (left) {
-                        const ssize_t n = pwrite(1, p, left, at);
-                        if (n < 0) { if (errno == EINTR) continue; perror("pwrite"); exit(1); }
-                        p += n; at += n; left -= (size_t) n;
-                    }
-                }
-                std::unique_ptr<ReadBatch> done;
-                {
-                    std::lock_guard<std::mutex> l(left_m);
-                    auto it = writing.find(w.b);
-                    if (--it->second.first == 0) { done = std::move(it->second.second); writing.erase(it); }
-                }
-                if (done) src.recycle(std::move(done));
-            }
-        });
-    std::thread writer([&] {
-        std::map<uint64_t, std::unique_ptr<ReadBatch>> pending;
-        uint64_t next = 0;
-        off_t at = out_pos;
-        std::unique_ptr<ReadBatch> b;
-        while (to_writer.pop(b)) {
-            pending[b->id] = std::move(b);
-            for (auto it = pending.find(next); it != pending.end(); it = pending.find(next)) {
-                if (positional) {
-                    ReadBatch* rbp = it->second.get();
-                    std::vector<WriteTask> tasks;
-                    for (size_t k = 0; k < rbp->n_text; ++k) {
-                        if (rbp->text[k].len) tasks.push_back(WriteTask{rbp, k, at});
-                        at += (off_t) rbp->text[k].len;
-                    }
-                    if (tasks.empty()) {
-                        src.recycle(std::move(it->second));
-                    } else {
-                        {
-                            std::lock_guard<std::mutex> l(left_m);
-                            writing[rbp] = std::make_pair(tasks.size(), std::move(it->second));
-                        }
-                        for (const WriteTask& w : tasks) to_pwrite.push(w);
-                    }
-                } else {
-                    {
-                        StageClock::Scope sw{clk_write};
-                        for (size_t k = 0; k < it->second->n_text; ++k) rbhost::write_all(1, it->second->text[k].p, it->second->text[k].len);
-                    }
-                    src.recycle(std::move(it->second));
-                }
-                pending.erase(it);
-                ++next;
-            }
-        }
-        to_pwrite.close();
-        for (auto& t : pwriters) t.join();
-        if (positional && lseek(1, at, SEEK_SET) < 0) { perror("lseek"); exit(1); }       // whatever is written next continues behind the report
-    });
-
-    for (;;) {
-        std::unique_ptr<ReadBatch> b;
-        {
-            StageClock::Scope sn{clk_next};
-            b = src.next();
-        }
-        if (!b) break;
-        ++n_batches;
-        n_reads_total += b->n;
-        StageClock::Scope sg{clk_wait_gpu};
-        to_gpu.push(std::move(b));
-    }
-    const int err = src.err();
-    to_gpu.close();
-    for (auto& w : workers) w.join();
-    to_format.close();
-    for (auto& f : formatters) f.join();
-    to_writer.close();
-    writer.join();
-    std::chrono::duration<double> query_time = clk::now() - q0;
-    if (getenv("RBG_HOST_STATS"))
-        fprintf(stderr, "host stages (busy seconds, summed over threads): pack %.3f  rbg_query %.3f  format %.3f  write %.3f | main thread: "
-                "waiting for parsed batches %.3f, waiting for a GPU worker %.3f | %llu batches, %llu reads, %d parser/formatter threads, %d GPU workers\n",
-                clk_pack.s(), clk_query.s(), clk_format.s(), clk_write.s(), clk_next.s(), clk_wait_gpu.s(),
-                (unsigned long long) n_batches, (unsigned long long) n_reads_total, args.threads, gpus);
-    for (auto* ix : idx) rbg_index_close(ix);
-    switch (err) {           // src/rb_align.cpp:181-191
-        case -2: fprintf(stderr, "ERROR: truncated quality string\n"); exit(1);
-        case -3: fprintf(stderr, "ERROR: error reading stream\n"); exit(1);
-        default: break;
-    }
-    std::cerr << load_time.count() << " " << query_time.count() << std::endl;
+    std::cerr << load_time.count() << " " << query_time << std::endl;
     return 0;
 }

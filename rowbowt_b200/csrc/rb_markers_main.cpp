@@ -14,21 +14,16 @@
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <iostream>
-#include <map>
 #include <memory>
 #include <random>
 #include <string>
 #include <thread>
 #include <vector>
 
-#include <atomic>
-#include <condition_variable>
-#include <mutex>
-
 #include "../../include/rowbowt_gpu.h"
-#include "fastx_parallel.hpp"
-#include "host_io.hpp"
+#include "driver_pipeline.hpp"
 
 namespace {
 
@@ -127,35 +122,36 @@ struct Seed {                           // MarkerSeed, src/rb_markers.cpp:255-30
     std::vector<uint64_t> markers;
 };
 
-void print_seed(std::string& o, const char* name, size_t name_len, const Seed& s) {      // MarkerSeed::print_buf :262-272
+// MarkerSeed::print_buf :262-272
+void print_seed(std::string& o, const char* name, size_t name_len, uint64_t range_size, int strand, uint64_t query_start,
+                uint64_t query_len, const uint64_t* mk, size_t n_mk) {
     o.append(name, name_len);
     o += ' ';
-    rbhost::put_u64(o, s.range_size);
-    o += s.strand ? " - " : " + ";
-    rbhost::put_u64(o, s.query_start);
+    rbhost::put_u64(o, range_size);
+    o += strand ? " - " : " + ";
+    rbhost::put_u64(o, query_start);
     o += ' ';
-    rbhost::put_u64(o, s.query_len);
-    if (!s.markers.empty()) {
-        for (uint64_t m : s.markers) {
-            o += ' ';
-            rbhost::put_u64(o, m_seq(m));
-            o += '/';
-            rbhost::put_u64(o, m_pos(m));
-            o += '/';
-            rbhost::put_u64(o, m_allele(m));
-        }
-    } else {
-        o += " .";
+    rbhost::put_u64(o, query_len);
+    for (size_t k = 0; k < n_mk; ++k) {
+        o += ' ';
+        rbhost::put_u64(o, m_seq(mk[k]));
+        o += '/';
+        rbhost::put_u64(o, m_pos(mk[k]));
+        o += '/';
+        rbhost::put_u64(o, m_allele(mk[k]));
     }
+    if (!n_mk) o += " .";
     o += '\n';
 }
+
+uint64_t seed_query_start(const rbg_seed& g) { return g.query_start == 0xFFFFFFFFu ? ~0ull : g.query_start; }      // the reference's size_t(-1)
 
 Seed make_seed(const rbg_seed_result& r, uint64_t j, int strand) {
     const rbg_seed& g = r.seeds[j];
     Seed s;
     s.strand = strand;
     s.range_size = g.hi - g.lo + 1;
-    s.query_start = g.query_start == 0xFFFFFFFFu ? ~0ull : g.query_start;      // the reference's size_t(-1)
+    s.query_start = seed_query_start(g);
     s.query_len = g.query_len;
     s.markers.assign(r.markers + g.mk_off, r.markers + g.mk_off + g.mk_cnt);
     return s;
@@ -182,34 +178,10 @@ void clear_if_conflicting(std::vector<uint64_t>& mk, size_t read_len) {
     if (m_seq(mk.back()) != m_seq(mk.front()) || m_pos(mk.back()) - m_pos(mk.front()) >= read_len) mk.clear();
 }
 
-// One seed of the plain worker straight from the result arrays (no Seed object: this path prints ~10 seeds per read).
-void print_raw_seed(std::string& o, const char* name, size_t name_len, const rbg_seed_result& r, uint64_t j, int strand) {
-    const rbg_seed& g = r.seeds[j];
-    o.append(name, name_len);
-    o += ' ';
-    rbhost::put_u64(o, g.hi - g.lo + 1);
-    o += strand ? " - " : " + ";
-    rbhost::put_u64(o, g.query_start == 0xFFFFFFFFu ? ~0ull : (uint64_t) g.query_start);     // the reference's size_t(-1)
-    o += ' ';
-    rbhost::put_u64(o, g.query_len);
-    if (g.mk_cnt) {
-        for (uint64_t k = 0; k < g.mk_cnt; ++k) {
-            const uint64_t m = r.markers[g.mk_off + k];
-            o += ' ';
-            rbhost::put_u64(o, m_seq(m));
-            o += '/';
-            rbhost::put_u64(o, m_pos(m));
-            o += '/';
-            rbhost::put_u64(o, m_allele(m));
-        }
-    } else {
-        o += " .";
-    }
-    o += '\n';
-}
-
-// The report of reads [i0, i1) of one batch.
-void format_slice(const Args& a, const rbg_seed_result& r, const ReadBatch& b, uint64_t i0, uint64_t i1, std::string& o) {
+// The report of reads [i0, i1) of one batch, built in a string of the formatter thread (it keeps its capacity from slice
+// to slice) and copied into the slice's buffer.
+void format_slice(const Args& a, const rbg_seed_result& r, const ReadBatch& b, uint64_t i0, uint64_t i1, rbhost::OutBuf& out) {
+    thread_local std::string o;
     o.clear();
     o.reserve((size_t) ((r.seed_off[2 * i1] - r.seed_off[2 * i0]) * 40 + (i1 - i0) * 16));
     std::vector<Seed> seeds;
@@ -217,8 +189,11 @@ void format_slice(const Args& a, const rbg_seed_result& r, const ReadBatch& b, u
         size_t nl;
         const char* nm = b.name(i, nl);
         if (!a.heuristic) {                                     // worker, :347-415
-            for (int s = 0; s < 2; ++s)
-                for (uint64_t j = r.seed_off[2 * i + s]; j < r.seed_off[2 * i + s + 1]; ++j) print_raw_seed(o, nm, nl, r, j, s);
+            for (int s = 0; s < 2; ++s)                         // straight from the result arrays: ~10 seeds per read
+                for (uint64_t j = r.seed_off[2 * i + s]; j < r.seed_off[2 * i + s + 1]; ++j) {
+                    const rbg_seed& g = r.seeds[j];
+                    print_seed(o, nm, nl, g.hi - g.lo + 1, s, seed_query_start(g), g.query_len, r.markers + g.mk_off, g.mk_cnt);
+                }
             continue;
         }
         // worker_heuristic, :416-507: a random strand first, the other one only if no seed of the first asked to stop
@@ -247,11 +222,12 @@ void format_slice(const Args& a, const rbg_seed_result& r, const ReadBatch& b, u
                 if (s.strand == strand) kept.push_back(std::move(s));
             seeds.swap(kept);
         }
-        for (const Seed& s : seeds) print_seed(o, nm, nl, s);
+        for (const Seed& s : seeds) print_seed(o, nm, nl, s.range_size, s.strand, s.query_start, s.query_len, s.markers.data(), s.markers.size());
     }
+    out.reserve(o.size());
+    if (!o.empty()) memcpy(out.p, o.data(), o.size());
+    out.len = o.size();
 }
-
-using rbhost::Channel;
 
 }  // namespace
 
@@ -262,138 +238,54 @@ int main(int argc, char** argv) {
     std::cerr << "(gpu) loading rowbowt + markers";
     if (args.ftab) std::cerr << " and ftab";
     std::cerr << std::endl;
-    const int ndev = rbg_device_count();
-    if (ndev <= 0) {
-        fprintf(stderr, "no CUDA device available (this build has no CPU path)\n");
+    const uint32_t flags = RBG_LOAD_MA | (args.ftab ? RBG_LOAD_FT : 0) | (args.fbb ? RBG_LOAD_FBB : 0) | (args.layout_cache ? RBG_LOAD_CACHE : 0);       // load_rbwt, src/rb_markers.cpp:534-542
+    rbhost::QueryPipeline<rbg_seed_result>::Options po;
+    po.fastq = args.fastq;
+    po.threads = args.threads > 1 ? (int) args.threads : (int) std::max(1u, std::thread::hardware_concurrency());
+    po.batch_reads = args.batch_reads;
+    po.gpus = args.gpus;
+    po.workers_per_gpu = 1;
+    po.slice_shift = 11;
+    rbhost::QueryPipeline<rbg_seed_result> pipe(std::move(po));
+    std::string msg;
+    if (pipe.open(args.inpre.c_str(), flags, nullptr, msg)) {
+        std::cerr << msg << std::endl;
         return 1;
     }
-    const int gpus = std::min(args.gpus, ndev);
-    const uint32_t flags = RBG_LOAD_MA | (args.ftab ? RBG_LOAD_FT : 0) | (args.fbb ? RBG_LOAD_FBB : 0) | (args.layout_cache ? RBG_LOAD_CACHE : 0);       // load_rbwt, src/rb_markers.cpp:534-542
-    std::vector<rbg_index*> idx(gpus, nullptr);
-    for (int g = 0; g < gpus; ++g) {
-        if (rbg_index_open(args.inpre.c_str(), flags, g, &idx[g]) != RBG_OK) {
-            std::cerr << rbg_last_error() << std::endl;
-            return 1;
-        }
-    }
+    const bool input_ok = pipe.finish_load();
     std::chrono::duration<double> diff = clk::now() - t0;
     std::cerr << "loading rowbowt + markers took: " << diff.count() << " seconds\n";
-    t0 = clk::now();
-    // host pipeline as in rb_align: parser threads over the mmap'ed FASTQ -> GPU workers -> formatter pool -> ordered writer
-    const int host_threads = args.threads > 1 ? (int) args.threads : (int) std::max(1u, std::thread::hardware_concurrency());
-    const size_t pool = 2 * (size_t) host_threads + 4 * (size_t) gpus + 4;
-    rbhost::FastxBatchSource src(args.fastq.c_str(), host_threads, 0, args.batch_reads, rbhost::HostAlloc{rbg_host_alloc, rbg_host_free}, pool);
-    if (!src.ok()) {
+    if (!input_ok) {
         fprintf(stderr, "invalid file\n");
         return 1;
     }
-    rbg_greedy_params gp{args.wsize, args.max_range, args.min_range, (uint32_t) args.ftab, 0};
-
-    struct Job {                                   // one batch between its query and its last formatted slice
-        std::unique_ptr<ReadBatch> b;
-        rbg_seed_result res;
-        std::atomic<int> left{0};
-        int gpu = 0;
-    };
-    struct Slice { Job* job; int s; uint64_t i0, i1; };
-    Channel<std::unique_ptr<ReadBatch>> to_gpu(2 * gpus), to_writer(pool);
-    Channel<Slice> to_format(64 * (size_t) host_threads);
-    std::mutex inflight_m;
-    std::condition_variable inflight_cv;
-    std::vector<int> inflight(gpus, 0);            // seed results of device g not yet freed
-
-    std::vector<std::thread> workers, formatters;
-    for (int g = 0; g < gpus; ++g)
-        workers.emplace_back([&, g] {
-            std::unique_ptr<ReadBatch> b;
-            while (to_gpu.pop(b)) {
-                {
-                    std::unique_lock<std::mutex> l(inflight_m);
-                    inflight_cv.wait(l, [&] { return inflight[g] < 3; });
-                    ++inflight[g];
-                }
-                Job* job = new Job;
-                rbg_batch in{b->n, b->bases.p, b->offs.p};
-                if (rbg_markers_greedy(idx[g], &in, &gp, &job->res) != RBG_OK) {
-                    // the reference exits (k - 1 > wsize) or dies on an uncaught std::out_of_range (read shorter than k) here
-                    fprintf(stderr, "ERROR: %s\n", rbg_last_error());
-                    exit(1);
-                }
-                job->gpu = g;
-                const uint64_t n = b->n;
-                const int slices = (int) std::max<uint64_t>(1, std::min<uint64_t>((uint64_t) host_threads, n >> 11));
-                b->out.resize(slices);
-                job->b = std::move(b);
-                job->left = slices;
-                for (int s = 0; s < slices; ++s)
-                    to_format.push(Slice{job, s, n * (uint64_t) s / slices, n * (uint64_t) (s + 1) / slices});
-            }
-        });
-    for (int t = 0; t < host_threads; ++t)
-        formatters.emplace_back([&] {
-            Slice sl;
-            while (to_format.pop(sl)) {
-                Job* job = sl.job;
-                format_slice(args, job->res, *job->b, sl.i0, sl.i1, job->b->out[sl.s]);
-                if (job->left.fetch_sub(1) == 1) {
-                    const int g = job->gpu;
-                    rbg_seed_result_free(&job->res);
-                    {
-                        std::lock_guard<std::mutex> l(inflight_m);
-                        --inflight[g];
-                    }
-                    inflight_cv.notify_all();
-                    to_writer.push(std::move(job->b));
-                    delete job;
-                }
-            }
-        });
-    std::thread writer([&] {
-        std::map<uint64_t, std::unique_ptr<ReadBatch>> pending;
-        uint64_t next = 0;
-        std::unique_ptr<ReadBatch> b;
-        while (to_writer.pop(b)) {
-            pending[b->id] = std::move(b);
-            for (auto it = pending.find(next); it != pending.end(); it = pending.find(next)) {
-                for (const std::string& o : it->second->out) rbhost::write_all(1, o.data(), o.size());
-                src.recycle(std::move(it->second));
-                pending.erase(it);
-                ++next;
-            }
-        }
-    });
-
+    const rbg_greedy_params gp{args.wsize, args.max_range, args.min_range, (uint32_t) args.ftab, 0};
     // RandomBoolGenerator, src/rb_markers.cpp:225-240: one bit per read IN INPUT ORDER, 32 per draw of a default-seeded
-    // mt19937 -- batches leave the source in input order, so the bits are dealt here, on the one thread that sees them all
+    // mt19937 -- batches leave the source in input order, so the bits are dealt on the one thread that sees them all
     std::mt19937 rng;
     uint32_t bits = 0;
     int bit_count = 0;
-    while (std::unique_ptr<ReadBatch> b = src.next()) {
-        if (args.heuristic) {
-            b->aux.resize(b->n);
-            for (uint64_t i = 0; i < b->n; ++i) {
+    const double counting = pipe.run(
+        [&](rbg_index* ix, ReadBatch& b, rbg_seed_result& res) {
+            rbg_batch in{b.n, b.bases.p, b.offs.p};
+            if (rbg_markers_greedy(ix, &in, &gp, &res) != RBG_OK) {
+                // the reference exits (k - 1 > wsize) or dies on an uncaught std::out_of_range (read shorter than k) here
+                fprintf(stderr, "ERROR: %s\n", rbg_last_error());
+                exit(1);
+            }
+        },
+        rbg_seed_result_free,
+        [&](const rbg_seed_result& res, const ReadBatch& b, uint64_t i0, uint64_t i1, rbhost::OutBuf& out) { format_slice(args, res, b, i0, i1, out); },
+        [&](ReadBatch& b) {
+            if (!args.heuristic) return;
+            b.aux.resize(b.n);
+            for (uint64_t i = 0; i < b.n; ++i) {
                 if (bit_count == 0) { bits = (uint32_t) rng(); bit_count = 32; }
-                b->aux[i] = (bits & 1u) ? 0 : 1;                // get_bool() ? FWD : REV
+                b.aux[i] = (bits & 1u) ? 0 : 1;                // get_bool() ? FWD : REV
                 bits >>= 1;
                 --bit_count;
             }
-        }
-        to_gpu.push(std::move(b));
-    }
-    const int err = src.err();
-    to_gpu.close();
-    for (auto& w : workers) w.join();
-    to_format.close();
-    for (auto& f : formatters) f.join();
-    to_writer.close();
-    writer.join();
-    for (auto* ix : idx) rbg_index_close(ix);
-    switch (err) {                      // src/rb_markers.cpp:584-593
-        case -2: fprintf(stderr, "ERROR: truncated quality string\n"); exit(1);
-        case -3: fprintf(stderr, "ERROR: error reading stream\n"); exit(1);
-        default: break;
-    }
-    diff = clk::now() - t0;
-    std::cerr << "counting markers took: " << diff.count() << " seconds" << std::endl;
+        });
+    std::cerr << "counting markers took: " << counting << " seconds" << std::endl;
     return 0;
 }

@@ -18,6 +18,7 @@ import rowbowt_b200 as rb
 
 HEADER = os.path.join(ROOT, "include", "rowbowt_gpu.h")
 RB_ALIGN = os.path.join(ROOT, "rowbowt_b200", "rb_align")
+RB_MARKERS = os.path.join(ROOT, "rowbowt_b200", "rb_markers")
 
 
 def declared_symbols():
@@ -100,9 +101,10 @@ def test_fails_loudly_without_gpu(tmp_path):
         rb.build_marker_array(raw, mps, str(tmp_path / "o.ma"))
     assert e.value.code == -4 and "no CPU fallback" in str(e.value)
     assert not os.path.exists(str(tmp_path / "built.rbwt")) and not os.path.exists(str(tmp_path / "o.ma"))
-    p = subprocess.run([RB_ALIGN, os.path.join(GOLDEN, "toy", "small.fa"), os.path.join(GOLDEN, "toy", "simple_query.fq")],
-                       capture_output=True, text=True)
-    assert p.returncode == 1 and p.stdout == "" and "no CUDA device" in p.stderr
+    for driver in (RB_ALIGN, RB_MARKERS):
+        p = subprocess.run([driver, os.path.join(GOLDEN, "toy", "small.fa"), os.path.join(GOLDEN, "toy", "simple_query.fq")],
+                           capture_output=True, text=True)
+        assert p.returncode == 1 and p.stdout == "" and "no CUDA device" in p.stderr, driver
 
 
 def test_open_errors_are_codes_not_aborts(tmp_path):

@@ -7,6 +7,7 @@ live binary when oracle/_ref is present.
 GPU (-m gpu): rbg_markers_greedy through the C ABI against the oracle (every seed record and marker
 word, bit-exact) and the host rb_markers binary against the reference's stdout, byte for byte.
 """
+import gzip
 import json
 import os
 import shutil
@@ -120,22 +121,70 @@ def test_gpu_seeds_match_oracle_and_reference_stdout(c):
     ix.close()
 
 
-@pytest.mark.gpu
-@pytest.mark.parametrize("c", CASES, ids=case_id)
-def test_rb_markers_binary_matches_reference_stdout(c, tmp_path):
-    """The host rb_markers over the C ABI prints byte-for-byte what the reference printed at --threads 1,
-    including the --heuristic post-filters (random first strand, best strand, conflicting / identical markers)."""
+def _case_prefix(c, tmp_path):
+    """The case's index prefix; with --ftab, a copy in tmp_path beside the committed seed table."""
     prefix = os.path.join(GOLDEN, c["fixture"], c["prefix"])
     if c["ftab_k"]:
         for suf in (".rbwt", ".mab"):
             shutil.copy(prefix + suf, tmp_path / (c["prefix"] + suf))
         shutil.copy(os.path.join(EXP, "%s.k%d.ftab" % (c["fixture"], c["ftab_k"])), tmp_path / (c["prefix"] + ".ftab"))
         prefix = str(tmp_path / c["prefix"])
+    return prefix
+
+
+def _gzipped_fastq(c, tmp_path):
+    """The case's FASTQ as one gzip stream: it goes through the sequential reader, which cuts batches of --batch reads."""
+    gz = tmp_path / (c["fastq"] + ".gz")
+    with open(os.path.join(GOLDEN, c["fixture"], c["fastq"]), "rb") as f, gzip.open(gz, "wb") as g:
+        g.write(f.read())
+    return str(gz)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("c", CASES, ids=case_id)
+def test_rb_markers_binary_matches_reference_stdout(c, tmp_path):
+    """The host rb_markers over the C ABI prints byte-for-byte what the reference printed at --threads 1,
+    including the --heuristic post-filters (random first strand, best strand, conflicting / identical markers)."""
+    prefix = _case_prefix(c, tmp_path)
     for batch in ("37", "100000"):
         p = subprocess.run([RB_MARKERS, "--batch", batch] + c["flags"] + [prefix, os.path.join(GOLDEN, c["fixture"], c["fastq"])],
                            capture_output=True)
         assert p.returncode == 0, p.stderr.decode()
         assert p.stdout == open(os.path.join(EXP, c["out"]), "rb").read()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("c", CASES, ids=case_id)
+def test_rb_markers_three_workers_ordered_reassembly(c, tmp_path):
+    """rb_markers --gpus 3 over batches of 37 reads: three GPU workers (mapped onto the visible devices modulo their
+    number, RBG_GPU_MODULO) feed the formatter pool and the ordered writer; stdout must still be the reference's."""
+    cmd = [RB_MARKERS, "--gpus", "3", "--threads", "4", "--batch", "37"] + c["flags"] + [_case_prefix(c, tmp_path), _gzipped_fastq(c, tmp_path)]
+    p = subprocess.run(cmd, capture_output=True, env=dict(os.environ, RBG_GPU_MODULO="1"))
+    assert p.returncode == 0, p.stderr.decode()
+    assert p.stdout == open(os.path.join(EXP, c["out"]), "rb").read()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("c", CASES, ids=case_id)
+def test_rb_markers_stdout_to_a_file_is_the_same_report(c, tmp_path):
+    """stdout redirected to a regular file takes the positional writer (slices pwritten concurrently at their offsets):
+    from offset 0, behind bytes already in the file, and -- opened O_APPEND, where pwrite ignores offsets -- the
+    sequential writer; the file must hold exactly the reference's report every time."""
+    want = open(os.path.join(EXP, c["out"]), "rb").read()
+    cmd = [RB_MARKERS, "--threads", "4", "--batch", "37"] + c["flags"] + [_case_prefix(c, tmp_path), _gzipped_fastq(c, tmp_path)]
+    out = str(tmp_path / "report.txt")
+    with open(out, "wb") as f:
+        assert subprocess.run(cmd, stdout=f, stderr=subprocess.PIPE).returncode == 0
+    assert open(out, "rb").read() == want
+    fd = os.open(out, os.O_WRONLY | os.O_CREAT | os.O_TRUNC)
+    os.write(fd, b"header line\n")
+    assert subprocess.run(cmd, stdout=fd, stderr=subprocess.PIPE).returncode == 0
+    os.write(fd, b"trailer\n")                        # the shared file position was left behind the report
+    os.close(fd)
+    assert open(out, "rb").read() == b"header line\n" + want + b"trailer\n"
+    with open(out, "ab") as f:
+        assert subprocess.run(cmd, stdout=f, stderr=subprocess.PIPE).returncode == 0
+    assert open(out, "rb").read() == b"header line\n" + want + b"trailer\n" + want
 
 
 @pytest.mark.gpu

@@ -5,6 +5,9 @@
 
   python tools/e2e_binaries.py [--config c2] [--reads 2000000] [--ref-reads 40000] [--out gpurun_out/e2e.json]
 
+--bin-dir times the rb_align of another build (for instance the parent commit's, built with
+`make -C rowbowt_b200/csrc OUTDIR=DIR`), so that two builds can be alternated on the same machine.
+
 For every flag set ("", -s, -m, -s -m):
   * wall time of our rb_align over the whole FASTQ (stdout to a file on the box's disk),
     its own "<load_s> <query_s>" stderr line, reads/s from both;
@@ -44,6 +47,7 @@ def main():
     ap.add_argument("--ref-reads", type=int, default=40_000)
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--skip-locate", action="store_true", help="leave out the -s runs (their text output is ~1.4 KB per read)")
+    ap.add_argument("--bin-dir", default=os.path.join(ROOT, "rowbowt_b200"), help="directory of the rb_align to time")
     ap.add_argument("--tmp", default="/tmp/rbg_e2e")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "e2e_binaries.json"))
     a = ap.parse_args()
@@ -57,11 +61,11 @@ def main():
     fq_ref = os.path.join(a.tmp, "reads_ref.fq")
     synth.write_fastq(reads, fq)
     synth.write_fastq(reads[:a.ref_reads], fq_ref)
-    ours = os.path.join(ROOT, "rowbowt_b200", "rb_align")
+    ours = os.path.join(os.path.abspath(a.bin_dir), "rb_align")
     ref = os.path.join(ROOT, "oracle", "_ref", "rb_align")
     have_ma = os.path.exists(prefix + ".mab")
     have_sa = os.path.exists(prefix + ".tsa")
-    res = {"config": a.config, "reads": a.reads, "ref_reads": a.ref_reads, "gpus": a.gpus, "host_cores": os.cpu_count(),
+    res = {"config": a.config, "bin_dir": os.path.dirname(ours), "reads": a.reads, "ref_reads": a.ref_reads, "gpus": a.gpus, "host_cores": os.cpu_count(),
            "fastq_bytes": os.path.getsize(fq), "runs": []}
     for flags in ([], ["-s"], ["-m"], ["-s", "-m"]):
         if ("-s" in flags and (not have_sa or a.skip_locate)) or ("-m" in flags and not have_ma):

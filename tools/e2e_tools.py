@@ -8,6 +8,9 @@ unmodified reference binaries under oracle/_ref:
 
   python tools/e2e_tools.py [--markers-config c2] [--reads 1000000] [--ref-reads 100000]
                             [--build-config medium] [--out gpurun_out/e2e_tools.json]
+
+--bin-dir times the rb_markers / rb_build of another build (for instance the parent commit's, built with
+`make -C rowbowt_b200/csrc OUTDIR=DIR`), so that two builds can be alternated on the same machine.
 """
 import argparse
 import filecmp
@@ -23,7 +26,6 @@ sys.path.insert(0, ROOT)
 from tools import synth  # noqa: E402
 
 REF = os.path.join(ROOT, "oracle", "_ref")
-OURS = os.path.join(ROOT, "rowbowt_b200")
 
 
 def timed(cmd, out_path=None):
@@ -57,17 +59,17 @@ def markers(a, res):
     synth.write_fastq(reads, fq)
     synth.write_fastq(reads[:a.ref_reads], fq_ref)
     cores = os.cpu_count() or 1
-    out = {"config": a.markers_config, "reads": a.reads, "ref_reads": a.ref_reads, "host_cores": cores, "runs": []}
+    out = {"config": a.markers_config, "bin_dir": a.bin_dir, "reads": a.reads, "ref_reads": a.ref_reads, "host_cores": cores, "runs": []}
     for extra in ([], ["--heuristic", "--read-len", "150"]):
         o_all = os.path.join(a.tmp, "mk_ours.txt")
-        wall, err = timed([os.path.join(OURS, "rb_markers")] + extra + [prefix, fq], o_all)
+        wall, err = timed([os.path.join(a.bin_dir, "rb_markers")] + extra + [prefix, fq], o_all)
         q = seconds(err, "counting markers took")
         row = {"flags": " ".join(extra), "ours": {"wall_s": wall, "query_s": q, "reads_per_s_query": a.reads / q if q else None}}
         if os.path.exists(os.path.join(REF, "rb_markers")):
             o_ref, o_sub = os.path.join(a.tmp, "mk_ref.txt"), os.path.join(a.tmp, "mk_ours_sub.txt")
             rwall, rerr = timed([os.path.join(REF, "rb_markers"), "--threads", str(cores)] + extra + [prefix, fq_ref], o_ref)
             rq = seconds(rerr, "counting markers took")
-            timed([os.path.join(OURS, "rb_markers")] + extra + [prefix, fq_ref], o_sub)
+            timed([os.path.join(a.bin_dir, "rb_markers")] + extra + [prefix, fq_ref], o_sub)
             same = sorted(open(o_ref, "rb").read().split(b"\n")) == sorted(open(o_sub, "rb").read().split(b"\n"))
             row["reference"] = {"wall_s": rwall, "query_s": rq, "threads": cores, "reads_per_s_query": a.ref_reads / rq if rq else None}
             row["lines_identical_as_multiset"] = bool(same)
@@ -86,8 +88,8 @@ def build(a, res):
     flags = ["-s"] + (["-m"] if os.path.exists(prefix + ".ma") else [])
     o_pre, r_pre = os.path.join(a.tmp, "b_ours"), os.path.join(a.tmp, "b_ref")
     out = {"config": a.build_config, "bwt_bytes": os.path.getsize(prefix + ".bwt"), "flags": " ".join(flags)}
-    timed([os.path.join(OURS, "rb_build")] + flags + ["-o", o_pre, prefix])          # warm the page cache / the driver
-    wall, err = timed([os.path.join(OURS, "rb_build")] + flags + ["-o", o_pre, prefix])
+    timed([os.path.join(a.bin_dir, "rb_build")] + flags + ["-o", o_pre, prefix])          # warm the page cache / the driver
+    wall, err = timed([os.path.join(a.bin_dir, "rb_build")] + flags + ["-o", o_pre, prefix])
     out["ours"] = {"wall_s": wall, "stderr_summary": err.strip().split("\n")[-1]}
     if os.path.exists(os.path.join(REF, "rb_build")):
         rwall, _ = timed([os.path.join(REF, "rb_build")] + flags + ["-o", r_pre, prefix])
@@ -105,9 +107,11 @@ def main():
     ap.add_argument("--reads", type=int, default=1_000_000)
     ap.add_argument("--ref-reads", type=int, default=100_000)
     ap.add_argument("--build-config", default="medium")
+    ap.add_argument("--bin-dir", default=os.path.join(ROOT, "rowbowt_b200"), help="directory of the rb_markers / rb_build to time")
     ap.add_argument("--tmp", default="/tmp/rbg_e2e")
     ap.add_argument("--out", default=os.path.join(ROOT, "gpurun_out", "e2e_tools.json"))
     a = ap.parse_args()
+    a.bin_dir = os.path.abspath(a.bin_dir)
     os.makedirs(a.tmp, exist_ok=True)
     os.makedirs(os.path.dirname(a.out), exist_ok=True)
     res = {}
