@@ -12,12 +12,12 @@
 #include <algorithm>
 #include <chrono>
 #include <condition_variable>
-#include <cstdlib>
 #include <cstring>
 #include <future>
 #include <memory>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "cuda_host.hpp"
@@ -27,6 +27,7 @@
 #include "raw_build.hpp"
 #include "sdsl_writer.hpp"
 #include "kernels.cuh"
+#include "knobs.hpp"
 #include "layout.hpp"
 #include "ma_build.hpp"
 
@@ -134,8 +135,7 @@ struct Lane {
         CU(cudaEventSynchronize(ev_done[slot]));
     }
     void create() {
-        const char* e = getenv("RBG_BLOCKING_SYNC");
-        blocking = e && atoi(e) > 0;
+        blocking = knob_blocking_sync();
         const unsigned wait_flags = cudaEventDisableTiming | (blocking ? cudaEventBlockingSync : 0u);
         for (auto& ev1 : ev_done) CU(cudaEventCreateWithFlags(&ev1, wait_flags));
         CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
@@ -382,22 +382,23 @@ void save_ftab(const rbg_index* ix, const std::string& path) {
 // Opening an index decodes the reference's serializations and re-lays them out for the GPU: ~1.3-2.2 s for the BASELINE
 // index where the reference maps its files in 0.05-0.5 s.  With RBG_LOAD_CACHE the device arrays of the finished layout are
 // written once to <prefix>.rbgcache and later opens upload them as they are.  The cache is valid only for exactly
-// these index files (size + mtime of each part), these load flags, this library's layout version and the layout knobs of
-// the environment; anything else rebuilds and rewrites it.  The index files stay the source of truth.
+// these index files (size + mtime of each part), these load flags, this library's layout version and the layout knobs the
+// open read; anything else rebuilds and rewrites it.  The index files stay the source of truth.
 constexpr uint64_t kCacheMagic = 0x3145484341434752ull;       // "RGCACHE1"
-constexpr uint32_t kCacheVersion = 3;                         // bump when a device structure or its meaning changes
+constexpr uint32_t kCacheVersion = 4;                         // bump when a device structure or its meaning changes
 
 struct CacheHeader {
     uint64_t magic;
     uint32_t version, flags;
     uint64_t file_size[3], file_mtime_ns[3];                  // .rbwt, .tsa, .mab (0 when not loaded)
-    uint32_t sizeof_dir, sizeof_toe, sizeof_phi, sizeof_mk, sizeof_info, sizeof_codes;
-    char knobs[160];                                           // RBG_LAYOUT / RBG_WINDOW / RBG_PHI_SHIFT / RBG_TOEHOLD_SHIFT as set
+    uint32_t sizeof_dir, sizeof_toe, sizeof_phi, sizeof_mk, sizeof_info, sizeof_codes, sizeof_knobs;
+    LayoutKnobs knobs;                                         // what the layout was built with
     uint32_t n_blobs;
     int32_t field_blob[15];                                    // which blob each device pointer of the structs refers to, -1 = null
 };
+static_assert(std::has_unique_object_representations_v<CacheHeader>, "headers are compared with memcmp: no padding");
 
-CacheHeader cache_stamp(const std::string& pre, uint32_t flags) {
+CacheHeader cache_stamp(const std::string& pre, uint32_t flags, const LayoutKnobs& knobs) {
     CacheHeader h{};
     h.magic = kCacheMagic;
     h.version = kCacheVersion;
@@ -413,12 +414,8 @@ CacheHeader cache_stamp(const std::string& pre, uint32_t flags) {
     }
     h.sizeof_dir = sizeof(DevLeafDir); h.sizeof_toe = sizeof(DevToehold); h.sizeof_phi = sizeof(DevPhi);
     h.sizeof_mk = sizeof(DevMarkers); h.sizeof_info = sizeof(rbg_info); h.sizeof_codes = sizeof(CodeTable);
-    std::string k;
-    for (const char* name : {"RBG_LAYOUT", "RBG_WINDOW", "RBG_PHI_SHIFT", "RBG_TOEHOLD_SHIFT"}) {
-        const char* v = getenv(name);
-        k += std::string(name) + "=" + (v ? v : "") + ";";
-    }
-    strncpy(h.knobs, k.c_str(), sizeof h.knobs - 1);
+    h.sizeof_knobs = sizeof(LayoutKnobs);
+    h.knobs = knobs;
     return h;
 }
 
@@ -436,8 +433,8 @@ void cache_fields(rbg_index* ix, const void*** f) {
 }
 
 // After open_from_arrays: dir.super already points into the hot region; its blob is the second upload (owned[1]).
-void write_layout_cache(rbg_index* ix, const std::string& pre, uint32_t flags) {
-    CacheHeader h = cache_stamp(pre, flags);
+void write_layout_cache(rbg_index* ix, const std::string& pre, uint32_t flags, const LayoutKnobs& knobs) {
+    CacheHeader h = cache_stamp(pre, flags, knobs);
     if (ix->owned.size() < 2) return;
     const void** f[15];
     cache_fields(ix, f);
@@ -482,12 +479,12 @@ std::unique_ptr<rbg_index> new_index(int device) {
     select_device(device);
     std::unique_ptr<rbg_index> ix(new rbg_index);
     ix->device = device;
-    if (const char* e = getenv("RBG_LANES")) ix->max_lanes = std::max(1, std::min(8, atoi(e)));
+    ix->max_lanes = knob_lanes();
     return ix;
 }
 
 // nullptr when there is no valid cache for (prefix, flags)
-std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t flags, int device) {
+std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t flags, int device, const LayoutKnobs& knobs) {
     const std::string path = pre + ".rbgcache";
     const int fd = open(path.c_str(), O_RDONLY);
     if (fd < 0) return nullptr;
@@ -500,7 +497,7 @@ std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t fl
     struct Unmap { const char* p; size_t n; ~Unmap() { munmap((void*) p, n); } } unmap{m, size};
     CacheHeader h;
     memcpy(&h, m, sizeof h);
-    CacheHeader want = cache_stamp(pre, flags);
+    CacheHeader want = cache_stamp(pre, flags, knobs);
     want.n_blobs = h.n_blobs;
     memcpy(want.field_blob, h.field_blob, sizeof want.field_blob);
     if (memcmp(&h, &want, sizeof h) != 0) return nullptr;      // other files, flags, library version or knobs
@@ -542,16 +539,15 @@ std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t fl
 // The pair directory, when the count search gains from it: a layout-5 index with n < 2^32 whose pair directory stays
 // within kPairBudget -- small enough to stay resident in L2 beside the single-base directory, where the search is bound by
 // instructions and two bases per step take fewer of them than two steps -- and whose superblock table fits shared memory.
-// Larger indexes are bound by their line gathers, which the pair directory would only multiply.  RBG_PAIR=0|1 (tests)
+// Larger indexes are bound by their line gathers, which the pair directory would only multiply.  knobs.pair = 0|1 (tests)
 // forces either form; 1 still needs layout 5, n < 2^32 and the shared-memory table.
 constexpr uint64_t kPairBudget = 64ull << 20;
-void build_pair(rbg_index* ix, const RunsBwt& bwt, const LeafDir& ld) {
-    const char* e = getenv("RBG_PAIR");
-    const int force = e && *e ? atoi(e) : -1;
+void build_pair(rbg_index* ix, const RunsBwt& bwt, const LeafDir& ld, const LayoutKnobs& knobs) {
+    const int force = knobs.pair;
     if (force == 0 || ld.version != 5 || (bwt.n >> 32)) return;
     // a line holds at most 12 runs of P, and P has at least as many runs as the BWT: skip what cannot fit without building it
     if (force != 1 && bwt.R * 64 / LeafFmt<6>::E > kPairBudget) return;
-    PairDir pd = build_pair_dir(bwt, ld);
+    PairDir pd = build_pair_dir(bwt, ld, knobs.pair_window);
     if (64 * pd.n_super > kPairMaxShared || (force != 1 && pd.bytes() > kPairBudget)) return;
     size_t acc = 0;
     DevPairDir& P = ix->pair;
@@ -575,7 +571,8 @@ void build_pair(rbg_index* ix, const RunsBwt& bwt, const LeafDir& ld) {
     ix->info.pair_window = pd.window;
 }
 
-std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerArrays* ma, int device) {
+std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArrays* tsa, const MarkerArrays* ma, int device,
+                                            const LayoutKnobs& knobs) {
     std::unique_ptr<rbg_index> ix = new_index(device);
 
     // caller-supplied arrays (rbg_index_open_arrays) and raw builds come here without passing a file reader
@@ -591,10 +588,10 @@ std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArr
     std::future<PhiDir> phi_job;
     if (tsa) {
         const uint64_t budget = phi_slot_budget();
-        phi_job = std::async(std::launch::async, [tsa, budget] { return build_phi_dir(*tsa, 0, budget); });
+        phi_job = std::async(std::launch::async, [tsa, budget, knobs] { return build_phi_dir(*tsa, knobs.phi_shift, knobs.phi_parts, budget); });
     }
     {
-        LeafDir ld = build_leaf_dir(bwt);
+        LeafDir ld = build_leaf_dir(bwt, knobs.window, knobs.layout);
         memcpy(F, ld.F, sizeof F);
         info.window = ld.window;
         info.layout = (uint32_t) ld.version;
@@ -613,12 +610,12 @@ std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArr
         set_fast_div(ix->dir);
         for (int t = 0; t < kMaxTerm; ++t) ix->dir.term_pos[t] = ld.term_pos[t];
         memcpy(ix->codes.code_of, ld.code_of, 256);
-        build_pair(ix.get(), bwt, ld);
+        build_pair(ix.get(), bwt, ld, knobs);
     }
     memcpy(info.F, F, sizeof info.F);
 
     if (tsa) {
-        ToeholdDir td = build_toehold_dir(bwt, F, *tsa);
+        ToeholdDir td = build_toehold_dir(bwt, F, *tsa, knobs.toehold_shift);
         acc = 0;
         ix->toe.table = upload(td.table, ix->owned, &acc);
         ix->toe.keys = upload(td.keys, ix->owned, &acc);
@@ -845,6 +842,7 @@ void collect_counters(Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t launches) {
 // path).  Leaves results on the device.
 void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mode, uint64_t max_hits, bool want_checksum) {
     const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS;
+    const QueryKnobs knobs = query_knobs(Lane::kMaxChunks);
     const LocForm lf(mode, ix->info.n);
     Views v = prepare(ix, rd, mode);
     DevBatch& b = v.b;
@@ -871,7 +869,7 @@ void run_staged(rbg_index* ix, Lane& L, rbg_stats& s, rbg_reads* rd, uint32_t mo
         if (lf.hi_plane) reserve(rd->locs_hi, rd->n_locs + 8);
         point_locs(rd, r, lf);
         CU(cudaEventRecord(L.ev[6], st));
-        launches += launch_locate(ix->phi, r, 0, n, rd->n_locs, L.d_ctr, &L.d_ctr->loc_cursor[0], st);
+        launches += launch_locate(ix->phi, r, 0, n, rd->n_locs, knobs.loc_draw, L.d_ctr, &L.d_ctr->loc_cursor[0], st);
     }
     CU(cudaEventRecord(L.ev[3], st));
     if (markers) {
@@ -949,6 +947,7 @@ void fetch_staged(rbg_index* ix, Lane& L, rbg_reads* rd, uint32_t mode, rbg_resu
 // Locate / marker output sizes are data dependent: see the comments at the locate and marker stages below.
 void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint32_t mode, uint64_t max_hits, rbg_result* out) {
     const bool locate = mode & RBG_LOCATE, markers = mode & RBG_MARKERS;
+    const QueryKnobs knobs = query_knobs(Lane::kMaxChunks);
     const LocForm lf(mode, ix->info.n);
     const size_t loc_item = lf.item();
     const bool narrow_rg = (mode & RBG_NARROW_RANGES) && !(ix->info.n >> 32);       // u32 planes of lo / hi on the wire
@@ -991,19 +990,11 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
     }
 
     // chunking: about 16 chunks, at least 64 K reads each
-    int n_chunks = (int) std::min<uint64_t>(16, std::max<uint64_t>(1, n >> 16));
-    if (const char* e = getenv("RBG_CHUNKS")) n_chunks = std::max(1, std::min(atoi(e), (int) Lane::kMaxChunks));
+    int n_chunks = knobs.chunks ? knobs.chunks : (int) std::min<uint64_t>(16, std::max<uint64_t>(1, n >> 16));
     if ((uint64_t) n_chunks > n) n_chunks = n ? (int) n : 1;
     auto cut = [&](int c) { return (uint64_t) ((__uint128_t) n * (uint64_t) c / (uint64_t) n_chunks); };
 
     uint32_t launches = 0;
-    // tests: RBG_TEST_STALL="a,b" stalls even chunks' stream for a microseconds in front of their pack and odd chunks' stream for
-    // b microseconds between their pack and their search
-    unsigned long long stall_ns[2] = {0, 0};
-    if (const char* e = getenv("RBG_TEST_STALL")) {
-        unsigned long long a = 0, bb = 0;
-        if (sscanf(e, "%llu,%llu", &a, &bb) >= 1) { stall_ns[0] = a * 1000ull; stall_ns[1] = bb * 1000ull; }
-    }
     CU(cudaEventRecord(L.ev_span[0], si));
     // offsets first (pack's flagging searches them), re-based to 0 when the caller's are not
     std::vector<uint64_t> rebased;
@@ -1056,9 +1047,9 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
         // first sizing: extrapolate from the chunks seen so far; later chunks only grow it when the guess was short
         uint64_t want = end;
         if (r1 < n && end > 0) want = std::max<uint64_t>(end, (uint64_t) ((double) end / (double) r1 * (double) n * 1.08) + 4096);
-        if (const char* e = getenv("RBG_LOC_EST")) want = std::max<uint64_t>(end, (uint64_t) atoll(e));      // tests: force regrowth
+        if (knobs.loc_est >= 0) want = std::max<uint64_t>(end, (uint64_t) knobs.loc_est);      // tests: force regrowth
         grow_locs(want);
-        launches += launch_locate(ix->phi, r, r0, r1, end - begin, L.d_ctr, &L.d_ctr->loc_cursor[c], sc);
+        launches += launch_locate(ix->phi, r, r0, r1, end - begin, knobs.loc_draw, L.d_ctr, &L.d_ctr->loc_cursor[c], sc);
         CU(cudaEventRecord(L.ev_loc[c], sc));
         CU(cudaStreamWaitEvent(so, L.ev_loc[c], 0));
         CU(cudaMemcpyAsync(out->loc_off + r0, r.loc_off + r0, (r1 - r0 + 1) * 8, cudaMemcpyDeviceToHost, so));
@@ -1097,11 +1088,11 @@ void run_pipelined(rbg_index* ix, Lane& L, rbg_stats& s, const BatchIn& in, uint
             // can land on top of the complete one while the later chunk is still searching (found by a parity failure under
             // compute-sanitizer's timing; RBG_TEST_STALL reproduces the order).  A search reading the word while the next
             // chunk's pack rewrites it sees the same bits for its own bases either way.
-            if (stall_ns[0] && !(c & 1)) launch_stall(stall_ns[0], ss);
+            if (knobs.stall_ns[0] && !(c & 1)) launch_stall(knobs.stall_ns[0], ss);
             if (c > 0) CU(cudaStreamWaitEvent(ss, L.ev_pack[c - 1], 0));
             launches += launch_pack(b, ix->codes, b1 - b0, ss);
             CU(cudaEventRecord(L.ev_pack[c], ss));
-            if (stall_ns[1] && (c & 1)) launch_stall(stall_ns[1], ss);
+            if (knobs.stall_ns[1] && (c & 1)) launch_stall(knobs.stall_ns[1], ss);
         }
         launches += launch_search(ix->dir, ix->pair, locate ? &ix->toe : nullptr, ix->ft, b, r, L.d_ctr, &L.d_ctr->cursor[c], ss);
         if (rd->has_bases) launches += launch_search_bytes(ix->dir, locate ? &ix->toe : nullptr, b, r, ix->codes, L.d_ctr, ss);
@@ -1287,8 +1278,9 @@ int rbg_index_open(const char* prefix, uint32_t flags, int device, rbg_index** o
         const std::string pre(prefix);
         if ((flags & RBG_LOAD_FBB) && (flags & RBG_LOAD_SA))
             return fail(RBG_E_ARG, "fbb_string does not support loading toehold suffix array");     // include/rowbowt_io.hpp:107
+        const LayoutKnobs knobs = layout_knobs();
         std::unique_ptr<rbg_index> ix;
-        if (flags & RBG_LOAD_CACHE) ix = open_layout_cache(pre, flags, device);
+        if (flags & RBG_LOAD_CACHE) ix = open_layout_cache(pre, flags, device, knobs);
         if (!ix) {
             // the three files are decoded at the same time (each reader is itself multi-threaded over its components)
             std::future<ToeholdArrays> tsa_job;
@@ -1300,10 +1292,10 @@ int rbg_index_open(const char* prefix, uint32_t flags, int device, rbg_index** o
             MarkerArrays ma;
             if (flags & RBG_LOAD_SA) tsa = tsa_job.get();
             if (flags & RBG_LOAD_MA) ma = ma_job.get();
-            ix = open_from_arrays(bwt, (flags & RBG_LOAD_SA) ? &tsa : nullptr, (flags & RBG_LOAD_MA) ? &ma : nullptr, device);
+            ix = open_from_arrays(bwt, (flags & RBG_LOAD_SA) ? &tsa : nullptr, (flags & RBG_LOAD_MA) ? &ma : nullptr, device, knobs);
             if (flags & RBG_LOAD_FBB) ix->codes.code_of[1] = -1;   // wt_fbb: terminator is byte 0, byte 1 is no symbol
             if (flags & RBG_LOAD_CACHE) {
-                try { write_layout_cache(ix.get(), pre, flags); } catch (...) { cudaGetLastError(); }      // best effort: the index is open either way
+                try { write_layout_cache(ix.get(), pre, flags, knobs); } catch (...) { cudaGetLastError(); }      // best effort: the index is open either way
             }
         }
         if (flags & RBG_LOAD_FT) {                  // ft_suffix :21, LoadRbwtFlag::FT :151
@@ -1356,7 +1348,7 @@ IndexArrays index_arrays_from_desc(const rbg_index_desc* d, bool tsa_only) {
 }
 
 std::unique_ptr<rbg_index> open_from_arrays(const IndexArrays& p, int device) {
-    return open_from_arrays(p.bwt, p.has_sa ? &p.tsa : nullptr, p.has_ma ? &p.ma : nullptr, device);
+    return open_from_arrays(p.bwt, p.has_sa ? &p.tsa : nullptr, p.has_ma ? &p.ma : nullptr, device, layout_knobs());
 }
 
 // rb_build's inputs (src/rb_build.cpp:76-87): <prefix>.bwt, .ssa/.esa, .ma
@@ -1422,7 +1414,7 @@ int rbg_build_index(const char* in_prefix, const char* out_prefix, uint32_t flag
         if (flags & RBG_LOAD_SA) write_tsa(p.tsa, out + ".tsa");           // :65-72
         st.s_write = wall_s() - t0;
         if (flags & RBG_LOAD_FT) {                                         // :82-88 (rb_build -f): build_ftab(k) + FTab::serialize
-            std::unique_ptr<rbg_index> ix = open_from_arrays(p.bwt, nullptr, nullptr, device);
+            std::unique_ptr<rbg_index> ix = open_from_arrays(p.bwt, nullptr, nullptr, device, layout_knobs());
             {
                 LaneHold hold(ix.get(), true);
                 build_ftab(ix.get(), hold.lane->stream, ftab_k ? ftab_k : 10);

@@ -1,5 +1,6 @@
 // See formats.hpp for the byte layouts and the reference lines they come from.
 #include "formats.hpp"
+#include "knobs.hpp"
 
 #include <algorithm>
 #include <thread>
@@ -493,8 +494,8 @@ RunsBwt read_rbwt_fbb(const std::string& path) {
         }
         part.n = sink.total;
     };
-    unsigned n_thr = n_sb >= 16 ? std::min<unsigned>(8, std::max(1u, std::thread::hardware_concurrency())) : 1;
-    if (const char* e = getenv("RBG_FBB_THREADS")) n_thr = (unsigned) std::max(1, std::min(64, atoi(e)));       // tests
+    unsigned n_thr = knob_fbb_threads();
+    if (n_thr == 0) n_thr = n_sb >= 16 ? std::min<unsigned>(8, std::max(1u, std::thread::hardware_concurrency())) : 1;
     n_thr = (unsigned) std::min<uint64_t>(n_thr, std::max<uint64_t>(1, n_sb));
     std::vector<RunsBwt> parts(n_thr);
     std::vector<std::string> errors(n_thr);

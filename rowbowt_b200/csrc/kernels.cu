@@ -9,7 +9,6 @@
 //   marker_*_kernel  rle_window_arr::at_range (pfbwt-f/include/rle_window_array.hpp:130-154)
 #include "kernels.cuh"
 
-#include <cstdlib>
 #include <stdexcept>
 
 #include <cub/device/device_scan.cuh>
@@ -652,11 +651,10 @@ static void launch_locate_form(bool draw, const DevPhi& P, const DevResult& r, u
     }
 }
 
-int launch_locate(const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, uint64_t n_locs, DevCounters* ctr,
+int launch_locate(const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, uint64_t n_locs, int force_draw, DevCounters* ctr,
                   unsigned long long* cursor, cudaStream_t st) {
     if (r1 <= r0) return 0;
-    const char* d = getenv("RBG_LOC_DRAW");                  // test override: 0 / 1 forces the static / drawing form
-    const bool draw = d ? atoi(d) != 0 : n_locs / (r1 - r0) >= 256;
+    const bool draw = force_draw >= 0 ? force_draw != 0 : n_locs / (r1 - r0) >= 256;
     if (r.locs_lo && r.locs_hi) launch_locate_form<true, true>(draw, P, r, r0, r1, ctr, cursor, st);
     else if (r.locs_lo) launch_locate_form<true, false>(draw, P, r, r0, r1, ctr, cursor, st);
     else launch_locate_form<false, false>(draw, P, r, r0, r1, ctr, cursor, st);

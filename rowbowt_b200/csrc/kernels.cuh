@@ -55,8 +55,9 @@ int launch_ftab_build(const DevLeafDir& D, uint32_t k, bool toehold, ulonglong2*
 int launch_search_bytes(const DevLeafDir& D, const DevToehold* T, const DevBatch& b, const DevResult& r,
                         const CodeTable& ct, DevCounters* ctr, cudaStream_t st);   // reads flagged kReadExotic
 int launch_locate_counts(const DevResult& r, uint64_t r0, uint64_t r1, uint64_t max_hits, cudaStream_t st);
-// n_locs: locations reads [r0, r1) will produce (chooses the static or the drawing kernel); cursor: zeroed device counter of this launch
-int launch_locate(const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, uint64_t n_locs, DevCounters* ctr,
+// n_locs: locations reads [r0, r1) will produce (chooses the static or the drawing kernel); force_draw: 0 / 1 forces the static /
+// drawing kernel, -1 lets n_locs choose; cursor: zeroed device counter of this launch
+int launch_locate(const DevPhi& P, const DevResult& r, uint64_t r0, uint64_t r1, uint64_t n_locs, int force_draw, DevCounters* ctr,
                   unsigned long long* cursor, cudaStream_t st);
 int launch_marker_counts(const DevMarkers& M, const DevResult& r, uint64_t r0, uint64_t r1, cudaStream_t st);
 int launch_marker_gather(const DevMarkers& M, const DevResult& r, uint64_t r0, uint64_t r1, DevCounters* ctr, cudaStream_t st);

@@ -3,7 +3,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <thread>
 
@@ -166,7 +165,7 @@ PredTable build_pred_table(std::vector<uint64_t>&& keys, uint64_t universe, doub
     return t;
 }
 
-LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window) {
+LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window, int layout) {
     LeafDir d;
     d.n = bwt.n;
     if (bwt.n == 0 || bwt.R == 0) throw format_error("empty BWT");
@@ -214,14 +213,10 @@ LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window) {
         else LeafWalker<4>{bwt, code, W, sb_shift_for(4, W)}.run(nullptr, c.children, c.clusters, d.Fcode, &c.stretch);
         return c;
     };
-    // Which layout: RBG_LAYOUT=4|5 forces one; otherwise 5 (no per-step superblock load) while its directory stays
+    // Which layout: `layout` 4|5 forces one; otherwise 5 (no per-step superblock load) while its directory stays
     // within the reach of the SM TLBs with room for the seed table and the reads (<= 224 MB), else 4 (3.8 instead of
     // 4.6 bytes per run: the gather rate falls 2.5x once the footprint passes 256 MB, profiles/r1_gather_sweep.jsonl).
-    int forced = 0;
-    if (const char* e = getenv("RBG_LAYOUT")) forced = atoi(e);
-    if (forced != 4 && forced != 5) forced = 0;
     uint32_t W = window;
-    if (W == 0) if (const char* e = getenv("RBG_WINDOW")) W = (uint32_t) atoi(e);
     auto choose_window = [&](int V, uint32_t& Wout, Count& chosen) {
         // aim at ~71 % of the entries used on average; try a ladder of eighths around it.  Cost of a candidate:
         // its lines (footprint decides the gather rate), inflated by the share of positions that fall inside a
@@ -252,10 +247,10 @@ LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window) {
         return ((bwt.n + Wout - 1) / Wout + chosen.children) * 64;       // directory bytes
     };
     Count chosen;
-    int V = forced ? forced : 5;
+    int V = layout ? layout : 5;
     if (W == 0) {
         uint64_t bytes = choose_window(V, W, chosen);
-        if (!forced && bytes > (224ull << 20)) {
+        if (!layout && bytes > (224ull << 20)) {
             V = 4;
             W = 0;
             bytes = choose_window(4, W, chosen);
@@ -417,7 +412,6 @@ PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window) {
         for (int c1 = 0; c1 < 4; ++c1) K[4 * c1 + c2] = (uint32_t) (d.Fcode[c1] + before[c1]);
     }
     uint32_t W = window;
-    if (W == 0) if (const char* e = getenv("RBG_PAIR_WINDOW")) W = (uint32_t) atoi(e);
     if (W == 0) {
         // the ladder of build_leaf_dir with E = 12; a rank in a CLUSTER window is answered by the whole warp from its raw
         // children, so those windows weigh as in the single-base cost model
@@ -444,7 +438,7 @@ PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window) {
     return P;
 }
 
-ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const ToeholdArrays& tsa) {
+ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const ToeholdArrays& tsa, uint32_t shift) {
     if (tsa.r != bwt.R || tsa.n != bwt.n) throw format_error("toehold SA does not match the BWT (r/n differ)");
     ToeholdDir t;
     // LF(end of run j) = F[c] + (#c in BWT[0, end_j]) - 1.  Visiting symbols in byte order and runs in
@@ -462,10 +456,12 @@ ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const
         rows[slot] = F[c] + seen[c] - 1;
         sample[slot] = tsa.samples_last[j];
     }
-    // bucket width: about three keys per bucket, so that the table (4 B per bucket) stays smaller than the keys' samples
-    uint32_t shift = 1;
-    while (shift < 32 && (double) (1ull << shift) < 2.0 * (double) bwt.n / (double) bwt.R) ++shift;
-    if (const char* e = getenv("RBG_TOEHOLD_SHIFT")) shift = (uint32_t) std::max(1, std::min(32, atoi(e)));      // tests: every key width
+    if (shift == 0) {
+        // bucket width: about three keys per bucket, so that the table (4 B per bucket) stays smaller than the keys' samples
+        shift = 1;
+        while (shift < 32 && (double) (1ull << shift) < 2.0 * (double) bwt.n / (double) bwt.R) ++shift;
+    }
+    if (shift > 32) throw std::runtime_error("toehold bucket shift out of range [1,32]");
     t.shift = shift;
     t.key_bytes = shift <= 8 ? 1 : shift <= 16 ? 2 : 4;
     t.n_keys = bwt.R;
@@ -508,7 +504,7 @@ uint64_t toehold_dir_rank(const ToeholdDir& t, uint64_t row) {
     return a;
 }
 
-PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift, uint64_t max_slot_bytes) {
+PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift, unsigned n_parts, uint64_t max_slot_bytes) {
     PhiDir p;
     const uint64_t r = tsa.r, n = tsa.n;
     if (r == 0) throw format_error("toehold SA without samples");
@@ -518,7 +514,6 @@ PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift, uint64_t max_slot
         // pred_to_run == 0 only for phi(SA[0]), which locate_range never evaluates (toehold_sa.hpp:65-66)
         return run ? tsa.samples_last[run - 1] : 0;
     };
-    if (shift == 0) if (const char* e = getenv("RBG_PHI_SHIFT")) shift = (uint32_t) atoi(e);
     if (shift == 0) {
         // 128-position buckets (the largest a BITMAP slot covers); larger ones only when the slots
         // would not fit the budget -- their crowded buckets are binary-searched instead
@@ -541,8 +536,7 @@ PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift, uint64_t max_slot
         std::string err;
     };
     auto group_of = [&](uint64_t k) { return (keys[k] >> shift) >> 5; };
-    unsigned n_parts = r > (1u << 20) ? std::min(8u, std::max(1u, std::thread::hardware_concurrency())) : 1u;
-    if (const char* e = getenv("RBG_PHI_PARTS")) n_parts = (unsigned) std::max(1, std::min(64, atoi(e)));      // tests
+    if (n_parts == 0) n_parts = r > (1u << 20) ? std::min(8u, std::max(1u, std::thread::hardware_concurrency())) : 1u;
     std::vector<Part> parts(n_parts);
     for (unsigned t = 0; t < n_parts; ++t) {
         uint64_t ka = r * t / n_parts;

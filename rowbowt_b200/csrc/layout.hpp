@@ -50,8 +50,9 @@ struct LeafDir {
     uint64_t term_pos[kMaxTerm] = {0};
 };
 
-// Validates the alphabet and builds the rank directory.  window = 0 -> choose automatically.
-LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window = 0);
+// Validates the alphabet and builds the rank directory.  window = 0 -> choose automatically; layout = 4 or 5 forces that
+// line format, 0 -> 5 while the directory stays small, else 4.
+LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window, int layout);
 
 // Pair directory (leaf.cuh, LeafFmt<6>): a rank directory over P[j] = (BWT[LF(j)], BWT[j]) with which the count search
 // takes two bases per LF step.  Built from the runs alone: the rows of BWT run k map under LF onto one contiguous interval
@@ -71,8 +72,8 @@ struct PairDir {
 // Runs of P in row order: code 0..15, or kPairBad for a row whose pair holds the terminator.
 constexpr uint8_t kPairBad = 16;
 void pair_runs(const RunsBwt& bwt, const LeafDir& d, std::vector<uint32_t>& lens, std::vector<uint8_t>& codes);
-// window = 0 -> choose (RBG_PAIR_WINDOW overrides).  Needs n < 2^32.
-PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window = 0);
+// window = 0 -> choose.  Needs n < 2^32.
+PairDir build_pair_dir(const RunsBwt& bwt, const LeafDir& d, uint32_t window);
 
 // Sorted u64 keys with a radix table: table[b] = #keys < (b << shift), b in [0, (universe>>shift)+1].
 struct PredTable {
@@ -126,9 +127,11 @@ struct PhiDir {
     uint64_t n_overflow = 0;             // BITMAP / SEARCH buckets
 };
 
-ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const ToeholdArrays& tsa);
-// shift = 0 -> choose (RBG_PHI_SHIFT overrides): 7, or the smallest larger one whose slots fit max_slot_bytes
-PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift = 0, uint64_t max_slot_bytes = 64ull << 30);
+// shift = 0 -> choose (about three keys per bucket), else buckets of 2^shift rows, shift <= 32
+ToeholdDir build_toehold_dir(const RunsBwt& bwt, const uint64_t (&F)[256], const ToeholdArrays& tsa, uint32_t shift);
+// shift = 0 -> choose: 7, or the smallest larger one whose slots fit max_slot_bytes.  n_parts = 0 -> choose how many host
+// threads build it (several only for large indexes)
+PhiDir build_phi_dir(const ToeholdArrays& tsa, uint32_t shift, unsigned n_parts, uint64_t max_slot_bytes);
 // phi(i) through the slots on the host (self-check): must equal ToeholdSA::phi for every i != SA[0]
 uint64_t phi_dir_eval(const PhiDir& p, uint64_t n, uint64_t i);
 PredTable build_pred_table(std::vector<uint64_t>&& keys, uint64_t universe, double keys_per_bucket);

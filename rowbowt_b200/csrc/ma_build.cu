@@ -18,13 +18,13 @@
 
 #include <algorithm>
 #include <cstdio>
-#include <cstdlib>
 #include <string>
 #include <vector>
 
 #include "ma_build.hpp"
 #include "cuda_host.hpp"
 #include "device_index.cuh"
+#include "knobs.hpp"
 #include "raw_build.hpp"
 #include "sdsl_writer.hpp"
 
@@ -138,7 +138,8 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
     const uint64_t j1 = (uint64_t) (std::upper_bound(start.begin(), start.end(), row_end - 1) - start.begin()) - 1;
 
     std::vector<Upload> owned;
-    const DevPhi P = upload_phi(build_phi_dir(tsa, 0, phi_slot_budget()), n, owned);
+    const LayoutKnobs knobs = layout_knobs();
+    const DevPhi P = upload_phi(build_phi_dir(tsa, knobs.phi_shift, knobs.phi_parts, phi_slot_budget()), n, owned);
 
     // directory over text positions: about one record per bucket, so it costs no more than the records themselves
     const uint64_t m = mps.first.size();
@@ -156,7 +157,7 @@ void build_marker_array(const RunsBwt& bwt, const ToeholdArrays& tsa, const MpsR
     CU(cudaMemGetInfo(&free_b, &total_b));
     const uint64_t per_row = 4 * 4 + 2 * sizeof(MaBlock);
     uint64_t cap = std::min<uint64_t>(kMaxChunkRows, (uint64_t) free_b / 2 / per_row);
-    if (const char* e = getenv("RBG_MA_CHUNK_ROWS")) cap = std::max<uint64_t>(1, std::min<uint64_t>(cap, strtoull(e, nullptr, 10)));
+    if (const uint64_t rows = knob_ma_chunk_rows()) cap = std::max<uint64_t>(1, std::min(cap, rows));
     uint64_t max_run = 0;
     for (uint64_t j = j0; j <= j1; ++j) max_run = std::max(max_run, bwt.lens[j]);
     const uint64_t rows_alloc = std::max(cap, std::min(max_run, row_end - row_begin));      // a chunk holds at least one run

@@ -14,6 +14,7 @@
 #include "../../include/rowbowt_gpu.h"
 #include "formats.hpp"
 #include "host_pack.hpp"
+#include "knobs.hpp"
 #include "layout.hpp"
 #include "leaf.cuh"
 #include "sdsl_writer.hpp"
@@ -72,10 +73,10 @@ extern "C" int rbg_selftest_layout(const char* prefix, uint32_t window, uint64_t
     try {
         RunsBwt bwt = read_rbwt(std::string(prefix) + ".rbwt");
         const uint32_t layout = window >> 16;                     // bits 16..: force layout 4 or 5 (0 = the loader's own choice)
-        window &= 0xFFFFu;
-        if (layout) setenv("RBG_LAYOUT", layout == 5 ? "5" : "4", 1);
-        LeafDir d = build_leaf_dir(bwt, window);
-        if (layout) unsetenv("RBG_LAYOUT");
+        LayoutKnobs k = layout_knobs();
+        if (window & 0xFFFFu) k.window = window & 0xFFFFu;
+        if (layout) k.layout = layout == 5 ? 5 : 4;
+        LeafDir d = build_leaf_dir(bwt, k.window, k.layout);
         if (layout && d.version != (int) layout) return 3;
         if (n_lines) *n_lines = d.n_lines();
         if (n_cluster) *n_cluster = d.n_cluster;
@@ -138,7 +139,9 @@ extern "C" int rbg_selftest_phi(const char* prefix, uint32_t shift, uint64_t str
                                 uint64_t* n_slots, uint64_t* n_overflow) {
     try {
         ToeholdArrays t = read_tsa(std::string(prefix) + ".tsa");
-        PhiDir p = build_phi_dir(t, shift & 0xFFu, (shift >> 8) ? (uint64_t) (shift >> 8) : ~0ull);     // bits 8.. = slot budget in bytes (0 = none)
+        LayoutKnobs k = layout_knobs();
+        if (shift & 0xFFu) k.phi_shift = shift & 0xFFu;
+        PhiDir p = build_phi_dir(t, k.phi_shift, k.phi_parts, (shift >> 8) ? (uint64_t) (shift >> 8) : ~0ull);     // bits 8.. = slot budget in bytes (0 = none)
         if (n_slots) *n_slots = p.n_slots;
         if (n_overflow) *n_overflow = p.n_overflow;
         auto direct = [&](uint64_t i) {
@@ -187,11 +190,10 @@ extern "C" int rbg_selftest_toehold(const char* prefix, uint32_t shift, uint64_t
     try {
         RunsBwt bwt = read_rbwt(std::string(prefix) + ".rbwt");
         ToeholdArrays t = read_tsa(std::string(prefix) + ".tsa");
-        LeafDir d = build_leaf_dir(bwt, 0);
-        char buf[16];
-        if (shift) { snprintf(buf, sizeof buf, "%u", shift); setenv("RBG_TOEHOLD_SHIFT", buf, 1); }
-        ToeholdDir td = build_toehold_dir(bwt, d.F, t);
-        if (shift) unsetenv("RBG_TOEHOLD_SHIFT");
+        LayoutKnobs k = layout_knobs();
+        if (shift) k.toehold_shift = shift;
+        LeafDir d = build_leaf_dir(bwt, k.window, k.layout);
+        ToeholdDir td = build_toehold_dir(bwt, d.F, t, k.toehold_shift);
         if (shift && td.shift != shift) return 3;
         if (dir_bytes) *dir_bytes = td.bytes();
         // per-symbol counts in front of every part's first run
@@ -268,10 +270,11 @@ extern "C" int rbg_selftest_pair(uint64_t n, const uint8_t* heads, const uint64_
         bwt.R = R;
         bwt.heads.assign(heads, heads + R);
         bwt.lens.assign(lens, lens + R);
-        setenv("RBG_LAYOUT", "5", 1);
-        LeafDir d = build_leaf_dir(bwt);
-        unsetenv("RBG_LAYOUT");
-        PairDir P = build_pair_dir(bwt, d, window);
+        LayoutKnobs k = layout_knobs();
+        k.layout = 5;
+        if (window) k.pair_window = window;
+        LeafDir d = build_leaf_dir(bwt, k.window, k.layout);
+        PairDir P = build_pair_dir(bwt, d, k.pair_window);
         if (n_lines) *n_lines = P.lines.size() / kLineWords;
         if (n_cluster) *n_cluster = P.n_cluster;
         std::vector<uint32_t> rl;

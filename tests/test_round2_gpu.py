@@ -292,6 +292,18 @@ def test_layout_cache_opens_the_same_index(name, tmp_path, monkeypatch):
     c = other.query(seqs, RBG_COUNT)
     assert np.array_equal(c.lo, want.lo) and np.array_equal(c.hi, want.hi)
     other.close()
+    monkeypatch.delenv("RBG_LAYOUT")
+    for knob, value in (("RBG_PAIR_WINDOW", "32"), ("RBG_PHI_PARTS", "3")):
+        served = []
+        for setting in (None, None, value):                   # rewritten without the knob, served, then the knob set
+            if setting:
+                monkeypatch.setenv(knob, setting)
+            ix = rb.GpuIndex.open(prefix, sa=True, markers=has_ma, cache=True)
+            served.append(ix.info().from_cache)
+            _same(want, ix.query(seqs, mode), mode)
+            ix.close()
+        monkeypatch.delenv(knob)
+        assert served[1:] == [1, 0], (knob, served)
 
 
 def test_layout_cache_concurrent_first_opens(tmp_path):
