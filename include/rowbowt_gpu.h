@@ -140,7 +140,8 @@ typedef struct {
     uint64_t n_cluster;             /* windows with more than 24 runs (densest stretch summarised, detail in raw children) */
     uint64_t dir_bytes, phi_bytes, toehold_bytes, marker_bytes;   /* device footprint */
     uint32_t ftab_k;                /* FTab::get_k() of the resident k-mer seed table, 0 = none */
-    uint32_t layout;                /* GPU layout of the rank directory: 4 (24 runs per line + L2-resident superblock counts) or 5 (20 runs, u32 counts in the line) */
+    uint32_t layout;                /* GPU layout of the rank directory: 4 (24 runs per line + L2-resident superblock counts), 5 (20 runs, u32 counts in the line)
+                                       or 7 (the BWT at 2 bits per row, 32-byte lines of 64 rows: indexes below 2^31 rows whose lines fit 32 MB) */
     uint64_t ftab_bytes;            /* seed table footprint */
     uint64_t hot_bytes;             /* superblock counts + seed table, held in one device allocation */
     uint64_t l2_pinned_bytes;       /* always 0: no persisting-L2 window is set (the field keeps the struct layout) */
@@ -351,12 +352,15 @@ double rbg_gather_roofline(int device, size_t footprint_bytes, int line_bytes, i
  * Each walks the SAME decode code the kernels run (csrc/leaf.cuh, csrc/phi_slot.cuh, the ToeholdDir lookup) on the
  * host over <prefix>.rbwt / .tsa and compares with a direct computation; 0 = every probe agreed.
  *   rbg_selftest_layout   rank_c(p), rank_c(p+1) for every stride-th position of every run (window & 0xFFFF = 0: automatic;
- *                         window >> 16 = 4 or 5 forces that line layout)
+ *                         window >> 16 = 4, 5 or 7 forces that line layout; layout 7 also checks BWT[p] as the toehold reads it)
+ *   rbg_selftest_layout_runs  the same over caller-supplied runs (n, heads, lens, R); *layout = the line layout built
  *   rbg_selftest_phi      phi(i) for every stride-th text position and the neighbours of every sample
  *   rbg_selftest_toehold  the toehold sample of every run end's LF image (shift = 0: automatic bucket width)
  *   rbg_selftest_rewrite  decode + re-serialize the index files (parts: 1 .rbwt, 2 .tsa, 4 .mab, 8 .rbwt is a wt_fbb)
  *   rbg_selftest_pack     rbg_pack_bytes with an explicit byte -> code table instead of an index handle */
 int rbg_selftest_layout(const char* prefix, uint32_t window, uint64_t stride, uint64_t* checked, uint64_t* n_lines, uint64_t* n_cluster);
+int rbg_selftest_layout_runs(uint64_t n, const uint8_t* heads, const uint64_t* lens, uint64_t R, uint32_t window, uint64_t stride,
+                             uint64_t* checked, uint64_t* n_lines, uint32_t* layout);
 int rbg_selftest_phi(const char* prefix, uint32_t shift, uint64_t stride, uint64_t* checked, uint64_t* n_slots, uint64_t* n_overflow);
 int rbg_selftest_toehold(const char* prefix, uint32_t shift, uint64_t* checked, uint64_t* dir_bytes);
 int rbg_selftest_rewrite(const char* prefix, const char* out_prefix, uint32_t parts);

@@ -167,6 +167,8 @@ def lib():
         L.rbg_gather_roofline.restype = C.c_double
         L.rbg_gather_roofline.argtypes = [C.c_int, C.c_size_t, C.c_int, C.c_int]
         L.rbg_selftest_layout.argtypes = [C.c_char_p, C.c_uint32, C.c_uint64, u64p, u64p, u64p]
+        L.rbg_selftest_layout_runs.argtypes = [C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, u64p, u64p,
+                                               C.POINTER(C.c_uint32)]
         L.rbg_selftest_phi.argtypes = [C.c_char_p, C.c_uint32, C.c_uint64, u64p, u64p, u64p]
         L.rbg_selftest_rewrite.argtypes = [C.c_char_p, C.c_char_p, C.c_uint32]
         L.rbg_selftest_toehold.argtypes = [C.c_char_p, C.c_uint32, u64p, u64p]

@@ -385,7 +385,7 @@ void save_ftab(const rbg_index* ix, const std::string& path) {
 // these index files (size + mtime of each part), these load flags, this library's layout version and the layout knobs the
 // open read; anything else rebuilds and rewrites it.  The index files stay the source of truth.
 constexpr uint64_t kCacheMagic = 0x3145484341434752ull;       // "RGCACHE1"
-constexpr uint32_t kCacheVersion = 4;                         // bump when a device structure or its meaning changes
+constexpr uint32_t kCacheVersion = 5;                         // bump when a device structure or its meaning changes
 
 struct CacheHeader {
     uint64_t magic;
@@ -540,7 +540,9 @@ std::unique_ptr<rbg_index> open_layout_cache(const std::string& pre, uint32_t fl
 // within kPairBudget -- small enough to stay resident in L2 beside the single-base directory, where the search is bound by
 // instructions and two bases per step take fewer of them than two steps -- and whose superblock table fits shared memory.
 // Larger indexes are bound by their line gathers, which the pair directory would only multiply.  knobs.pair = 0|1 (tests)
-// forces either form; 1 still needs layout 5, n < 2^32 and the shared-memory table.
+// forces either form; 1 still needs layout 5, n < 2^32 and the shared-memory table.  Every index small enough for it opens
+// in layout 7 unless a layout is forced (RBG_PAIR=1 asks for layout 5, LayoutKnobs::leaf_layout), so automatically it is
+// built only under RBG_LAYOUT=5.
 constexpr uint64_t kPairBudget = 64ull << 20;
 void build_pair(rbg_index* ix, const RunsBwt& bwt, const LeafDir& ld, const LayoutKnobs& knobs) {
     const int force = knobs.pair;
@@ -591,7 +593,7 @@ std::unique_ptr<rbg_index> open_from_arrays(const RunsBwt& bwt, const ToeholdArr
         phi_job = std::async(std::launch::async, [tsa, budget, knobs] { return build_phi_dir(*tsa, knobs.phi_shift, knobs.phi_parts, budget); });
     }
     {
-        LeafDir ld = build_leaf_dir(bwt, knobs.window, knobs.layout);
+        LeafDir ld = build_leaf_dir(bwt, knobs.window, knobs.leaf_layout());
         memcpy(F, ld.F, sizeof F);
         info.window = ld.window;
         info.layout = (uint32_t) ld.version;

@@ -12,17 +12,17 @@ constexpr int kDevMaxTerm = 8;
 constexpr int kMaxSuper5Dev = 256;      // == kMaxSuper5 (layout.hpp): layout 5 keeps at most 4 x 256 superblock bases
 constexpr uint64_t kPairMaxShared = 48 << 10;   // the pair superblock table search_kernel holds in shared memory (16 x 4 x n_super bytes)
 
-// The rank directory (LeafDir, layout.hpp): the line of BWT position p is p >> g.
+// The rank directory (LeafDir, layout.hpp): the line of BWT position p is p / window.
 struct DevLeafDir {
-    const uint32_t* lines;      // 64-byte mixed leaves: [n_direct] direct, then RAW children of CLUSTER windows
-    const uint64_t* super;      // [4][n_super]: F[c] + #c in BWT[0, superblock_start)
+    const uint32_t* lines;      // 64-byte mixed leaves: [n_direct] direct, then RAW children of CLUSTER windows (layout 7: 32-byte plain lines)
+    const uint64_t* super;      // [4][n_super]: F[c] + #c in BWT[0, superblock_start) (layout 7: unused)
     uint64_t n;
     uint64_t magic;             // i / window == umul64hi(i, magic)
     uint64_t n_super;
     uint32_t window;
     uint32_t sb_shift;
     uint32_t n_term;
-    uint32_t version;           // leaf.cuh LeafFmt: 4 or 5
+    uint32_t version;           // leaf.cuh: LeafFmt 4 or 5, or 7 (plain lines)
     // i / window without the 64 x 64 -> 128 bit product: window = m * 2^div_k (m odd), so i / window = (i >> div_k) / m, and for
     // (n >> div_k) < 2^31 that is ((i >> div_k) * div_mul) >> div_s with a 32-bit multiplier (set_fast_div below):
     // 3 instructions instead of 9, twice per LF step.  div_fast == 0 (odd windows over huge n): umul64hi(i, magic).
@@ -188,10 +188,65 @@ __device__ __forceinline__ bool lf_step_v(const DevLeafDir& D, uint32_t c, uint6
     return true;
 }
 
-// One thread, either layout (seed-table build, byte-wise search, greedy seeding: not the hot loop).
+// One 32-byte plain line (layout 7, leaf.cuh) as one 256-bit read-only load.
+__device__ __forceinline__ void load_plain_line(const uint32_t* p, uint32_t (&w)[kPlainWords]) {
+    asm("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+        : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]), "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7])
+        : "l"(p));
+}
+
+// LF step on the plain lines (layout 7, n < 2^31): rank_c(lo) from lo's line, rank_c(hi+1) from hi's line -- the match word
+// and the count of one line serve both once the range is narrow -- and BWT[hi] == c as bit q of hi's match word.  WARP: every
+// lane of the warp calls (search_kernel; `act` says whether the lane has a step, an inactive lane reads line 0 and keeps its
+// range), so the TERM path costs the common path one flag test and one vote.  Otherwise one thread (lf_step).
+template <bool TOEHOLD, bool WARP>
+__device__ __forceinline__ bool lf_step_plain(const DevLeafDir& D, uint32_t c, uint64_t& lo, uint64_t& hi, bool act,
+                                              bool& hi_is_c, uint32_t& lines_touched) {
+    const uint32_t l = act ? (uint32_t) lo : 0u, h = act ? (uint32_t) hi : 0u;
+    const uint32_t wa = l >> kPlainShift, wb = h >> kPlainShift, qa = l & (kPlainRows - 1u), qb = h & (kPlainRows - 1u);
+    uint32_t A[kPlainWords];
+    load_plain_line(D.lines + (uint64_t) wa * kPlainWords, A);
+    const uint64_t ma = plain_match(A, c);
+    const uint32_t ca = plain_count(A, c);
+    uint64_t mb = ma;
+    uint32_t cb = ca, flags = A[0];
+    if (wb == wa) {
+        lines_touched += act ? 1u : 0u;
+    } else {
+        uint32_t B[kPlainWords];
+        load_plain_line(D.lines + (uint64_t) wb * kPlainWords, B);
+        mb = plain_match(B, c);
+        cb = plain_count(B, c);
+        flags |= B[0];
+        lines_touched += 2;
+    }
+    uint32_t new_lo = ca + plain_rank_before(ma, qa);            // F[c] + #c in BWT[0, lo)
+    uint32_t new_end = cb + plain_rank_upto(mb, qb);             // F[c] + #c in BWT[0, hi]
+    hi_is_c = TOEHOLD && ((mb >> qb) & 1ull);
+    const bool term = act && (flags & kPlainTerm) && c == 0u;
+    if (WARP ? __any_sync(0xFFFFFFFFu, term) : term) {            // a terminator in lo's or hi's line, counted as 'A'
+        if (term) {
+#pragma unroll
+            for (uint32_t t = 0; t < (uint32_t) kDevMaxTerm; ++t) {     // constant indices: term_pos stays in the parameter bank
+                const bool on = t < D.n_term;
+                const uint64_t p = D.term_pos[t];
+                new_lo -= (on && p >= ((uint64_t) wa << kPlainShift) && p < l) ? 1u : 0u;
+                new_end -= (on && p >= ((uint64_t) wb << kPlainShift) && p <= h) ? 1u : 0u;
+                hi_is_c = hi_is_c && !(on && p == h);
+            }
+        }
+    }
+    if (!act || new_end == new_lo) return false;
+    lo = new_lo;
+    hi = new_end - 1u;
+    return true;
+}
+
+// One thread, any layout (seed-table build, byte-wise search, greedy seeding: not the hot loop).
 template <bool TOEHOLD>
 __device__ __forceinline__ bool lf_step(const DevLeafDir& D, uint32_t c, uint64_t& lo, uint64_t& hi,
                                         bool& hi_is_c, uint32_t& lines_touched) {
+    if (D.version == 7) return lf_step_plain<TOEHOLD, false>(D, c, lo, hi, true, hi_is_c, lines_touched);
     return D.version == 5 ? lf_step_v<TOEHOLD, 5>(D, c, lo, hi, hi_is_c, lines_touched)
                           : lf_step_v<TOEHOLD, 4>(D, c, lo, hi, hi_is_c, lines_touched);
 }
@@ -260,8 +315,12 @@ __device__ __forceinline__ bool lf_step_lines(const DevLeafDir& D, const uint64_
 template <bool TOEHOLD, int V>
 __device__ __forceinline__ bool lf_step_warp(const DevLeafDir& D, const uint64_t* sup, uint32_t c, uint64_t& lo, uint64_t& hi, bool act,
                                              bool& hi_is_c, uint32_t& lines_touched) {
-    const uint64_t l = act ? lo : 0ull, h = act ? hi : 0ull;
-    return lf_step_lines<TOEHOLD, V>(D, sup, c, lo, hi, act, line_of(D, l), line_of(D, h), hi_is_c, lines_touched);
+    if constexpr (V == 7) {
+        return lf_step_plain<TOEHOLD, true>(D, c, lo, hi, act, hi_is_c, lines_touched);
+    } else {
+        const uint64_t l = act ? lo : 0ull, h = act ? hi : 0ull;
+        return lf_step_lines<TOEHOLD, V>(D, sup, c, lo, hi, act, line_of(D, l), line_of(D, h), hi_is_c, lines_touched);
+    }
 }
 
 // Same with the line indexes of lo and hi already known (0, 0 for an inactive lane).

@@ -160,6 +160,7 @@ struct ToeholdTrack {
 // whole warp (device_index.cuh).
 // Layout 5 (V == 5): the superblock bases (<= 4 x 256 u64) are copied to shared memory once per CTA, so an LF step
 // issues no load besides its one or two directory lines.
+// Layout 7 (V == 7): the plain 2-bit lines of an L2-resident index (lf_step_plain); nothing to stage in shared memory.
 // PAIR (count search only): two bases per step from the pair directory (lf_pair_warp), whose superblock table (16 x n_super
 // u32, <= kPairMaxShared bytes) is the kernel's dynamic shared memory.  A lane whose read has an odd number of bases left
 // first takes one step on the single-base directory, which then reads its superblock bases from global memory.
@@ -597,6 +598,9 @@ int launch_search(const DevLeafDir& D, const DevPairDir& PD, const DevToehold* T
     if (!T && PD.lines) {                                   // the pair directory is built only over a layout-5 directory
         if (D.version != 5 || 64ull * PD.n_super > kPairMaxShared) throw std::logic_error("pair directory without its layout");
         search_kernel<false, 5, true><<<grid, kBlock, 64 * PD.n_super, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
+    } else if (D.version == 7) {
+        if (T) search_kernel<true, 7, false><<<grid, kBlock, 0, st>>>(D, PD, *T, ft, b, r, ctr, cursor);
+        else search_kernel<false, 7, false><<<grid, kBlock, 0, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
     } else if (D.version == 5) {
         if (T) search_kernel<true, 5, false><<<grid, kBlock, 0, st>>>(D, PD, *T, ft, b, r, ctr, cursor);
         else search_kernel<false, 5, false><<<grid, kBlock, 0, st>>>(D, PD, t0, ft, b, r, ctr, cursor);

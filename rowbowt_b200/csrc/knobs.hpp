@@ -20,18 +20,22 @@ inline std::optional<long long> env_int(const char* name) {
 // What shapes an index's device layout; read once per open and passed to the builders (layout.hpp).  0 = the builder's
 // own choice.  The layout cache stamps it, so every field is part of what a cache is valid for.
 struct LayoutKnobs {
-    int32_t layout = 0;                  // RBG_LAYOUT: 4 or 5 forces the line format of the rank directory
+    int32_t layout = 0;                  // RBG_LAYOUT: 4, 5 or 7 forces the line format of the rank directory
     uint32_t window = 0;                 // RBG_WINDOW: window of the rank directory
     int32_t pair = -1;                   // RBG_PAIR: 0 / 1 builds the pair directory never / whenever allowed; -1 automatic
     uint32_t pair_window = 0;            // RBG_PAIR_WINDOW: window of the pair directory
     uint32_t toehold_shift = 0;          // RBG_TOEHOLD_SHIFT: bucket width 2^s of the toehold directory, 1..32
     uint32_t phi_shift = 0;              // RBG_PHI_SHIFT: bucket width 2^s of the phi directory
     uint32_t phi_parts = 0;              // RBG_PHI_PARTS: parts the phi directory is built in, 1..64
+
+    // The line format asked of build_leaf_dir: RBG_LAYOUT, else layout 5 when RBG_PAIR=1 asks for the pair directory (which
+    // is built over layout 5 only), else 0, the builder's own choice.
+    int leaf_layout() const { return layout ? layout : pair == 1 ? 5 : 0; }
 };
 
 inline LayoutKnobs layout_knobs() {
     LayoutKnobs k;
-    if (auto v = env_int("RBG_LAYOUT")) k.layout = *v == 4 || *v == 5 ? (int32_t) *v : 0;
+    if (auto v = env_int("RBG_LAYOUT")) k.layout = *v == 4 || *v == 5 || *v == 7 ? (int32_t) *v : 0;
     if (auto v = env_int("RBG_WINDOW")) k.window = (uint32_t) *v;
     if (auto v = env_int("RBG_PAIR")) k.pair = (int32_t) *v;
     if (auto v = env_int("RBG_PAIR_WINDOW")) k.pair_window = (uint32_t) *v;

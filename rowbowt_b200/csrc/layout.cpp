@@ -143,6 +143,72 @@ struct LeafWalker {
     }
 };
 
+// Layout 7 (leaf.cuh, plain lines): the runs expanded into 2-bit planes, 64 rows per line, with the counts in front of each
+// line.  O(n / 64 + R), cut into contiguous parts of lines, one per host thread.
+void build_plain_lines(const RunsBwt& bwt, const int8_t* code, LeafDir& d) {
+    d.version = 7;
+    d.window = kPlainRows;
+    d.magic = ~0ull / kPlainRows + 1;
+    d.n_direct = (bwt.n + kPlainRows - 1) / kPlainRows;
+    d.sb_shift = 31 - kPlainShift;                      // one superblock (all zero) covers every line of an index below 2^31 rows
+    d.n_super = 1;
+    d.super.assign(4, 0);
+    d.n_cluster = 0;
+    d.lines.assign(d.n_direct * kPlainWords, 0);
+    const unsigned n_parts = d.n_direct >= (1u << 16) ? std::max(1u, std::min(16u, std::thread::hardware_concurrency())) : 1u;
+    struct Start { uint64_t j, jstart, cum[4]; };         // the run covering a part's first row, its start, counts in front of it
+    std::vector<Start> start(n_parts);
+    {
+        Start s{0, 0, {0, 0, 0, 0}};
+        for (unsigned p = 0; p < n_parts; ++p) {
+            const uint64_t P0 = d.n_direct * p / n_parts * kPlainRows;
+            while (s.jstart + bwt.lens[s.j] <= P0) {
+                const int8_t c = code[bwt.heads[s.j]];
+                if (c < 4) s.cum[c] += bwt.lens[s.j];
+                s.jstart += bwt.lens[s.j];
+                ++s.j;
+            }
+            start[p] = s;
+        }
+    }
+    auto part = [&](unsigned p) {
+        Start s = start[p];
+        const uint64_t t1 = d.n_direct * (p + 1) / n_parts;
+        for (uint64_t t = d.n_direct * p / n_parts; t < t1; ++t) {
+            const uint64_t P = t * kPlainRows, Pend = std::min<uint64_t>(P + kPlainRows, bwt.n);
+            while (s.jstart + bwt.lens[s.j] <= P) {
+                const int8_t c = code[bwt.heads[s.j]];
+                if (c < 4) s.cum[c] += bwt.lens[s.j];
+                s.jstart += bwt.lens[s.j];
+                ++s.j;
+            }
+            uint32_t* w = d.lines.data() + t * kPlainWords;
+            const int8_t c0 = code[bwt.heads[s.j]];
+            for (int c = 0; c < 4; ++c) w[c] = (uint32_t) (d.Fcode[c] + s.cum[c] + (c == c0 ? P - s.jstart : 0));
+            uint64_t plane[2] = {0, 0};
+            for (uint64_t i = s.j, at = s.jstart; i < bwt.R && at < Pend; at += bwt.lens[i], ++i) {
+                const uint64_t a = std::max(at, P), z = std::min(at + bwt.lens[i], Pend);
+                const uint64_t m = (z - a == kPlainRows ? ~0ull : (1ull << (z - a)) - 1ull) << (a - P);
+                uint32_t c = (uint32_t) code[bwt.heads[i]];
+                if (c == 4) { c = 0; w[0] |= kPlainTerm; }     // the terminator rides as 'A', uncounted
+                if (c & 1u) plane[0] |= m;
+                if (c & 2u) plane[1] |= m;
+            }
+            w[4] = (uint32_t) plane[0];
+            w[5] = (uint32_t) (plane[0] >> 32);
+            w[6] = (uint32_t) plane[1];
+            w[7] = (uint32_t) (plane[1] >> 32);
+        }
+    };
+    if (n_parts == 1) {
+        part(0);
+    } else {
+        std::vector<std::thread> th;
+        for (unsigned p = 0; p < n_parts; ++p) th.emplace_back(part, p);
+        for (auto& t : th) t.join();
+    }
+}
+
 }  // namespace
 
 PredTable build_pred_table(std::vector<uint64_t>&& keys, uint64_t universe, double keys_per_bucket) {
@@ -198,6 +264,14 @@ LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window, int layout) {
     memset(d.code_of, -1, sizeof d.code_of);
     for (int c = 0; c < 4; ++c) if (d.count[c]) d.code_of[sym[c]] = (int8_t) c;
     if (d.n_term) d.code_of[1] = 4;
+
+    // layout 7 while the plain lines stay L2-resident (kPlainMaxBytes); a forced window asks for a run-length layout
+    const uint64_t plain_bytes = (bwt.n + kPlainRows - 1) / kPlainRows * kPlainWords * 4;
+    if (layout == 7 || (layout == 0 && window == 0 && (bwt.n >> 31) == 0 && plain_bytes <= kPlainMaxBytes)) {
+        if (bwt.n >> 31) throw std::runtime_error("layout 7: BWT of 2^31 positions or more");
+        build_plain_lines(bwt, code, d);
+        return d;
+    }
 
     // layout 4: a superblock is <= 65535 positions (u16 counts); layout 5: <= 2^32 positions (u32 counts)
     auto sb_shift_for = [](int V, uint32_t W) {

@@ -29,19 +29,24 @@ constexpr uint32_t kMinWindow = 16;
 constexpr uint32_t kMaxWindow = 32767;  // starts are u16 and values >= 0x8000 must read as "unused"
 constexpr int kMaxTerm = 8;             // terminator positions carried in kernel params
 constexpr int kMaxSuper5 = 256;         // layout 5: superblocks of 2^32 positions at most, n < 2^40
+// Layout 7 (plain 2-bit lines, leaf.cuh) is the automatic choice while its lines stay this small: resident in L2, where the
+// search is bound by instructions and a plain rank takes far fewer than a run-length decode.  Needs n < 2^31.
+constexpr uint64_t kPlainMaxBytes = 32ull << 20;
 
 struct LeafDir {
     uint64_t n = 0;
-    int version = 4;                     // leaf.cuh LeafFmt: 4 (24 entries, u16 counts, L2-resident superblock array) or 5 (20 entries, u32 counts)
+    int version = 4;                     // leaf.cuh LeafFmt: 4 (24 entries, u16 counts, L2-resident superblock array) or 5 (20 entries,
+                                         // u32 counts); 7: plain 2-bit lines of 64 rows (n_super = 1, super all zero, no children)
     uint32_t window = 0;                 // W: BWT positions per direct line
     uint64_t magic = 0;                  // floor(2^64 / W) + 1: i / W == umul64hi(i, magic) for i * W < 2^64
     uint32_t sb_shift = 0;               // a superblock is 2^sb_shift windows (<= 65535 positions; layout 5: <= 2^32)
     uint64_t n_direct = 0;               // ceil(n / W)
     uint64_t n_super = 0;                // ceil(n_direct / 2^sb_shift)
     uint64_t n_cluster = 0;              // windows with a collapsed stretch (CLUSTER lines)
-    std::vector<uint32_t> lines;         // [(n_direct + raw children) * 16]
+    std::vector<uint32_t> lines;         // [(n_direct + raw children) * 16]; layout 7: [n_direct * 8]
     std::vector<uint64_t> super;         // [4][n_super]: F[c] + #c in BWT[0, superblock_start) (layout 5: at most 4 x 256, kept in shared memory)
-    uint64_t n_lines() const { return lines.size() / kLineWords; }
+    uint64_t line_words() const { return version == 7 ? kPlainWords : kLineWords; }
+    uint64_t n_lines() const { return lines.size() / line_words(); }
     uint64_t F[256] = {0};               // RowBowt::build_f (include/rowbowt.hpp:770-778), by byte value
     uint64_t Fcode[4] = {0, 0, 0, 0};    // F of A,C,G,T
     uint64_t count[4] = {0, 0, 0, 0};    // occurrences of A,C,G,T
@@ -50,8 +55,9 @@ struct LeafDir {
     uint64_t term_pos[kMaxTerm] = {0};
 };
 
-// Validates the alphabet and builds the rank directory.  window = 0 -> choose automatically; layout = 4 or 5 forces that
-// line format, 0 -> 5 while the directory stays small, else 4.
+// Validates the alphabet and builds the rank directory.  window = 0 -> choose automatically; layout = 4, 5 or 7 forces that
+// line format; 0 -> 7 when n < 2^31, its lines fit kPlainMaxBytes and no window is forced, else 5 while the directory
+// stays small, else 4.
 LeafDir build_leaf_dir(const RunsBwt& bwt, uint32_t window, int layout);
 
 // Pair directory (leaf.cuh, LeafFmt<6>): a rank directory over P[j] = (BWT[LF(j)], BWT[j]) with which the count search

@@ -96,6 +96,13 @@ RBG_HD uint32_t rbg_popc(uint32_t x) {
     return (uint32_t) __builtin_popcount(x);
 #endif
 }
+RBG_HD uint32_t rbg_popc64(uint64_t x) {
+#if defined(__CUDA_ARCH__)
+    return (uint32_t) __popcll(x);
+#else
+    return (uint32_t) __builtin_popcountll(x);
+#endif
+}
 
 // Bit position of entry e's head inside its head word (w[2] for e < 16, w[15] for e >= 16).
 RBG_HD uint32_t leaf_head_bit(uint32_t e) { return 8u * (e & 3u) + 2u * ((e & 15u) >> 2); }
@@ -251,5 +258,34 @@ RBG_HD uint32_t pair_raw_word_count(uint32_t word, uint32_t ppat, int first, int
     const uint32_t m = rem >= 8 ? 0xFFFFFFFFu : (rem <= 0 ? 0u : (1u << (4 * rem)) - 1u);
     return rbg_popc(pair_eq_nibbles(word ^ ppat) & 0x11111111u & m);
 }
+
+// ---- plain lines (layout 7) -------------------------------------------------------------------
+// An index whose BWT is small enough to stay in L2 (n < 2^31, <= kPlainMaxBytes of lines) keeps the BWT itself at 2 bits
+// per row, in 32-byte lines of 64 rows: the line of row i is i >> 6, with no division, no superblock table and no run decode.
+//   w[0..3]   4 x u32: F[c] + #c in BWT[0, line_start), c = A,C,G,T; bit 31 of w[0] is the TERM flag (free: n < 2^31)
+//   w[4..5]   the low bit of each row's code, row line_start + j at bit j of the 64-bit word w[5]:w[4]
+//   w[6..7]   the high bit, in the same order
+// rank_c(line_start + q) = w[c] + popc(match_c & ((1 << q) - 1)), match_c = the rows whose two bits spell c; the count
+// up to and including row q uses the mask (2 << q) - 1, so q never reaches 64, and BWT[line_start + q] == c is bit q of
+// match_c.  TERM: a terminator rides as code 0 ('A') in the planes but is not counted in w[0]; rank_A in such a line
+// subtracts the terminator rows it counted, from the (<= 8) terminator positions kept in the kernel parameters.
+constexpr uint32_t kPlainWords = 8, kPlainRows = 64, kPlainShift = 6;
+constexpr uint32_t kPlainTerm = 1u << 31;
+
+// the rows of the line that hold code c, row j at bit j
+RBG_HD uint64_t plain_match(const uint32_t (&w)[kPlainWords], uint32_t c) {
+    const uint32_t xl = (c & 1u) ? 0u : ~0u, xh = (c & 2u) ? 0u : ~0u;
+    const uint32_t m0 = (w[4] ^ xl) & (w[6] ^ xh), m1 = (w[5] ^ xl) & (w[7] ^ xh);
+    return (uint64_t) m0 | ((uint64_t) m1 << 32);
+}
+// F[c] + #c in BWT[0, line_start)
+RBG_HD uint32_t plain_count(const uint32_t (&w)[kPlainWords], uint32_t c) {
+    const uint32_t a = (c & 1u) ? w[1] : w[0] & ~kPlainTerm, b = (c & 1u) ? w[3] : w[2];
+    return (c & 2u) ? b : a;
+}
+// #c among rows [0, q) of the line, q < 64
+RBG_HD uint32_t plain_rank_before(uint64_t match, uint32_t q) { return rbg_popc64(match & ((1ull << q) - 1ull)); }
+// #c among rows [0, q] of the line, q < 64
+RBG_HD uint32_t plain_rank_upto(uint64_t match, uint32_t q) { return rbg_popc64(match & ((2ull << q) - 1ull)); }
 
 }  // namespace rbg

@@ -22,9 +22,40 @@
 using namespace rbg;
 
 namespace {
+// Layout 7 (plain lines, leaf.cuh): F[c] + rank_c(pos) in both forms the kernel takes it -- from the line of pos counting the
+// rows before it (lo) and from the line of pos - 1 counting up to and including that row (hi + 1) -- ~0 when they disagree.
+uint64_t plain_dir_rank(const LeafDir& d, uint32_t c, uint64_t pos) {
+    uint64_t out = ~0ull;
+    for (int upto = 0; upto < 2; ++upto) {
+        if (upto ? pos == 0 : pos == d.n) continue;
+        const uint64_t at = upto ? pos - 1 : pos, line = at >> kPlainShift;
+        const uint32_t q = (uint32_t) (at & (kPlainRows - 1));
+        uint32_t w[kPlainWords];
+        memcpy(w, d.lines.data() + line * kPlainWords, sizeof w);
+        const uint64_t m = plain_match(w, c);
+        uint64_t r = plain_count(w, c) + (upto ? plain_rank_upto(m, q) : plain_rank_before(m, q));
+        if ((w[0] & kPlainTerm) && c == 0)
+            for (uint32_t t = 0; t < d.n_term; ++t) r -= (d.term_pos[t] >= (line << kPlainShift) && d.term_pos[t] < pos) ? 1 : 0;
+        if (out != ~0ull && out != r) return ~0ull;
+        out = r;
+    }
+    return out;
+}
+
+// Layout 7: BWT[pos] == c as the toehold step reads it, bit q of the match word of c, not at a terminator row.
+bool plain_dir_is(const LeafDir& d, uint32_t c, uint64_t pos) {
+    uint32_t w[kPlainWords];
+    memcpy(w, d.lines.data() + (pos >> kPlainShift) * kPlainWords, sizeof w);
+    bool is = (plain_match(w, c) >> (pos & (kPlainRows - 1))) & 1ull;
+    if ((w[0] & kPlainTerm) && c == 0)
+        for (uint32_t t = 0; t < d.n_term; ++t) is = is && d.term_pos[t] != pos;
+    return is;
+}
+
 // F[c] + rank_c(pos) through the directory, pos in [0, n]; mirrors lf_step / leaf_rank_slow
 // (device_index.cuh): rank at pos is taken in the window of position `at` with offset q.
 uint64_t dir_rank(const LeafDir& d, uint32_t c, uint64_t pos) {
+    if (d.version == 7) return plain_dir_rank(d, c, pos);
     const bool use_prev = pos == d.n || (pos % d.window == 0 && pos > 0 && (pos & 1));   // also exercise the "hi" form (q = W)
     const uint64_t at = use_prev ? pos - 1 : pos;
     const uint64_t widx = (uint64_t) (((__uint128_t) at * d.magic) >> 64);
@@ -66,67 +97,92 @@ int parallel_parts(uint64_t n_items, unsigned n_parts, Fn&& fn) {
     return out;
 }
 unsigned selftest_threads() { return std::max(1u, std::min(32u, std::thread::hardware_concurrency())); }
+
+// rank_c(p) and rank_c(p + 1) (hence BWT[p] == c) decoded from the directory at the first and last position of every run and
+// every stride-th position inside, against a direct count over the runs.  window & 0xFFFF forces the window, window >> 16
+// the layout (4, 5 or 7; 0 = the loader's own choice).
+int check_layout(const RunsBwt& bwt, uint32_t window, uint64_t stride, uint64_t* checked, uint64_t* n_lines, uint64_t* n_cluster,
+                 uint32_t* layout_out) {
+    const uint32_t layout = window >> 16;
+    LayoutKnobs k = layout_knobs();
+    if (window & 0xFFFFu) k.window = window & 0xFFFFu;
+    if (layout) k.layout = layout == 5 || layout == 7 ? (int32_t) layout : 4;
+    LeafDir d = build_leaf_dir(bwt, k.window, k.leaf_layout());
+    if (layout && d.version != (int) k.layout) return 3;
+    if (n_lines) *n_lines = d.n_lines();
+    if (n_cluster) *n_cluster = d.n_cluster;
+    if (layout_out) *layout_out = (uint32_t) d.version;
+    static const uint8_t sym[4] = {'A', 'C', 'G', 'T'};
+    if (stride == 0) stride = 1;
+    int8_t code_of_head[256];
+    memset(code_of_head, -1, sizeof code_of_head);
+    for (int c = 0; c < 4; ++c) code_of_head[sym[c]] = (int8_t) c;
+    // where every part starts: position and per-symbol counts in front of its first run
+    const unsigned n_parts = selftest_threads();
+    struct Start { uint64_t pos, cum[4]; };
+    std::vector<Start> start(n_parts + 1, Start{0, {0, 0, 0, 0}});
+    {
+        Start cur{0, {0, 0, 0, 0}};
+        unsigned p = 0;
+        for (uint64_t j = 0; j <= bwt.R; ++j) {
+            while (p <= n_parts && j == bwt.R * p / n_parts) start[p++] = cur;
+            if (j == bwt.R) break;
+            const int hc = code_of_head[bwt.heads[j]];
+            if (hc >= 0) cur.cum[hc] += bwt.lens[j];
+            cur.pos += bwt.lens[j];
+        }
+    }
+    std::atomic<uint64_t> total{0};
+    const int rc = parallel_parts(bwt.R, n_parts, [&](unsigned part, uint64_t j0, uint64_t j1) {
+        uint64_t cum[4], pos = start[part].pos, n_checked = 0;
+        memcpy(cum, start[part].cum, sizeof cum);
+        for (uint64_t j = j0; j < j1; ++j) {
+            const int hc = code_of_head[bwt.heads[j]];
+            // the first and last position of every run and every stride-th position inside
+            for (uint64_t t = 0; t < bwt.lens[j]; t = (t + stride < bwt.lens[j] || t == bwt.lens[j] - 1) ? t + stride : bwt.lens[j] - 1) {
+                const uint64_t p = pos + t;
+                for (uint32_t c = 0; c < 4; ++c) {
+                    if (!d.count[c]) continue;
+                    const uint64_t want = d.Fcode[c] + cum[c] + ((int) c == hc ? t : 0);
+                    if (dir_rank(d, c, p) != want) return 1;
+                    if (dir_rank(d, c, p + 1) != want + ((int) c == hc ? 1 : 0)) return 2;
+                    if (d.version == 7 && plain_dir_is(d, c, p) != ((int) c == hc)) return 4;
+                    ++n_checked;
+                }
+            }
+            if (hc >= 0) cum[hc] += bwt.lens[j];
+            pos += bwt.lens[j];
+        }
+        total += n_checked;
+        return 0;
+    });
+    if (rc) return rc;
+    const uint64_t n_checked = total;
+    if (checked) *checked = n_checked;
+    return 0;
+}
 }  // namespace
 
 extern "C" int rbg_selftest_layout(const char* prefix, uint32_t window, uint64_t stride, uint64_t* checked,
                                    uint64_t* n_lines, uint64_t* n_cluster) {
     try {
-        RunsBwt bwt = read_rbwt(std::string(prefix) + ".rbwt");
-        const uint32_t layout = window >> 16;                     // bits 16..: force layout 4 or 5 (0 = the loader's own choice)
-        LayoutKnobs k = layout_knobs();
-        if (window & 0xFFFFu) k.window = window & 0xFFFFu;
-        if (layout) k.layout = layout == 5 ? 5 : 4;
-        LeafDir d = build_leaf_dir(bwt, k.window, k.layout);
-        if (layout && d.version != (int) layout) return 3;
-        if (n_lines) *n_lines = d.n_lines();
-        if (n_cluster) *n_cluster = d.n_cluster;
-        static const uint8_t sym[4] = {'A', 'C', 'G', 'T'};
-        if (stride == 0) stride = 1;
-        int8_t code_of_head[256];
-        memset(code_of_head, -1, sizeof code_of_head);
-        for (int c = 0; c < 4; ++c) code_of_head[sym[c]] = (int8_t) c;
-        // where every part starts: position and per-symbol counts in front of its first run
-        const unsigned n_parts = selftest_threads();
-        struct Start { uint64_t pos, cum[4]; };
-        std::vector<Start> start(n_parts + 1, Start{0, {0, 0, 0, 0}});
-        {
-            Start cur{0, {0, 0, 0, 0}};
-            unsigned p = 0;
-            for (uint64_t j = 0; j <= bwt.R; ++j) {
-                while (p <= n_parts && j == bwt.R * p / n_parts) start[p++] = cur;
-                if (j == bwt.R) break;
-                const int hc = code_of_head[bwt.heads[j]];
-                if (hc >= 0) cur.cum[hc] += bwt.lens[j];
-                cur.pos += bwt.lens[j];
-            }
-        }
-        std::atomic<uint64_t> total{0};
-        const int rc = parallel_parts(bwt.R, n_parts, [&](unsigned part, uint64_t j0, uint64_t j1) {
-            uint64_t cum[4], pos = start[part].pos, n_checked = 0;
-            memcpy(cum, start[part].cum, sizeof cum);
-            for (uint64_t j = j0; j < j1; ++j) {
-                const int hc = code_of_head[bwt.heads[j]];
-                // the first and last position of every run and every stride-th position inside
-                for (uint64_t t = 0; t < bwt.lens[j]; t = (t + stride < bwt.lens[j] || t == bwt.lens[j] - 1) ? t + stride : bwt.lens[j] - 1) {
-                    const uint64_t p = pos + t;
-                    for (uint32_t c = 0; c < 4; ++c) {
-                        if (!d.count[c]) continue;
-                        const uint64_t want = d.Fcode[c] + cum[c] + ((int) c == hc ? t : 0);
-                        if (dir_rank(d, c, p) != want) return 1;
-                        if (dir_rank(d, c, p + 1) != want + ((int) c == hc ? 1 : 0)) return 2;
-                        ++n_checked;
-                    }
-                }
-                if (hc >= 0) cum[hc] += bwt.lens[j];
-                pos += bwt.lens[j];
-            }
-            total += n_checked;
-            return 0;
-        });
-        if (rc) return rc;
-        const uint64_t n_checked = total;
-        if (checked) *checked = n_checked;
-        return 0;
+        return check_layout(read_rbwt(std::string(prefix) + ".rbwt"), window, stride, checked, n_lines, n_cluster, nullptr);
+    } catch (const std::exception&) {
+        return -1;
+    }
+}
+
+// The same over caller-supplied runs; *layout receives the line format the directory was built in, which is what an open
+// of these runs under the same environment would pick.
+extern "C" int rbg_selftest_layout_runs(uint64_t n, const uint8_t* heads, const uint64_t* lens, uint64_t R, uint32_t window,
+                                        uint64_t stride, uint64_t* checked, uint64_t* n_lines, uint32_t* layout) {
+    try {
+        RunsBwt bwt;
+        bwt.n = n;
+        bwt.R = R;
+        bwt.heads.assign(heads, heads + R);
+        bwt.lens.assign(lens, lens + R);
+        return check_layout(bwt, window, stride, checked, n_lines, nullptr, layout);
     } catch (const std::exception&) {
         return -1;
     }
@@ -192,7 +248,7 @@ extern "C" int rbg_selftest_toehold(const char* prefix, uint32_t shift, uint64_t
         ToeholdArrays t = read_tsa(std::string(prefix) + ".tsa");
         LayoutKnobs k = layout_knobs();
         if (shift) k.toehold_shift = shift;
-        LeafDir d = build_leaf_dir(bwt, k.window, k.layout);
+        LeafDir d = build_leaf_dir(bwt, k.window, k.leaf_layout());
         ToeholdDir td = build_toehold_dir(bwt, d.F, t, k.toehold_shift);
         if (shift && td.shift != shift) return 3;
         if (dir_bytes) *dir_bytes = td.bytes();

@@ -63,10 +63,11 @@ def branch_target(full):
     return int(mm.group(1), 16) if mm else None
 
 
-def loop_parts(ins):
+def loop_parts(ins, anchor="IDP", lead=0x200):
     """Splits the outer loop of search_kernel into (refill, common step path, rare path) by structure:
-    the loop = the longest backward branch; the step starts at the last branch-join before the first IDP.2A (the read
-    refill sits in front of it); the rare block is what the first forward branch after the decode's VOTE skips."""
+    the loop = the longest backward branch; the step starts at the last branch-join at least `lead` bytes before the first
+    `anchor` instruction of the ranks (IDP.2A on the run-length lines, POPC on the plain lines; the read refill sits in
+    front of it); the rare block is what the first forward branch after the decode's VOTE skips."""
     best = None
     first_exit = min([x[0] for x in ins if x[2] == "EXIT"] + [1 << 30])      # the loop ends before the kernel's epilogue
     for addr, full, op, body in ins:
@@ -77,14 +78,15 @@ def loop_parts(ins):
             best = (tgt, addr)
     start, end = best
     loop = [x for x in ins if start <= x[0] <= end]
-    idp = [x[0] for x in loop if x[2] == "IDP"]
+    first_line = next(x[0] for x in loop if x[2] == "LDG" and ".256" in x[1])     # the step's first directory line load
+    idp = [x[0] for x in loop if x[2] == anchor and x[0] > first_line]
     first_idp = idp[0]
     last_core_idp = first_idp
     for a in idp:                                              # the first dense run of IDPs = the two ranks of the common path
         if a - last_core_idp <= 0x280:
             last_core_idp = a
     joins = sorted({branch_target(x[1]) for x in loop if x[2] == "BRA" and branch_target(x[1]) is not None and branch_target(x[1]) > x[0]})
-    step_start = max([j for j in joins if j <= first_idp - 0x200] + [start])
+    step_start = max([j for j in joins if j <= first_idp - lead] + [start])
     vote = next(x[0] for x in loop if x[0] > last_core_idp and x[2] == "VOTE")
     rb = next(x for x in loop if x[0] > vote and x[2] == "BRA" and branch_target(x[1]) and branch_target(x[1]) > x[0])
     rare = (rb[0], branch_target(rb[1]))
@@ -103,11 +105,13 @@ def main():
            "variants the `common path` column also holds the block of the third rank, which runs in about one warp step in six.",
            "`common path` = what every warp step executes; `rare path` = the forward-branched block that runs only when some lane's",
            "rank position lies inside a collapsed variant cluster / the terminator window (warp-cooperative child-line walk).", ""]
-    for variant, label in (("ILb0ELi5ELb0EE", "count, layout 5"),
-                           ("ILb1ELi5ELb0EE", "toehold (-s), layout 5"),
-                           ("ILb0ELi4ELb0EE", "count, layout 4")):
+    for variant, label, anchor, lead in (("ILb0ELi7ELb0EE", "count, layout 7", "POPC", 0x100),
+                                         ("ILb1ELi7ELb0EE", "toehold (-s), layout 7", "POPC", 0x100),
+                                         ("ILb0ELi5ELb0EE", "count, layout 5", "IDP", 0x200),
+                                         ("ILb1ELi5ELb0EE", "toehold (-s), layout 5", "IDP", 0x200),
+                                         ("ILb0ELi4ELb0EE", "count, layout 4", "IDP", 0x200)):
         ins = sass_of(variant)
-        (start, end, step_start, rare), refill, common, rare_ins = loop_parts(ins)
+        (start, end, step_start, rare), refill, common, rare_ins = loop_parts(ins, anchor, lead)
         out += ["## %s — `search_kernel<%s>`" % (label, variant), "",
                 "loop 0x%04x..0x%04x; LF step from 0x%04x: **%d instructions on the common path** of a step, %d in the rare block "
                 "(0x%04x..0x%04x), %d in the read refill in front of the step (runs when a quarter of the warp is idle)" % (
@@ -117,7 +121,7 @@ def main():
         for name in sorted(set(cc) | set(rc) | set(fc), key=lambda k: -cc.get(k, 0)):
             out.append("| %s | %d | %d | %d |" % (name, cc.get(name, 0), rc.get(name, 0), fc.get(name, 0)))
         out.append("")
-        if variant == "ILb0ELi5ELb0EE":
+        if variant in ("ILb0ELi7ELb0EE", "ILb0ELi5ELb0EE"):
             out += ["<details><summary>common path, full listing</summary>", "", "```"]
             out += ["/*%04x*/ %s ;" % (x[0], x[1]) for x in common]
             out += ["```", "", "</details>", ""]
