@@ -35,7 +35,8 @@ enum {
     RBG_E_ALPHABET = -3,    /* BWT symbols outside {terminator,A,C,G,T} (build with pfbwt-f --non-acgt-to-a) */
     RBG_E_CUDA = -4,        /* CUDA runtime failure, including "no device" */
     RBG_E_ARG = -5,         /* invalid argument / mode needs a part that was not loaded */
-    RBG_E_NOMEM = -6
+    RBG_E_NOMEM = -6,
+    RBG_E_INTERNAL = -7     /* a result failed its own check (the BWT builder's suffix-array certificate); nothing was written */
 };
 
 /* rbwt::LoadRbwtFlag, include/rowbowt_io.hpp:146-158 (same numeric values) */
@@ -229,10 +230,15 @@ int rbg_build_marker_array_arrays(const rbg_index_desc* desc, const char* mps_pa
  * Input: FASTA, plain, gzip or BGZF, multi-line records joined.  Uppercase A C G T are kept, any other uppercase letter
  * becomes 'A'.  Refused before any CUDA call: a missing or unreadable file RBG_E_IO; no records, or a record without bases
  * RBG_E_FORMAT; a lowercase letter or a non-letter byte in a sequence RBG_E_ALPHABET (record and offset named: soft-masked
- * input must be uppercased first); n >= 2^32 RBG_E_ARG.  When the build does not fit the device's free memory RBG_E_NOMEM
+ * input must be uppercased first); n >= 2^40 RBG_E_ARG.  When the build does not fit the device's free memory RBG_E_NOMEM
  * (the bytes needed are named), before anything is allocated.  Outputs are written to temporary files and renamed.
- * rbg_build_bwt_text takes len ACGT bytes without the terminator (tests) and writes no .docs; len is checked before the
- * buffer is read.  `stats` may be NULL. */
+ * Below 2^32 positions the build keeps positions and ranks in u32 (37 bytes of device memory per position); from 2^32 on
+ * (or at any n with RBG_BWT_WIDE=1 in the environment) in u64, with the suffix array sorted in parts of at most M rows:
+ * 21 bytes per position + 32 per part row + 391 MB of prefix counts + scratch, M taken from the free memory (capped by
+ * RBG_BWT_PART_ROWS).  An 11-symbol prefix shared by more than M suffixes is refused with RBG_E_NOMEM naming it.  That
+ * build certifies its suffix array before writing anything; a failure is RBG_E_INTERNAL naming the row.
+ * rbg_build_bwt_text takes len ACGT bytes without the terminator (tests) and writes no .docs; len (n < 2^32) is checked
+ * before the buffer is read.  `stats` may be NULL. */
 #define RBG_BWT_MAX_ROUNDS 32
 typedef struct {
     uint64_t n, r;                  /* text length (terminator included), BWT runs */
@@ -242,8 +248,14 @@ typedef struct {
     uint64_t max_active;            /* most suffixes one round sorted */
     uint64_t active[RBG_BWT_MAX_ROUNDS];   /* suffixes round i sorted (i < rounds): those whose group was still larger than 1 */
     double s_parse, s_sort, s_write, s_total;   /* wall time: FASTA -> text; upload, sort, BWT and samples back; file writes; all */
-    float ms_sort, ms_gather;       /* CUDA-event time of the initial sort + rounds, and of the BWT gather + run boundaries + samples */
+    float ms_sort, ms_gather;       /* CUDA-event time of the initial sort + rounds, and of the BWT gather + run boundaries + samples
+                                       (the u64 build: with the copy of the BWT to the host, which its run chunks are cut by) */
     uint64_t peak_bytes;            /* device memory the build allocates (checked against the free memory first) */
+    uint32_t wide;                  /* 1: u64 positions and ranks, the suffix array sorted in parts */
+    uint32_t parts;                 /* parts the rows were cut into (1 for the u32 build) */
+    uint64_t part_rows;             /* rows of the largest part */
+    float ms_verify;                /* CUDA-event time of the suffix-array certificate (0 for the u32 build, which has none) */
+    uint32_t _pad2;
 } rbg_bwt_stats;
 int rbg_build_bwt(const char* fasta_path, const char* out_prefix, int device, rbg_bwt_stats* stats);
 int rbg_build_bwt_text(const uint8_t* text, uint64_t len, const char* out_prefix, int device, rbg_bwt_stats* stats);
@@ -347,6 +359,12 @@ void rbg_host_free(void* p);
  * thread reads whole lines (as the kernels do); -64: 64-byte lines read by lane pairs, one request per line;
  * iters < 0: each address depends on the data just read. */
 double rbg_gather_roofline(int device, size_t footprint_bytes, int line_bytes, int iters);
+
+/* The BWT builder's suffix-array certificate over a caller's suffix array: sa[0, len + 1) of text[0, len) (A, C, G, T) + the
+ * terminator.  *first_bad = len + 1 when sa is the suffix array, else the smallest row i where sa[i] >= len + 1, sa[i]
+ * appeared at an earlier row, or (T[sa[i]], rank[sa[i] + 1]) is not below (T[sa[i + 1]], rank[sa[i + 1] + 1]) -- rank being
+ * the first row holding each value, the terminator the smallest symbol. */
+int rbg_check_suffix_array(const uint8_t* text, uint64_t len, const uint64_t* sa, int device, uint64_t* first_bad);
 
 /* ---- diagnostics (host only, no CUDA call): the load-time re-layout checked against the flat arrays ----------
  * Each walks the SAME decode code the kernels run (csrc/leaf.cuh, csrc/phi_slot.cuh, the ToeholdDir lookup) on the

@@ -8,6 +8,7 @@ CPU fallback — if the library is missing or there is no GPU, calls raise.
 from .binding import (  # noqa: F401
     RBG_COUNT, RBG_LOCATE, RBG_MARKERS, RBG_NARROW_LOCS, RBG_NARROW_RANGES, RBG_READ_DEAD, RBG_READ_EXOTIC, RBG_LOAD_SA, RBG_LOAD_MA,
     BuildStats, BwtStats, GpuIndex, MaStats, RbgError, SEED_DTYPE, StagedReads, build_bwt, build_bwt_text, build_index, build_marker_array,
+    check_suffix_array,
     build_marker_array_arrays, lib,
     lib_path, result_checksum,
 )

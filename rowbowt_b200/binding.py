@@ -95,10 +95,12 @@ class BwtStats(C.Structure):
     _fields_ = [("n", C.c_uint64), ("r", C.c_uint64), ("records", C.c_uint64), ("rounds", C.c_uint32), ("_pad", C.c_uint32),
                 ("max_active", C.c_uint64), ("active", C.c_uint64 * BWT_MAX_ROUNDS),
                 ("s_parse", C.c_double), ("s_sort", C.c_double), ("s_write", C.c_double), ("s_total", C.c_double),
-                ("ms_sort", C.c_float), ("ms_gather", C.c_float), ("peak_bytes", C.c_uint64)]
+                ("ms_sort", C.c_float), ("ms_gather", C.c_float), ("peak_bytes", C.c_uint64),
+                ("wide", C.c_uint32), ("parts", C.c_uint32), ("part_rows", C.c_uint64), ("ms_verify", C.c_float),
+                ("_pad2", C.c_uint32)]
 
     def as_dict(self):
-        d = {k: getattr(self, k) for k, _ in self._fields_ if k not in ("_pad", "active")}
+        d = {k: getattr(self, k) for k, _ in self._fields_ if k not in ("_pad", "_pad2", "active")}
         d["active"] = list(self.active)[:min(self.rounds, BWT_MAX_ROUNDS)]
         return d
 
@@ -166,6 +168,7 @@ def lib():
         L.rbg_host_free.argtypes = [C.c_void_p]
         L.rbg_gather_roofline.restype = C.c_double
         L.rbg_gather_roofline.argtypes = [C.c_int, C.c_size_t, C.c_int, C.c_int]
+        L.rbg_check_suffix_array.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_int, u64p]
         L.rbg_selftest_layout.argtypes = [C.c_char_p, C.c_uint32, C.c_uint64, u64p, u64p, u64p]
         L.rbg_selftest_layout_runs.argtypes = [C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, u64p, u64p,
                                                C.POINTER(C.c_uint32)]
@@ -249,7 +252,8 @@ def build_index(in_prefix: str, out_prefix: str, sa: bool = False, markers: bool
 
 def build_bwt(fasta: str, out_prefix: str, device: int = 0) -> "BwtStats":
     """pfbwt-f64 --non-acgt-to-a --print-docs -r on the GPU: a FASTA (plain, gzip or BGZF) -> <out>.bwt/.ssa/.esa/.docs, the
-    files rb_build reads.  The text is every record followed by 10 'A's, then the terminator; it must have n < 2^32."""
+    files rb_build reads.  The text is every record followed by 10 'A's, then the terminator; it must have n < 2^40 (from
+    2^32 on, u64 positions and the suffix array sorted in parts: `stats.wide`)."""
     st = BwtStats()
     _check(lib().rbg_build_bwt(fasta.encode(), out_prefix.encode(), device, C.byref(st)))
     return st
@@ -261,6 +265,18 @@ def build_bwt_text(text: np.ndarray, out_prefix: str, device: int = 0) -> "BwtSt
     st = BwtStats()
     _check(lib().rbg_build_bwt_text(t.ctypes.data, len(t), out_prefix.encode(), device, C.byref(st)))
     return st
+
+
+def check_suffix_array(text: np.ndarray, sa: np.ndarray, device: int = 0) -> int:
+    """The BWT builder's suffix-array certificate on the GPU over sa (len(text) + 1 values) of an ACGT text + terminator:
+    len(sa) when sa is its suffix array, else the smallest failing row (rbg_check_suffix_array)."""
+    t = np.ascontiguousarray(text, np.uint8)
+    a = np.ascontiguousarray(sa, np.uint64)
+    if len(a) != len(t) + 1:
+        raise ValueError("sa must hold len(text) + 1 values")
+    bad = C.c_uint64(0)
+    _check(lib().rbg_check_suffix_array(t.ctypes.data, len(t), a.ctypes.data, device, C.byref(bad)))
+    return bad.value
 
 
 def _ma_window(rows):

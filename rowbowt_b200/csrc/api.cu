@@ -666,6 +666,7 @@ int guarded(Fn&& fn) {
     } catch (const alphabet_error& e) { return fail(RBG_E_ALPHABET, e.what());
     } catch (const cuda_error& e) { cudaGetLastError(); return fail(RBG_E_CUDA, e.what());
     } catch (const nomem_error& e) { return fail(RBG_E_NOMEM, e.what());
+    } catch (const internal_error& e) { return fail(RBG_E_INTERNAL, e.what());
     } catch (const std::bad_alloc&) { return fail(RBG_E_NOMEM, "out of host memory");
     } catch (const std::exception& e) { return fail(RBG_E_ARG, e.what()); }
 }
@@ -1511,11 +1512,13 @@ int rbg_build_bwt(const char* fasta_path, const char* out_prefix, int device, rb
         rbg_bwt_stats st;
         memset(&st, 0, sizeof st);
         const double t_begin = wall_s();
-        const FastaText ft = read_fasta_text(fasta_path);
+        const BwtKnobs knobs = bwt_knobs();
+        const FastaText ft = read_fasta_text(fasta_path, kBwtWideMaxN);
         st.records = ft.names.size();
         st.s_parse = wall_s() - t_begin;
         select_device(device);
-        build_bwt_files(ft.text.data(), ft.text.size(), device, out_prefix, st);
+        if (knobs.wide || ft.text.size() + 1 > kBwtMaxN) build_bwt_files_wide(ft.text.data(), ft.text.size(), device, knobs.part_rows, out_prefix, st);
+        else build_bwt_files(ft.text.data(), ft.text.size(), device, out_prefix, st);
         const double t_docs = wall_s();
         write_docs(ft, std::string(out_prefix) + ".docs");
         st.s_write += wall_s() - t_docs;
@@ -1532,11 +1535,13 @@ int rbg_build_bwt_text(const uint8_t* text, uint64_t len, const char* out_prefix
         rbg_bwt_stats st;
         memset(&st, 0, sizeof st);
         const double t_begin = wall_s();
-        check_bwt_length(std::min(len, kBwtMaxN) + 1, "a text of " + std::to_string(len) + " bases");    // before the buffer is read
+        check_bwt_length(std::min(len, kBwtMaxN) + 1, "a text of " + std::to_string(len) + " bases", kBwtMaxN);   // before the buffer is read
+        const BwtKnobs knobs = bwt_knobs();
         check_acgt(text, len);
         st.s_parse = wall_s() - t_begin;
         select_device(device);
-        build_bwt_files(text, len, device, out_prefix, st);
+        if (knobs.wide) build_bwt_files_wide(text, len, device, knobs.part_rows, out_prefix, st);
+        else build_bwt_files(text, len, device, out_prefix, st);
         st.s_total = wall_s() - t_begin;
         if (stats) *stats = st;
         return (int) RBG_OK;
@@ -1757,6 +1762,17 @@ void* rbg_host_alloc(size_t bytes) {
 
 void rbg_host_free(void* p) {
     if (p) cudaFreeHost(p);
+}
+
+int rbg_check_suffix_array(const uint8_t* text, uint64_t len, const uint64_t* sa, int device, uint64_t* first_bad) {
+    if (!text || !sa || !first_bad) return fail(RBG_E_ARG, "null argument");
+    if (len == 0) return fail(RBG_E_ARG, "empty text");
+    return guarded([&] {
+        check_acgt(text, len);
+        select_device(device);
+        *first_bad = check_suffix_array(text, len, sa, device);
+        return (int) RBG_OK;
+    });
 }
 
 double rbg_gather_roofline(int device, size_t footprint_bytes, int line_bytes, int iters) {

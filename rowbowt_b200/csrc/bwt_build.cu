@@ -28,6 +28,7 @@
 #include <string>
 #include <vector>
 
+#include "bwt_build.cuh"
 #include "bwt_build.hpp"
 #include "cuda_host.hpp"
 #include "formats.hpp"
@@ -37,17 +38,8 @@
 namespace rbg {
 
 // Kernels outside the anonymous namespace: their names stay the same from build to build (traces, profiles).
-constexpr int kBwtBlock = 256;
-constexpr int kBwtK = 27;                          // 27 base-5 digits fit 63 bits
 constexpr uint32_t kBwtSorted = 0xFFFFFFFFu;      // item whose group is a singleton (no row reaches 2^32 - 1)
 constexpr uint64_t kBwtBytesPerPos = 37;
-
-__device__ __forceinline__ uint64_t bwt_code(uint8_t c) { return c == 'A' ? 1 : c == 'C' ? 2 : c == 'G' ? 3 : c == 'T' ? 4 : 0; }
-
-__device__ __forceinline__ uint64_t bwt_item() { return (uint64_t) blockIdx.x * kBwtBlock + threadIdx.x; }
-
-// Item k starts a group of equal keys.
-__device__ __forceinline__ bool bwt_is_head(const uint64_t* __restrict__ keys, uint64_t k) { return k == 0 || keys[k] != keys[k - 1]; }
 
 __global__ void __launch_bounds__(kBwtBlock) bwt_init_keys_kernel(const uint8_t* __restrict__ text, uint64_t n, uint64_t* __restrict__ keys,
                                                                   uint32_t* __restrict__ pos) {
@@ -93,23 +85,6 @@ __global__ void __launch_bounds__(kBwtBlock) bwt_scatter_kernel(const uint64_t* 
     hd[k] = single ? kBwtSorted : row;
 }
 
-__global__ void __launch_bounds__(kBwtBlock) bwt_gather_kernel(const uint8_t* __restrict__ text, const uint32_t* __restrict__ sa, uint64_t n,
-                                                               uint8_t* __restrict__ bwt) {
-    const uint64_t i = bwt_item();
-    if (i >= n) return;
-    const uint32_t p = sa[i];
-    bwt[i] = text[p ? p - 1 : n - 1];
-}
-
-__global__ void __launch_bounds__(kBwtBlock) bwt_samples_kernel(const uint32_t* __restrict__ starts, uint64_t r, uint64_t n,
-                                                                const uint32_t* __restrict__ sa, uint32_t* __restrict__ sa_first,
-                                                                uint32_t* __restrict__ sa_last) {
-    const uint64_t j = bwt_item();
-    if (j >= r) return;
-    sa_first[j] = sa[starts[j]];
-    sa_last[j] = sa[(j + 1 < r ? (uint64_t) starts[j + 1] : n) - 1];
-}
-
 namespace {
 
 struct MaxU32 {
@@ -125,7 +100,15 @@ struct RunStart {
 
 unsigned grid(uint64_t items) { return (unsigned) ((items + kBwtBlock - 1) / kBwtBlock); }
 
-// The whole file to a temporary name, then renamed into place.
+std::string printable(uint8_t c) {
+    char buf[16];
+    if (c >= 0x20 && c < 0x7f) snprintf(buf, sizeof buf, "'%c'", c);
+    else snprintf(buf, sizeof buf, "0x%02x", c);
+    return buf;
+}
+
+}  // namespace
+
 void write_file(const std::string& path, const void* data, size_t bytes) {
     const std::string tmp = path + ".tmp." + std::to_string((long) getpid());
     FILE* f = fopen(tmp.c_str(), "wb");
@@ -139,19 +122,13 @@ void write_file(const std::string& path, const void* data, size_t bytes) {
     }
 }
 
-std::string printable(uint8_t c) {
-    char buf[16];
-    if (c >= 0x20 && c < 0x7f) snprintf(buf, sizeof buf, "'%c'", c);
-    else snprintf(buf, sizeof buf, "0x%02x", c);
-    return buf;
-}
-
-}  // namespace
-
-void check_bwt_length(uint64_t n, const std::string& what) {
-    if (n > kBwtMaxN)
-        throw std::invalid_argument(what + " would have n >= 2^32 positions (terminator included); this BWT builder keeps "
-                                    "positions in 32 bits and takes n <= " + std::to_string(kBwtMaxN));
+void check_bwt_length(uint64_t n, const std::string& what, uint64_t max_n) {
+    if (n > max_n) {
+        int bits = 0;
+        while (bits < 64 && (max_n >> bits)) ++bits;
+        throw std::invalid_argument(what + " would have n >= 2^" + std::to_string(bits) + " positions (terminator included); this "
+                                    "BWT builder takes n <= " + std::to_string(max_n));
+    }
 }
 
 void check_acgt(const uint8_t* text, uint64_t len) {
@@ -162,7 +139,7 @@ void check_acgt(const uint8_t* text, uint64_t len) {
     }
 }
 
-FastaText read_fasta_text(const std::string& path) {
+FastaText read_fasta_text(const std::string& path, uint64_t max_n) {
     struct stat sb;
     if (stat(path.c_str(), &sb) != 0) throw io_error("bad file: " + path);
     rbhost::FastxReader rd(path.c_str());
@@ -174,7 +151,7 @@ FastaText read_fasta_text(const std::string& path) {
     map['G'] = 'G';
     map['T'] = 'T';
     FastaText ft;
-    if (S_ISREG(sb.st_mode)) ft.text.reserve(std::min<uint64_t>((uint64_t) sb.st_size + 1024, kBwtMaxN));
+    if (S_ISREG(sb.st_mode)) ft.text.reserve(std::min<uint64_t>((uint64_t) sb.st_size + 1024, max_n));
     std::string name, seq;
     for (;;) {
         seq.clear();
@@ -184,7 +161,7 @@ FastaText read_fasta_text(const std::string& path) {
         if (rc == -3) throw io_error("cannot read " + path);
         if (seq.empty()) throw format_error("record '" + name + "' of " + path + " has no bases");
         const uint64_t start = ft.text.size();
-        check_bwt_length(start + seq.size() + kBwtPad + 1, "the text of " + path);
+        check_bwt_length(start + seq.size() + kBwtPad + 1, "the text of " + path, max_n);
         ft.text.resize(start + seq.size() + kBwtPad, 'A');
         uint8_t* out = ft.text.data() + start;
         uint8_t bad = 0xff;
@@ -214,9 +191,11 @@ void write_docs(const FastaText& ft, const std::string& path) {
 
 void build_bwt_files(const uint8_t* text, uint64_t len, int device, const std::string& out_prefix, rbg_bwt_stats& st) {
     const uint64_t n = len + 1;
-    check_bwt_length(n, "the text");
+    check_bwt_length(n, "the text", kBwtMaxN);
     const double t_sort = wall_s();
     st.n = n;
+    st.parts = 1;
+    st.part_rows = n;
 
     // scratch of every CUB call, for the largest item count, before anything is allocated
     size_t tmp_sort = 0, tmp_scan = 0, tmp_sel = 0, tmp_runs = 0;
@@ -315,14 +294,14 @@ void build_bwt_files(const uint8_t* text, uint64_t len, int device, const std::s
     uint8_t* bwt = d_rank.as<uint8_t>();
     uint32_t* starts = d_k[0].as<uint32_t>();
     uint32_t *sa_first = d_k[1].as<uint32_t>(), *sa_last = sa_first + n;
-    bwt_gather_kernel<<<grid(n), kBwtBlock, 0, s>>>(text_d, sa, n, bwt);
+    bwt_gather_kernel<uint32_t><<<grid(n), kBwtBlock, 0, s>>>(text_d, sa, n, bwt);
     CU(cudaGetLastError());
     size_t tb = tmp_bytes;
     CU(cub::DeviceSelect::If(d_tmp.p, tb, thrust::counting_iterator<uint32_t>(0), starts, cnt, (int64_t) n, RunStart{bwt}, s));
     uint64_t r = 0;
     CU(cudaMemcpyAsync(&r, cnt, 8, cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
-    bwt_samples_kernel<<<grid(r), kBwtBlock, 0, s>>>(starts, r, n, sa, sa_first, sa_last);
+    bwt_samples_kernel<uint32_t, uint32_t><<<grid(r), kBwtBlock, 0, s>>>(starts, r, n, sa, sa_first, sa_last);
     CU(cudaGetLastError());
     CU(cudaEventRecord(ev[1], s));
     std::vector<uint8_t> h_bwt(n);

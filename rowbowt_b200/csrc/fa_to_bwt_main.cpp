@@ -18,7 +18,6 @@ void print_help() {
     fprintf(stderr, "    -o <out_prefix>      writes <out_prefix>.bwt/.ssa/.esa/.docs (default <in.fa[.gz]>)\n");
     fprintf(stderr, "    --device <D>         CUDA device to build on (default 0)\n");
     fprintf(stderr, "    Uppercase A C G T are kept and other uppercase letters become A; lowercase input is refused.\n");
-    fprintf(stderr, "    The text (every record + 10 A's, then the terminator) must have fewer than 2^32 positions.\n");
 }
 
 }  // namespace
@@ -48,10 +47,10 @@ int main(int argc, char** argv) {
         return 1;
     }
     fprintf(stderr,
-            "n=%llu r=%llu  records %llu  rounds %u (largest active set %llu)  parse %.3fs  sort %.3fs (kernels %.1f ms, gather %.1f ms)  "
-            "write %.3fs  total %.3fs  device memory %.2f GB\n",
-            (unsigned long long) st.n, (unsigned long long) st.r, (unsigned long long) st.records, st.rounds,
-            (unsigned long long) st.max_active, st.s_parse, st.s_sort, st.ms_sort, st.ms_gather, st.s_write, st.s_total,
+            "n=%llu r=%llu  records %llu  wide %u  parts %u  rounds %u (largest active set %llu)  parse %.3fs  sort %.3fs (kernels %.1f ms, "
+            "verify %.1f ms, gather %.1f ms)  write %.3fs  total %.3fs  device memory %.2f GB\n",
+            (unsigned long long) st.n, (unsigned long long) st.r, (unsigned long long) st.records, st.wide, st.parts, st.rounds,
+            (unsigned long long) st.max_active, st.s_parse, st.s_sort, st.ms_sort, st.ms_verify, st.ms_gather, st.s_write, st.s_total,
             st.peak_bytes / 1e9);
     return 0;
 }

@@ -78,6 +78,19 @@ inline unsigned knob_fbb_threads() {
     return v ? (unsigned) std::clamp(*v, 1ll, 64ll) : 0u;
 }
 
+// Read by every BWT build (rbg_build_bwt, rbg_build_bwt_text) and passed to the builder.
+struct BwtKnobs {
+    bool wide = false;                   // RBG_BWT_WIDE=1: the u64 builder (parts) at any n
+    uint64_t part_rows = 0;              // RBG_BWT_PART_ROWS: rows of one part of that builder at most, >= 1 (0: from free memory)
+};
+
+inline BwtKnobs bwt_knobs() {
+    BwtKnobs k;
+    if (auto v = env_int("RBG_BWT_WIDE")) k.wide = *v == 1;
+    if (auto v = env_int("RBG_BWT_PART_ROWS")) k.part_rows = (uint64_t) std::max(*v, 1ll);
+    return k;
+}
+
 // RBG_MA_CHUNK_ROWS: rows of one device pass of the marker-array build at most, >= 1 (0: from free device memory).
 inline uint64_t knob_ma_chunk_rows() {
     const auto v = env_int("RBG_MA_CHUNK_ROWS");

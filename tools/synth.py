@@ -16,6 +16,7 @@ Seeds (§8(d)): reference seed=1, panel/genotypes seed=2, reads seed=3.
 from __future__ import annotations
 
 import argparse
+import json
 import os
 import subprocess
 import sys
@@ -288,7 +289,8 @@ def build_index_from_fasta_gpu(panel: Panel, prefix: str, markers: bool = True, 
     t = {}
     fa = prefix + ".fa"
     t0 = time.time(); write_fasta(panel, fa); t["fasta"] = time.time() - t0
-    t0 = time.time(); rb.build_bwt(fa, prefix, device=device); t["bwt"] = time.time() - t0
+    t0 = time.time(); st = rb.build_bwt(fa, prefix, device=device); t["bwt"] = time.time() - t0
+    print("build_bwt %s" % json.dumps(st.as_dict()), file=log, flush=True)
     t0 = time.time(); rb.build_index(prefix, prefix, sa=True, device=device); t["rb_build"] = time.time() - t0
     if markers:
         t0 = time.time(); write_mps(panel, prefix + ".mps"); t["mps"] = time.time() - t0
