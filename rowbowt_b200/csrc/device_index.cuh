@@ -188,8 +188,9 @@ __device__ __forceinline__ bool lf_step_v(const DevLeafDir& D, uint32_t c, uint6
     return true;
 }
 
-// One 32-byte plain line (layout 7, leaf.cuh) as one 256-bit read-only load.
-__device__ __forceinline__ void load_plain_line(const uint32_t* p, uint32_t (&w)[kPlainWords]) {
+// 32 bytes as one 256-bit read-only load without L1 allocation (p 32-byte aligned): a plain line (layout 7, leaf.cuh), a
+// group of raw read bytes (pack_kernel).
+__device__ __forceinline__ void load_nc_32B(const void* p, uint32_t (&w)[8]) {
     asm("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
         : "=r"(w[0]), "=r"(w[1]), "=r"(w[2]), "=r"(w[3]), "=r"(w[4]), "=r"(w[5]), "=r"(w[6]), "=r"(w[7])
         : "l"(p));
@@ -205,7 +206,7 @@ __device__ __forceinline__ bool lf_step_plain(const DevLeafDir& D, uint32_t c, u
     const uint32_t l = act ? (uint32_t) lo : 0u, h = act ? (uint32_t) hi : 0u;
     const uint32_t wa = l >> kPlainShift, wb = h >> kPlainShift, qa = l & (kPlainRows - 1u), qb = h & (kPlainRows - 1u);
     uint32_t A[kPlainWords];
-    load_plain_line(D.lines + (uint64_t) wa * kPlainWords, A);
+    load_nc_32B(D.lines + (uint64_t) wa * kPlainWords, A);
     const uint64_t ma = plain_match(A, c);
     const uint32_t ca = plain_count(A, c);
     uint64_t mb = ma;
@@ -214,7 +215,7 @@ __device__ __forceinline__ bool lf_step_plain(const DevLeafDir& D, uint32_t c, u
         lines_touched += act ? 1u : 0u;
     } else {
         uint32_t B[kPlainWords];
-        load_plain_line(D.lines + (uint64_t) wb * kPlainWords, B);
+        load_nc_32B(D.lines + (uint64_t) wb * kPlainWords, B);
         mb = plain_match(B, c);
         cb = plain_count(B, c);
         flags |= B[0];

@@ -33,7 +33,12 @@ namespace {
 constexpr int kBlock = 256;
 // Resident CTAs per SM search_kernel is built and launched for: 4 x 256 threads at 64 registers.  5 x 256 at 48 registers
 // and 9 x 128 at 56 registers spill and measured 26.8 / 22.7 ms against 21.2 ms (profiles/r2_search_occupancy_variants.jsonl).
+// Layout 7 is not bound by its L2-resident lines (DESIGN.md 2.1b) and its step needs fewer registers, so more resident warps
+// hide more of each step's dependent latency.  Count: 6 x 256 at 40 registers (no spill), toehold: 5 x 256 at 46 (at 6 it
+// spills and is slower); on `small` (B200) search_kernel 7.19 -> 6.69 ms and the toehold search 7.83 -> 7.52 ms
+// (profiles/plain_occupancy_small.jsonl).
 constexpr int kSearchCtas = 4;
+constexpr int search_ctas(int V, bool toehold) { return V == 7 ? (toehold ? 5 : 6) : kSearchCtas; }
 
 __device__ __forceinline__ uint64_t mix64(uint64_t z) {
     z += 0x9E3779B97F4A7C15ull;
@@ -57,69 +62,87 @@ __device__ __forceinline__ unsigned long long warp_sum(unsigned long long v) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// pack: thread t converts bytes [32t, 32t+32) into one u64 of 2-bit codes.  Coalesced 2 x 16-byte
-// loads, no dependence on read boundaries.  A byte that is not A/C/G/T marks its read through a
+// pack: group t = bytes [32t, 32t+32) becomes one u64 of 2-bit codes.  One coalesced 32-byte load
+// per group, no dependence on read boundaries.  A byte that is not A/C/G/T marks its read through a
 // binary search over the offsets (rare path).  One launch covers the words that hold reads
 // [r0, r1); bytes at or beyond offs[r1] may not have arrived yet (chunked H2D) and are ignored --
 // the word that straddles the chunk boundary is packed again, complete, by the next chunk.
+// A group's eight words stay in registers: every index into them is a compile-time constant, the tail group's too (writing
+// them through a byte pointer would put them in local memory for every group).
+
+// The bytes of group t; past `limit` they read as 0.
+__device__ __forceinline__ void pack_load(const DevBatch& b, uint64_t t, uint64_t limit, uint32_t (&vw)[8]) {
+    const uint64_t x0 = t << 5;
+    if (x0 + 32 <= limit) {
+        load_nc_32B(b.bases + x0, vw);
+        return;
+    }
+#pragma unroll
+    for (int wd = 0; wd < 8; ++wd) {
+        uint32_t x = 0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            if (x0 + 4 * wd + k < limit) x |= (uint32_t) b.bases[x0 + 4 * wd + k] << (8 * k);
+        vw[wd] = x;
+    }
+}
+
+__device__ __forceinline__ void pack_group(const DevBatch& b, const CodeTable& ct, const int8_t* lut, uint64_t t, uint64_t limit,
+                                           const uint32_t (&vw)[8]) {
+    const uint64_t x0 = t << 5;
+    uint64_t out = 0;
+    uint32_t bad = 0;
+    // fast path (every index built by the documented pipeline maps A,C,G,T -> 0..3): four bytes at a time, SIMD-in-register.
+    // A=0x41 C=0x43 G=0x47 T=0x54: ((c >> 1) ^ (c >> 2)) & 3 = 0,1,2,3; the four 2-bit fields of a word are gathered
+    // into one byte by a multiply (fields land at bits 24..31, nothing else does).
+    uint32_t all_ok = 0xFFFFFFFFu;
+    if (ct.plain) {
+#pragma unroll
+        for (int wd = 0; wd < 8; ++wd) {
+            const uint32_t x = vw[wd];
+            all_ok &= __vcmpeq4(x, 0x41414141u) | __vcmpeq4(x, 0x43434343u) | __vcmpeq4(x, 0x47474747u) | __vcmpeq4(x, 0x54545454u);
+            const uint32_t f = ((x >> 1) ^ (x >> 2)) & 0x03030303u;
+            out |= (uint64_t) ((f * 0x01041040u) >> 24) << (8 * wd);
+        }
+    }
+    if (!ct.plain || all_ok != 0xFFFFFFFFu || x0 + 32 > limit) {        // byte by byte through the table: flags / bad bits
+        out = 0;
+#pragma unroll
+        for (int i = 0; i < 32; ++i) {
+            const uint32_t byte = (vw[i >> 2] >> (8 * (i & 3))) & 0xFFu;
+            const int code = lut[byte];
+            if (code >= 0 && code < 4) {
+                out |= (uint64_t) code << (2 * i);
+            } else if (b.bad) {
+                bad |= 1u << i;                       // greedy seeding: such a base fails its seed, not its read
+            } else if (x0 + i < limit) {
+                // which read owns byte x0+i: last offset <= x
+                const uint64_t x = x0 + i;
+                uint64_t lo = 0, hi = b.n_reads;      // invariant offs[lo] <= x < offs[hi]
+                while (hi - lo > 1) {
+                    const uint64_t mid = (lo + hi) >> 1;
+                    if (b.offs[mid] <= x) lo = mid; else hi = mid;
+                }
+                flag_read(b.flags, lo, code == 4 ? kReadExotic : kReadDead);
+            }
+        }
+    }
+    b.packed[t] = out;
+    if (b.bad) b.bad[t] = bad;
+}
+
+// One group per thread and iteration: two per iteration, both loads issued before either group is converted, measured
+// 0.586 against 0.574 ms for the 1.5 GB of the `small` batch (B200, profiles/pack_bench_small.jsonl).
 __global__ void __launch_bounds__(kBlock) pack_kernel(DevBatch b, CodeTable ct) {
     __shared__ int8_t lut[256];
     for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = ct.code_of[i];
     __syncthreads();
     const uint64_t limit = b.offs[b.r1];
     const uint64_t w0 = b.offs[b.r0] >> 5, w1 = (limit + 31) >> 5;
-    for (uint64_t t = w0 + (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; t < w1;
-         t += (uint64_t) gridDim.x * blockDim.x) {
-        const uint64_t x0 = t << 5;
-        uint4 v[2] = {make_uint4(0, 0, 0, 0), make_uint4(0, 0, 0, 0)};
-        if (x0 + 32 <= limit) {
-            const uint4* p = reinterpret_cast<const uint4*>(b.bases + x0);
-            v[0] = __ldg(p);
-            v[1] = __ldg(p + 1);
-        } else {
-            uint8_t* vb = reinterpret_cast<uint8_t*>(v);
-            for (uint64_t i = 0; x0 + i < limit; ++i) vb[i] = b.bases[x0 + i];
-        }
-        const uint32_t* vw = reinterpret_cast<const uint32_t*>(v);
-        uint64_t out = 0;
-        uint32_t bad = 0;
-        // fast path (every index built by the documented pipeline maps A,C,G,T -> 0..3): four bytes at a time, SIMD-in-register.
-        // A=0x41 C=0x43 G=0x47 T=0x54: ((c >> 1) ^ (c >> 2)) & 3 = 0,1,2,3; the four 2-bit fields of a word are gathered
-        // into one byte by a multiply (fields land at bits 24..31, nothing else does).
-        uint32_t all_ok = 0xFFFFFFFFu;
-        if (ct.plain) {
-#pragma unroll
-            for (int wd = 0; wd < 8; ++wd) {
-                const uint32_t x = vw[wd];
-                all_ok &= __vcmpeq4(x, 0x41414141u) | __vcmpeq4(x, 0x43434343u) | __vcmpeq4(x, 0x47474747u) | __vcmpeq4(x, 0x54545454u);
-                const uint32_t f = ((x >> 1) ^ (x >> 2)) & 0x03030303u;
-                out |= (uint64_t) ((f * 0x01041040u) >> 24) << (8 * wd);
-            }
-        }
-        if (!ct.plain || all_ok != 0xFFFFFFFFu || x0 + 32 > limit) {        // byte by byte through the table: flags / bad bits
-            out = 0;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-                const uint32_t byte = (vw[i >> 2] >> (8 * (i & 3))) & 0xFFu;
-                const int code = lut[byte];
-                if (code >= 0 && code < 4) {
-                    out |= (uint64_t) code << (2 * i);
-                } else if (b.bad) {
-                    bad |= 1u << i;                       // greedy seeding: such a base fails its seed, not its read
-                } else if (x0 + i < limit) {
-                    // which read owns byte x0+i: last offset <= x
-                    const uint64_t x = x0 + i;
-                    uint64_t lo = 0, hi = b.n_reads;      // invariant offs[lo] <= x < offs[hi]
-                    while (hi - lo > 1) {
-                        const uint64_t mid = (lo + hi) >> 1;
-                        if (b.offs[mid] <= x) lo = mid; else hi = mid;
-                    }
-                    flag_read(b.flags, lo, code == 4 ? kReadExotic : kReadDead);
-                }
-            }
-        }
-        b.packed[t] = out;
-        if (b.bad) b.bad[t] = bad;
+    for (uint64_t t = w0 + (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; t < w1; t += (uint64_t) gridDim.x * blockDim.x) {
+        uint32_t vw[8];
+        pack_load(b, t, limit, vw);
+        pack_group(b, ct, lut, t, limit, vw);
     }
 }
 
@@ -165,7 +188,7 @@ struct ToeholdTrack {
 // u32, <= kPairMaxShared bytes) is the kernel's dynamic shared memory.  A lane whose read has an odd number of bases left
 // first takes one step on the single-base directory, which then reads its superblock bases from global memory.
 template <bool TOEHOLD, int V, bool PAIR>
-__global__ void __launch_bounds__(kBlock, kSearchCtas) search_kernel(DevLeafDir D, DevPairDir PD, DevToehold T, DevFtab ft, DevBatch b,
+__global__ void __launch_bounds__(kBlock, search_ctas(V, TOEHOLD)) search_kernel(DevLeafDir D, DevPairDir PD, DevToehold T, DevFtab ft, DevBatch b,
                                                                      DevResult r, DevCounters* ctr, unsigned long long* cursor) {
     constexpr uint32_t kFull = 0xFFFFFFFFu;
     __shared__ uint64_t s_base[V == 5 && !PAIR ? 4 * kMaxSuper5Dev : 1];
@@ -594,7 +617,7 @@ int launch_search(const DevLeafDir& D, const DevPairDir& PD, const DevToehold* T
     if (b.r1 <= b.r0) return 0;
     DevToehold t0{};
     // reads are handed out by the device cursor, so ONE wave of CTAs is the whole grid: resident CTAs per SM x SMs.
-    const int grid = grid_for(b.r1 - b.r0, kBlock, kSearchCtas);
+    const int grid = grid_for(b.r1 - b.r0, kBlock, search_ctas((int) D.version, T != nullptr));
     if (!T && PD.lines) {                                   // the pair directory is built only over a layout-5 directory
         if (D.version != 5 || 64ull * PD.n_super > kPairMaxShared) throw std::logic_error("pair directory without its layout");
         search_kernel<false, 5, true><<<grid, kBlock, 64 * PD.n_super, st>>>(D, PD, t0, ft, b, r, ctr, cursor);
